@@ -4,6 +4,7 @@
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
     python bench.py --impl reference ...       # the CPU path (oracle port) on the box's host cores
+    python bench.py --dump-outputs DIR ...     # also write the outputs of the last timed step as DIR/<name>.npy
 
 A "step" is one pass of the hot path over one batch: detector loss on both images + dense descriptor loss,
 forward and backward, on 32 synthetic 240x320 pairs per GPU (head outputs `semi`/`desc` are the inputs; the
@@ -160,6 +161,29 @@ class ClockSampler(object):
                 "reasons": reasons, "samples": len(sm)}
 
 
+DUMP_MAX_BYTES = 64 * 10**6
+DUMP_SAMPLE = 1 << 22  # elements kept of a larger output (the two descriptor gradients, 9.8 M elements each at B32)
+
+
+def dump_outputs(path, out):
+    """Write what one loss step returns -- the loss scalars and the gradients of the four head outputs -- to path/<name>.npy in
+    float32.  An output of more than DUMP_SAMPLE elements is reduced to the same seeded sample of its flattened elements in
+    every run, so that the files of two builds can be compared element for element."""
+    grads = dict(zip(("grad_semi", "grad_semi_warp", "grad_desc", "grad_desc_warp"), out["grads"]))
+    arrays = {k: v for k, v in out.items() if k != "grads"}
+    arrays.update(grads)
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    for k, a in arrays.items():
+        if a.size > DUMP_SAMPLE:
+            idx = np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))
+            arrays[k] = a.reshape(-1)[idx]
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, total
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------
 # our arm
 # ------------------------------------------------------------------------------------------------
@@ -197,11 +221,13 @@ def run_ours(args):
     h2d_bytes = sum(pinned[0][k].numel() * pinned[0][k].element_size() for k in in_keys)
 
     def step(d):
+        """One eager step; returns what GraphedLossStep.replay() returns: the loss scalars and "grads" of the four leaves."""
         leaves = [d[k].detach().requires_grad_(True) for k in ("semi", "semi_warp", "desc", "desc_warp")]
         out = S.step.loss_step(leaves[0], leaves[1], leaves[2], leaves[3], d["labels_2D"], d["warped_labels"], d["mask_2D"],
                                d["mask_warp_2D"], d["mat_H"], dist_group=group)
         out["loss"].backward()
-        return out["loss"], leaves
+        out["grads"] = [l.grad for l in leaves]
+        return out
 
     def barrier():
         if world > 1:
@@ -217,9 +243,9 @@ def run_ours(args):
     if use_graph:
         # fwd+bwd of the whole step captured once per input set and replayed: the step is ~25 short kernels
         graphs = [S.step.GraphedLossStep(d, dist_group=group) for d in dsets]
-        run = lambda i: graphs[i % NSETS].replay()["loss"]
+        run = lambda i: graphs[i % NSETS].replay()
     else:
-        run = lambda i: step(dsets[i % NSETS])[0]
+        run = lambda i: step(dsets[i % NSETS])
     for i in range(max(args.warmup, 3)):
         run(i)
     barrier()
@@ -232,14 +258,16 @@ def run_ours(args):
     barrier()
     ev0.record()
     for i in range(args.steps):
-        loss = run(i)
+        out = run(i)
     ev1.record()
     barrier()
     ms = ev0.elapsed_time(ev1)
     kernels = kernels_per_step * args.steps
     ms = sdist.max_over_ranks(ms, dev)
     value = B * world * args.steps / (ms * 1e-3)
-    loss_val = float(loss)
+    loss_val = float(out["loss"])
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)  # before any later phase reuses the buffers
 
     # ---- everything below is secondary to the timed region above: if a later phase fails (or, with several ranks, a peer
     #      is lost and rank 0 would wait forever) the line is still printed, with e2e / roofline marked as failed
@@ -292,7 +320,7 @@ def run_ours(args):
                 ready[slot].record(copy_stream)
 
         def run_slot(slot):
-            return slots[slot].replay()["loss"] if use_graph else step(bufs[slot])[0]
+            return slots[slot].replay()["loss"] if use_graph else step(bufs[slot])["loss"]
 
         def e2e_loop(n):
             for f in freed:
@@ -627,7 +655,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-variants", action="store_true", help="skip the timings of the other engines / fused=False")
     ap.add_argument("--no-semantic", action="store_true", help="skip the auxiliary step timing with the semantic head")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the loss scalars and input gradients of the last timed step "
+                    "(rank 0) to DIR/<name>.npy; the inputs are seeded, so runs with the same arguments are comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -7,8 +7,7 @@ the reference file:line it follows.  Only tests/, __graft_entry__.smoke() and be
 Pinning: the reference ships no golden vectors or assertions for this path (SURVEY 4, 8c), so this oracle is
 pinned against outputs of the LIVE reference functions, generated in the authoring container by
 tests/golden/make_golden.py (which imports /root/reference) and committed as tests/golden/*.npz;
-tests/test_oracle_golden.py replays them (and checks nn_match_two_way against the one fixture the reference ships,
-datasets/kitti/kitti_test/0000000000.npz).  Third-party arithmetic on the path that is restated here:
+tests/test_oracle_golden.py replays them.  Third-party arithmetic on the path that is restated here:
 torch 2.11 (F.grid_sample bilinear/nearest zeros-padding align_corners=True, softmax, BCELoss with the
 -100 log clamp, torch.norm), torchvision 0.26 ops.nms, opencv 4.13 getStructuringElement(MORPH_ELLIPSE) +
 erode (reference pins opencv-python 3.4.2.16).  The only torch call kept is torch.linspace for the

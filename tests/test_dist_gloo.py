@@ -36,6 +36,10 @@ def _sem_inputs():
 
 def _worker(rank, world, port, q):
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    if torch.cuda.is_available():
+        # with a CUDA device the default exchange is the peer-memory kernel (covered by the -m gpu tests); this test
+        # drives the torch.distributed form with CPU tensors
+        os.environ["SSP_EXCHANGE"] = "allreduce"
     import torch.distributed as tdist
     from ssp_b200.dist import (LossExchange, get_exchange, globalize_descriptor, globalize_detector, globalize_semantic,
                                init_from_env, shard_range)

@@ -154,22 +154,6 @@ def test_sparse_descriptors_and_matching(golden):
     assert O.sample_desc_from_points(coarse, np.zeros((3, 0))).shape == (256, 0)
 
 
-def test_matching_oracle_against_the_reference_shipped_fixture():
-    """The one fixture the reference ships for this code path: datasets/kitti/kitti_test/0000000000.npz holds
-    keypoints / descriptors of an image pair and their `matches` (SURVEY 4).  nn_match_two_way at the reference default
-    nn_thresh = 0.7 reproduces all 584 rows, in order.  Runs where /root/reference is mounted (authoring container)."""
-    import os
-    import pytest
-    path = "/root/reference/datasets/kitti/kitti_test/0000000000.npz"
-    if not os.path.exists(path):
-        pytest.skip("reference checkout not mounted")
-    g = np.load(path)
-    m = O.nn_match_two_way(g["desc1"], g["desc2"], 0.7)
-    pred = np.concatenate([g["keypoints1"][m[0].astype(int)], g["keypoints2"][m[1].astype(int)]], axis=1)
-    assert pred.shape == g["matches"].shape == (584, 4)
-    assert np.array_equal(pred, g["matches"])
-
-
 def test_warp_labels_oracle(golden):
     """SURVEY 8f rank 4 (oracle pinned ahead of the kernels): datasets/data_tools.warpLabels incl. the bilinear label map."""
     g = golden("warp_labels")
