@@ -35,9 +35,9 @@ int ssp_warp_keypoints_f64(const double* kp /*[K,2] x,y pixels*/, int K, const d
 
 /* ---- a2: inv_warp_image_batch / inv_warp_image (utils/utils.py:347-405).
  *      xs[W], ys[H] = the normalised sampling grid (torch.linspace(-1,1,n) of the reference, :375).
- *      mode 0 = bilinear, 1 = nearest; zeros padding, align_corners=True.  Default kernel: 32x32 output tiles whose
- *      source footprint is staged through shared memory with 16-byte cp.async; mode + 2 forces the per-pixel gather
- *      kernel (also taken automatically for W % 4 != 0 or a misaligned image).  Same results either way. ---- */
+ *      mode 0 = bilinear, 1 = nearest (any other value is an argument error); zeros padding, align_corners=True.
+ *      One gather kernel: each thread computes the source coordinates of 4 output pixels once and reads their taps
+ *      straight from global memory for every channel. ---- */
 int ssp_inv_warp_image(const float* img /*[B,C,H,W]*/, int B, int C, int H, int W, const float* Hinv /*[B,3,3]*/,
                        const float* xs, const float* ys, int mode, float* out /*[B,C,H,W]*/, void* stream);
 
@@ -82,24 +82,6 @@ int ssp_flatten_detection_masked(const float* semi /*[N,65,Hc,Wc]*/, const float
 int ssp_combine_heatmap(const float* heat /*[I,N,H,W]*/, const float* mask /*[I,N,H,W]*/,
                         const float* Hinv /*[I,N,3,3]*/, int I, int N, int H, int W, const float* xs, const float* ys,
                         float* out /*[I,H,W]*/, void* stream);
-/* Same arguments and results through the shared-memory staged kernel (32x32 output tiles, source footprints copied with
- * 16-byte cp.async); needs W % 4 == 0 and 16-byte aligned maps.  Opt-in: measured slower than the gather kernel at
- * 240x320 (see heatmap.cu). */
-int ssp_combine_heatmap_tiled(const float* heat, const float* mask, const float* Hinv, int I, int N, int H, int W,
-                              const float* xs, const float* ys, float* out, void* stream);
-
-/* Bit-mask form of the same aggregation (default of the batched export path): the 0/1 valid masks of homography adaptation
- * (compute_valid_mask, datasets/Coco.py:284-288) as one bit per pixel, bits [rows, ceil(W/32)], bit x&31 of word x>>5.
- * ssp_mask_pack_bits converts float masks (flag, a zeroed device int, is set on a value other than 0/1 and makes the
- * aggregation return NaN); ssp_valid_mask_bits is compute_valid_mask(erosion_radius=0) straight to bits.  Results are
- * bit-identical to ssp_combine_heatmap on binary masks. */
-size_t ssp_mask_bits_words(int rows, int W);
-int ssp_mask_pack_bits(const float* mask /*[rows,W]*/, long long rows, int W, uint32_t* bits, int* flag, void* stream);
-int ssp_valid_mask_bits(int B, int H, int W, const float* Hinv /*[B,3,3]*/, const float* xs, const float* ys,
-                        uint32_t* bits /*[B,H,ceil(W/32)]*/, void* stream);
-int ssp_combine_heatmap_bits(const float* heat /*[I,N,H,W]*/, const uint32_t* mbits /*[I,N,H,ceil(W/32)]*/,
-                             const float* Hinv /*[I,N,3,3]*/, int I, int N, int H, int W, const float* xs, const float* ys,
-                             const int* flag /*or NULL*/, float* out /*[I,H,W]*/, void* stream);
 /* the same aggregation from the signed heat of ssp_flatten_detection_masked: one gather per tap (bit-identical results for
  * 0/1 masks; a raised flag turns the output into NaN) */
 int ssp_combine_heatmap_signed(const float* heat_signed /*[I,N,H,W]*/, const float* Hinv /*[I,N,3,3]*/, int I, int N, int H,

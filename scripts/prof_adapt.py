@@ -28,7 +28,6 @@ for rep in range(2):
     out = S.step.adaptation_step(semi, Hw, mask, binary_mask=True)
     w = S.inv_warp_image_batch(img, Hinv[0], device=dev)
     wn = S.inv_warp_image_batch(img, Hinv[0], device=dev, mode="nearest")
-    wg = S.inv_warp_image_batch(img, Hinv[0], device=dev, staged=True)
     wp = S.warp_points(pts, Hinv[0], device=dev)
 torch.cuda.synchronize()
 print("done", len(out), out[0].shape)

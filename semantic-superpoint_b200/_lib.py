@@ -38,11 +38,6 @@ SIGNATURES = {
     "ssp_flatten_detection": (_I, [_P, _I, _I, _I, _P, _P]),
     "ssp_flatten_detection_masked": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "ssp_combine_heatmap": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
-    "ssp_combine_heatmap_tiled": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
-    "ssp_mask_bits_words": (_Z, [_I, _I]),
-    "ssp_mask_pack_bits": (_I, [_P, _c.c_longlong, _I, _P, _P, _P]),
-    "ssp_valid_mask_bits": (_I, [_I, _I, _I, _P, _P, _P, _P, _P]),
-    "ssp_combine_heatmap_bits": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_combine_heatmap_signed": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_nms_ws_bytes": (_Z, [_I, _I, _I, _I]),
     "ssp_nms_fast": (_I, [_P, _I, _I, _I, _F, _I, _P, _I, _I, _P, _P, _P, _Z, _P]),

@@ -5,7 +5,6 @@
 // intermediate [N,1,H,W] warped stacks of the reference never exist.  HBM traffic = the algorithmic
 // (2N+1)*H*W*4 bytes.  A block owns an 8x8 output tile x 4 interleaved view groups.
 #include "common.cuh"
-#include <cstdlib>
 
 #define CH_PIX 64
 #define CH_GROUPS 4
@@ -13,10 +12,16 @@
 // ncu of the first version (32 x 100 views of 240x320): 140 SASS instructions per (pixel, view), issue slots 63 % busy, DRAM 14 %:
 // instruction-bound.  This version keeps the per-view work lean: homographies padded to 12 floats (three 16-byte shared loads),
 // 32-bit tap offsets against per-view base pointers, the four corner predicates folded once.
+// SIGNED = false: heat and a float mask, two gathers per tap (the reference's heat * mask product formed at the gather).
+// SIGNED = true: heat is flatten_detection_masked's array (heat where the view's mask is 1, -1 where it is 0), so a tap is ONE
+// gather and a sign test; mask is ignored and flag (its non-binary-mask flag, or NULL) turns the output into NaN.  The gather
+// kernels are bound by L1 wavefronts (ncu: l1tex 89 %, ~6 lines per warp-wide load under rotation), so half the loads is what
+// moves them.  Same arithmetic for m in {0, 1}: bit-identical results.
+template <bool SIGNED>
 __global__ void __launch_bounds__(CH_PIX * CH_GROUPS)
 combine_heatmap_kernel(const float* __restrict__ heat, const float* __restrict__ mask,
                        const float* __restrict__ Hinv, int N, int H, int W, const float* __restrict__ xs,
-                       const float* __restrict__ ys, float* __restrict__ out) {
+                       const float* __restrict__ ys, const int* __restrict__ flag, float* __restrict__ out) {
   extern __shared__ __align__(16) float sh[];  // N x 12 floats (homography + pad), then 2*CH_PIX*CH_GROUPS partial sums
   float4* hs = reinterpret_cast<float4*>(sh);
   float* part = sh + N * 12;
@@ -61,83 +66,22 @@ combine_heatmap_kernel(const float* __restrict__ heat, const float* __restrict__
       const bool xin0 = x0 >= 0, xin1 = x0 + 1 < W, yin0 = y0 >= 0, yin1 = y0 + 1 < H;
       const int o = y0 * W + x0;
       float ah = 0.f, am = 0.f;
-      if (yin0 && xin0) { const float m = __ldg(mp + o), w = wx0 * wy0; am += m * w; ah += (__ldg(hp + o) * m) * w; }
-      if (yin0 && xin1) { const float m = __ldg(mp + o + 1), w = wx1 * wy0; am += m * w; ah += (__ldg(hp + o + 1) * m) * w; }
-      if (yin1 && xin0) { const float m = __ldg(mp + o + W), w = wx0 * wy1; am += m * w; ah += (__ldg(hp + o + W) * m) * w; }
-      if (yin1 && xin1) { const float m = __ldg(mp + o + W + 1), w = wx1 * wy1; am += m * w; ah += (__ldg(hp + o + W + 1) * m) * w; }
-      sum_h += ah;
-      sum_m += am;
-    }
-  }
-  part[threadIdx.x] = sum_h;
-  part[CH_PIX * CH_GROUPS + threadIdx.x] = sum_m;
-  __syncthreads();
-  if (g == 0 && inside) {
-    float th = 0.f, tm = 0.f;
-#pragma unroll
-    for (int q = 0; q < CH_GROUPS; ++q) {
-      th += part[q * CH_PIX + lp];
-      tm += part[CH_PIX * CH_GROUPS + q * CH_PIX + lp];
-    }
-    out[y * W + x] = th / tm;  // 0/0 -> NaN exactly like the reference when no view covers the pixel
-  }
-}
-
-
-// Signed-heat variant: the input is flatten_detection_masked's array (heat where the view's mask is 1, -1 where it is 0), so a
-// tap is ONE gather and a sign test instead of two gathers.  The gather kernels are bound by L1 wavefronts (ncu: l1tex 89 %,
-// ~6 lines per warp-wide load under rotation), so half the loads is what moves them.  Same arithmetic as the float-mask
-// kernel for m in {0, 1}: bit-identical results.
-__global__ void __launch_bounds__(CH_PIX * CH_GROUPS)
-combine_heatmap_signed_kernel(const float* __restrict__ heat, const float* __restrict__ Hinv, int N, int H, int W,
-                              const float* __restrict__ xs, const float* __restrict__ ys, const int* __restrict__ flag,
-                              float* __restrict__ out) {
-  extern __shared__ __align__(16) float sh[];  // N x 12 floats (homography + pad), then 2*CH_PIX*CH_GROUPS partial sums
-  float4* hs = reinterpret_cast<float4*>(sh);
-  float* part = sh + N * 12;
-  const int plane = H * W;
-  heat += (size_t)blockIdx.y * N * plane;
-  Hinv += (size_t)blockIdx.y * N * 9;
-  out += (size_t)blockIdx.y * plane;
-  for (int i = threadIdx.x; i < N * 12; i += blockDim.x) {
-    const int n = i / 12, k = i - n * 12;
-    sh[i] = k < 9 ? Hinv[n * 9 + k] : 0.f;
-  }
-  __syncthreads();
-  const int lp = threadIdx.x % CH_PIX, g = threadIdx.x / CH_PIX;
-  const int tiles_x = (W + 7) / 8;
-  const int x = (blockIdx.x % tiles_x) * 8 + (lp & 7), y = (blockIdx.x / tiles_x) * 8 + (lp >> 3);
-  const bool inside = x < W && y < H;
-  float sum_h = 0.f, sum_m = 0.f;
-  if (inside) {
-    const float gx = __ldg(xs + x), gy = __ldg(ys + y);
-    const float fW = (float)W, fH = (float)H, sx = (float)(W - 1), sy = (float)(H - 1);
-    const float* hp = heat + (size_t)g * plane;
-    const size_t step = (size_t)CH_GROUPS * plane;
-    for (int n = g; n < N; n += CH_GROUPS, hp += step) {
-      const float4 h0 = hs[3 * n], h1 = hs[3 * n + 1], h2 = hs[3 * n + 2];
-      const float X = fmaf(h0.y, gy, h0.x * gx) + h0.z;
-      const float Y = fmaf(h1.x, gy, h0.w * gx) + h1.y;
-      const float Z = fmaf(h1.w, gy, h1.z * gx) + h2.x;
-      const float ix = ((X / Z + 1.f) / 2.f) * sx;
-      const float iy = ((Y / Z + 1.f) / 2.f) * sy;
-      const float fx = floorf(ix), fy = floorf(iy);
-      if (!(fx >= -1.f && fx < fW && fy >= -1.f && fy < fH)) continue;
-      const int x0 = (int)fx, y0 = (int)fy;
-      const float wx1 = ix - fx, wx0 = (fx + 1.f) - ix;
-      const float wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
-      const bool xin0 = x0 >= 0, xin1 = x0 + 1 < W, yin0 = y0 >= 0, yin1 = y0 + 1 < H;
-      const int o = y0 * W + x0;
-      // out-of-image taps read as "masked"
-      const float p00 = (yin0 && xin0) ? __ldg(hp + o) : -1.f;
-      const float p01 = (yin0 && xin1) ? __ldg(hp + o + 1) : -1.f;
-      const float p10 = (yin1 && xin0) ? __ldg(hp + o + W) : -1.f;
-      const float p11 = (yin1 && xin1) ? __ldg(hp + o + W + 1) : -1.f;
-      float ah = 0.f, am = 0.f;
-      if (p00 >= 0.f) { const float w = wx0 * wy0; am += w; ah += p00 * w; }
-      if (p01 >= 0.f) { const float w = wx1 * wy0; am += w; ah += p01 * w; }
-      if (p10 >= 0.f) { const float w = wx0 * wy1; am += w; ah += p10 * w; }
-      if (p11 >= 0.f) { const float w = wx1 * wy1; am += w; ah += p11 * w; }
+      if constexpr (SIGNED) {
+        // out-of-image taps read as "masked"
+        const float p00 = (yin0 && xin0) ? __ldg(hp + o) : -1.f;
+        const float p01 = (yin0 && xin1) ? __ldg(hp + o + 1) : -1.f;
+        const float p10 = (yin1 && xin0) ? __ldg(hp + o + W) : -1.f;
+        const float p11 = (yin1 && xin1) ? __ldg(hp + o + W + 1) : -1.f;
+        if (p00 >= 0.f) { const float w = wx0 * wy0; am += w; ah += p00 * w; }
+        if (p01 >= 0.f) { const float w = wx1 * wy0; am += w; ah += p01 * w; }
+        if (p10 >= 0.f) { const float w = wx0 * wy1; am += w; ah += p10 * w; }
+        if (p11 >= 0.f) { const float w = wx1 * wy1; am += w; ah += p11 * w; }
+      } else {
+        if (yin0 && xin0) { const float m = __ldg(mp + o), w = wx0 * wy0; am += m * w; ah += (__ldg(hp + o) * m) * w; }
+        if (yin0 && xin1) { const float m = __ldg(mp + o + 1), w = wx1 * wy0; am += m * w; ah += (__ldg(hp + o + 1) * m) * w; }
+        if (yin1 && xin0) { const float m = __ldg(mp + o + W), w = wx0 * wy1; am += m * w; ah += (__ldg(hp + o + W) * m) * w; }
+        if (yin1 && xin1) { const float m = __ldg(mp + o + W + 1), w = wx1 * wy1; am += m * w; ah += (__ldg(hp + o + W + 1) * m) * w; }
+      }
       sum_h += ah;
       sum_m += am;
     }
@@ -153,413 +97,35 @@ combine_heatmap_signed_kernel(const float* __restrict__ heat, const float* __res
       tm += part[CH_PIX * CH_GROUPS + q * CH_PIX + lp];
     }
     float r = th / tm;  // 0/0 -> NaN exactly like the reference when no view covers the pixel
-    if (flag && *flag) r = __int_as_float(0x7fc00000);  // a mask that was not 0/1: refuse loudly
+    if constexpr (SIGNED) {
+      if (flag && *flag) r = __int_as_float(0x7fc00000);  // a mask that was not 0/1: refuse loudly
+    }
     out[y * W + x] = r;
   }
 }
 
-// ----------------------------------------------------------------------------------------------
-// Bit-mask variant (the default of the batched export path).  The valid masks of homography adaptation are 0/1 images
-// (compute_valid_mask, datasets/Coco.py:284-288); as floats they are half of the aggregation's traffic and half of its
-// gather instructions.  Packed to one bit per pixel (40 bytes per row at W = 320) a warp's mask taps fall into 2-3 cache
-// lines instead of ~6 per load, and the two taps of a row come out of ONE word load.  Arithmetic is unchanged
-// (m in {0.0f, 1.0f}), so results are bit-identical to the float-mask kernel.
-// ----------------------------------------------------------------------------------------------
-// float mask -> bits; flag[0] is set when a value other than 0 / 1 is seen (the aggregation then returns NaN: loud)
-__global__ void __launch_bounds__(256)
-mask_pack_bits_kernel(const float* __restrict__ mask, size_t rows, int W, int WP, uint32_t* __restrict__ bits,
-                      int* __restrict__ flag) {
-  const int lane = threadIdx.x & 31;
-  const size_t warp = (size_t)blockIdx.x * 8 + (threadIdx.x >> 5);  // one warp per (row, word)
-  if (warp >= rows * WP) return;
-  const size_t row = warp / WP;
-  const int wi = (int)(warp - row * WP), x = wi * 32 + lane;
-  float m = 0.f;
-  if (x < W) m = __ldg(mask + row * W + x);
-  const uint32_t word = __ballot_sync(0xffffffffu, m != 0.f);
-  const bool odd = __any_sync(0xffffffffu, m != 0.f && m != 1.f);
-  if (lane == 0) {
-    bits[warp] = word;
-    if (odd) *flag = 1;
-  }
-}
-
-// compute_valid_mask(erosion_radius = 0) straight to bits: nearest warp of an all-ones image = in-bounds predicate of the
-// rounded source coordinate (same arithmetic as valid_mask_kernel in warp.cu); nothing but 1 bit per pixel reaches HBM
-__global__ void __launch_bounds__(256)
-valid_mask_bits_kernel(int H, int W, int WP, const float* __restrict__ Hinv, const float* __restrict__ xs,
-                       const float* __restrict__ ys, uint32_t* __restrict__ bits) {
-  __shared__ float h[9];
-  const int b = blockIdx.z;
-  if (threadIdx.x < 9) h[threadIdx.x] = Hinv[b * 9 + threadIdx.x];
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  const int wi = blockIdx.x, y = blockIdx.y * 8 + (threadIdx.x >> 5);
-  if (y >= H) return;
-  const int x = wi * 32 + lane;
-  bool v = false;
-  if (x < W) {
-    float nx, ny;
-    homography_apply(h, __ldg(xs + x), __ldg(ys + y), nx, ny);
-    const float ix = ((nx + 1.f) / 2.f) * (float)(W - 1), iy = ((ny + 1.f) / 2.f) * (float)(H - 1);
-    const float rx = rintf(ix), ry = rintf(iy);
-    v = rx >= 0.f && rx < (float)W && ry >= 0.f && ry < (float)H;
-  }
-  const uint32_t word = __ballot_sync(0xffffffffu, v);
-  if (lane == 0) bits[((size_t)b * H + y) * WP + wi] = word;
-}
-
-__global__ void __launch_bounds__(CH_PIX * CH_GROUPS)
-combine_heatmap_bits_kernel(const float* __restrict__ heat, const uint32_t* __restrict__ mbits,
-                            const float* __restrict__ Hinv, int N, int H, int W, int WP, const float* __restrict__ xs,
-                            const float* __restrict__ ys, const int* __restrict__ flag, float* __restrict__ out) {
-  extern __shared__ float sh[];  // N*9 homographies, then 2*CH_PIX*CH_GROUPS partial sums
-  float* hs = sh;
-  float* part = sh + N * 9;
-  heat += (size_t)blockIdx.y * N * H * W;
-  mbits += (size_t)blockIdx.y * N * H * WP;
-  Hinv += (size_t)blockIdx.y * N * 9;
-  out += (size_t)blockIdx.y * H * W;
-  for (int i = threadIdx.x; i < N * 9; i += blockDim.x) hs[i] = Hinv[i];
-  __syncthreads();
-  int lp = threadIdx.x % CH_PIX, g = threadIdx.x / CH_PIX;
-  int tiles_x = (W + 7) / 8;
-  int x = (blockIdx.x % tiles_x) * 8 + (lp & 7), y = (blockIdx.x / tiles_x) * 8 + (lp >> 3);
-  bool inside = x < W && y < H;
-  int pix = y * W + x;
-  float sum_h = 0.f, sum_m = 0.f;
-  if (inside) {
-    float gx = __ldg(xs + x), gy = __ldg(ys + y);
-    size_t plane = (size_t)H * W;
-    for (int n = g; n < N; n += CH_GROUPS) {
-      const float* h = hs + n * 9;
-      float nx, ny;
-      homography_apply(h, gx, gy, nx, ny);
-      float ix = ((nx + 1.f) / 2.f) * (float)(W - 1);
-      float iy = ((ny + 1.f) / 2.f) * (float)(H - 1);
-      float fx = floorf(ix), fy = floorf(iy);
-      if (!(fx >= -1.f && fx < (float)W && fy >= -1.f && fy < (float)H)) continue;
-      int x0 = (int)fx, y0 = (int)fy, x1 = x0 + 1, y1 = y0 + 1;
-      float wx1 = ix - fx, wx0 = (fx + 1.f) - ix;
-      float wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
-      bool xin0 = x0 >= 0, xin1 = x1 < W, yin0 = y0 >= 0, yin1 = y1 < H;
-      const float* hp = heat + n * plane;
-      const uint32_t* mp = mbits + (size_t)n * H * WP;
-      const int xa = xin0 ? x0 : x1;  // a column inside the image: its word holds both taps unless they straddle a word
-      const bool straddle = xin0 && xin1 && (x1 & 31) == 0;
-      float ah = 0.f, am = 0.f;
-      if (yin0) {
-        const uint32_t* mr = mp + (size_t)y0 * WP;
-        const uint32_t wa = __ldg(mr + (xa >> 5));
-        const uint32_t wb = straddle ? __ldg(mr + (x1 >> 5)) : wa;
-        size_t r = (size_t)y0 * W;
-        if (xin0) { float m = (float)((wa >> (x0 & 31)) & 1u), w = wx0 * wy0; am += m * w; ah += (__ldg(hp + r + x0) * m) * w; }
-        if (xin1) { float m = (float)((wb >> (x1 & 31)) & 1u), w = wx1 * wy0; am += m * w; ah += (__ldg(hp + r + x1) * m) * w; }
-      }
-      if (yin1) {
-        const uint32_t* mr = mp + (size_t)y1 * WP;
-        const uint32_t wa = __ldg(mr + (xa >> 5));
-        const uint32_t wb = straddle ? __ldg(mr + (x1 >> 5)) : wa;
-        size_t r = (size_t)y1 * W;
-        if (xin0) { float m = (float)((wa >> (x0 & 31)) & 1u), w = wx0 * wy1; am += m * w; ah += (__ldg(hp + r + x0) * m) * w; }
-        if (xin1) { float m = (float)((wb >> (x1 & 31)) & 1u), w = wx1 * wy1; am += m * w; ah += (__ldg(hp + r + x1) * m) * w; }
-      }
-      sum_h += ah;
-      sum_m += am;
-    }
-  }
-  part[threadIdx.x] = sum_h;
-  part[CH_PIX * CH_GROUPS + threadIdx.x] = sum_m;
-  __syncthreads();
-  if (g == 0 && inside) {
-    float th = 0.f, tm = 0.f;
-#pragma unroll
-    for (int q = 0; q < CH_GROUPS; ++q) {
-      th += part[q * CH_PIX + lp];
-      tm += part[CH_PIX * CH_GROUPS + q * CH_PIX + lp];
-    }
-    float v = th / tm;  // 0/0 -> NaN exactly like the reference when no view covers the pixel
-    if (flag && *flag) v = __int_as_float(0x7fc00000);  // the packed mask was not binary
-    out[pix] = v;
-  }
-}
-
-// ----------------------------------------------------------------------------------------------
-// Tiled variant: shared-memory staging of the source footprint.
-// The gather kernel above is bound by L1 wavefronts: a warp's 8x4 output patch lands on ~8 different 128 B lines per
-// load under rotation, 8 loads per (pixel, view).  Here a block owns a 32x32 output tile; for every view the source
-// footprint of the tile (bounding box of its four warped corners -- a homography with Z > 0 maps the tile to a convex
-// quadrilateral -- widened to 16 B columns, +1 pixel of slack) is copied row by row with 16-byte cp.async
-// (coalesced, double buffered: view n+1 streams in while view n is sampled) and the 8 bilinear taps come from
-// shared memory (8x4 patches per warp, row stride = 4 mod 8 floats: conflict-free along x, y and diagonals).
-// Views whose footprint does not fit (or with a non-positive Z at a corner) take the global gather for that view.
-// ----------------------------------------------------------------------------------------------
-#define CT_TILE 32
-#define CT_THREADS 256
-#define CT_CAP 4096  // floats per plane and buffer
-
-struct CtMeta { int bx0, by0, bw, bh; };  // bw = staged width (multiple of 4), bh = rows; bh == 0: nothing to sample; bw < 0: gather path
-
-__device__ __forceinline__ void cp_async16(void* smem_dst, const void* gsrc) {
-  unsigned int d = (unsigned int)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
-}
-__device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commit_group;" ::: "memory"); }
-template <int N_>
-__device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N_) : "memory"); }
-
-__device__ __forceinline__ int ct_stride(int bw) {  // multiple of 4, congruent 4 mod 8
-  return (bw & 4) ? bw : bw + 4;
-}
-
-__global__ void __launch_bounds__(CT_THREADS)
-combine_heatmap_tiled_kernel(const float* __restrict__ heat, const float* __restrict__ mask,
-                             const float* __restrict__ Hinv, int N, int H, int W, const float* __restrict__ xs,
-                             const float* __restrict__ ys, float* __restrict__ out) {
-  extern __shared__ __align__(16) float sh[];
-  float* bufs = sh;                                  // 2 buffers x 2 planes x CT_CAP
-  float* hs = bufs + 4 * CT_CAP;                     // N*9
-  CtMeta* meta = reinterpret_cast<CtMeta*>(hs + ((N * 9 + 3) & ~3));  // N
-  heat += (size_t)blockIdx.y * N * H * W;
-  mask += (size_t)blockIdx.y * N * H * W;
-  Hinv += (size_t)blockIdx.y * N * 9;
-  out += (size_t)blockIdx.y * H * W;
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-  const int tiles_x = (W + CT_TILE - 1) / CT_TILE;
-  const int tx0 = (blockIdx.x % tiles_x) * CT_TILE, ty0 = (blockIdx.x / tiles_x) * CT_TILE;
-  for (int i = tid; i < N * 9; i += CT_THREADS) hs[i] = Hinv[i];
-  __syncthreads();
-  // footprint of the tile under every view
-  for (int n = tid; n < N; n += CT_THREADS) {
-    const float* h = hs + n * 9;
-    const int cx[2] = {tx0, min(tx0 + CT_TILE - 1, W - 1)}, cy[2] = {ty0, min(ty0 + CT_TILE - 1, H - 1)};
-    float xmin = 3.0e38f, xmax = -3.0e38f, ymin = 3.0e38f, ymax = -3.0e38f;
-    bool ok = true;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      float gx = __ldg(xs + cx[c & 1]), gy = __ldg(ys + cy[c >> 1]);
-      float Z = fmaf(h[7], gy, h[6] * gx) + h[8];
-      float nx, ny;
-      homography_apply(h, gx, gy, nx, ny);
-      float ix = ((nx + 1.f) / 2.f) * (float)(W - 1), iy = ((ny + 1.f) / 2.f) * (float)(H - 1);
-      ok = ok && Z > 1e-6f && fabsf(ix) < 1.0e6f && fabsf(iy) < 1.0e6f;
-      xmin = fminf(xmin, ix); xmax = fmaxf(xmax, ix); ymin = fminf(ymin, iy); ymax = fmaxf(ymax, iy);
-    }
-    CtMeta m;
-    m.bx0 = m.by0 = m.bh = 0;
-    m.bw = -1;
-    if (ok) {
-      int x0 = max((int)floorf(xmin) - 1, 0) & ~3, x1 = min(((int)floorf(xmax) + 3 + 3) & ~3, W);
-      int y0 = max((int)floorf(ymin) - 1, 0), y1 = min((int)floorf(ymax) + 3, H);
-      if (x1 <= x0 || y1 <= y0) {
-        m.bw = 4; m.bh = 0;  // the whole footprint is outside the image: every tap is zero
-      } else if (ct_stride(x1 - x0) * (y1 - y0) <= CT_CAP) {
-        m.bx0 = x0; m.by0 = y0; m.bw = x1 - x0; m.bh = y1 - y0;
-      }
-    }
-    meta[n] = m;
-  }
-  __syncthreads();
-
-  auto prefetch = [&](int n) {
-    const CtMeta m = meta[n];
-    if (m.bw > 0 && m.bh > 0) {
-      float* bh_ = bufs + (n & 1) * 2 * CT_CAP;
-      float* bm_ = bh_ + CT_CAP;
-      const int vpr = m.bw >> 2, stride = ct_stride(m.bw), nvec = vpr * m.bh;
-      const float* hp = heat + (size_t)n * H * W + (size_t)m.by0 * W + m.bx0;
-      const float* mp = mask + (size_t)n * H * W + (size_t)m.by0 * W + m.bx0;
-      for (int v = tid; v < nvec; v += CT_THREADS) {
-        int row = v / vpr, c4 = (v - row * vpr) << 2;
-        cp_async16(bh_ + row * stride + c4, hp + (size_t)row * W + c4);
-        cp_async16(bm_ + row * stride + c4, mp + (size_t)row * W + c4);
-      }
-    }
-    cp_async_commit();
-  };
-
-  // pixel k of this thread: 8x4 patch p = warp + 8k of the 4 x 8 patch grid of the tile
-  float gxv[4], gyv[4], sum_h[4], sum_m[4];
-  bool inside[4];
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    int p = warp + 8 * k;
-    int x = tx0 + (p & 3) * 8 + (lane & 7), y = ty0 + (p >> 2) * 4 + (lane >> 3);
-    inside[k] = x < W && y < H;
-    gxv[k] = inside[k] ? __ldg(xs + x) : 0.f;
-    gyv[k] = inside[k] ? __ldg(ys + y) : 0.f;
-    sum_h[k] = 0.f;
-    sum_m[k] = 0.f;
-  }
-  const size_t plane = (size_t)H * W;
-  prefetch(0);
-  for (int n = 0; n < N; ++n) {
-    if (n + 1 < N) {
-      prefetch(n + 1);
-      cp_async_wait<1>();
-    } else {
-      cp_async_wait<0>();
-    }
-    __syncthreads();
-    const CtMeta m = meta[n];
-    if (m.bh != 0 || m.bw < 0) {
-      const float* h = hs + n * 9;
-      const bool staged = m.bw > 0;
-      const float* bh_ = bufs + (n & 1) * 2 * CT_CAP;
-      const float* bm_ = bh_ + CT_CAP;
-      const int stride = ct_stride(m.bw > 0 ? m.bw : 4);
-      const float* hp = heat + n * plane;
-      const float* mp = mask + n * plane;
-#pragma unroll
-      for (int k = 0; k < 4; ++k) {
-        if (!inside[k]) continue;
-        float nx, ny;
-        homography_apply(h, gxv[k], gyv[k], nx, ny);
-        float ix = ((nx + 1.f) / 2.f) * (float)(W - 1);
-        float iy = ((ny + 1.f) / 2.f) * (float)(H - 1);
-        float fx = floorf(ix), fy = floorf(iy);
-        if (!(fx >= -1.f && fx < (float)W && fy >= -1.f && fy < (float)H)) continue;
-        int x0 = (int)fx, y0 = (int)fy, x1 = x0 + 1, y1 = y0 + 1;
-        float wx1 = ix - fx, wx0 = (fx + 1.f) - ix;
-        float wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
-        bool xin0 = x0 >= 0, xin1 = x1 < W, yin0 = y0 >= 0, yin1 = y1 < H;
-        // staged taps must also lie inside the staged box (they do, by construction; the test keeps a rounding
-        // surprise from reading the wrong pixel: such a tap goes to global memory instead)
-        bool box = staged && x0 >= m.bx0 - (xin0 ? 0 : 1) && x1 < m.bx0 + m.bw + (xin1 ? 0 : 1) &&
-                   y0 >= m.by0 - (yin0 ? 0 : 1) && y1 < m.by0 + m.bh + (yin1 ? 0 : 1);
-        float ah = 0.f, am = 0.f;
-        if (box) {
-          const int o00 = (y0 - m.by0) * stride + (x0 - m.bx0);
-          if (yin0) {
-            if (xin0) { float mm = bm_[o00], w = wx0 * wy0; am += mm * w; ah += (bh_[o00] * mm) * w; }
-            if (xin1) { float mm = bm_[o00 + 1], w = wx1 * wy0; am += mm * w; ah += (bh_[o00 + 1] * mm) * w; }
-          }
-          if (yin1) {
-            if (xin0) { float mm = bm_[o00 + stride], w = wx0 * wy1; am += mm * w; ah += (bh_[o00 + stride] * mm) * w; }
-            if (xin1) { float mm = bm_[o00 + stride + 1], w = wx1 * wy1; am += mm * w; ah += (bh_[o00 + stride + 1] * mm) * w; }
-          }
-        } else {
-          if (yin0) {
-            size_t r = (size_t)y0 * W;
-            if (xin0) { float mm = __ldg(mp + r + x0), w = wx0 * wy0; am += mm * w; ah += (__ldg(hp + r + x0) * mm) * w; }
-            if (xin1) { float mm = __ldg(mp + r + x1), w = wx1 * wy0; am += mm * w; ah += (__ldg(hp + r + x1) * mm) * w; }
-          }
-          if (yin1) {
-            size_t r = (size_t)y1 * W;
-            if (xin0) { float mm = __ldg(mp + r + x0), w = wx0 * wy1; am += mm * w; ah += (__ldg(hp + r + x0) * mm) * w; }
-            if (xin1) { float mm = __ldg(mp + r + x1), w = wx1 * wy1; am += mm * w; ah += (__ldg(hp + r + x1) * mm) * w; }
-          }
-        }
-        sum_h[k] += ah;
-        sum_m[k] += am;
-      }
-    }
-    __syncthreads();  // buffer (n & 1) is refilled by the prefetch of view n + 2
-  }
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (!inside[k]) continue;
-    int p = warp + 8 * k;
-    int x = tx0 + (p & 3) * 8 + (lane & 7), y = ty0 + (p >> 2) * 4 + (lane >> 3);
-    out[(size_t)y * W + x] = sum_h[k] / sum_m[k];  // 0/0 -> NaN exactly like the reference when no view covers the pixel
-  }
-}
-
-static int combine_launch(int variant /*0 gather, 1 tiled, -1 default*/, const float* heat, const float* mask,
-                          const float* Hinv, int I, int N, int H, int W, const float* xs, const float* ys, float* out,
-                          void* stream) {
-  SSP_REQUIRE(heat && mask && Hinv && xs && ys && out, "ssp_combine_heatmap: null pointer");
-  SSP_REQUIRE(I > 0 && I <= 65535 && N > 0 && H > 0 && W > 0, "ssp_combine_heatmap: bad sizes I=%d N=%d H=%d W=%d", I, N, H, W);
-  // The direct-gather kernel is the default: measured on B200 (16 images x 100 views per call) the adaptation step ran
-  // 9.5 k images/s with it and 8.6 k with the tiled kernel -- three 69 KB blocks per SM and two barriers per view hide
-  // less latency than eight gather blocks, although the tiled kernel issues a third of the L1 wavefronts.
-  // SSP_COMBINE=tiled makes the staged kernel the default (kept for larger images / future tuning, parity-tested).
-  static const bool env_tiled = [] { const char* e = getenv("SSP_COMBINE"); return e && e[0] == 't'; }();
-  size_t smem_t = (4 * (size_t)CT_CAP + (((size_t)N * 9 + 3) & ~(size_t)3)) * sizeof(float) + (size_t)N * sizeof(CtMeta);
-  bool can_tile = W % 4 == 0 && ((((uintptr_t)heat | (uintptr_t)mask) & 15) == 0) && smem_t <= 200 * 1024;
-  SSP_REQUIRE(variant != 1 || can_tile, "ssp_combine_heatmap_tiled: needs W %% 4 == 0, 16-byte aligned maps and N <= ~3500 views");
-  bool tiled = variant == 1 || (variant < 0 && env_tiled && can_tile);
-  if (tiled) {
-    static bool attr_done = false;
-    if (!attr_done) {
-      SSP_CUDA_CALL(cudaFuncSetAttribute(combine_heatmap_tiled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
-      attr_done = true;
-    }
-    dim3 nblk(ssp_ceil_div(W, CT_TILE) * ssp_ceil_div(H, CT_TILE), I);
-    combine_heatmap_tiled_kernel<<<nblk, CT_THREADS, smem_t, (cudaStream_t)stream>>>(heat, mask, Hinv, N, H, W, xs, ys, out);
-    SSP_CUDA_CHECK_LAUNCH("combine_heatmap_tiled_kernel");
-    return SSP_OK;
-  }
+template <bool SIGNED>
+static int combine_launch(const char* name, const float* heat, const float* mask, const float* Hinv, int I, int N, int H,
+                          int W, const float* xs, const float* ys, const int* flag, float* out, void* stream) {
+  SSP_REQUIRE(I > 0 && I <= 65535 && N > 0 && H > 0 && W > 0, "%s: bad sizes I=%d N=%d H=%d W=%d", name, I, N, H, W);
   size_t smem = ((size_t)N * 12 + 2 * CH_PIX * CH_GROUPS) * sizeof(float);
-  SSP_REQUIRE(smem <= 48 * 1024, "ssp_combine_heatmap: N=%d views exceed the shared-memory table (max ~900)", N);
+  SSP_REQUIRE(smem <= 48 * 1024, "%s: N=%d views exceed the shared-memory table (max ~900)", name, N);
   dim3 nblk(ssp_ceil_div(W, 8) * ssp_ceil_div(H, 8), I);
-  combine_heatmap_kernel<<<nblk, CH_PIX * CH_GROUPS, smem, (cudaStream_t)stream>>>(heat, mask, Hinv, N, H, W, xs, ys, out);
+  combine_heatmap_kernel<SIGNED><<<nblk, CH_PIX * CH_GROUPS, smem, (cudaStream_t)stream>>>(heat, mask, Hinv, N, H, W, xs, ys,
+                                                                                          flag, out);
   SSP_CUDA_CHECK_LAUNCH("combine_heatmap_kernel");
   return SSP_OK;
 }
 
 extern "C" int ssp_combine_heatmap(const float* heat, const float* mask, const float* Hinv, int I, int N, int H, int W,
                                    const float* xs, const float* ys, float* out, void* stream) {
-  return combine_launch(-1, heat, mask, Hinv, I, N, H, W, xs, ys, out, stream);
-}
-
-// the shared-memory staged variant, explicitly (same arguments and results)
-extern "C" int ssp_combine_heatmap_tiled(const float* heat, const float* mask, const float* Hinv, int I, int N, int H,
-                                         int W, const float* xs, const float* ys, float* out, void* stream) {
-  return combine_launch(1, heat, mask, Hinv, I, N, H, W, xs, ys, out, stream);
+  SSP_REQUIRE(heat && mask && Hinv && xs && ys && out, "ssp_combine_heatmap: null pointer");
+  return combine_launch<false>("ssp_combine_heatmap", heat, mask, Hinv, I, N, H, W, xs, ys, nullptr, out, stream);
 }
 
 // heat = flatten_detection_masked output [I,N,H,W]; flag = its non-binary-mask flag (device int) or NULL
 extern "C" int ssp_combine_heatmap_signed(const float* heat, const float* Hinv, int I, int N, int H, int W, const float* xs,
                                           const float* ys, const int* flag, float* out, void* stream) {
   SSP_REQUIRE(heat && Hinv && xs && ys && out, "ssp_combine_heatmap_signed: null pointer");
-  SSP_REQUIRE(I > 0 && I <= 65535 && N > 0 && H > 0 && W > 0, "ssp_combine_heatmap_signed: bad sizes I=%d N=%d H=%d W=%d", I, N, H, W);
-  size_t smem = ((size_t)N * 12 + 2 * CH_PIX * CH_GROUPS) * sizeof(float);
-  SSP_REQUIRE(smem <= 48 * 1024, "ssp_combine_heatmap_signed: N=%d views exceed the shared-memory table (max ~900)", N);
-  dim3 nblk(ssp_ceil_div(W, 8) * ssp_ceil_div(H, 8), I);
-  combine_heatmap_signed_kernel<<<nblk, CH_PIX * CH_GROUPS, smem, (cudaStream_t)stream>>>(heat, Hinv, N, H, W, xs, ys, flag, out);
-  SSP_CUDA_CHECK_LAUNCH("combine_heatmap_signed_kernel");
-  return SSP_OK;
-}
-
-// ---- bit-mask path ----
-extern "C" size_t ssp_mask_bits_words(int rows, int W) { return (size_t)rows * ((W + 31) / 32); }
-
-// mask [rows, W] float 0/1 -> bits [rows, ceil(W/32)] (bit x & 31 of word x >> 5).  flag (device int, zeroed by the caller) is set
-// when a value other than 0 / 1 was seen.
-extern "C" int ssp_mask_pack_bits(const float* mask, long long rows, int W, uint32_t* bits, int* flag, void* stream) {
-  SSP_REQUIRE(mask && bits && flag, "ssp_mask_pack_bits: null pointer");
-  SSP_REQUIRE(rows > 0 && W > 0, "ssp_mask_pack_bits: bad sizes");
-  const int WP = (W + 31) / 32;
-  const size_t warps = (size_t)rows * WP;
-  SSP_REQUIRE((warps + 7) / 8 <= 0x7fffffffull, "ssp_mask_pack_bits: too many rows");
-  mask_pack_bits_kernel<<<(unsigned)((warps + 7) / 8), 256, 0, (cudaStream_t)stream>>>(mask, (size_t)rows, W, WP, bits, flag);
-  SSP_CUDA_CHECK_LAUNCH("mask_pack_bits_kernel");
-  return SSP_OK;
-}
-
-// compute_valid_mask(image_shape, inv_homography, erosion_radius = 0) as bits [B, H, ceil(W/32)]
-extern "C" int ssp_valid_mask_bits(int B, int H, int W, const float* Hinv, const float* xs, const float* ys, uint32_t* bits,
-                                   void* stream) {
-  SSP_REQUIRE(Hinv && xs && ys && bits, "ssp_valid_mask_bits: null pointer");
-  SSP_REQUIRE(B > 0 && B <= 65535 && H > 0 && W > 0, "ssp_valid_mask_bits: bad sizes");
-  const int WP = (W + 31) / 32;
-  dim3 grid(WP, ssp_ceil_div(H, 8), B);
-  valid_mask_bits_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(H, W, WP, Hinv, xs, ys, bits);
-  SSP_CUDA_CHECK_LAUNCH("valid_mask_bits_kernel");
-  return SSP_OK;
-}
-
-// combine_heatmap with the valid masks given as bits (flag: optional device int from ssp_mask_pack_bits)
-extern "C" int ssp_combine_heatmap_bits(const float* heat, const uint32_t* mbits, const float* Hinv, int I, int N, int H, int W,
-                                        const float* xs, const float* ys, const int* flag, float* out, void* stream) {
-  SSP_REQUIRE(heat && mbits && Hinv && xs && ys && out, "ssp_combine_heatmap_bits: null pointer");
-  SSP_REQUIRE(I > 0 && I <= 65535 && N > 0 && H > 0 && W > 0, "ssp_combine_heatmap_bits: bad sizes I=%d N=%d H=%d W=%d", I, N, H, W);
-  size_t smem = ((size_t)N * 9 + 2 * CH_PIX * CH_GROUPS) * sizeof(float);
-  SSP_REQUIRE(smem <= 48 * 1024, "ssp_combine_heatmap_bits: N=%d views exceed the shared-memory table (max ~1100)", N);
-  dim3 nblk(ssp_ceil_div(W, 8) * ssp_ceil_div(H, 8), I);
-  combine_heatmap_bits_kernel<<<nblk, CH_PIX * CH_GROUPS, smem, (cudaStream_t)stream>>>(heat, mbits, Hinv, N, H, W, (W + 31) / 32, xs,
-                                                                                          ys, flag, out);
-  SSP_CUDA_CHECK_LAUNCH("combine_heatmap_bits_kernel");
-  return SSP_OK;
+  return combine_launch<true>("ssp_combine_heatmap_signed", heat, nullptr, Hinv, I, N, H, W, xs, ys, flag, out, stream);
 }

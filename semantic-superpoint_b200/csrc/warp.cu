@@ -3,7 +3,6 @@
 // (Gabriel-SGama/Semantic-SuperPoint).  All kernels are HBM-bound streaming kernels; the source
 // image of a warp is gathered through L1/L2 (one image is 0.3-1.2 MB, far below the 126 MB L2).
 #include "common.cuh"
-#include <cstdlib>
 
 // ----------------------------------------------------------------------------------------------
 // a1: warp_points   out[b,p,:] = (H_b [x,y,1]^T)[:2] / (H_b [x,y,1]^T)[2]
@@ -92,36 +91,6 @@ extern "C" int ssp_warp_keypoints_f64(const double* kp, int K, const double* Hm,
 // The normalised grid values xs[W], ys[H] are passed in as tables (the reference builds them with a
 // CPU torch.linspace, utils/utils.py:375) so that sampling coordinates are reproduced exactly.
 // ----------------------------------------------------------------------------------------------
-__device__ __forceinline__ float bilinear_zero(const float* __restrict__ im, int H, int W, float ix, float iy) {
-  float fx = floorf(ix), fy = floorf(iy);
-  int x0 = (int)fx, y0 = (int)fy;
-  int x1 = x0 + 1, y1 = y0 + 1;
-  // weights exactly as ATen grid_sampler: nw=(x1-ix)(y1-iy) ne=(ix-x0)(y1-iy) sw=(x1-ix)(iy-y0) se=(ix-x0)(iy-y0)
-  float wx1 = ix - fx, wx0 = (fx + 1.f) - ix;
-  float wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
-  bool xin0 = (x0 >= 0) & (x0 < W), xin1 = (x1 >= 0) & (x1 < W);
-  bool yin0 = (y0 >= 0) & (y0 < H), yin1 = (y1 >= 0) & (y1 < H);
-  float acc = 0.f;
-  if (yin0) {
-    const float* r = im + (size_t)y0 * W;
-    if (xin0) acc += __ldg(r + x0) * (wx0 * wy0);
-    if (xin1) acc += __ldg(r + x1) * (wx1 * wy0);
-  }
-  if (yin1) {
-    const float* r = im + (size_t)y1 * W;
-    if (xin0) acc += __ldg(r + x0) * (wx0 * wy1);
-    if (xin1) acc += __ldg(r + x1) * (wx1 * wy1);
-  }
-  return acc;
-}
-
-__device__ __forceinline__ float nearest_zero(const float* __restrict__ im, int H, int W, float ix, float iy) {
-  // std::nearbyint under the default rounding mode = round half to even = rintf
-  float rx = rintf(ix), ry = rintf(iy);
-  if (rx >= 0.f && rx < (float)W && ry >= 0.f && ry < (float)H) return __ldg(im + (size_t)(int)ry * W + (int)rx);
-  return 0.f;
-}
-
 // src pixel coordinate of output pixel (x,y): grid_sampler unnormalize with align_corners=True
 __device__ __forceinline__ void src_coord(const float* h, float gx, float gy, int H, int W, float& ix, float& iy) {
   float nx, ny;
@@ -204,147 +173,12 @@ inv_warp_gather_kernel(const float* __restrict__ img, int C, int H, int W, const
   }
 }
 
-// Staged kernel (north_star's "float4 reads with shared-memory tile staging"; measured on B200 at 100 x 240 x 320: 103 us against
-// 53 us for the gather kernel above -- the warp is instruction-bound, not memory-bound -- so it is opt-in): a block owns a
-// 32x32 output tile of one image.  The source footprint of the tile (bounding
-// box of its four warped corners -- a homography with Z > 0 maps the tile to a convex quadrilateral -- widened to 16-byte
-// columns, +-2 pixels of slack) is copied row by row with 16-byte cp.async (fully coalesced 128-bit reads), the taps
-// come from shared memory, and every output row is one coalesced 128-byte store per warp.  Source coordinates are computed
-// once per pixel and reused for all channels.  A tap outside the staged box (rounding surprise) reads global memory, a
-// tile whose footprint does not fit (strong magnification, Z <= 0) takes the gather path per pixel.
-#define IW_TILE 32
-#define IW_CAP 6144  // floats staged per tile and channel (24 KB): a 32x32 tile rotated by 45 degrees at scale 1.25 needs ~60x60
-
-__device__ __forceinline__ void iw_cp_async16(void* smem_dst, const void* gsrc) {
-  unsigned int d = (unsigned int)__cvta_generic_to_shared(smem_dst);
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(d), "l"(gsrc) : "memory");
-}
-
-template <int MODE>
-__global__ void __launch_bounds__(256)
-inv_warp_staged_kernel(const float* __restrict__ img, int C, int H, int W, const float* __restrict__ Hinv,
-                       const float* __restrict__ xs, const float* __restrict__ ys, float* __restrict__ out) {
-  __shared__ __align__(16) float buf[IW_CAP];
-  __shared__ float h[9];
-  __shared__ int box[4];  // bx0, by0, bw (multiple of 4; 0 = nothing inside the image; -1 = does not fit), bh
-  const int b = blockIdx.z, tid = threadIdx.x;
-  const int tx0 = blockIdx.x * IW_TILE, ty0 = blockIdx.y * IW_TILE;
-  if (tid < 9) h[tid] = Hinv[b * 9 + tid];
-  __syncthreads();
-  if (tid == 0) {
-    const int cx[2] = {tx0, min(tx0 + IW_TILE - 1, W - 1)}, cy[2] = {ty0, min(ty0 + IW_TILE - 1, H - 1)};
-    float xmin = 3.0e38f, xmax = -3.0e38f, ymin = 3.0e38f, ymax = -3.0e38f;
-    bool ok = true;
-#pragma unroll
-    for (int c = 0; c < 4; ++c) {
-      const float gx = __ldg(xs + cx[c & 1]), gy = __ldg(ys + cy[c >> 1]);
-      const float Z = fmaf(h[7], gy, h[6] * gx) + h[8];
-      float ix, iy;
-      src_coord(h, gx, gy, H, W, ix, iy);
-      ok = ok && Z > 1e-6f && fabsf(ix) < 1.0e6f && fabsf(iy) < 1.0e6f;
-      xmin = fminf(xmin, ix); xmax = fmaxf(xmax, ix); ymin = fminf(ymin, iy); ymax = fmaxf(ymax, iy);
-    }
-    int bx0 = 0, by0 = 0, bw = -1, bh = 0;
-    if (ok) {
-      const int x0 = max((int)floorf(xmin) - 2, 0) & ~3, x1 = min(((int)floorf(xmax) + 4 + 3) & ~3, W);
-      const int y0 = max((int)floorf(ymin) - 2, 0), y1 = min((int)floorf(ymax) + 4, H);
-      if (x1 <= x0 || y1 <= y0) { bw = 0; bh = 0; }                      // footprint entirely outside: every tap is zero
-      else if ((x1 - x0) * (y1 - y0) <= IW_CAP) { bx0 = x0; by0 = y0; bw = x1 - x0; bh = y1 - y0; }
-    }
-    box[0] = bx0; box[1] = by0; box[2] = bw; box[3] = bh;
-  }
-  __syncthreads();
-  const int bx0 = box[0], by0 = box[1], bw = box[2], bh = box[3];
-  // this thread's four pixels: column tid & 31, rows (tid >> 5) + 8k -- a warp writes one 128-byte output row segment
-  const int x = tx0 + (tid & 31);
-  float ixv[4], iyv[4];
-  const float gx = x < W ? __ldg(xs + x) : 0.f;
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    const int y = ty0 + (tid >> 5) + 8 * k;
-    ixv[k] = 0.f; iyv[k] = 0.f;
-    if (x < W && y < H) src_coord(h, gx, __ldg(ys + y), H, W, ixv[k], iyv[k]);
-  }
-  const size_t plane = (size_t)H * W;
-  for (int c = 0; c < C; ++c) {
-    const float* im = img + ((size_t)b * C + c) * plane;
-    if (bw > 0) {
-      const int vpr = bw >> 2, nvec = vpr * bh;
-      const float* src = im + (size_t)by0 * W + bx0;
-      for (int v = tid; v < nvec; v += 256) {
-        const int row = v / vpr, c4 = (v - row * vpr) << 2;
-        iw_cp_async16(buf + row * bw + c4, src + (size_t)row * W + c4);
-      }
-      asm volatile("cp.async.commit_group;" ::: "memory");
-      asm volatile("cp.async.wait_group 0;" ::: "memory");
-    }
-    __syncthreads();
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-      const int y = ty0 + (tid >> 5) + 8 * k;
-      if (x >= W || y >= H) continue;
-      const float ix = ixv[k], iy = iyv[k];
-      float v = 0.f;
-      if (bw < 0) {
-        v = MODE == 0 ? bilinear_zero(im, H, W, ix, iy) : nearest_zero(im, H, W, ix, iy);
-      } else if (bw > 0) {
-        if (MODE == 0) {
-          const float fx = floorf(ix), fy = floorf(iy);
-          if (fx >= -1.f && fx < (float)W && fy >= -1.f && fy < (float)H) {  // else: all four taps outside, v = 0
-            const int x0 = (int)fx, y0 = (int)fy, x1 = x0 + 1, y1 = y0 + 1;
-            const float wx1 = ix - fx, wx0 = (fx + 1.f) - ix, wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
-            const bool xin0 = x0 >= 0, xin1 = x1 < W, yin0 = y0 >= 0, yin1 = y1 < H;
-            const bool inbox = x0 >= bx0 - (xin0 ? 0 : 1) && x1 < bx0 + bw + (xin1 ? 0 : 1) && y0 >= by0 - (yin0 ? 0 : 1) &&
-                               y1 < by0 + bh + (yin1 ? 0 : 1);
-            if (inbox) {
-              const int o = (y0 - by0) * bw + (x0 - bx0);
-              // same tap order and arithmetic as bilinear_zero: nw, ne, sw, se
-              if (yin0) {
-                if (xin0) v += buf[o] * (wx0 * wy0);
-                if (xin1) v += buf[o + 1] * (wx1 * wy0);
-              }
-              if (yin1) {
-                if (xin0) v += buf[o + bw] * (wx0 * wy1);
-                if (xin1) v += buf[o + bw + 1] * (wx1 * wy1);
-              }
-            } else {
-              v = bilinear_zero(im, H, W, ix, iy);
-            }
-          }
-        } else {
-          const float rx = rintf(ix), ry = rintf(iy);
-          if (rx >= 0.f && rx < (float)W && ry >= 0.f && ry < (float)H) {
-            const int xi = (int)rx, yi = (int)ry;
-            v = (xi >= bx0 && xi < bx0 + bw && yi >= by0 && yi < by0 + bh) ? buf[(yi - by0) * bw + (xi - bx0)]
-                                                                            : __ldg(im + (size_t)yi * W + xi);
-          }
-        }
-      }
-      out[((size_t)b * C + c) * plane + (size_t)y * W + x] = v;
-    }
-    if (c + 1 < C) __syncthreads();  // the buffer is refilled for the next channel
-  }
-}
-
 extern "C" int ssp_inv_warp_image(const float* img, int B, int C, int H, int W, const float* Hinv,
                                   const float* xs, const float* ys, int mode, float* out, void* stream) {
   SSP_REQUIRE(img && Hinv && xs && ys && out, "ssp_inv_warp_image: null pointer");
   SSP_REQUIRE(B > 0 && C > 0 && H > 0 && W > 0, "ssp_inv_warp_image: bad sizes B=%d C=%d H=%d W=%d", B, C, H, W);
-  SSP_REQUIRE(mode >= 0 && mode <= 3, "ssp_inv_warp_image: mode must be 0 (bilinear) or 1 (nearest), +2 to force the gather kernel; got %d", mode);
+  SSP_REQUIRE(mode == 0 || mode == 1, "ssp_inv_warp_image: mode must be 0 (bilinear) or 1 (nearest); got %d", mode);
   SSP_REQUIRE(B <= 65535, "ssp_inv_warp_image: batch %d exceeds grid.z limit", B);
-  // 16-byte staging needs rows that start on 16-byte boundaries; anything else takes the gather kernel
-  const bool force_gather = (mode & 2) != 0;
-  mode &= 1;
-  const bool staged = !force_gather && W % 4 == 0 && (((uintptr_t)img) & 15) == 0;  // host side: staged only on request
-  if (staged) {
-    dim3 grid(ssp_ceil_div(W, IW_TILE), ssp_ceil_div(H, IW_TILE), B);
-    if (mode == 0)
-      inv_warp_staged_kernel<0><<<grid, 256, 0, (cudaStream_t)stream>>>(img, C, H, W, Hinv, xs, ys, out);
-    else
-      inv_warp_staged_kernel<1><<<grid, 256, 0, (cudaStream_t)stream>>>(img, C, H, W, Hinv, xs, ys, out);
-    SSP_CUDA_CHECK_LAUNCH("inv_warp_staged_kernel");
-    return SSP_OK;
-  }
   dim3 block(32, 8);
   dim3 grid(ssp_ceil_div(W, 32), ssp_ceil_div(H, 8 * IWG_PX), B);
   if (mode == 0)

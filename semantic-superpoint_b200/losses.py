@@ -6,8 +6,6 @@ numerators / mask sums are exchanged by ONE peer-memory kernel (dist.LossExchang
 the loss scalars and normalisers in place, stream ordered, before the forward returns; the backward kernels
 scale by the global normaliser.
 """
-import os
-
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -15,10 +13,6 @@ from . import _lib
 from ._lib import call, f32c, ptr, stream_of
 
 _ENGINES = ("bf16x3", "bf16", "fp32")
-# The fused step folds the (binary) cell mask into the indicator words of the tensor-core engines, so the backward needs no
-# pack pass (measured: 0.339 -> 0.330 ms per step).  SSP_BG_ALPHA=pack restores the general path (alpha * Dw packed into
-# its own planes), which is also what the reference-signature `descriptor_loss` always uses (its mask may be anything).
-FOLD_ALPHA = os.environ.get("SSP_BG_ALPHA", "fold") != "pack"
 _engine = "bf16x3"
 CHECK_LIST_OVERFLOW = False  # tests turn this on (costs a host sync per call)
 
@@ -494,8 +488,12 @@ class LossStepFn(torch.autograd.Function):
             raise RuntimeError("loss_step: mask_warp_2D must be [B,1,%d,%d]" % (Hc * 8, Wc * 8))
         c2 = _Ctx((ctx.needs_input_grad[6], ctx.needs_input_grad[7]) + (False,) * 8)
         total = torch.empty((1,), dtype=torch.float32, device=dev)
+        # fold_alpha=True: the cell mask is folded into the indicator words of the tensor-core engines, so the backward needs
+        # no pack pass (measured: 0.339 -> 0.330 ms per step).  Fold requires a binary mask and g_neg = 0; the latter holds
+        # because only `loss` is differentiable, and a non-binary mask turns the loss into NaN.  A soft mask belongs on
+        # fused=False, whose descriptor_loss packs alpha * Dw into its own planes.
         ld, pos, neg, _wpts = DescriptorLossFn.forward(c2, desc, desc_w, Hm, ("2d", mw), 8, lamda_d, dist, engine,
-                                                       None, None, FOLD_ALPHA, (c1.out, lambda_loss, total, fork))
+                                                       None, None, True, (c1.out, lambda_loss, total, fork))
         if dist_group is not None:
             # multi-GPU: ONE exchange kernel turns the three local results into global-batch values in place (the scalars
             # above are views of c1.out / c2.out8) and rewrites the weighted total; the backward kernels read the global

@@ -65,27 +65,21 @@ def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2
 
 
 @torch.no_grad()
-def adaptation_step(semi, inv_homographies, mask_2D=None, conf_thresh=0.015, nms_dist=4, top_k=600, binary_mask=False,
-                    mask_homographies=None):
+def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist=4, top_k=600, binary_mask=False):
     """semi [I,N,65,Hc,Wc] (or [N,65,Hc,Wc]), inv_homographies [I,N,3,3], mask_2D [I,N,H,W] -> list of [K,3] arrays
     (x, y, prob), K <= top_k, per source image.
     mask_2D is the stack of valid masks of the warped views; binary_mask=True promises a 0/1 mask (compute_valid_mask's output,
     what the export path always passes): the mask is folded into the flattened heatmap as its sign and the aggregation gathers
-    one array instead of two (bit-identical results; a non-binary mask then yields NaN heatmaps).
-    mask_2D=None + mask_homographies [I,N,3,3]: the masks are compute_valid_mask(shape, mask_homographies, 0) as in
-    datasets/Coco.py:284-288 and are generated as bits on the device."""
+    one array instead of two (bit-identical results; a non-binary mask then yields NaN heatmaps)."""
     if semi.dim() == 4:
         semi, inv_homographies = semi.unsqueeze(0), inv_homographies.reshape(1, -1, 3, 3)
-        if mask_2D is not None:
-            mask_2D = mask_2D.reshape(1, semi.shape[1], mask_2D.shape[-2], mask_2D.shape[-1])
-        if mask_homographies is not None:
-            mask_homographies = mask_homographies.reshape(1, -1, 3, 3)
+        mask_2D = mask_2D.reshape(1, semi.shape[1], mask_2D.shape[-2], mask_2D.shape[-1])
     I, N, C, Hc, Wc = semi.shape
-    if binary_mask and mask_2D is not None:
+    if binary_mask:
         agg = U.combine_from_logits_batch(semi, inv_homographies, mask_2D)
     else:
         heat = U.flattenDetection(semi.reshape(I * N, C, Hc, Wc)).reshape(I, N, Hc * 8, Wc * 8)
-        agg = U.combine_heatmap_batch(heat, inv_homographies, mask_2D, mask_homographies=mask_homographies)
+        agg = U.combine_heatmap_batch(heat, inv_homographies, mask_2D)
     pts = U.heatmap_to_pts_batch(agg, conf_thresh, nms_dist, top_k=top_k)
     return [p.transpose() for p in pts]
 

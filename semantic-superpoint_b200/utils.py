@@ -174,9 +174,8 @@ def denormPts(pts, shape):
 # ------------------------------------------------------------------------------------------------
 # a2 / a3  image warps
 # ------------------------------------------------------------------------------------------------
-def inv_warp_image_batch(img, mat_homo_inv, device="cpu", mode="bilinear", staged=False):
-    """reference: utils/utils.py:347-385.  img [B,C,H,W] (2-D/3-D viewed as [1,1,H,W]), H^-1 [B,3,3] / [3,3].
-    staged=True selects the shared-memory staged kernel instead of the per-pixel gather (same results, measured slower)."""
+def inv_warp_image_batch(img, mat_homo_inv, device="cpu", mode="bilinear"):
+    """reference: utils/utils.py:347-385.  img [B,C,H,W] (2-D/3-D viewed as [1,1,H,W]), H^-1 [B,3,3] / [3,3]."""
     _no_grad_inputs("inv_warp_image_batch", img, mat_homo_inv)
     if img.dim() == 2 or img.dim() == 3:
         img = img.view(1, 1, img.shape[0], img.shape[1])
@@ -193,7 +192,7 @@ def inv_warp_image_batch(img, mat_homo_inv, device="cpu", mode="bilinear", stage
         raise RuntimeError("inv_warp_image_batch: %d images but %d homographies" % (B, Hm.shape[0]))
     out = torch.empty_like(x)
     call("ssp_inv_warp_image", ptr(x), B, C, H, W, ptr(Hm), ptr(_linspace_grid(W, dev)), ptr(_linspace_grid(H, dev)),
-         (0 if mode == "bilinear" else 1) + (0 if staged else 2), ptr(out), stream_of(out))  # +2: gather kernel
+         0 if mode == "bilinear" else 1, ptr(out), stream_of(out))
     return out.to(out_dev)
 
 
@@ -353,35 +352,13 @@ def combine_heatmap(heatmap, inv_homographies, mask_2D, device="cpu"):
     return out.to(out_dev)
 
 
-def combine_heatmap_batch(heatmap, inv_homographies, mask_2D=None, tiled=False, binary_mask=False, mask_homographies=None):
-    """Batched export form: heatmap/mask [I,N,H,W], inv_homographies [I,N,3,3] -> [I,H,W] in one launch.
-    tiled=True runs the shared-memory staged kernel (same results; see csrc/heatmap.cu for when it pays).
-    binary_mask=True: mask_2D is a 0/1 image (what compute_valid_mask returns): it is packed to one bit per pixel first and the
-    bit-mask kernel runs (bit-identical results, a third fewer gather instructions; a non-binary mask gives NaN).
-    mask_2D=None with mask_homographies [I,N,3,3]: the masks of the export path, compute_valid_mask(shape, mask_homographies,
-    erosion_radius=0) (datasets/Coco.py:284-288), are generated directly as bits -- no float mask ever exists."""
+def combine_heatmap_batch(heatmap, inv_homographies, mask_2D):
+    """Batched export form: heatmap/mask [I,N,H,W], inv_homographies [I,N,3,3] -> [I,H,W] in one launch."""
     dev = _cuda_device("cuda", heatmap)
-    h, Hm = f32c(heatmap, dev), f32c(inv_homographies, dev)
+    h, Hm, m = f32c(heatmap, dev), f32c(inv_homographies, dev), f32c(mask_2D, dev)
     I, N, H, W = h.shape
     out = torch.empty((I, H, W), dtype=torch.float32, device=dev)
-    xs, ys = _linspace_grid(W, dev), _linspace_grid(H, dev)
-    if mask_2D is None or binary_mask:
-        words = _lib.load().ssp_mask_bits_words(I * N * H, W)
-        bits = torch.empty((words,), dtype=torch.int32, device=dev)
-        flag = None
-        if mask_2D is None:
-            if mask_homographies is None:
-                raise ValueError("combine_heatmap_batch: give mask_2D or the homographies the valid masks are built from")
-            Hmask = f32c(mask_homographies, dev).reshape(-1, 3, 3)
-            call("ssp_valid_mask_bits", I * N, H, W, ptr(Hmask), ptr(xs), ptr(ys), ptr(bits), stream_of(out))
-        else:
-            m = f32c(mask_2D, dev)
-            flag = torch.zeros((1,), dtype=torch.int32, device=dev)
-            call("ssp_mask_pack_bits", ptr(m), I * N * H, W, ptr(bits), ptr(flag), stream_of(out))
-        call("ssp_combine_heatmap_bits", ptr(h), ptr(bits), ptr(Hm), I, N, H, W, ptr(xs), ptr(ys), ptr(flag), ptr(out), stream_of(out))
-        return out
-    m = f32c(mask_2D, dev)
-    call("ssp_combine_heatmap_tiled" if tiled else "ssp_combine_heatmap", ptr(h), ptr(m), ptr(Hm), I, N, H, W, ptr(xs), ptr(ys),
+    call("ssp_combine_heatmap", ptr(h), ptr(m), ptr(Hm), I, N, H, W, ptr(_linspace_grid(W, dev)), ptr(_linspace_grid(H, dev)),
          ptr(out), stream_of(out))
     return out
 

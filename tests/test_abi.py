@@ -2,6 +2,7 @@
 import ctypes
 import os
 import re
+import subprocess
 
 from conftest import ROOT
 
@@ -21,6 +22,15 @@ def test_library_builds_and_exports_header_symbols():
     for s in syms:
         assert hasattr(lib, s), "missing export %s" % s
     assert lib.ssp_version() >= 100
+
+
+def test_library_exports_only_header_symbols():
+    """Every ssp_* symbol the library defines is declared in the header: no entry point outlives its declaration."""
+    import ssp_b200
+    path = ssp_b200.build.build_library()
+    out = subprocess.run(["nm", "-D", "--defined-only", path], capture_output=True, text=True, check=True).stdout
+    exported = sorted({line.split()[-1] for line in out.splitlines() if line.split() and line.split()[-1].startswith("ssp_")})
+    assert exported == header_symbols()
 
 
 def test_python_signatures_match_header():
@@ -46,6 +56,9 @@ def test_argument_errors_without_gpu():
     assert b"null pointer" in lib.ssp_last_error()
     assert lib.ssp_labels2d_to_3d(ctypes.c_void_p(16), 1, 12, 12, 1, ctypes.c_void_p(16), None) < 0
     assert b"multiples of 8" in lib.ssp_last_error()
+    p = ctypes.c_void_p(16)
+    assert lib.ssp_inv_warp_image(p, 1, 1, 8, 8, p, p, p, 2, p, None) < 0  # mode is 0 (bilinear) or 1 (nearest)
+    assert b"mode" in lib.ssp_last_error()
     assert lib.ssp_detector_loss_ws_bytes(32, 30, 40) >= 16 + 300 * 16
 
 

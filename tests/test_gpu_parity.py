@@ -121,23 +121,20 @@ def test_inv_warp_240x320():
             assert_only_rounding_ties(out, ref, Hinv)
 
 
-def test_inv_warp_staged_equals_gather():
-    """The shared-memory staged kernel (default) and the per-pixel gather kernel are the same function, bit for bit:
-    multi-channel images, strong warps (footprints that overflow the staging buffer fall back per tile), identity,
-    and a width that is not a multiple of 4 (always gather)."""
-    rng = np.random.default_rng(5)
+def test_inv_warp_multichannel_strong_warps():
+    """Multi-channel images under identity, magnifying and strongly minifying homographies, and a width that is not a
+    multiple of 4, against the oracle in both modes."""
     _, Hinv = homographies(6, 13)
     Hinv[0] = np.eye(3)
-    Hinv[1] = np.array([[0.3, 0, 0], [0, 0.3, 0], [0, 0, 1]], np.float32)      # 3.3x magnification of the sampled region... footprint small
-    Hinv[2] = np.array([[3.0, 0.4, 0.1], [-0.5, 2.5, 0], [0.2, 0.1, 1]], np.float32)  # minification: footprint overflows the buffer
+    Hinv[1] = np.array([[0.3, 0, 0], [0, 0.3, 0], [0, 0, 1]], np.float32)            # 3.3x magnification
+    Hinv[2] = np.array([[3.0, 0.4, 0.1], [-0.5, 2.5, 0], [0.2, 0.1, 1]], np.float32)  # strong minification
     img = synth.uniform((6, 2, 240, 320), 6)
-    for mode in ("bilinear", "nearest"):
-        a = S.inv_warp_image_batch(cu(img), cu(Hinv), device=DEV, mode=mode, staged=True)
-        b = S.inv_warp_image_batch(cu(img), cu(Hinv), device=DEV, mode=mode, staged=False)
-        assert torch.equal(a, b), mode
     odd = synth.uniform((2, 1, 47, 61), 7)
-    a = S.inv_warp_image_batch(cu(odd), cu(Hinv[3:5]), device=DEV)
-    close(a, O.inv_warp_image_batch(odd, Hinv[3:5], "bilinear"), atol=1e-5)
+    for im, Hm, atol in ((img, Hinv, 1e-4), (odd, Hinv[3:5], 1e-5)):
+        out = S.inv_warp_image_batch(cu(im), cu(Hm), device=DEV).cpu().numpy()
+        close(out, O.inv_warp_image_batch(im, Hm, "bilinear"), atol=atol)
+        out = S.inv_warp_image_batch(cu(im), cu(Hm), device=DEV, mode="nearest").cpu().numpy()
+        assert_only_rounding_ties(out, O.inv_warp_image_batch(im, Hm, "nearest"), Hm)
 
 
 def test_inv_warp_100x240x320_oracle():
@@ -230,12 +227,6 @@ def test_flatten_combine(golden):
     close(np.nan_to_num(out), np.nan_to_num(c["out"]), atol=2e-6)
 
 
-def test_combine_heatmap_tiled_golden(golden):
-    g = golden("combine")
-    out = S.combine_heatmap_batch(cu(g["heat"][None, :, 0]), cu(g["Hwarp"][None]), cu(g["mask"][None, :, 0]), tiled=True)
-    close(out[0], g["out"][0] if g["out"].ndim == 3 else g["out"], atol=2e-6)
-
-
 def test_combine_heatmap_n100():
     N = 100
     Hs, Hinv = homographies(N, 14, identity_first=True)
@@ -249,48 +240,24 @@ def test_combine_heatmap_n100():
                                    cu(np.stack([mask[:, 0], mask[::-1, 0]]))).cpu().numpy()
     close(both[0], ref[0] if ref.ndim == 3 else ref, atol=2e-6)
     close(both[1], both[0], atol=2e-6)  # same set of views in another order
-    # the shared-memory staged kernel gives the same map (also on the small golden case with a partial tile)
-    tiled = S.combine_heatmap_batch(cu(np.stack([heat[:, 0], heat[::-1, 0]])), cu(np.stack([Hs, Hs[::-1]])),
-                                    cu(np.stack([mask[:, 0], mask[::-1, 0]])), tiled=True).cpu().numpy()
-    close(tiled, both, atol=2e-6)
-
-
-def test_combine_heatmap_bit_masks():
-    """Bit-mask aggregation (default of the export path) == float-mask aggregation, bit for bit, at N = 100; masks generated
-    directly as bits from the homographies == compute_valid_mask(r=0) packed; a non-binary mask is refused loudly (NaN)."""
-    I, N = 2, 100
-    Hs, Hinv = homographies(I * N, 31, identity_first=True)
-    heat = synth.uniform((I, N, 240, 320), 9)
-    mask = S.compute_valid_mask(torch.tensor([240, 320]), cu(Hinv), device=DEV).reshape(I, N, 240, 320)
-    Hw = cu(Hs).reshape(I, N, 3, 3)
-    ref = S.combine_heatmap_batch(cu(heat), Hw, mask)
-    bits = S.combine_heatmap_batch(cu(heat), Hw, mask, binary_mask=True)
-    auto = S.combine_heatmap_batch(cu(heat), Hw, None, mask_homographies=cu(Hinv).reshape(I, N, 3, 3))
-    assert torch.equal(torch.nan_to_num(ref, nan=-1.0), torch.nan_to_num(bits, nan=-1.0))
-    assert torch.equal(torch.nan_to_num(ref, nan=-1.0), torch.nan_to_num(auto, nan=-1.0))
-    soft = mask * 0.5
-    assert torch.isnan(S.combine_heatmap_batch(cu(heat), Hw, soft, binary_mask=True)).all()
-    # narrow image: a row of bits does not fill its last word
-    h2 = synth.uniform((1, 5, 24, 40), 10)
-    H2s, H2i = homographies(5, 32)
-    m2 = S.compute_valid_mask(torch.tensor([24, 40]), cu(H2i), device=DEV).reshape(1, 5, 24, 40)
-    a = S.combine_heatmap_batch(cu(h2), cu(H2s).reshape(1, 5, 3, 3), m2)
-    b = S.combine_heatmap_batch(cu(h2), cu(H2s).reshape(1, 5, 3, 3), m2, binary_mask=True)
-    assert torch.equal(torch.nan_to_num(a, nan=-1.0), torch.nan_to_num(b, nan=-1.0))
 
 
 def test_combine_from_logits_signed_heat():
     """flatten fused with the 0/1 mask (sign = mask) + one-gather aggregation == flattenDetection + float-mask aggregation, bit for
-    bit, at N = 100; the whole adaptation step returns the same keypoints either way; a soft mask is refused loudly (NaN)."""
-    I, N = 2, 100
-    Hs, Hinv = homographies(I * N, 33, identity_first=True)
-    semi = cu(synth.pseudo_normal((I, N, 65, 30, 40), 12))
-    mask = S.compute_valid_mask(torch.tensor([240, 320]), cu(Hinv), device=DEV).reshape(I, N, 240, 320)
-    Hw = cu(Hs).reshape(I, N, 3, 3)
-    heat = S.flattenDetection(semi.reshape(I * N, 65, 30, 40)).reshape(I, N, 240, 320)
-    ref = S.combine_heatmap_batch(heat, Hw, mask)
-    got = S.utils.combine_from_logits_batch(semi, Hw, mask)
-    assert torch.equal(torch.nan_to_num(ref, nan=-1.0), torch.nan_to_num(got, nan=-1.0))
+    bit, on a narrow image (5 views of 24x40) and at N = 100; at N = 100 the whole adaptation step returns the same keypoints
+    either way, and a soft mask is refused loudly (NaN)."""
+    def case(I, N, Hc, Wc, seed_h, seed_s, identity_first):
+        Hs, Hinv = homographies(I * N, seed_h, identity_first=identity_first)
+        semi = cu(synth.pseudo_normal((I, N, 65, Hc, Wc), seed_s))
+        mask = S.compute_valid_mask(torch.tensor([8 * Hc, 8 * Wc]), cu(Hinv), device=DEV).reshape(I, N, 8 * Hc, 8 * Wc)
+        return semi, cu(Hs).reshape(I, N, 3, 3), mask
+
+    for semi, Hw, mask in (case(1, 5, 3, 5, 32, 10, False), case(2, 100, 30, 40, 33, 12, True)):
+        I, N, _, Hc, Wc = semi.shape
+        heat = S.flattenDetection(semi.reshape(I * N, 65, Hc, Wc)).reshape(I, N, 8 * Hc, 8 * Wc)
+        ref = S.combine_heatmap_batch(heat, Hw, mask)
+        got = S.utils.combine_from_logits_batch(semi, Hw, mask)
+        assert torch.equal(torch.nan_to_num(ref, nan=-1.0), torch.nan_to_num(got, nan=-1.0)), (I, N)
     assert torch.isnan(S.utils.combine_from_logits_batch(semi, Hw, mask * 0.5)).all()
     a = S.step.adaptation_step(semi, Hw, mask)
     b = S.step.adaptation_step(semi, Hw, mask, binary_mask=True)
