@@ -445,11 +445,36 @@ def descriptor_loss(descriptors, descriptors_warped, homographies, mask_valid=No
     return res
 
 
+def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2D, mask_warp_2D, mat_H, lamda_d=250,
+              descriptor_dist=4, lambda_loss=1.0, weighting="uniform"):
+    """Train_model_heatmap_all.py:295-365: detector_loss of both images (:155-179, targets labels2Dto3D, masks
+    getMasks(mask_2D) / getMasks(mask_warp_2D)), descriptor_loss with mask_valid = getMasks(mask_warp_2D), then the total
+      weighting="uniform":    loss_det + loss_det_warp + lambda_loss * loss_desc   (:361-365)
+      weighting="multi_task": loss_det + loss_det_warp + positive_dist + negative_dist (:355-359 at unit weights)
+    and its gradients with respect to the four head outputs.  Returns a dict of the six fp32 scalars (loss, loss_det,
+    loss_det_warp, loss_desc, positive_dist, negative_dist) and "grads" = (d semi, d semi_warp, d desc, d desc_warp)."""
+    if weighting not in ("uniform", "multi_task"):
+        raise ValueError("weighting must be 'uniform' or 'multi_task'")
+    m3, mw3 = getMasks(mask_2D), getMasks(mask_warp_2D)
+    l_det, d_semi = detector_loss(semi, labels2Dto3D(labels_2D), m3, grad=True)
+    l_detw, d_semiw = detector_loss(semi_warp, labels2Dto3D(warped_labels), mw3, grad=True)
+    g = (float(lambda_loss), 0.0, 0.0) if weighting == "uniform" else (0.0, 1.0, 1.0)
+    l_desc, _, pos, neg, d_desc, d_descw = descriptor_loss(desc, desc_warp, mat_H, mw3[:, None], lamda_d=lamda_d,
+                                                           descriptor_dist=descriptor_dist, grad=g)
+    if weighting == "uniform":
+        total = float(l_det) + float(l_detw) + float(lambda_loss) * float(l_desc)
+    else:
+        total = float(l_det) + float(l_detw) + float(pos) + float(neg)
+    return {"loss": f32(total), "loss_det": l_det, "loss_det_warp": l_detw, "loss_desc": l_desc, "positive_dist": pos,
+            "negative_dist": neg, "grads": (d_semi, d_semiw, d_desc, d_descw)}
+
+
 def descriptor_boundary_slack(descriptors, descriptors_warped, homographies, mask_valid=None, cell_size=8, lamda_d=250,
-                              descriptor_dist=4, eps=1e-3):
+                              descriptor_dist=4, eps=1e-3, per_term=False):
     """Largest change of (loss, pos_sum, neg_sum) if every pair whose centre distance lies within `eps` of
     descriptor_dist flipped its mask bit (the mask is a step function of fp32 coordinates ~1e3 in magnitude, so
-    1-ulp differences in the warp arithmetic flip such pairs; each flip moves the numerator by up to lamda_d)."""
+    1-ulp differences in the warp arithmetic flip such pairs; each flip moves the numerator by up to lamda_d).
+    per_term=True returns the bound of each of the three scalars: (loss, pos_sum, neg_sum)."""
     D = np.asarray(descriptors, dtype=f32)
     Dw = np.asarray(descriptors_warped, dtype=f32)
     B, Dch, Hc, Wc = D.shape
@@ -460,14 +485,17 @@ def descriptor_boundary_slack(descriptors, descriptors_warped, homographies, mas
     cx = (ll.reshape(-1) * cell_size + cell_size // 2).astype(np.float64)
     mv = np.ones((B, Nc), f32) if mask_valid is None else np.asarray(mask_valid, dtype=f32).reshape(B, Nc)
     norm = float(B) * (float(mv.sum()) + 1.0) * Hc * Wc
-    slack = 0.0
+    s_pos = s_neg = 0.0
     for b in range(B):
         d = np.sqrt((cy[None, :] - w[b, :, 1:2].astype(np.float64)) ** 2 + (cx[None, :] - w[b, :, 0:1].astype(np.float64)) ** 2)
         rr, cc = np.nonzero(np.abs(d - descriptor_dist) < eps)
         for r, c in zip(rr, cc):
             dot = float(D[b].reshape(Dch, Nc)[:, r].astype(np.float64) @ Dw[b].reshape(Dch, Nc)[:, c].astype(np.float64))
-            slack += lamda_d * max(1.0 - dot, 0.0) + max(dot - 0.2, 0.0)
-    return slack / norm
+            s_pos += lamda_d * max(1.0 - dot, 0.0)
+            s_neg += max(dot - 0.2, 0.0)
+    if per_term:
+        return (s_pos + s_neg) / norm, s_pos / norm, s_neg / norm
+    return (s_pos + s_neg) / norm
 
 
 def descriptor_unstable_cells(descriptors, descriptors_warped, homographies, cell_size=8, descriptor_dist=4, eps_dot=1e-5,

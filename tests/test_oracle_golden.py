@@ -117,6 +117,51 @@ def test_descriptor_identity_kat(golden):
     assert abs(float(pos)) < 1e-6
 
 
+def test_loss_step_composition_and_gradients():
+    """oracle.loss_step at a tiny shape: its scalars are those of detector_loss / descriptor_loss on getMasks of the two
+    masks, the total follows the chosen weighting, and each of the four gradients is the derivative of that total
+    (central differences along a fixed direction, in float64 around the fp32 inputs)."""
+    B, Hc, Wc = 2, 3, 4
+    inp = {"semi": synth.pseudo_normal((B, 65, Hc, Wc), 1), "semi_warp": synth.pseudo_normal((B, 65, Hc, Wc), 2),
+           "desc": synth.unit_descriptors(B, 256, Hc, Wc, 3, smooth=0.3),
+           "desc_warp": synth.unit_descriptors(B, 256, Hc, Wc, 4, smooth=0.3),
+           "labels_2D": synth.keypoint_labels(B, 8 * Hc, 8 * Wc, 5, p=0.05),
+           "warped_labels": synth.keypoint_labels(B, 8 * Hc, 8 * Wc, 6, p=0.05),
+           "mask_2D": np.ones((B, 1, 8 * Hc, 8 * Wc), np.float32),
+           "mask_warp_2D": np.ones((B, 1, 8 * Hc, 8 * Wc), np.float32),
+           "mat_H": np.stack([np.eye(3), [[0.9, 0.05, 0.1], [0.0, 1.1, -0.05], [0.0, 0.0, 1.0]]]).astype(np.float32)}
+    inp["mask_warp_2D"][0, 0, 3, 12] = 0    # one pixel: getMasks zeroes cell (0, 1)
+    inp["mask_warp_2D"][1, 0, 16:, :8] = 0  # cell (2, 0)
+    mw3 = O.getMasks(inp["mask_warp_2D"])
+    assert mw3.sum() == B * Hc * Wc - 2
+    ld = O.detector_loss(inp["semi"], O.labels2Dto3D(inp["labels_2D"]), O.getMasks(inp["mask_2D"]))
+    ldw = O.detector_loss(inp["semi_warp"], O.labels2Dto3D(inp["warped_labels"]), mw3)
+    desc = O.descriptor_loss(inp["desc"], inp["desc_warp"], inp["mat_H"], mw3[:, None], lamda_d=250, descriptor_dist=6)
+    assert float(desc[2]) > 0  # positive pairs exist
+    keys = ("semi", "semi_warp", "desc", "desc_warp")
+    for weighting, lam in (("uniform", 2.5), ("multi_task", 1.0)):
+        kw = dict(descriptor_dist=6, lambda_loss=lam, weighting=weighting)
+        r = O.loss_step(**inp, **kw)
+        assert float(r["loss_det"]) == float(ld) and float(r["loss_det_warp"]) == float(ldw)
+        assert (float(r["loss_desc"]), float(r["positive_dist"]), float(r["negative_dist"])) == tuple(float(x) for x in (desc[0], desc[2], desc[3]))
+        terms = (lam * float(desc[0]),) if weighting == "uniform" else (float(desc[2]), float(desc[3]))
+        close(r["loss"], float(ld) + float(ldw) + sum(terms))
+        for i, k in enumerate(keys):
+            v = synth.pseudo_normal(inp[k].shape, 40 + i).astype(np.float64)
+            eps = (3e-2 if k.startswith("semi") else 1e-3) / np.abs(v).max()  # the detector loss is smooth, the hinges are not
+
+            def total(t):
+                moved = dict(inp)
+                moved[k] = (inp[k].astype(np.float64) + t * v).astype(np.float32)
+                return float(O.loss_step(**moved, **kw)["loss"])
+
+            fd = (total(eps) - total(-eps)) / (2 * eps)
+            an = float((r["grads"][i].astype(np.float64) * v).sum())
+            assert r["grads"][i].shape == inp[k].shape
+            noise = 3 * float(np.spacing(np.float32(abs(r["loss"])))) / (2 * eps)  # the fp32 rounding of three scalars
+            np.testing.assert_allclose(an, fd, rtol=1e-3, atol=noise, err_msg="%s %s" % (weighting, k))
+
+
 def test_semantic_head(golden):
     """SURVEY 8f rank 1: x8 bilinear upsample (reference model forward) + CrossEntropyLoss(ignore_index=133)."""
     g = golden("semantic")
