@@ -244,6 +244,20 @@ int ssp_sparse_desc_loss_fwd(const float* Dt, const float* Dwt, const int* ia, c
 int ssp_sparse_desc_loss_bwd(const float* Dt, const float* Dwt, const int* ia, const int* ib, const float* dots,
                              const float* stats, const float* g3 /*device [3]*/, int B, int Nc, int Dch, int K, int Kn,
                              float lamda, float mpos, float mneg, float* dDt, float* dDwt, void* stream);
+/* ssp_sparse_sample draws those lists on the device, with the distribution of the reference's sample_correspondences
+ * (sparse_loss.py:170-255, correspondence_finder.py:191-320), not its RNG stream.  Per image b: the candidates are the cells
+ * a whose warp by T^-1 mat_H[b] T (normalised -> cell coordinates), rounded half to even, lands in [0,Wc-1] x [0,Hc-1]
+ * (M[b] of them); the K matches are a uniformly random K-subset of them in random order (M >= K), or all M in random order
+ * followed by K - M draws with replacement (M < K); the K*nper non-matches pair matches_a[k] (repeated nper times) with
+ * uniform cells.  ia / ib [B, K + K*nper] int32, matches first.  Hc * Wc <= 8192.  state [4] uint64 device: {seed, launch
+ * counter, 0, images with M = 0 so far}; the launch reads the counter and advances it by one (no host involvement: graph
+ * replays draw fresh lists).  An image with M = 0 gets ia = ib = -1 (it adds nothing to the loss) and counts in state[3].
+ * ssp_sparse_finalize (optional M, total) turns out3 into NaN when some M[b] = 0 and writes
+ * total = det0[0] + det1[0] + lambda_loss * out3[0] (det0 / det1: detector-loss triples) when total is not NULL. */
+int ssp_sparse_sample(const float* mat_H /*[B,3,3]*/, int B, int Hc, int Wc, int K, int nper, unsigned long long* state,
+                      int* ia, int* ib, int* M /*[B]*/, void* stream);
+int ssp_sparse_finalize(const int* M /*[B] or NULL*/, int B, float* out3, const float* det0, const float* det1,
+                        float lambda_loss, float* total /*or NULL*/, void* stream);
 
 /* ---- label warping of the warped training pair (SURVEY 8f rank 4): datasets/data_tools.py:37-63 warpLabels (+ :6-34
  * get_labels_bi), call sites datasets/Coco.py:330,367.  pnts [B,Pmax,2] (x, y) fp32, counts[b] valid points per image

@@ -12,6 +12,7 @@
 // apart), one warp per sampled pair for the dot products, a fixed-order per-image reduction, and for the backward a
 // warp-per-pair scatter (fp32 atomics into cell-major gradient buffers) followed by the transpose back.
 #include "common.cuh"
+#include <cub/block/block_radix_sort.cuh>
 
 // [B, Dch, Nc] <-> [B, Nc, Dch] through a 32 x 32 shared tile (both directions coalesced)
 __global__ void __launch_bounds__(256)
@@ -164,5 +165,177 @@ extern "C" int ssp_sparse_desc_loss_bwd(const float* Dt, const float* Dwt, const
   dim3 grid(ssp_ceil_div(K + Kn, 8), B);
   sparse_bwd_kernel<<<grid, 256, 0, st>>>(Dt, Dwt, ia, ib, dots, stats, g3, B, Nc, Dch, K, Kn, lamda, mpos, mneg, dDt, dDwt);
   SSP_CUDA_CHECK_LAUNCH("sparse_bwd_kernel");
+  return SSP_OK;
+}
+
+// ------------------------------------------------------------------------------------------------------------------------
+// Correspondence sampling on the device: the distribution of sample_correspondences (sparse_loss.py:170-255 with
+// correspondence_finder.py:191-320), not its host RNG stream.  One block per image:
+//   candidates  every cell a = (u, v) warped by T^-1 H T (scale_homography_torch, shift -1), rounded half to even, kept when
+//               0 <= p <= (Wc-1, Hc-1); M = their count
+//   matches     every candidate gets a 31-bit Philox key (non-candidates sort behind them) and one BlockRadixSort orders the
+//               block: the first min(M, K) ranks are a uniformly random K-subset in random order (M >= K), or all M in random
+//               order (M < K) followed by K - M draws with replacement from them -- crop_or_pad_choice (sparse_loss.py:44-48)
+//   non-matches non_a[k n + j] = matches_a[k], non_b a uniform cell (the reference's perturbation is identically zero)
+// Random numbers: Philox4x32-10, key = seed, counter = (item, image << 2 | purpose, launch counter).  The seed and the launch
+// counter live in the caller's state buffer; every block reads the counter, and the last block to finish advances it, so
+// consecutive launches (and graph replays) draw fresh lists with no host involvement.
+constexpr int SAMPLE_THREADS = 1024, SAMPLE_ITEMS = 8, SAMPLE_MAX_CELLS = SAMPLE_THREADS * SAMPLE_ITEMS;
+
+__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
+#pragma unroll
+  for (int r = 0; r < 10; ++r) {
+    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
+    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
+    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
+    k.x += 0x9E3779B9u;
+    k.y += 0xBB67AE85u;
+  }
+  return c;
+}
+
+// uniform integer in [0, n) from 64 random bits (bias below n / 2^64)
+__device__ __forceinline__ int uniform_below(unsigned lo, unsigned hi, int n) {
+  return (int)__umul64hi(((unsigned long long)hi << 32) | lo, (unsigned long long)n);
+}
+
+__global__ void __launch_bounds__(SAMPLE_THREADS, 1)
+sparse_sample_kernel(const float* __restrict__ mat_H, int Hc, int Wc, int K, int nper, unsigned long long* state, int* ia,
+                     int* ib, int* Mout) {
+  using Sort = cub::BlockRadixSort<unsigned, SAMPLE_THREADS, SAMPLE_ITEMS, int>;
+  __shared__ typename Sort::TempStorage sort_tmp;
+  __shared__ float hcell[9];
+  __shared__ unsigned long long s_seed, s_ctr;
+  __shared__ int s_count;
+  const int b = blockIdx.x, t = threadIdx.x, Nc = Hc * Wc;
+  const int Kn = K * nper, Kt = K + Kn;
+  ia += (size_t)b * Kt;
+  ib += (size_t)b * Kt;
+  if (t == 0) {
+    s_seed = *(volatile unsigned long long*)&state[0];
+    s_ctr = *(volatile unsigned long long*)&state[1];
+    s_count = 0;
+    // T^-1 H T, T = [[2/Wc, 0, -1], [0, 2/Hc, -1], [0, 0, 1]] (sparse.py:20-24), in double and rounded once to fp32
+    const float* h = mat_H + (size_t)b * 9;
+    const double sx = 2.0 / Wc, sy = 2.0 / Hc;
+    double ht[9];  // H T
+    for (int r = 0; r < 3; ++r) {
+      ht[3 * r] = (double)h[3 * r] * sx;
+      ht[3 * r + 1] = (double)h[3 * r + 1] * sy;
+      ht[3 * r + 2] = -(double)h[3 * r] - (double)h[3 * r + 1] + (double)h[3 * r + 2];
+    }
+    for (int c = 0; c < 3; ++c) {  // T^-1 = [[Wc/2, 0, Wc/2], [0, Hc/2, Hc/2], [0, 0, 1]]
+      hcell[c] = (float)(0.5 * Wc * (ht[c] + ht[6 + c]));
+      hcell[3 + c] = (float)(0.5 * Hc * (ht[3 + c] + ht[6 + c]));
+      hcell[6 + c] = (float)ht[6 + c];
+    }
+  }
+  __syncthreads();
+  const uint2 key = make_uint2((unsigned)s_seed, (unsigned)(s_seed >> 32));
+  const unsigned clo = (unsigned)s_ctr, chi = (unsigned)(s_ctr >> 32);
+
+  // candidates, blocked arrangement: thread t holds cells 8t .. 8t+7
+  unsigned keys[SAMPLE_ITEMS];
+  int vals[SAMPLE_ITEMS];
+  int mine = 0;
+#pragma unroll
+  for (int j = 0; j < SAMPLE_ITEMS; j += 4) {
+    const uint4 r = philox4x32_10(make_uint4(t * (SAMPLE_ITEMS / 4) + j / 4, (unsigned)b << 2, clo, chi), key);
+    const unsigned rr[4] = {r.x, r.y, r.z, r.w};
+#pragma unroll
+    for (int q = 0; q < 4; ++q) {
+      const int cell = t * SAMPLE_ITEMS + j + q;
+      keys[j + q] = 0xFFFFFFFFu;
+      vals[j + q] = 0;
+      if (cell < Nc) {
+        const int v = cell / Wc, u = cell - v * Wc;
+        float x, y;
+        homography_apply(hcell, (float)u, (float)v, x, y);
+        x = rintf(x);  // torch.round: half to even
+        y = rintf(y);
+        if (x >= 0.f && x <= (float)(Wc - 1) && y >= 0.f && y <= (float)(Hc - 1)) {
+          keys[j + q] = rr[q] >> 1;
+          vals[j + q] = cell | (((int)y * Wc + (int)x) << 16);
+          ++mine;
+        }
+      }
+    }
+  }
+  if (mine) atomicAdd(&s_count, mine);
+  __syncthreads();
+  const int M = s_count;
+  Sort(sort_tmp).Sort(keys, vals);
+
+  if (M == 0) {  // the homography maps no cell into the image: out-of-range lists (they contribute nothing), M[b] = 0 and the flag
+    for (int k = t; k < Kt; k += SAMPLE_THREADS) {
+      ia[k] = -1;
+      ib[k] = -1;
+    }
+    if (t == 0) atomicAdd(&state[3], 1ull);
+  } else {
+#pragma unroll
+    for (int j = 0; j < SAMPLE_ITEMS; ++j) {
+      const int rank = t * SAMPLE_ITEMS + j;
+      if (rank < M && rank < K) {
+        ia[rank] = vals[j] & 0xFFFF;
+        ib[rank] = vals[j] >> 16;
+      }
+    }
+    __syncthreads();  // the block's global writes above are visible to the block from here on
+    for (int k = M + t; k < K; k += SAMPLE_THREADS) {  // M < K: pad with draws with replacement from the M candidates
+      const uint4 r = philox4x32_10(make_uint4(k, ((unsigned)b << 2) | 1u, clo, chi), key);
+      const int src = uniform_below(r.x, r.y, M);
+      ia[k] = ia[src];
+      ib[k] = ib[src];
+    }
+    __syncthreads();
+    for (int k = t; k < Kn; k += SAMPLE_THREADS) {
+      const uint4 r = philox4x32_10(make_uint4(k, ((unsigned)b << 2) | 2u, clo, chi), key);
+      ia[K + k] = ia[k / nper];
+      ib[K + k] = uniform_below(r.x, r.y, Nc);
+    }
+  }
+  if (t == 0) {
+    Mout[b] = M;
+    // the last block to finish advances the launch counter: every other block has read it by then
+    __threadfence();
+    const unsigned prev = atomicInc((unsigned*)&state[2], gridDim.x - 1);  // wraps back to 0 for the next launch
+    if (prev == gridDim.x - 1) state[1] = s_ctr + 1;
+  }
+}
+
+extern "C" int ssp_sparse_sample(const float* mat_H, int B, int Hc, int Wc, int K, int nper, unsigned long long* state, int* ia,
+                                 int* ib, int* M, void* stream) {
+  SSP_REQUIRE(mat_H && state && ia && ib && M, "ssp_sparse_sample: null pointer");
+  SSP_REQUIRE(B > 0 && B <= 65535 && Hc > 0 && Wc > 0, "ssp_sparse_sample: bad sizes");
+  SSP_REQUIRE((long long)Hc * Wc <= SAMPLE_MAX_CELLS, "ssp_sparse_sample: %d x %d cells exceed the supported %d cells", Hc, Wc,
+              SAMPLE_MAX_CELLS);
+  SSP_REQUIRE(K > 0 && nper >= 0 && (long long)K * (nper + 1) <= 0x7FFFFFFF,
+              "ssp_sparse_sample: need K > 0 and n >= 0 (got K = %d, n = %d)", K, nper);
+  sparse_sample_kernel<<<B, SAMPLE_THREADS, 0, (cudaStream_t)stream>>>(mat_H, Hc, Wc, K, nper, state, ia, ib, M);
+  SSP_CUDA_CHECK_LAUNCH("sparse_sample_kernel");
+  return SSP_OK;
+}
+
+// out3 (ssp_sparse_desc_loss_fwd's batch means) becomes NaN when an image had no candidate (M[b] = 0); with total set,
+// total = (det0[0] + det1[0]) + lambda_loss * out3[0], the sparse loss step's weighted sum (Train_model_heatmap_all.py:361-365)
+__global__ void sparse_finalize_kernel(const int* __restrict__ M, int B, float* __restrict__ out3, const float* __restrict__ det0,
+                                       const float* __restrict__ det1, float lambda_loss, float* __restrict__ total) {
+  bool empty = false;
+  if (M != nullptr)
+    for (int b = threadIdx.x; b < B; b += 32) empty |= M[b] == 0;
+  empty = __any_sync(0xffffffffu, empty);
+  if (threadIdx.x == 0) {
+    if (empty) out3[0] = out3[1] = out3[2] = __int_as_float(0x7fc00000);
+    if (total != nullptr) total[0] = __fadd_rn(__fadd_rn(det0[0], det1[0]), __fmul_rn(lambda_loss, out3[0]));
+  }
+}
+
+extern "C" int ssp_sparse_finalize(const int* M, int B, float* out3, const float* det0, const float* det1, float lambda_loss,
+                                   float* total, void* stream) {
+  SSP_REQUIRE(out3 && (total == nullptr || (det0 && det1)), "ssp_sparse_finalize: null pointer");
+  SSP_REQUIRE(B > 0, "ssp_sparse_finalize: bad sizes");
+  sparse_finalize_kernel<<<1, 32, 0, (cudaStream_t)stream>>>(M, B, out3, det0, det1, lambda_loss, total);
+  SSP_CUDA_CHECK_LAUNCH("sparse_finalize_kernel");
   return SSP_OK;
 }

@@ -534,6 +534,48 @@ class LossStepFn(torch.autograd.Function):
         return d0, None, None, d1, None, None, dD, dDw, None, None, None, None, None, None
 
 
+class SparseLossStepFn(torch.autograd.Function):
+    """The loss step of the shipped configs (sparse_loss.enable) as ONE autograd node: both detector losses plus the sparse
+    descriptor loss on device-sampled lists ia / ib [B, K + Kn] with candidate counts M,
+    loss = loss_det + loss_det_warp + lambda_loss * loss_desc (Train_model_heatmap_all.py:333-365, uniform weighting).
+    Returns (loss, loss_det, loss_det_warp, loss_desc, pos, neg); only `loss` is differentiable.  The total is formed by
+    ssp_sparse_finalize, which also turns it into NaN when an image had no candidate."""
+
+    @staticmethod
+    def forward(ctx, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, desc, desc_w, ia, ib, M, K, lamda_d,
+                lambda_loss):
+        from .sparse import SparseDescriptorLossFn
+        c1 = _Ctx((ctx.needs_input_grad[0], False, False, ctx.needs_input_grad[3], False, False, False, False))
+        l0, l1, _cm = DetectorLossPairFn.forward(c1, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, True)
+        c2 = _Ctx((ctx.needs_input_grad[6], ctx.needs_input_grad[7]) + (False,) * 6)
+        ld, pos, neg = SparseDescriptorLossFn.forward(c2, desc, desc_w, ia, ib, K, ia.shape[1] - K, lamda_d)
+        total = torch.empty((1,), dtype=torch.float32, device=semi.device)
+        call("ssp_sparse_finalize", ptr(M), M.shape[0], ptr(c2.out3), ptr(c1.out[0]), ptr(c1.out[1]), float(lambda_loss),
+             ptr(total), stream_of(total))
+        ctx.c1, ctx.c2, ctx.lambda_loss = c1, c2, float(lambda_loss)
+        ctx.mark_non_differentiable(l0, l1, ld, pos, neg)
+        ctx.set_materialize_grads(False)
+        return total[0], l0, l1, ld, pos, neg
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g, *_unused):
+        from .sparse import sparse_loss_backward
+        if g is None:
+            return (None,) * 14
+        dev = g.device
+        g = f32c(g.reshape(1), dev)
+        d0 = d1 = dD = dDw = None
+        if ctx.needs_input_grad[0] or ctx.needs_input_grad[3]:
+            d0, _, _, d1 = DetectorLossPairFn.backward(ctx.c1, g, _SAME, None)[:4]
+        if ctx.needs_input_grad[6] or ctx.needs_input_grad[7]:
+            key = (dev.index, ctx.lambda_loss)
+            if key not in _lam3:
+                _lam3[key] = torch.tensor([ctx.lambda_loss, 0.0, 0.0], dtype=torch.float32, device=dev)
+            dD, dDw = sparse_loss_backward(ctx.c2, g * _lam3[key])
+        return d0, None, None, d1, None, None, dD, dDw, None, None, None, None, None, None
+
+
 # ------------------------------------------------------------------------------------------------
 class LazyPairMask(object):
     """The [B,Hc,Wc,Hc,Wc] float correspondence mask of descriptor_loss (utils/utils.py:854-860), built only

@@ -8,6 +8,11 @@ The reference draws its correspondences on the HOST with numpy / torch CPU rando
 same calls in the same order (np.random.permutation [+ np.random.choice], torch.rand, torch.rand, torch.randn), so under the
 same RNG state it returns the reference's own index lists (tests pin this against fixtures of the live reference).  The
 lists go to the device once per batch; the loss and its gradient are CUDA kernels (csrc/sparse.cu).
+
+DeviceSampler draws lists with the same distribution on the device (ssp_sparse_sample) from a seed and a launch counter held
+in device memory: no host RNG call and no host synchronisation, so the whole sparse step can be captured into a CUDA graph
+whose replays draw fresh lists.  Its draws are not the reference's RNG stream; batch_descriptor_loss_sparse uses it only
+when it is passed one.
 """
 import numpy as np
 import torch
@@ -15,6 +20,8 @@ from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import call, f32c, ptr, stream_of
+
+CHECK_EMPTY_IMAGES = False  # DeviceSampler.sample raises when an image had no candidate (costs a host sync per call)
 
 
 def scale_homography_torch(H, shape, shift=(-1, -1), dtype=torch.float32):
@@ -65,11 +72,61 @@ def sample_correspondences(homography, Hc, Wc, num_matching_attempts=1000, num_m
     return matches_a, matches_b, non_a.long(), non_b.long()
 
 
+class DeviceSampler(object):
+    """Correspondence lists of the sparse loss drawn on the device (ssp_sparse_sample, csrc/sparse.cu): per image, the cells
+    whose warp lands in the image are the candidates; K matches are a random K-subset of them (or all of them plus draws
+    with replacement when there are fewer than K), and every match gets n non-matches at uniform cells.
+
+    The random numbers are Philox4x32-10 keyed by (seed, image, launch counter).  The seed and the counter live in a device
+    buffer that every launch reads and advances, so eager calls and graph replays draw fresh lists without the host, and
+    get_state() / set_state() reproduce a sequence bit for bit.  An image whose homography maps no cell into the image turns
+    the loss into NaN and counts in a device flag (empty_images(); CHECK_EMPTY_IMAGES raises on it).  Grids up to 8192
+    cells (one block of 1024 threads x 8 cells per image: 30x40, 60x80 and KITTI's 47x155 fit); larger ones are an error."""
+
+    def __init__(self, seed=0, device="cuda"):
+        self.device = torch.device(device)
+        if self.device.type != "cuda":
+            raise RuntimeError("DeviceSampler samples on a CUDA device, got %s" % self.device)
+        seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+        seed = seed - (1 << 64) if seed >= (1 << 63) else seed
+        # {seed, launch counter, blocks done (0 between launches), images with M = 0 so far}, as uint64 bits
+        self.state = torch.tensor([seed, 0, 0, 0], dtype=torch.int64).to(self.device)
+        self.last = None  # (ia, ib, M) of the last call
+
+    def sample(self, mat_H, Hc, Wc, K=1000, n=10):
+        """mat_H [B,3,3] (normalised coordinates) -> ia, ib int32 [B, K + K*n] (cell indices u + v*Wc into the descriptors
+        and the warped descriptors, the K matches first) and M int32 [B], the candidate count of every image."""
+        Hm = f32c(mat_H.detach().reshape(-1, 3, 3), self.device)
+        B, K, n = Hm.shape[0], int(K), int(n)
+        ia = torch.empty((B, K + K * n), dtype=torch.int32, device=self.device)
+        ib = torch.empty_like(ia)
+        M = torch.empty((B,), dtype=torch.int32, device=self.device)
+        call("ssp_sparse_sample", ptr(Hm), B, int(Hc), int(Wc), K, n, ptr(self.state), ptr(ia), ptr(ib), ptr(M), stream_of(Hm))
+        self.last = (ia, ib, M)
+        if CHECK_EMPTY_IMAGES and int(self.state[3]) != 0:  # host sync: debugging / tests only (the NaN loss is the signal)
+            n_empty = int(self.state[3])
+            self.state[3] = 0
+            raise RuntimeError("DeviceSampler: the homography maps no cell into the image (%d images)" % n_empty)
+        return ia, ib, M
+
+    def get_state(self):
+        """{seed, launch counter} as a device int64 tensor [2] (a copy)."""
+        return self.state[:2].clone()
+
+    def set_state(self, state):
+        self.state[:2].copy_(torch.as_tensor(state, dtype=torch.int64))
+
+    def empty_images(self):
+        """Images that had no candidate since the sampler was created (host sync)."""
+        return int(self.state[3])
+
+
 class SparseDescriptorLossFn(torch.autograd.Function):
-    """(loss, match, nonmatch) batch means from descriptors [B,Dch,Hc,Wc] and index lists ia / ib [B, K + Kn] (int32)."""
+    """(loss, match, nonmatch) batch means from descriptors [B,Dch,Hc,Wc] and index lists ia / ib [B, K + Kn] (int32).
+    M: the candidate counts of DeviceSampler.sample, or None; a zero count turns the three means into NaN."""
 
     @staticmethod
-    def forward(ctx, D, Dw, ia, ib, K, Kn, lamda):
+    def forward(ctx, D, Dw, ia, ib, K, Kn, lamda, M=None):
         _lib.require_cuda(D, Dw)
         dev = D.device
         Dc, Dwc = f32c(D.detach(), dev), f32c(Dw.detach(), dev)
@@ -85,29 +142,39 @@ class SparseDescriptorLossFn(torch.autograd.Function):
         out3 = torch.empty((3,), dtype=torch.float32, device=dev)
         call("ssp_sparse_desc_loss_fwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), B, Nc, Dch, K, Kn, float(lamda), 1.0, 0.2,
              ptr(dots), ptr(stats), ptr(out3), st)
+        if M is not None:
+            call("ssp_sparse_finalize", ptr(M), B, ptr(out3), None, None, 0.0, None, st)
         ctx.save_for_backward(Dt, Dwt, ia, ib, dots, stats)
         ctx.meta = (B, Dch, Hc, Wc, K, Kn, float(lamda))
+        ctx.out3 = out3  # attribute, not a saved tensor (the fused sparse step writes its total from it)
         return out3[0], out3[1], out3[2]
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g_loss, g_match, g_non):
-        Dt, Dwt, ia, ib, dots, stats = ctx.saved_tensors
-        B, Dch, Hc, Wc, K, Kn, lamda = ctx.meta
-        dev = Dt.device
-        Nc = Hc * Wc
-        st = stream_of(Dt)
-        zero = torch.zeros((), dtype=torch.float32, device=dev)
+        zero = torch.zeros((), dtype=torch.float32, device=ctx.saved_tensors[0].device)
         g3 = torch.stack([(g if g is not None else zero).reshape(()).to(torch.float32) for g in (g_loss, g_match, g_non)]).contiguous()
-        dDt = torch.empty_like(Dt)
-        dDwt = torch.empty_like(Dwt)
-        call("ssp_sparse_desc_loss_bwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), ptr(dots), ptr(stats), ptr(g3), B, Nc, Dch, K, Kn,
-             lamda, 1.0, 0.2, ptr(dDt), ptr(dDwt), st)
-        dD = torch.empty((B, Dch, Hc, Wc), dtype=torch.float32, device=dev)
-        dDw = torch.empty_like(dD)
-        call("ssp_transpose_batched", ptr(dDt), B, Nc, Dch, ptr(dD), st)
-        call("ssp_transpose_batched", ptr(dDwt), B, Nc, Dch, ptr(dDw), st)
-        return dD, dDw, None, None, None, None, None
+        dD, dDw = sparse_loss_backward(ctx, g3)
+        return dD, dDw, None, None, None, None, None, None
+
+
+def sparse_loss_backward(ctx, g3):
+    """Gradients (dD, dDw) [B,Dch,Hc,Wc] of SparseDescriptorLossFn's forward saved in ctx, for g3 = device {dL/dloss,
+    dL/dmatch, dL/dnonmatch}."""
+    Dt, Dwt, ia, ib, dots, stats = ctx.saved_tensors
+    B, Dch, Hc, Wc, K, Kn, lamda = ctx.meta
+    dev = Dt.device
+    Nc = Hc * Wc
+    st = stream_of(Dt)
+    dDt = torch.empty_like(Dt)
+    dDwt = torch.empty_like(Dwt)
+    call("ssp_sparse_desc_loss_bwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), ptr(dots), ptr(stats), ptr(g3), B, Nc, Dch, K, Kn,
+         lamda, 1.0, 0.2, ptr(dDt), ptr(dDwt), st)
+    dD = torch.empty((B, Dch, Hc, Wc), dtype=torch.float32, device=dev)
+    dDw = torch.empty_like(dD)
+    call("ssp_transpose_batched", ptr(dDt), B, Nc, Dch, ptr(dD), st)
+    call("ssp_transpose_batched", ptr(dDwt), B, Nc, Dch, ptr(dDw), st)
+    return dD, dDw
 
 
 def sparse_loss_from_lists(descriptors, descriptors_warped, matches_a, matches_b, non_matches_a, non_matches_b, lamda_d=250):
@@ -121,12 +188,19 @@ def sparse_loss_from_lists(descriptors, descriptors_warped, matches_a, matches_b
 
 def batch_descriptor_loss_sparse(descriptors, descriptors_warped, homographies, mask_valid=None, cell_size=8, device="cpu",
                                  descriptor_dist=4, lamda_d=250, num_matching_attempts=1000,
-                                 num_masked_non_matches_per_match=10, dist="cos", method="1d", **config):
-    """reference: utils/loss_functions/sparse_loss.py:267-284.  Returns (loss, None, positive, negative), batch means."""
+                                 num_masked_non_matches_per_match=10, dist="cos", method="1d", sampler=None, **config):
+    """reference: utils/loss_functions/sparse_loss.py:267-284.  Returns (loss, None, positive, negative), batch means.
+    sampler=None samples on the host like the reference (its RNG call order); a DeviceSampler samples on the device."""
     if dist != "cos" or method != "1d":
         raise NotImplementedError("descriptor_loss_sparse: only dist='cos', method='1d' (what every shipped config uses)")
     _lib.require_cuda(descriptors, descriptors_warped)
     B, _, Hc, Wc = descriptors.shape
+    if sampler is not None:
+        K = int(num_matching_attempts)
+        ia, ib, M = sampler.sample(homographies, Hc, Wc, K, num_masked_non_matches_per_match)
+        loss, pos, neg = SparseDescriptorLossFn.apply(descriptors, descriptors_warped, ia, ib, K, ia.shape[1] - K,
+                                                      float(lamda_d), M)
+        return loss, None, pos, neg
     lists = [sample_correspondences(homographies[i].detach().float().cpu(), Hc, Wc, num_matching_attempts,
                                     num_masked_non_matches_per_match) for i in range(B)]
     ma, mb, na, nb = (torch.stack([l[j] for l in lists]) for j in range(4))

@@ -12,7 +12,8 @@ from . import utils as U
 
 def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2D, mask_warp_2D, mat_H,
               lamda_d=250, descriptor_dist=4, lambda_loss=1.0, engine=None, dist_group=None, side_stream=None,
-              sem_pred=None, sem=None, sem_warp_pred=None, warped_sem=None, fused=True):
+              sem_pred=None, sem=None, sem_warp_pred=None, warped_sem=None, fused=True, descriptor_loss="dense",
+              sampler=None, num_matching_attempts=1000, num_masked_non_matches_per_match=10):
     """Returns dict(loss, loss_det, loss_det_warp, loss_desc, positive_dist, negative_dist[, loss_sem, loss_sem_warp]).
 
     loss = loss_det + loss_det_warp [+ loss_sem + loss_sem_warp] + lambda_loss * loss_desc
@@ -23,7 +24,17 @@ def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2
     fused=True: the step is one autograd node and only `loss` carries gradient; the component scalars are
     values for logging.  Pass fused=False to differentiate through loss_det / positive_dist / negative_dist separately
     (the reference's multi_task_loss weighting, Train_model_heatmap_all.py:355-359).
+    descriptor_loss="sparse": the descriptor term is the sparse loss of the shipped configs (sparse_loss.py:65-284,
+    Train_model_heatmap_all.py:333-347) on lists that `sampler` (a sparse.DeviceSampler) draws on the device with
+    num_matching_attempts matches and num_masked_non_matches_per_match non-matches per match; descriptor_dist and engine
+    do not apply.  Single GPU only.
     """
+    if descriptor_loss == "sparse":
+        return _sparse_loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2D, mask_warp_2D, mat_H,
+                                 lamda_d, lambda_loss, dist_group, sem_pred, sem, sem_warp_pred, warped_sem, fused, sampler,
+                                 num_matching_attempts, num_masked_non_matches_per_match)
+    if descriptor_loss != "dense":
+        raise ValueError("descriptor_loss must be 'dense' or 'sparse', got %r" % (descriptor_loss,))
     if fused:
         # fast path: the whole step is one autograd node (no scalar-glue kernels), see losses.LossStepFn; with dist_group
         # set, one peer-memory exchange kernel makes the normalisers global (dist.LossExchange)
@@ -58,6 +69,35 @@ def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2
         out["loss_sem_warp"] = U.sem_loss(sem_warp_pred, warped_sem, dist_group=dist_group)
     loss = loss_det + loss_det_warp + lambda_loss * loss_desc
     if sem_pred is not None:
+        loss = loss + out["loss_sem"] + out["loss_sem_warp"]
+    out.update({"loss": loss, "loss_det": loss_det, "loss_det_warp": loss_det_warp, "loss_desc": loss_desc,
+                "positive_dist": pos, "negative_dist": neg})
+    return out
+
+
+def _sparse_loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2D, mask_warp_2D, mat_H, lamda_d,
+                      lambda_loss, dist_group, sem_pred, sem, sem_warp_pred, warped_sem, fused, sampler, K, n):
+    """loss_step(descriptor_loss="sparse"): sampler launch, detector pair, sparse loss; no host sync, no host RNG."""
+    from .sparse import DeviceSampler, SparseDescriptorLossFn
+    if dist_group is not None:
+        raise NotImplementedError("loss_step: the sparse descriptor loss runs on one GPU (dist_group is not supported)")
+    if not isinstance(sampler, DeviceSampler):
+        raise ValueError("loss_step(descriptor_loss='sparse') needs sampler=sparse.DeviceSampler(seed, device)")
+    K = int(K)
+    ia, ib, M = sampler.sample(mat_H, desc.shape[2], desc.shape[3], K, n)
+    out = {}
+    if fused:
+        from .losses import SparseLossStepFn
+        loss, loss_det, loss_det_warp, loss_desc, pos, neg = SparseLossStepFn.apply(
+            semi, labels_2D, mask_2D, semi_warp, warped_labels, mask_warp_2D, desc, desc_warp, ia, ib, M, K, float(lamda_d),
+            float(lambda_loss))
+    else:
+        loss_det, loss_det_warp, _ = U.detector_loss_pair_2d(semi, labels_2D, mask_2D, semi_warp, warped_labels, mask_warp_2D)
+        loss_desc, pos, neg = SparseDescriptorLossFn.apply(desc, desc_warp, ia, ib, K, ia.shape[1] - K, float(lamda_d), M)
+        loss = loss_det + loss_det_warp + lambda_loss * loss_desc
+    if sem_pred is not None:
+        out["loss_sem"] = U.sem_loss(sem_pred, sem)
+        out["loss_sem_warp"] = U.sem_loss(sem_warp_pred, warped_sem)
         loss = loss + out["loss_sem"] + out["loss_sem_warp"]
     out.update({"loss": loss, "loss_det": loss_det, "loss_det_warp": loss_det_warp, "loss_desc": loss_desc,
                 "positive_dist": pos, "negative_dist": neg})
@@ -110,7 +150,10 @@ def collate_warped_pair(img, pnts_list, homographies, erosion_radius=3, bilinear
 class GraphedLossStep(object):
     """loss_step forward + backward captured once into a CUDA graph and replayed (the step is a chain of ~25 short
     kernels; replay removes the per-launch host cost).  Inputs are copied into static buffers; outputs (loss
-    scalars and the four gradients) live in static buffers that the next replay overwrites."""
+    scalars and the four gradients) live in static buffers that the next replay overwrites.
+    With descriptor_loss="sparse" the sampler launch is part of the graph: every replay draws new lists, the first replay
+    draws what an eager step from the sampler's state at construction would (the warm-up steps restore that state), and
+    the outputs hold the last replay's lists as "lists" = (ia, ib, M)."""
 
     IN_KEYS = ("semi", "semi_warp", "desc", "desc_warp", "labels_2D", "warped_labels", "mask_2D", "mask_warp_2D", "mat_H")
     SEM_KEYS = ("sem_pred", "sem_warp_pred", "sem", "warped_sem")  # optional: SSp configuration
@@ -125,6 +168,8 @@ class GraphedLossStep(object):
         if self.semantic:
             self.IN_KEYS = self.IN_KEYS + self.SEM_KEYS
         self.static = {k: example[k].detach().clone() for k in self.IN_KEYS}
+        sampler = kw.get("sampler") if kw.get("descriptor_loss") == "sparse" else None
+        state = sampler.get_state() if sampler is not None else None
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
@@ -132,6 +177,8 @@ class GraphedLossStep(object):
                 self._run()
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
+        if sampler is not None:
+            sampler.set_state(state)
         self.graph = torch.cuda.CUDAGraph()
         with torch.cuda.graph(self.graph):
             self.out = self._run()
@@ -153,6 +200,8 @@ class GraphedLossStep(object):
         total.backward(gradient=self._one)
         res = {k: v.detach() for k, v in out.items()}
         res["grads"] = [l.grad for l in leaves]
+        if kw.get("descriptor_loss") == "sparse":
+            res["lists"] = kw["sampler"].last
         return res
 
     def load(self, inputs, non_blocking=True):
