@@ -6,6 +6,9 @@ numerators / mask sums are exchanged by ONE peer-memory kernel (dist.LossExchang
 the loss scalars and normalisers in place, stream ordered, before the forward returns; the backward kernels
 scale by the global normaliser.
 """
+import functools
+from collections import namedtuple
+
 import torch
 from torch.autograd.function import once_differentiable
 
@@ -30,7 +33,6 @@ def get_descriptor_engine():
 
 
 _side_streams = {}
-_SAME = object()  # marker: "second gradient == first gradient" (no stack / cat kernels)
 
 
 class _Fork(object):
@@ -171,61 +173,266 @@ class SemanticLossFn(torch.autograd.Function):
         return d, None, None, None
 
 
+def grad_vector(grads, dev):
+    """The upstream gradients of a node's scalar outputs as one contiguous fp32 device vector, zero where none came."""
+    zero = torch.zeros((), dtype=torch.float32, device=dev)
+    return torch.stack([(g if g is not None else zero).reshape(()).to(torch.float32) for g in grads]).contiguous()
+
+
+@functools.lru_cache(maxsize=None)
+def _lam3_vector(lam, dev):
+    """The device vector [lam, 0, 0]: g * it is the gradient vector of a descriptor loss weighted by lam."""
+    return torch.tensor([lam, 0.0, 0.0], dtype=torch.float32, device=dev)
+
+
+# ------------------------------------------------------------------------------------------------
+DetPair = namedtuple("DetPair", "saved out fused2d")  # saved = fp32 (x0, t0, m0, x1, t1, m1); out [2,3]: a triple per image
+
+
+def det_pair_forward(semi, target, mask, semi_w, target_w, mask_w, fused2d):
+    """Both detector losses in one launch -> (DetPair, getMasks() of the warped mask [B,Hc,Wc])."""
+    _lib.require_cuda(semi, semi_w)
+    dev = semi.device
+    x0, t0, m0 = f32c(semi.detach(), dev), f32c(target.detach(), dev), f32c(mask.detach(), dev)
+    x1, t1, m1 = f32c(semi_w.detach(), dev), f32c(target_w.detach(), dev), f32c(mask_w.detach(), dev)
+    B, C, Hc, Wc = x0.shape
+    if C != 65 or x1.shape != x0.shape:
+        raise RuntimeError("detector_loss: inputs must be two [B,65,Hc,Wc] tensors of the same shape")
+    n2d = B * Hc * Wc * 64
+    for t, m in ((t0, m0), (t1, m1)):
+        ok = (t.numel() == n2d and m.numel() == n2d) if fused2d else (t.shape == x0.shape and m.numel() == B * Hc * Wc)
+        if not ok:
+            raise RuntimeError("detector_loss: target / mask shapes do not match the logits")
+    out = torch.empty((2, 3), dtype=torch.float32, device=dev)
+    cellmask = torch.empty((B, Hc, Wc), dtype=torch.float32, device=dev)
+    per = (_lib.load().ssp_detector_loss_ws_bytes(B, Hc, Wc) + 15) // 16 * 16
+    ws = torch.empty((2 * per,), dtype=torch.uint8, device=dev)
+    call("ssp_detector_loss_fwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
+         1 if fused2d else 0, ptr(out[0]), ptr(out[1]), ptr(cellmask), ptr(ws), 2 * per, stream_of(x0))
+    return DetPair((x0, t0, m0, x1, t1, m1), out, fused2d), cellmask
+
+
+def det_pair_backward(st, g0, g1):
+    """(d semi, d semi_w) for upstream gradients g0, g1: 1-element device tensors (the fused step passes one twice)."""
+    x0, t0, m0, x1, t1, m1 = st.saved
+    B, C, Hc, Wc = x0.shape
+    d0, d1 = torch.empty_like(x0), torch.empty_like(x1)
+    call("ssp_detector_loss_bwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
+         1 if st.fused2d else 0, ptr(st.out[0]), ptr(st.out[1]), ptr(g0), ptr(g1), ptr(d0), ptr(d1), stream_of(x0))
+    return d0, d1
+
+
 class DetectorLossPairFn(torch.autograd.Function):
     """Both detector losses of a training pair (image, warped image) in ONE launch each way, plus getMasks() of the
     warped mask as a by-product (it is the descriptor loss's mask_valid).  Returns (loss, loss_warp, cell_mask_warp)."""
 
     @staticmethod
     def forward(ctx, semi, target, mask, semi_w, target_w, mask_w, fused2d, dist_group=None):
-        _lib.require_cuda(semi, semi_w)
-        dev = semi.device
-        x0, t0, m0 = f32c(semi.detach(), dev), f32c(target.detach(), dev), f32c(mask.detach(), dev)
-        x1, t1, m1 = f32c(semi_w.detach(), dev), f32c(target_w.detach(), dev), f32c(mask_w.detach(), dev)
-        B, C, Hc, Wc = x0.shape
-        if C != 65 or x1.shape != x0.shape:
-            raise RuntimeError("detector_loss: inputs must be two [B,65,Hc,Wc] tensors of the same shape")
-        n2d = B * Hc * Wc * 64
-        for t, m in ((t0, m0), (t1, m1)):
-            ok = (t.numel() == n2d and m.numel() == n2d) if fused2d else (t.shape == x0.shape and m.numel() == B * Hc * Wc)
-            if not ok:
-                raise RuntimeError("detector_loss: target / mask shapes do not match the logits")
-        out = torch.empty((2, 3), dtype=torch.float32, device=dev)
-        cellmask = torch.empty((B, Hc, Wc), dtype=torch.float32, device=dev)
-        per = (_lib.load().ssp_detector_loss_ws_bytes(B, Hc, Wc) + 15) // 16 * 16
-        ws = torch.empty((2 * per,), dtype=torch.uint8, device=dev)
-        call("ssp_detector_loss_fwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
-             1 if fused2d else 0, ptr(out[0]), ptr(out[1]), ptr(cellmask), ptr(ws), 2 * per, stream_of(x0))
-        ctx.save_for_backward(x0, t0, m0, x1, t1, m1)
-        ctx.out = out  # see DetectorLossFn
-        ctx.fused2d = fused2d
+        st, cellmask = det_pair_forward(semi, target, mask, semi_w, target_w, mask_w, fused2d)
+        ctx.save_for_backward(*st.saved)
+        ctx.st = st._replace(saved=None)  # out is an attribute, see DetectorLossFn
         ctx.mark_non_differentiable(cellmask)
         if dist_group is not None:
             from .dist import get_exchange
-            get_exchange(dist_group).run(det0=out[0], det1=out[1])
-        return out[0, 0], out[1, 0], cellmask
+            get_exchange(dist_group).run(det0=st.out[0], det1=st.out[1])
+        return st.out[0, 0], st.out[1, 0], cellmask
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g0, g1, _gm):
-        x0, t0, m0, x1, t1, m1 = ctx.saved_tensors
-        out = ctx.out
-        B, C, Hc, Wc = x0.shape
-        dev = x0.device
-        if g1 is _SAME:  # fused step: both losses share one upstream gradient scalar
-            g = f32c(g0.reshape(1), dev).expand(2)
-        else:
-            zero = torch.zeros((), dtype=torch.float32, device=dev)
-            g = torch.stack([(a if a is not None else zero).reshape(()).to(torch.float32) for a in (g0, g1)]).contiguous()
-        d0, d1 = torch.empty_like(x0), torch.empty_like(x1)
-        call("ssp_detector_loss_bwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
-             1 if ctx.fused2d else 0, ptr(out[0]), ptr(out[1]), ptr(g[0:1]), ptr(g[1:2]) if g1 is not _SAME else ptr(g[0:1]),
-             ptr(d0), ptr(d1), stream_of(x0))
+        st = ctx.st._replace(saved=ctx.saved_tensors)
+        g = grad_vector((g0, g1), st.out.device)
+        d0, d1 = det_pair_backward(st, g[0:1], g[1:2])
         return d0, None, None, d1, None, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------
+_MPOS, _MNEG = 1.0, 0.2  # hinge margins, hard-coded in the reference (utils/utils.py:817-818)
+
+
 def _nc_pad(nc):
     return (nc + 255) // 256 * 256
+
+
+# What desc_backward needs of desc_forward: saved = (Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f, Ahi, Alo, Bhi, Blo), None
+# where the engine or need_grad has none; out8 = [loss, pos, neg, norm, num_loss, num_pos, num_neg, sum(mask_valid)].
+DescState = namedtuple("DescState", "saved out8 dims lamda engine fold")
+
+
+def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist, engine, need_grad, fold, debug_S=None):
+    """The dense descriptor loss up to desc_finalize -> (DescState, partial sums for desc_finalize, wpts [B,Ncp,2]).
+    mask_valid [B,Hc*Wc] or mask_2d [B,1,8Hc,8Wc] (getMasks fused into the geometry kernel).  fold (tensor-core engines with
+    need_grad): the mask is folded into the indicator words and the backward needs no pack pass.  Exact only for a 0/1 mask
+    and g_neg = 0; a non-binary mask poisons the normaliser with NaN in the geometry kernel (loud, no sync)."""
+    lib = _lib.load()
+    dev = D.device
+    Dc = f32c(D.detach(), dev)
+    Dwc = f32c(Dw.detach(), dev)
+    if Dc.shape != Dwc.shape:
+        raise RuntimeError("descriptor_loss: descriptor shapes differ")
+    B, Dch, Hc, Wc = Dc.shape
+    Nc = Hc * Wc
+    Ncp = _nc_pad(Nc)
+    s = stream_of(Dc)
+    if engine not in _ENGINES:
+        raise ValueError("descriptor engine must be one of %s" % (_ENGINES,))
+    if Dch != 256:
+        engine = "fp32"  # the tcgen05 kernels are specialised for 256 channels
+    split = engine == "bf16x3"
+    fold = bool(fold and need_grad and engine != "fp32")
+
+    wpts = torch.empty((B, Ncp, 2), dtype=torch.float32, device=dev)
+    mv_pad = torch.empty((B, Ncp), dtype=torch.float32, device=dev)
+    mvbits = torch.empty((B, Ncp // 32), dtype=torch.int32, device=dev) if fold else None
+    nmv = lib.ssp_desc_geometry_nblocks(B, Nc)
+    mv_part = torch.empty((nmv,), dtype=torch.float64, device=dev)
+    geom_args = (ptr(Hm), ptr(mask_valid), ptr(mask_2d), cell, ptr(wpts), ptr(mv_pad), ptr(mv_part), ptr(mvbits))
+    if engine == "fp32":
+        call("ssp_desc_geometry", geom_args[0], geom_args[1], geom_args[2], B, Hc, Wc, *geom_args[3:], s)
+    # tensor-core engines: the geometry blocks ride in the operand pack's launch (independent work, one launch instead of two)
+
+    # sparse positive pairs: exact dots, partial sums, pair lists for the backward
+    maxp = lib.ssp_desc_maxp()
+    npos = lib.ssp_desc_pos_planes_nblocks(B, Nc) if split else lib.ssp_desc_pos_nblocks(B, Nc)
+    pos_part = torch.empty((npos, 4), dtype=torch.float64, device=dev)
+    lists_i = torch.empty((3, B, Ncp, maxp), dtype=torch.int32, device=dev)   # rowcol, colrow, (colcnt in [2,:,:,0])
+    lists_f = torch.empty((2, B, Ncp, maxp), dtype=torch.float32, device=dev)  # rowdot, coldot
+    rowcol, colrow, colcnt = lists_i[0], lists_i[1], lists_i[2].view(-1)[: B * Ncp + 1]
+    rowdot, coldot = lists_f[0], lists_f[1]
+    overflow = colcnt[B * Ncp:]  # pairs that did not fit a list: desc_finalize turns a non-zero count into NaN
+    bitsR = bitsC = None
+    if need_grad:
+        bitsR = torch.empty((B, Ncp // 32, Ncp), dtype=torch.int32, device=dev)
+        bitsC = torch.empty((B, Ncp // 32, Ncp), dtype=torch.int32, device=dev)
+    Ahi = Alo = Bhi = Blo = None
+    # every buffer of the forward is allocated before the fork (see _Fork)
+    if engine == "fp32":
+        nneg = lib.ssp_desc_dense_simt_nblocks(B, Nc)
+    else:
+        nneg = lib.ssp_desc_dense_tc_nblocks(B, Nc)
+        # hi (and lo) planes of one tensor in ONE allocation, lo above hi: the backward's TMA box spans both planes
+        PA = torch.empty((2 if split else 1, B, Ncp, Dch), dtype=torch.bfloat16, device=dev)
+        PB = torch.empty_like(PA)
+        Ahi, Alo = PA[0], (PA[1] if split else None)
+        Bhi, Blo = PB[0], (PB[1] if split else None)
+    neg_part = torch.empty((nneg, 2), dtype=torch.float64, device=dev)
+    out8 = torch.empty((8,), dtype=torch.float32, device=dev)
+    if split:
+        # bf16x3: the positive pairs read the packed hi/lo planes (2 x 512 contiguous bytes per cell instead of 256
+        # strided channels), so they run right after the pack, in front of the tensor-core kernel
+        call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), *geom_args, s)
+        call("ssp_desc_pos_fwd_planes", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(wpts), ptr(mv_pad), B, Hc, Wc, cell,
+             dist, lamda, _MPOS, _MNEG, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), s)
+        # bitsC (the column-orientation indicator words) is only read by the backward GEMM: it is transposed from bitsR by
+        # extra blocks of the backward's coefficient launch, not here
+        call("ssp_desc_dense_fwd_tc", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(mv_pad), ptr(mvbits), B, Hc, Wc, _MNEG,
+             ptr(neg_part), ptr(bitsR), None, ptr(debug_S), s)
+    else:
+        # the HBM-bound exact positive-pair kernel overlaps the pack + tensor-core kernels
+        if engine != "fp32":  # single-pass bf16: pack + geometry first (the positive-pair kernel needs the warped points)
+            call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), None, ptr(Bhi), None, *geom_args, s)
+        with _Fork(dev) as fork:
+            call("ssp_desc_pos_fwd", ptr(Dc), ptr(Dwc), ptr(wpts), ptr(mv_pad), B, Hc, Wc, Dch, cell, dist, lamda, _MPOS,
+                 _MNEG, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), stream_of(Dc))
+        if engine == "fp32":
+            call("ssp_desc_dense_fwd_simt", ptr(Dc), ptr(Dwc), ptr(mv_pad), B, Hc, Wc, Dch, _MNEG, ptr(neg_part),
+                 ptr(bitsR), ptr(bitsC), ptr(debug_S), s)
+        else:
+            call("ssp_desc_dense_fwd_tc", ptr(Ahi), None, ptr(Bhi), None, ptr(mv_pad), ptr(mvbits), B, Hc, Wc, _MNEG,
+                 ptr(neg_part), ptr(bitsR), None, ptr(debug_S), s)
+        fork.join()
+    st = DescState((Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f, Ahi, Alo, Bhi, Blo), out8, (B, Dch, Hc, Wc), lamda,
+                   engine, fold)
+    return st, (pos_part, npos, neg_part, nneg, mv_part, nmv, overflow), wpts
+
+
+def desc_finalize(st, parts, det_out=None, lambda_loss=0.0, total=None):
+    """ssp_desc_finalize: reduces the partial sums of desc_forward into st.out8 (a positive pair that did not fit the lists
+    turns the loss into NaN).  With det_out ([2,3], det_pair_forward's out) it also writes the fused step's total
+    det_out[0,0] + det_out[1,0] + lambda_loss * loss_desc into total [1]."""
+    pos_part, npos, neg_part, nneg, mv_part, nmv, overflow = parts
+    B, _, Hc, Wc = st.dims
+    call("ssp_desc_finalize", ptr(pos_part), npos, ptr(neg_part), nneg, ptr(mv_part), nmv, B, Hc, Wc, ptr(overflow),
+         ptr(st.out8), ptr(None if det_out is None else det_out[0]), ptr(None if det_out is None else det_out[1]),
+         float(lambda_loss), ptr(total), stream_of(pos_part))
+    if CHECK_LIST_OVERFLOW and int(overflow[0]) != 0:  # host sync: debugging / tests only (the NaN above is the product signal)
+        raise RuntimeError("descriptor_loss: %d positive pairs overflowed the sparse lists" % int(overflow[0]))
+
+
+def desc_backward(st, g3, gscale=1.0, gmode=0, det=None):
+    """(dD, dDw) for g3 = device {dL/dloss, dL/dpos, dL/dneg} (gmode 0) or, folded mask only, the fused step's upstream
+    gradient scaled by gscale in the coefficient kernel (gmode 1).  det = (DetPair, g, d0, d1), folded mask only: the
+    detector-pair backward for g into d0 / d1 rides in the coefficient launch."""
+    if det is not None and not st.fold:
+        raise ValueError("desc_backward: the detector backward merges only into the folded-mask backward")
+    Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f, Ahi, Alo, Bhi, Blo = st.saved
+    out8, lamda, fold = st.out8, st.lamda, st.fold
+    B, Dch, Hc, Wc = st.dims
+    dev = Dc.device
+    Nc = Hc * Wc
+    Ncp = _nc_pad(Nc)
+    s = stream_of(Dc)
+    tc_engine = st.engine != "fp32"
+    split = st.engine == "bf16x3"
+    # alpha[b,c] = (g_loss * mv[c] + g_neg) / norm: coefficient of the negative hinge of column c; srow = alpha at mv = 1
+    # (row scale of the folded backward).  Folded: both come out of the coefficient kernel below.
+    alpha = torch.empty((B, Ncp), dtype=torch.float32, device=dev)
+    srow = torch.empty((B, Ncp), dtype=torch.float32, device=dev) if fold else None
+    if not fold:
+        call("ssp_desc_alpha", ptr(mv_pad), ptr(g3), ptr(out8), B, Ncp, ptr(alpha), None, s)
+    rowcol, colrow, colcnt = lists_i[0], lists_i[1], lists_i[2]
+    rowdot, coldot = lists_f[0], lists_f[1]
+    coefs = torch.empty((2,) + tuple(rowdot.shape), dtype=torch.float32, device=dev)
+    colrow_sorted = torch.empty_like(colrow)  # the saved lists stay as the forward wrote them (retain_graph safe)
+    dD = torch.empty_like(Dc)
+    dDw = torch.empty_like(Dwc)
+    if tc_engine and not fold:
+        PS = torch.empty((2 if split else 1, B, Ncp, Dch), dtype=torch.bfloat16, device=dev)
+        Shi, Slo = PS[0], (PS[1] if split else None)
+    # dD [b,:,r] = sum_c I[r,c] alpha[c] Dw[b,:,c] + sum_n rowcoef[r,n] Dw[b,:,rowcol[r,n]]
+    # dDw[b,:,c] = alpha[c] sum_r I[r,c] D[b,:,r]  + sum_n colcoef[c,n] D [b,:,colrow[c,n]]
+    # tensor-core engines: both GEMMs run in ONE persistent launch, the positive pairs are applied inside the GEMM
+    # epilogues (dedicated epilogue warps hide the gathers behind the next item's main loop);
+    # fp32 engine: one streaming apply kernel after the GEMMs.
+    # stream plan:  [pos_coef]  ||  [pack(alpha * Dw), unless folded]  ->  GEMM pair
+    if fold:
+        # bitsR / bitsC already exclude the columns with mask_valid = 0: dD = srow * (I' @ Dw) on the forward planes
+        if det is not None:
+            # fused step: the detector-loss backward of both images rides in the same launch (heterogeneous blocks)
+            dst, dg, d0, d1 = det
+            x0, t0, m0, x1, t1, m1 = dst.saved
+            call("ssp_step_bwd_prologue", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc, ptr(dst.out[0]),
+                 ptr(dst.out[1]), ptr(dg), ptr(d0), ptr(d1),
+                 ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR), ptr(mv_pad), ptr(g3), gscale,
+                 gmode, ptr(out8), lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(alpha), ptr(srow),
+                 ptr(bitsC), s)
+        else:
+            call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
+                 ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted),
+                 ptr(coefs[1]), ptr(alpha), ptr(srow), ptr(bitsC), Nc, s)
+    else:
+        # on the tensor-core engines the coefficient launch also transposes bitsR into bitsC (fp32: the forward wrote it)
+        with _Fork(dev) as f1:
+            call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
+                 ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted),
+                 ptr(coefs[1]), None, None, ptr(bitsC) if tc_engine else None, Nc if tc_engine else 0, stream_of(Dc))
+        if not tc_engine:
+            call("ssp_desc_bits_gemm_simt", ptr(bitsR), ptr(Dwc), ptr(alpha), None, None, None, None, B, Dch, Nc, ptr(dD), s)
+            call("ssp_desc_bits_gemm_simt", ptr(bitsC), ptr(Dc), None, ptr(alpha), None, None, None, B, Dch, Nc, ptr(dDw), s)
+            f1.join()
+            call("ssp_desc_pos_apply", ptr(rowcol), ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(Dc), ptr(Dwc), B, Dch,
+                 Nc, 0, ptr(dD), ptr(dDw), s)
+            return dD, dDw
+        call("ssp_desc_pack", ptr(Dwc), ptr(alpha), B, Dch, Nc, ptr(Shi), ptr(Slo), s)
+        f1.join()
+    # the dD GEMM reads the forward planes of Dw (rows scaled by srow) when folded, the packed alpha * Dw otherwise; the
+    # positive-pair partners come from the packed planes of the forward (Dw for dD, D for dDw)
+    Whi, Wlo = (Bhi, Blo) if fold else (Shi, Slo)
+    call("ssp_desc_bits_gemm_tc_pair",
+         ptr(bitsR), ptr(Whi), ptr(Wlo), ptr(srow), ptr(rowcol), ptr(coefs[0]), ptr(Bhi), ptr(Blo), ptr(dD),
+         ptr(bitsC), ptr(Ahi), ptr(Alo), ptr(alpha), ptr(colrow_sorted), ptr(coefs[1]), ptr(Ahi), ptr(Alo), ptr(dDw),
+         B, Nc, s)
+    return dD, dDw
 
 
 class DescriptorLossFn(torch.autograd.Function):
@@ -233,236 +440,30 @@ class DescriptorLossFn(torch.autograd.Function):
     differentiable w.r.t. descriptors and descriptors_warped, wpts (warped cell centres) is not."""
 
     @staticmethod
-    def forward(ctx, D, Dw, Hm, mv, cell, lamda, dist, engine, dist_group=None, debug_S=None, fold_alpha=False, step_total=None):
-        # step_total (LossStepFn only): (det_out [2,3], lambda_loss, total [1]) -- the finalize kernel also writes the weighted
-        # sum of the fused step, so no torch add / mul kernels are needed for it
-        lib = _lib.load()
-        dev = D.device
-        Dc = f32c(D.detach(), dev)
-        Dwc = f32c(Dw.detach(), dev)
-        if Dc.shape != Dwc.shape:
-            raise RuntimeError("descriptor_loss: descriptor shapes differ")
-        B, Dch, Hc, Wc = Dc.shape
-        Nc = Hc * Wc
-        Ncp = _nc_pad(Nc)
-        st = stream_of(Dc)
-        mpos, mneg = 1.0, 0.2  # hard-coded in the reference (utils/utils.py:817-818)
-        if engine not in _ENGINES:
-            raise ValueError("descriptor engine must be one of %s" % (_ENGINES,))
-        if Dch != 256:
-            engine = "fp32"  # the tcgen05 kernels are specialised for 256 channels
+    def forward(ctx, D, Dw, Hm, mv, cell, lamda, dist, engine, dist_group=None, debug_S=None):
         need_grad = bool(ctx.needs_input_grad[0] or ctx.needs_input_grad[1])
-        split = engine == "bf16x3"
-        # "fold": the (binary) mask is folded into the indicator words, the dD GEMM runs on the forward planes of Dw and
-        # the backward needs no pack pass.  Exact only for a 0/1 mask and g_neg = 0 (LossStepFn guarantees the latter);
-        # a non-binary mask poisons the normaliser with NaN in the geometry kernel (loud, no sync).
-        fold_alpha = bool(fold_alpha and need_grad and engine != "fp32")
-
-        wpts = torch.empty((B, Ncp, 2), dtype=torch.float32, device=dev)
-        mv_pad = torch.empty((B, Ncp), dtype=torch.float32, device=dev)
-        mvbits = torch.empty((B, Ncp // 32), dtype=torch.int32, device=dev) if fold_alpha else None
-        nmv = lib.ssp_desc_geometry_nblocks(B, Nc)
-        mv_part = torch.empty((nmv,), dtype=torch.float64, device=dev)
-        mask2d = None
-        if isinstance(mv, tuple):  # ("2d", mask [B,1,8Hc,8Wc]): LossStepFn -- getMasks is fused into the geometry kernel
-            mask2d, mv = mv[1], None
-        geom_args = (ptr(Hm), ptr(mv), ptr(mask2d), cell, ptr(wpts), ptr(mv_pad), ptr(mv_part), ptr(mvbits))
-        if engine == "fp32":
-            call("ssp_desc_geometry", geom_args[0], geom_args[1], geom_args[2], B, Hc, Wc, *geom_args[3:], st)
-        # tensor-core engines: the geometry blocks ride in the operand pack's launch (independent work, one launch instead of two)
-
-        # sparse positive pairs: exact dots, partial sums, pair lists for the backward
-        maxp = lib.ssp_desc_maxp()
-        npos = lib.ssp_desc_pos_planes_nblocks(B, Nc) if split else lib.ssp_desc_pos_nblocks(B, Nc)
-        pos_part = torch.empty((npos, 4), dtype=torch.float64, device=dev)
-        lists_i = torch.empty((3, B, Ncp, maxp), dtype=torch.int32, device=dev)   # rowcol, colrow, (colcnt in [2,:,:,0])
-        lists_f = torch.empty((2, B, Ncp, maxp), dtype=torch.float32, device=dev)  # rowdot, coldot
-        rowcol, colrow, colcnt = lists_i[0], lists_i[1], lists_i[2].view(-1)[: B * Ncp + 1]
-        rowdot, coldot = lists_f[0], lists_f[1]
-        overflow = colcnt[B * Ncp:]  # pairs that did not fit a list: desc_finalize turns a non-zero count into NaN
-        bitsR = bitsC = None
-        if need_grad:
-            bitsR = torch.empty((B, Ncp // 32, Ncp), dtype=torch.int32, device=dev)
-            bitsC = torch.empty((B, Ncp // 32, Ncp), dtype=torch.int32, device=dev)
-        planes = None
-        # every buffer of the forward is allocated before the fork (see _Fork)
-        if engine == "fp32":
-            nneg = lib.ssp_desc_dense_simt_nblocks(B, Nc)
-        else:
-            nneg = lib.ssp_desc_dense_tc_nblocks(B, Nc)
-            # hi (and lo) planes of one tensor in ONE allocation, lo above hi: the backward's TMA box spans both planes
-            PA = torch.empty((2 if split else 1, B, Ncp, Dch), dtype=torch.bfloat16, device=dev)
-            PB = torch.empty_like(PA)
-            Ahi, Alo = PA[0], (PA[1] if split else None)
-            Bhi, Blo = PB[0], (PB[1] if split else None)
-        neg_part = torch.empty((nneg, 2), dtype=torch.float64, device=dev)
-        out8 = torch.empty((8,), dtype=torch.float32, device=dev)
-        if split:
-            # bf16x3: the positive pairs read the packed hi/lo planes (2 x 512 contiguous bytes per cell instead of 256
-            # strided channels), so they run right after the pack, in front of the tensor-core kernel
-            call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), *geom_args, st)
-            call("ssp_desc_pos_fwd_planes", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(wpts), ptr(mv_pad), B, Hc, Wc, cell,
-                 dist, lamda, mpos, mneg, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), st)
-            # bitsC (the column-orientation indicator words) is only read by the backward GEMM: it is transposed from bitsR by
-            # extra blocks of the backward's coefficient launch, not here
-            call("ssp_desc_dense_fwd_tc", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(mv_pad), ptr(mvbits), B, Hc, Wc, mneg,
-                 ptr(neg_part), ptr(bitsR), None, ptr(debug_S), st)
-            planes = (Ahi, Alo, Bhi, Blo)
-        else:
-            # the HBM-bound exact positive-pair kernel overlaps the pack + tensor-core kernels
-            if engine != "fp32":  # single-pass bf16: pack + geometry first (the positive-pair kernel needs the warped points)
-                call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), None, ptr(Bhi), None, *geom_args, st)
-            with _Fork(dev) as fork:
-                call("ssp_desc_pos_fwd", ptr(Dc), ptr(Dwc), ptr(wpts), ptr(mv_pad), B, Hc, Wc, Dch, cell, dist, lamda, mpos,
-                     mneg, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), stream_of(Dc))
-            if engine == "fp32":
-                call("ssp_desc_dense_fwd_simt", ptr(Dc), ptr(Dwc), ptr(mv_pad), B, Hc, Wc, Dch, mneg, ptr(neg_part),
-                     ptr(bitsR), ptr(bitsC), ptr(debug_S), st)
-            else:
-                call("ssp_desc_dense_fwd_tc", ptr(Ahi), None, ptr(Bhi), None, ptr(mv_pad), ptr(mvbits), B, Hc, Wc, mneg,
-                     ptr(neg_part), ptr(bitsR), None, ptr(debug_S), st)
-                planes = (Ahi, None, Bhi, None)
-            fork.join()
-
-        if step_total is not None:
-            det_out, lam_loss, total = step_total[:3]
-            if len(step_total) > 3 and step_total[3] is not None:
-                step_total[3].join()  # the detector losses ran on a forked stream (LossStepFn)
-            call("ssp_desc_finalize", ptr(pos_part), npos, ptr(neg_part), nneg, ptr(mv_part), nmv, B, Hc, Wc, ptr(overflow),
-                 ptr(out8), ptr(det_out[0]), ptr(det_out[1]), float(lam_loss), ptr(total), st)
-        else:
-            call("ssp_desc_finalize", ptr(pos_part), npos, ptr(neg_part), nneg, ptr(mv_part), nmv, B, Hc, Wc, ptr(overflow),
-                 ptr(out8), None, None, 0.0, None, st)
-        if CHECK_LIST_OVERFLOW and int(overflow[0]) != 0:  # host sync: debugging / tests only (the NaN above is the product signal)
-            raise RuntimeError("descriptor_loss: %d positive pairs overflowed the sparse lists" % int(overflow[0]))
+        st, parts, wpts = desc_forward(D, Dw, Hm, mask_valid=mv, cell=cell, lamda=lamda, dist=dist, engine=engine,
+                                       need_grad=need_grad, fold=False, debug_S=debug_S)
+        desc_finalize(st, parts)
         if dist_group is not None:
             from .dist import globalize_descriptor
-            globalize_descriptor(out8, B, Hc, Wc, dist_group)
-
+            B, _, Hc, Wc = st.dims
+            globalize_descriptor(st.out8, B, Hc, Wc, dist_group)
         if need_grad:
-            ctx.save_for_backward(Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f,
-                                  *([p for p in planes if p is not None] if planes else []))
-            ctx.out8 = out8  # see DetectorLossFn
-        ctx.meta = (B, Dch, Hc, Wc, cell, lamda, dist, mpos, engine, planes is not None and planes[1] is not None)
-        ctx.fold_alpha = fold_alpha
+            ctx.save_for_backward(*st.saved)
+        ctx.st = st._replace(saved=None)  # out8 is an attribute, see DetectorLossFn
         ctx.mark_non_differentiable(wpts)
-        return out8[0], out8[1], out8[2], wpts
+        return st.out8[0], st.out8[1], st.out8[2], wpts
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g_loss, g_pos, g_neg, _g_wpts):
-        saved = ctx.saved_tensors
-        Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f = saved[:7]
-        out8 = ctx.out8
-        B, Dch, Hc, Wc, cell, lamda, dist, mpos, engine, split = ctx.meta
-        dev = Dc.device
-        Nc = Hc * Wc
-        Ncp = _nc_pad(Nc)
-        st = stream_of(Dc)
-        tc_engine = engine != "fp32"
-        fold = tc_engine and getattr(ctx, "fold_alpha", False)
-        gscale, gmode = 1.0, 0
-        if g_pos is _SAME:  # fused step: g_loss is the upstream gradient of the step total (one element), to be scaled by lambda_loss
-            lam = float(getattr(ctx, "gscale", 1.0))
-            if fold:
-                g3, gscale, gmode = g_loss, lam, 1  # the coefficient kernel applies the scale itself: no torch kernel here
-            else:
-                key = (dev.index, lam)
-                if key not in _lam3:
-                    _lam3[key] = torch.tensor([lam, 0.0, 0.0], dtype=torch.float32, device=dev)
-                g3 = g_loss * _lam3[key]
-        else:
-            zero = torch.zeros((), dtype=torch.float32, device=dev)
-            g3 = torch.stack([(g if g is not None else zero).reshape(()).to(torch.float32) for g in (g_loss, g_pos, g_neg)])
-            g3 = g3.contiguous()
-        # alpha[b,c] = (g_loss * mv[c] + g_neg) / norm: coefficient of the negative hinge of column c; srow = alpha at mv = 1
-        # (row scale of the folded backward).  Folded: both come out of the coefficient kernel below.
-        alpha = torch.empty((B, Ncp), dtype=torch.float32, device=dev)
-        srow = torch.empty((B, Ncp), dtype=torch.float32, device=dev) if fold else None
-        if not fold:
-            call("ssp_desc_alpha", ptr(mv_pad), ptr(g3), ptr(out8), B, Ncp, ptr(alpha), None, st)
-        rowcol, colrow, colcnt = lists_i[0], lists_i[1], lists_i[2]
-        rowdot, coldot = lists_f[0], lists_f[1]
-        coefs = torch.empty((2,) + tuple(rowdot.shape), dtype=torch.float32, device=dev)
-        colrow_sorted = torch.empty_like(colrow)  # the saved lists stay as the forward wrote them (retain_graph safe)
-        dD = torch.empty_like(Dc)
-        dDw = torch.empty_like(Dwc)
-        if tc_engine:
-            if split:
-                Ahi, Alo, Bhi, Blo = saved[7:11]
-            else:
-                (Ahi, Bhi), Alo, Blo = saved[7:9], None, None
-            if not fold:
-                PS = torch.empty((2 if split else 1, B, Ncp, Dch), dtype=torch.bfloat16, device=dev)
-                Shi, Slo = PS[0], (PS[1] if split else None)
-        # dD [b,:,r] = sum_c I[r,c] alpha[c] Dw[b,:,c] + sum_n rowcoef[r,n] Dw[b,:,rowcol[r,n]]
-        # dDw[b,:,c] = alpha[c] sum_r I[r,c] D[b,:,r]  + sum_n colcoef[c,n] D [b,:,colrow[c,n]]
-        # tensor-core engines: both GEMMs run in ONE persistent launch, the positive pairs are applied inside the GEMM
-        # epilogues (dedicated epilogue warps hide the gathers behind the next item's main loop);
-        # fp32 engine: one streaming apply kernel after the GEMMs.
-        # stream plan:  [pos_coef]  ||  [pack(alpha * Dw), unless folded]  ->  GEMM pair
-        if fold:
-            # bitsR / bitsC already exclude the columns with mask_valid = 0: dD = s * (I' @ Dw) on the forward planes, s = g_loss / norm
-            det_job = getattr(ctx, "det_job", None)
-            if det_job is not None:
-                # fused step: the detector-loss backward of both images rides in the same launch (heterogeneous blocks)
-                x0, t0, m0, x1, t1, m1, dout, dg, d0, d1 = det_job
-                call("ssp_step_bwd_prologue", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc, ptr(dout[0]),
-                     ptr(dout[1]), ptr(dg), ptr(d0), ptr(d1),
-                     ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR), ptr(mv_pad), ptr(g3), gscale,
-                     gmode, ptr(out8), lamda, mpos, ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(alpha), ptr(srow),
-                     ptr(bitsC), st)
-            else:
-                call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
-                     ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, mpos, ptr(coefs[0]), ptr(colrow_sorted),
-                     ptr(coefs[1]), ptr(alpha), ptr(srow), ptr(bitsC), Nc, st)
-            call("ssp_desc_bits_gemm_tc_pair",
-                 ptr(bitsR), ptr(Bhi), ptr(Blo), ptr(srow), ptr(rowcol), ptr(coefs[0]), ptr(Bhi), ptr(Blo), ptr(dD),
-                 ptr(bitsC), ptr(Ahi), ptr(Alo), ptr(alpha), ptr(colrow_sorted), ptr(coefs[1]), ptr(Ahi), ptr(Alo), ptr(dDw),
-                 B, Nc, st)
-        elif tc_engine:
-            with _Fork(dev) as f1:
-                call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
-                     ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, mpos, ptr(coefs[0]), ptr(colrow_sorted),
-                     ptr(coefs[1]), None, None, ptr(bitsC), Nc, stream_of(Dc))
-            call("ssp_desc_pack", ptr(Dwc), ptr(alpha), B, Dch, Nc, ptr(Shi), ptr(Slo), st)
-            f1.join()
-            # positive-pair partners from the packed planes of the forward (Dw for dD, D for dDw)
-            call("ssp_desc_bits_gemm_tc_pair",
-                 ptr(bitsR), ptr(Shi), ptr(Slo), None, ptr(rowcol), ptr(coefs[0]), ptr(Bhi), ptr(Blo), ptr(dD),
-                 ptr(bitsC), ptr(Ahi), ptr(Alo), ptr(alpha), ptr(colrow_sorted), ptr(coefs[1]), ptr(Ahi), ptr(Alo), ptr(dDw),
-                 B, Nc, st)
-        else:
-            with _Fork(dev) as f1:
-                call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
-                     ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, mpos, ptr(coefs[0]), ptr(colrow_sorted),
-                     ptr(coefs[1]), None, None, None, 0, stream_of(Dc))
-            call("ssp_desc_bits_gemm_simt", ptr(bitsR), ptr(Dwc), ptr(alpha), None, None, None, None, B, Dch, Nc, ptr(dD), st)
-            call("ssp_desc_bits_gemm_simt", ptr(bitsC), ptr(Dc), None, ptr(alpha), None, None, None, B, Dch, Nc, ptr(dDw), st)
-            f1.join()
-            call("ssp_desc_pos_apply", ptr(rowcol), ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(Dc), ptr(Dwc), B, Dch, Nc, 0,
-                 ptr(dD), ptr(dDw), st)
-        return dD, dDw, None, None, None, None, None, None, None, None, None, None
+        st = ctx.st._replace(saved=ctx.saved_tensors)
+        dD, dDw = desc_backward(st, grad_vector((g_loss, g_pos, g_neg), st.out8.device))
+        return dD, dDw, None, None, None, None, None, None, None, None
 
 
 # ------------------------------------------------------------------------------------------------
-class _Ctx(object):
-    """Stand-in for the autograd context so LossStepFn can run the bodies of the two Functions above."""
-
-    def __init__(self, needs):
-        self.needs_input_grad = needs
-        self.saved_tensors = ()
-
-    def save_for_backward(self, *tensors):
-        self.saved_tensors = tensors
-
-    def mark_non_differentiable(self, *tensors):
-        pass
-
-
-_lam3 = {}
-
-
 class LossStepFn(torch.autograd.Function):
     """The whole loss step (Train_model_heatmap_all.py:295-365, uniform weighting) as ONE autograd node:
     loss = loss_det + loss_det_warp + lambda_loss * loss_desc.  Same kernels as DetectorLossPairFn + DescriptorLossFn;
@@ -473,7 +474,6 @@ class LossStepFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, desc, desc_w, Hm, lamda_d, dist,
                 lambda_loss, engine, dist_group=None):
-        c1 = _Ctx((ctx.needs_input_grad[0], False, False, ctx.needs_input_grad[3], False, False, False, False))
         B, _, Hc, Wc = semi.shape
         dev = semi.device
         # The two detector losses (HBM-bound, + their one-block finalize) run on a forked stream next to the first half of
@@ -482,55 +482,52 @@ class LossStepFn(torch.autograd.Function):
         # in).  The streams join in front of desc_finalize, which reads both detector triples for the step total.
         fork = _Fork(dev)
         with fork:
-            l0, l1, _cm = DetectorLossPairFn.forward(c1, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, True)
+            det, _ = det_pair_forward(semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, True)
         mw = f32c(mask_warp_2D.detach(), dev)
         if mw.numel() != B * Hc * Wc * 64:
             raise RuntimeError("loss_step: mask_warp_2D must be [B,1,%d,%d]" % (Hc * 8, Wc * 8))
-        c2 = _Ctx((ctx.needs_input_grad[6], ctx.needs_input_grad[7]) + (False,) * 8)
+        want_desc = bool(ctx.needs_input_grad[6] or ctx.needs_input_grad[7])
         total = torch.empty((1,), dtype=torch.float32, device=dev)
-        # fold_alpha=True: the cell mask is folded into the indicator words of the tensor-core engines, so the backward needs
-        # no pack pass (measured: 0.339 -> 0.330 ms per step).  Fold requires a binary mask and g_neg = 0; the latter holds
-        # because only `loss` is differentiable, and a non-binary mask turns the loss into NaN.  A soft mask belongs on
-        # fused=False, whose descriptor_loss packs alpha * Dw into its own planes.
-        ld, pos, neg, _wpts = DescriptorLossFn.forward(c2, desc, desc_w, Hm, ("2d", mw), 8, lamda_d, dist, engine,
-                                                       None, None, True, (c1.out, lambda_loss, total, fork))
+        # fold=True (measured: 0.339 -> 0.330 ms per step): g_neg = 0 holds because only `loss` is differentiable, and a
+        # non-binary mask turns the loss into NaN.  A soft mask belongs on fused=False, whose descriptor_loss packs
+        # alpha * Dw into its own planes.
+        st, parts, _wpts = desc_forward(desc, desc_w, Hm, mask_2d=mw, cell=8, lamda=lamda_d, dist=dist, engine=engine,
+                                        need_grad=want_desc, fold=True)
+        fork.join()
+        desc_finalize(st, parts, det.out, lambda_loss, total)
         if dist_group is not None:
             # multi-GPU: ONE exchange kernel turns the three local results into global-batch values in place (the scalars
-            # above are views of c1.out / c2.out8) and rewrites the weighted total; the backward kernels read the global
+            # below are views of det.out / st.out8) and rewrites the weighted total; the backward kernels read the global
             # normalisers from the same buffers
             from .dist import get_exchange
-            get_exchange(dist_group).run(det0=c1.out[0], det1=c1.out[1], desc8=c2.out8, B_local=B, Hc=Hc, Wc=Wc,
+            get_exchange(dist_group).run(det0=det.out[0], det1=det.out[1], desc8=st.out8, B_local=B, Hc=Hc, Wc=Wc,
                                          lambda_loss=lambda_loss, total=total)
-        loss = total[0]
-        ctx.c1, ctx.c2, ctx.lambda_loss = c1, c2, float(lambda_loss)
-        ctx.mark_non_differentiable(l0, l1, ld, pos, neg)
+        ctx.det, ctx.desc, ctx.lambda_loss = det, (st if want_desc else None), float(lambda_loss)
+        outs = (det.out[0, 0], det.out[1, 0], st.out8[0], st.out8[1], st.out8[2])
+        ctx.mark_non_differentiable(*outs)
         ctx.set_materialize_grads(False)  # no zero-filled gradient tensors for the five logging outputs
-        return loss, l0, l1, ld, pos, neg
+        return (total[0],) + outs
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g, *_unused):
         if g is None:
             return (None,) * 14
-        dev = g.device
-        g = f32c(g.reshape(1), dev)
+        g = f32c(g.reshape(1), g.device)
+        det, desc, lam = ctx.det, ctx.desc, ctx.lambda_loss
         d0 = d1 = dD = dDw = None
         want_det = ctx.needs_input_grad[0] or ctx.needs_input_grad[3]
-        want_desc = ctx.needs_input_grad[6] or ctx.needs_input_grad[7]
-        c2 = ctx.c2
-        c2.det_job = None
-        merged = (want_det and want_desc and getattr(c2, "fold_alpha", False) and c2.meta[8] != "fp32" and ctx.c1.fused2d)
+        # folded mask: one launch runs the detector backward and the descriptor backward's coefficient / transpose blocks
+        merged = want_det and desc is not None and desc.fold
         if merged:
-            # one launch for the detector backward and the descriptor backward's coefficient / transpose blocks
-            x0, t0, m0, x1, t1, m1 = ctx.c1.saved_tensors
-            d0, d1 = torch.empty_like(x0), torch.empty_like(x1)
-            c2.det_job = (x0, t0, m0, x1, t1, m1, ctx.c1.out, g, d0, d1)
+            d0, d1 = torch.empty_like(det.saved[0]), torch.empty_like(det.saved[3])
         elif want_det:
-            d0, _, _, d1 = DetectorLossPairFn.backward(ctx.c1, g, _SAME, None)[:4]
-        if want_desc:
-            c2.gscale = ctx.lambda_loss
-            dD, dDw = DescriptorLossFn.backward(c2, g, _SAME, None, None)[:2]
-            c2.det_job = None
+            d0, d1 = det_pair_backward(det, g, g)
+        if desc is not None:
+            if desc.fold:  # the coefficient kernel scales g by lambda_loss itself: no torch kernel here
+                dD, dDw = desc_backward(desc, g, lam, 1, det=(det, g, d0, d1) if merged else None)
+            else:
+                dD, dDw = desc_backward(desc, g * _lam3_vector(lam, g.device))
         return d0, None, None, d1, None, None, dD, dDw, None, None, None, None, None, None
 
 
@@ -544,35 +541,30 @@ class SparseLossStepFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, desc, desc_w, ia, ib, M, K, lamda_d,
                 lambda_loss):
-        from .sparse import SparseDescriptorLossFn
-        c1 = _Ctx((ctx.needs_input_grad[0], False, False, ctx.needs_input_grad[3], False, False, False, False))
-        l0, l1, _cm = DetectorLossPairFn.forward(c1, semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, True)
-        c2 = _Ctx((ctx.needs_input_grad[6], ctx.needs_input_grad[7]) + (False,) * 6)
-        ld, pos, neg = SparseDescriptorLossFn.forward(c2, desc, desc_w, ia, ib, K, ia.shape[1] - K, lamda_d)
+        from .sparse import sparse_forward
+        det, _ = det_pair_forward(semi, labels_2D, mask_2D, semi_w, warped_labels, mask_warp_2D, True)
+        sp = sparse_forward(desc, desc_w, ia, ib, K, ia.shape[1] - K, lamda_d)
         total = torch.empty((1,), dtype=torch.float32, device=semi.device)
-        call("ssp_sparse_finalize", ptr(M), M.shape[0], ptr(c2.out3), ptr(c1.out[0]), ptr(c1.out[1]), float(lambda_loss),
+        call("ssp_sparse_finalize", ptr(M), M.shape[0], ptr(sp.out3), ptr(det.out[0]), ptr(det.out[1]), float(lambda_loss),
              ptr(total), stream_of(total))
-        ctx.c1, ctx.c2, ctx.lambda_loss = c1, c2, float(lambda_loss)
-        ctx.mark_non_differentiable(l0, l1, ld, pos, neg)
+        ctx.det, ctx.sparse, ctx.lambda_loss = det, sp, float(lambda_loss)
+        outs = (det.out[0, 0], det.out[1, 0], sp.out3[0], sp.out3[1], sp.out3[2])
+        ctx.mark_non_differentiable(*outs)
         ctx.set_materialize_grads(False)
-        return total[0], l0, l1, ld, pos, neg
+        return (total[0],) + outs
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g, *_unused):
-        from .sparse import sparse_loss_backward
+        from .sparse import sparse_backward
         if g is None:
             return (None,) * 14
-        dev = g.device
-        g = f32c(g.reshape(1), dev)
+        g = f32c(g.reshape(1), g.device)
         d0 = d1 = dD = dDw = None
         if ctx.needs_input_grad[0] or ctx.needs_input_grad[3]:
-            d0, _, _, d1 = DetectorLossPairFn.backward(ctx.c1, g, _SAME, None)[:4]
+            d0, d1 = det_pair_backward(ctx.det, g, g)
         if ctx.needs_input_grad[6] or ctx.needs_input_grad[7]:
-            key = (dev.index, ctx.lambda_loss)
-            if key not in _lam3:
-                _lam3[key] = torch.tensor([ctx.lambda_loss, 0.0, 0.0], dtype=torch.float32, device=dev)
-            dD, dDw = sparse_loss_backward(ctx.c2, g * _lam3[key])
+            dD, dDw = sparse_backward(ctx.sparse, g * _lam3_vector(ctx.lambda_loss, g.device))
         return d0, None, None, d1, None, None, dD, dDw, None, None, None, None, None, None
 
 

@@ -14,12 +14,15 @@ in device memory: no host RNG call and no host synchronisation, so the whole spa
 whose replays draw fresh lists.  Its draws are not the reference's RNG stream; batch_descriptor_loss_sparse uses it only
 when it is passed one.
 """
+from collections import namedtuple
+
 import numpy as np
 import torch
 from torch.autograd.function import once_differentiable
 
 from . import _lib
 from ._lib import call, f32c, ptr, stream_of
+from .losses import grad_vector
 
 CHECK_EMPTY_IMAGES = False  # DeviceSampler.sample raises when an image had no candidate (costs a host sync per call)
 
@@ -121,60 +124,66 @@ class DeviceSampler(object):
         return int(self.state[3])
 
 
+# What sparse_backward needs of sparse_forward: saved = (Dt, Dwt, ia, ib, dots, stats), out3 = [loss, match, nonmatch]
+SparseState = namedtuple("SparseState", "saved out3 dims K Kn lamda")
+
+
+def sparse_forward(D, Dw, ia, ib, K, Kn, lamda, M=None):
+    """SparseDescriptorLossFn's forward -> SparseState."""
+    _lib.require_cuda(D, Dw)
+    dev = D.device
+    Dc, Dwc = f32c(D.detach(), dev), f32c(Dw.detach(), dev)
+    B, Dch, Hc, Wc = Dc.shape
+    Nc = Hc * Wc
+    s = stream_of(Dc)
+    Dt = torch.empty((B, Nc, Dch), dtype=torch.float32, device=dev)
+    Dwt = torch.empty_like(Dt)
+    call("ssp_transpose_batched", ptr(Dc), B, Dch, Nc, ptr(Dt), s)
+    call("ssp_transpose_batched", ptr(Dwc), B, Dch, Nc, ptr(Dwt), s)
+    dots = torch.empty((B, K + Kn), dtype=torch.float32, device=dev)
+    stats = torch.empty((B, 4), dtype=torch.float32, device=dev)
+    out3 = torch.empty((3,), dtype=torch.float32, device=dev)
+    call("ssp_sparse_desc_loss_fwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), B, Nc, Dch, K, Kn, float(lamda), 1.0, 0.2,
+         ptr(dots), ptr(stats), ptr(out3), s)
+    if M is not None:
+        call("ssp_sparse_finalize", ptr(M), B, ptr(out3), None, None, 0.0, None, s)
+    return SparseState((Dt, Dwt, ia, ib, dots, stats), out3, (B, Dch, Hc, Wc), K, Kn, float(lamda))
+
+
+def sparse_backward(st, g3):
+    """Gradients (dD, dDw) [B,Dch,Hc,Wc] of sparse_forward's loss for g3 = device {dL/dloss, dL/dmatch, dL/dnonmatch}."""
+    Dt, Dwt, ia, ib, dots, stats = st.saved
+    B, Dch, Hc, Wc = st.dims
+    Nc = Hc * Wc
+    s = stream_of(Dt)
+    dDt = torch.empty_like(Dt)
+    dDwt = torch.empty_like(Dwt)
+    call("ssp_sparse_desc_loss_bwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), ptr(dots), ptr(stats), ptr(g3), B, Nc, Dch, st.K,
+         st.Kn, st.lamda, 1.0, 0.2, ptr(dDt), ptr(dDwt), s)
+    dD = torch.empty((B, Dch, Hc, Wc), dtype=torch.float32, device=Dt.device)
+    dDw = torch.empty_like(dD)
+    call("ssp_transpose_batched", ptr(dDt), B, Nc, Dch, ptr(dD), s)
+    call("ssp_transpose_batched", ptr(dDwt), B, Nc, Dch, ptr(dDw), s)
+    return dD, dDw
+
+
 class SparseDescriptorLossFn(torch.autograd.Function):
     """(loss, match, nonmatch) batch means from descriptors [B,Dch,Hc,Wc] and index lists ia / ib [B, K + Kn] (int32).
     M: the candidate counts of DeviceSampler.sample, or None; a zero count turns the three means into NaN."""
 
     @staticmethod
     def forward(ctx, D, Dw, ia, ib, K, Kn, lamda, M=None):
-        _lib.require_cuda(D, Dw)
-        dev = D.device
-        Dc, Dwc = f32c(D.detach(), dev), f32c(Dw.detach(), dev)
-        B, Dch, Hc, Wc = Dc.shape
-        Nc = Hc * Wc
-        st = stream_of(Dc)
-        Dt = torch.empty((B, Nc, Dch), dtype=torch.float32, device=dev)
-        Dwt = torch.empty_like(Dt)
-        call("ssp_transpose_batched", ptr(Dc), B, Dch, Nc, ptr(Dt), st)
-        call("ssp_transpose_batched", ptr(Dwc), B, Dch, Nc, ptr(Dwt), st)
-        dots = torch.empty((B, K + Kn), dtype=torch.float32, device=dev)
-        stats = torch.empty((B, 4), dtype=torch.float32, device=dev)
-        out3 = torch.empty((3,), dtype=torch.float32, device=dev)
-        call("ssp_sparse_desc_loss_fwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), B, Nc, Dch, K, Kn, float(lamda), 1.0, 0.2,
-             ptr(dots), ptr(stats), ptr(out3), st)
-        if M is not None:
-            call("ssp_sparse_finalize", ptr(M), B, ptr(out3), None, None, 0.0, None, st)
-        ctx.save_for_backward(Dt, Dwt, ia, ib, dots, stats)
-        ctx.meta = (B, Dch, Hc, Wc, K, Kn, float(lamda))
-        ctx.out3 = out3  # attribute, not a saved tensor (the fused sparse step writes its total from it)
-        return out3[0], out3[1], out3[2]
+        st = sparse_forward(D, Dw, ia, ib, K, Kn, lamda, M)
+        ctx.save_for_backward(*st.saved)
+        ctx.st = st._replace(saved=None)
+        return st.out3[0], st.out3[1], st.out3[2]
 
     @staticmethod
     @once_differentiable
     def backward(ctx, g_loss, g_match, g_non):
-        zero = torch.zeros((), dtype=torch.float32, device=ctx.saved_tensors[0].device)
-        g3 = torch.stack([(g if g is not None else zero).reshape(()).to(torch.float32) for g in (g_loss, g_match, g_non)]).contiguous()
-        dD, dDw = sparse_loss_backward(ctx, g3)
+        st = ctx.st._replace(saved=ctx.saved_tensors)
+        dD, dDw = sparse_backward(st, grad_vector((g_loss, g_match, g_non), st.out3.device))
         return dD, dDw, None, None, None, None, None, None
-
-
-def sparse_loss_backward(ctx, g3):
-    """Gradients (dD, dDw) [B,Dch,Hc,Wc] of SparseDescriptorLossFn's forward saved in ctx, for g3 = device {dL/dloss,
-    dL/dmatch, dL/dnonmatch}."""
-    Dt, Dwt, ia, ib, dots, stats = ctx.saved_tensors
-    B, Dch, Hc, Wc, K, Kn, lamda = ctx.meta
-    dev = Dt.device
-    Nc = Hc * Wc
-    st = stream_of(Dt)
-    dDt = torch.empty_like(Dt)
-    dDwt = torch.empty_like(Dwt)
-    call("ssp_sparse_desc_loss_bwd", ptr(Dt), ptr(Dwt), ptr(ia), ptr(ib), ptr(dots), ptr(stats), ptr(g3), B, Nc, Dch, K, Kn,
-         lamda, 1.0, 0.2, ptr(dDt), ptr(dDwt), st)
-    dD = torch.empty((B, Dch, Hc, Wc), dtype=torch.float32, device=dev)
-    dDw = torch.empty_like(dD)
-    call("ssp_transpose_batched", ptr(dDt), B, Nc, Dch, ptr(dD), st)
-    call("ssp_transpose_batched", ptr(dDwt), B, Nc, Dch, ptr(dDw), st)
-    return dD, dDw
 
 
 def sparse_loss_from_lists(descriptors, descriptors_warped, matches_a, matches_b, non_matches_a, non_matches_b, lamda_d=250):

@@ -44,14 +44,8 @@ def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2
             semi, labels_2D, mask_2D, semi_warp, warped_labels, mask_warp_2D, desc, desc_warp,
             Hm.to(device=semi.device, dtype=torch.float32).contiguous(), float(lamda_d), float(descriptor_dist),
             float(lambda_loss), engine or get_descriptor_engine(), dist_group)
-        out = {}
-        if sem_pred is not None:
-            out["loss_sem"] = U.sem_loss(sem_pred, sem, dist_group=dist_group)
-            out["loss_sem_warp"] = U.sem_loss(sem_warp_pred, warped_sem, dist_group=dist_group)
-            loss = loss + out["loss_sem"] + out["loss_sem_warp"]
-        out.update({"loss": loss, "loss_det": loss_det, "loss_det_warp": loss_det_warp, "loss_desc": loss_desc,
-                    "positive_dist": pos, "negative_dist": neg})
-        return out
+        return _result(loss, loss_det, loss_det_warp, loss_desc, pos, neg,
+                       _sem_losses(sem_pred, sem, sem_warp_pred, warped_sem, dist_group))
     # separately differentiable components (the reference's multi_task_loss weighting); with dist_group each loss runs
     # its own exchange kernel
     # both detector losses in one launch each way; getMasks(mask_warp_2D) comes out of the same kernel
@@ -63,13 +57,24 @@ def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2
         kw["engine"] = engine
     loss_desc, _mask, pos, neg = U.descriptor_loss(desc, desc_warp, mat_H, mask_valid=mask_desc, device=semi.device,
                                                    lamda_d=lamda_d, descriptor_dist=descriptor_dist, **kw)
-    out = {}
-    if sem_pred is not None:
-        out["loss_sem"] = U.sem_loss(sem_pred, sem, dist_group=dist_group)
-        out["loss_sem_warp"] = U.sem_loss(sem_warp_pred, warped_sem, dist_group=dist_group)
+    sem_terms = _sem_losses(sem_pred, sem, sem_warp_pred, warped_sem, dist_group)
     loss = loss_det + loss_det_warp + lambda_loss * loss_desc
-    if sem_pred is not None:
-        loss = loss + out["loss_sem"] + out["loss_sem_warp"]
+    return _result(loss, loss_det, loss_det_warp, loss_desc, pos, neg, sem_terms)
+
+
+def _sem_losses(sem_pred, sem, sem_warp_pred, warped_sem, dist_group=None):
+    """(loss_sem, loss_sem_warp), or None without semantic terms."""
+    if sem_pred is None:
+        return None
+    return U.sem_loss(sem_pred, sem, dist_group=dist_group), U.sem_loss(sem_warp_pred, warped_sem, dist_group=dist_group)
+
+
+def _result(loss, loss_det, loss_det_warp, loss_desc, pos, neg, sem_terms):
+    """loss_step's result dict; the semantic terms, if any, are added to the total."""
+    out = {}
+    if sem_terms is not None:
+        out["loss_sem"], out["loss_sem_warp"] = sem_terms
+        loss = loss + sem_terms[0] + sem_terms[1]
     out.update({"loss": loss, "loss_det": loss_det, "loss_det_warp": loss_det_warp, "loss_desc": loss_desc,
                 "positive_dist": pos, "negative_dist": neg})
     return out
@@ -85,7 +90,6 @@ def _sparse_loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels
         raise ValueError("loss_step(descriptor_loss='sparse') needs sampler=sparse.DeviceSampler(seed, device)")
     K = int(K)
     ia, ib, M = sampler.sample(mat_H, desc.shape[2], desc.shape[3], K, n)
-    out = {}
     if fused:
         from .losses import SparseLossStepFn
         loss, loss_det, loss_det_warp, loss_desc, pos, neg = SparseLossStepFn.apply(
@@ -95,13 +99,7 @@ def _sparse_loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels
         loss_det, loss_det_warp, _ = U.detector_loss_pair_2d(semi, labels_2D, mask_2D, semi_warp, warped_labels, mask_warp_2D)
         loss_desc, pos, neg = SparseDescriptorLossFn.apply(desc, desc_warp, ia, ib, K, ia.shape[1] - K, float(lamda_d), M)
         loss = loss_det + loss_det_warp + lambda_loss * loss_desc
-    if sem_pred is not None:
-        out["loss_sem"] = U.sem_loss(sem_pred, sem)
-        out["loss_sem_warp"] = U.sem_loss(sem_warp_pred, warped_sem)
-        loss = loss + out["loss_sem"] + out["loss_sem_warp"]
-    out.update({"loss": loss, "loss_det": loss_det, "loss_det_warp": loss_det_warp, "loss_desc": loss_desc,
-                "positive_dist": pos, "negative_dist": neg})
-    return out
+    return _result(loss, loss_det, loss_det_warp, loss_desc, pos, neg, _sem_losses(sem_pred, sem, sem_warp_pred, warped_sem))
 
 
 @torch.no_grad()

@@ -551,7 +551,7 @@ def descriptor_loss(descriptors, descriptors_warped, homographies, mask_valid=No
     engine = config.get("engine", None) or get_descriptor_engine()
     out = DescriptorLossFn.apply(descriptors, descriptors_warped, Hm, mv, int(cell_size), float(lamda_d),
                                  float(descriptor_dist), engine, config.get("dist_group", None),
-                                 config.get("debug_S", None), False, None)
+                                 config.get("debug_S", None))
     loss, pos_sum, neg_sum, wpts = out
     mask = LazyPairMask(wpts, B, Hc, Wc, int(cell_size), float(descriptor_dist))
     return loss, mask, pos_sum, neg_sum

@@ -410,6 +410,43 @@ def test_step_deterministic(engine):
     assert_identical(a, r1, "eager vs replay")
 
 
+def test_backward_twice_over_retained_graph():
+    """Two backward(retain_graph=True) calls over one graph give the same gradients: the backward leaves the saved pair
+    lists as the forward wrote them.  Bit-identical on descriptor_loss (each engine) and the fused dense step, whose
+    summation order is fixed; within 1e-5 of the largest element on the fused sparse step, whose scatter backward adds
+    with fp32 atomics."""
+    d = bench_set(0)
+    mv = S.getMasks(d["mask_warp_2D"], 8, device=DEV).unsqueeze(1)
+
+    def step(**kw):
+        return lambda *leaves: S.step.loss_step(*leaves, d["labels_2D"], d["warped_labels"], d["mask_2D"], d["mask_warp_2D"],
+                                                d["mat_H"], **kw)["loss"]
+
+    def desc(engine):
+        def run(semi, semi_w, D, Dw):
+            loss, _, pos, neg = S.descriptor_loss(D, Dw, d["mat_H"], mask_valid=mv, device=DEV, engine=engine)
+            return loss + 0.5 * pos + 0.25 * neg
+        return run
+
+    cases = [("descriptor_loss " + e, desc(e), 0.0) for e in ("bf16x3", "bf16", "fp32")]
+    cases += [("fused dense step", step(), 0.0),
+              ("fused sparse step", step(descriptor_loss="sparse", sampler=S.sparse.DeviceSampler(11, DEV)), 1e-5)]
+    for what, run, rtol in cases:
+        leaves = [d[k].detach().requires_grad_(True) for k in LEAVES]
+        total = run(*leaves)
+        grads = []
+        for _ in range(2):
+            for t in leaves:
+                t.grad = None
+            total.backward(retain_graph=True)
+            grads.append([t.grad for t in leaves])
+        torch.cuda.synchronize()
+        for name, a, b in zip(LEAVES, *grads):
+            assert (a is None) == (b is None), (what, name)
+            if a is not None:
+                assert float((a - b).abs().max()) <= rtol * float(a.abs().max()), (what, name)
+
+
 # ------------------------------------------------------------------ tile edges of the descriptor kernels
 # Hc x Wc: exact multiples of 256 cells (no padding rows), 264 (a 16-wide last column tile: 8 cells per CTA in the TMA
 # box), 255, 1023, and fewer than 128 cells (the second CTA of a pair holds only padding)

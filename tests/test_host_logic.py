@@ -131,11 +131,11 @@ def test_shard_range_covers_everything():
 
 def test_orchestration_call_sequences(monkeypatch):
     """The host side of the loss step with the C library faked out (every entry point recorded, nothing computed): the
-    Python orchestration -- buffer shapes, autograd plumbing, engine dispatch, fused / unfused / semantic variants -- runs
-    on a CPU-only box and issues the documented kernel sequence (DESIGN 4.3)."""
-    from ssp_b200 import _lib, losses, step, utils
+    Python orchestration -- buffer shapes, autograd plumbing, engine dispatch, fused / unfused / semantic / sparse variants,
+    partial gradients -- runs on a CPU-only box and issues the documented kernel sequence (DESIGN 4.3)."""
+    from ssp_b200 import _lib, losses, sparse, step, utils
     calls = []
-    for m in (_lib, losses, utils):
+    for m in (_lib, losses, sparse, utils):
         monkeypatch.setattr(m, "call", lambda name, *a: calls.append(name))
         monkeypatch.setattr(m, "stream_of", lambda t: None)
     monkeypatch.setattr(_lib, "require_cuda", lambda *t: None)
@@ -161,10 +161,16 @@ def test_orchestration_call_sequences(monkeypatch):
     semi, semi_w, D, Dw = leaf(B, 65, Hc, Wc), leaf(B, 65, Hc, Wc), leaf(B, 256, Hc, Wc), leaf(B, 256, Hc, Wc)
     lab, m, H = torch.zeros(B, 1, Hc * 8, Wc * 8), torch.ones(B, 1, Hc * 8, Wc * 8), torch.eye(3).repeat(B, 1, 1)
 
-    def run(**kw):
+    def run(loss_keys=("loss",), grad_on=(semi, semi_w, D, Dw), **kw):
         del calls[:]
+        for t in (semi, semi_w, D, Dw):
+            t.grad = None
+            t.requires_grad_(any(t is g for g in grad_on))
         out = step.loss_step(semi, semi_w, D, Dw, lab, lab, m, m, H, **kw)
-        out["loss"].backward()
+        sum(out[k] for k in loss_keys).backward()
+        for t in (semi, semi_w, D, Dw):
+            assert (t.grad is not None) == any(t is g for g in grad_on)
+            t.requires_grad_()
         return list(calls)
 
     fwd = ["ssp_detector_loss_fwd_pair", "ssp_desc_pack2_geometry", "ssp_desc_pos_fwd_planes",
@@ -172,10 +178,16 @@ def test_orchestration_call_sequences(monkeypatch):
     # one-node fused step: the mask is folded into the indicator words, no pack pass in the backward, both GEMMs in one launch
     # backward of the one-node fused step: detector backward + coefficient / alpha / transpose blocks in ONE launch, then both GEMMs
     assert run() == fwd + ["ssp_step_bwd_prologue", "ssp_desc_bits_gemm_tc_pair"]
+    # one side of the step differentiated: no merged launch
+    assert run(grad_on=(D, Dw)) == fwd + ["ssp_desc_pos_coef", "ssp_desc_bits_gemm_tc_pair"]
+    assert run(grad_on=(semi, semi_w)) == fwd + ["ssp_detector_loss_bwd_pair"]
     # separately differentiable components (reference multi_task_loss weighting): general mask path with the pack pass
     bwd_desc = ["ssp_desc_alpha", "ssp_desc_pos_coef", "ssp_desc_pack", "ssp_desc_bits_gemm_tc_pair"]
     unfused = run(fused=False)
     assert unfused[:5] == fwd and sorted(unfused[5:]) == sorted(bwd_desc + ["ssp_detector_loss_bwd_pair"])
+    multi = run(fused=False, loss_keys=("loss_det", "loss_det_warp", "positive_dist", "negative_dist"))
+    assert multi[:5] == fwd and sorted(multi[5:]) == sorted(bwd_desc + ["ssp_detector_loss_bwd_pair"])
+    assert run(fused=False, grad_on=(D, Dw), loss_keys=("positive_dist", "negative_dist")) == fwd + bwd_desc
     assert [c for c in run(engine="fp32") if "_desc_" in c] == [
         "ssp_desc_geometry", "ssp_desc_pos_fwd", "ssp_desc_dense_fwd_simt", "ssp_desc_finalize", "ssp_desc_alpha",
         "ssp_desc_pos_coef", "ssp_desc_bits_gemm_simt", "ssp_desc_bits_gemm_simt", "ssp_desc_pos_apply"]
@@ -188,3 +200,23 @@ def test_orchestration_call_sequences(monkeypatch):
     assert sem.count("ssp_sem_ce_fwd") == 2 and sem.count("ssp_sem_ce_bwd") == 2          # full-resolution logits
     with pytest.raises(RuntimeError, match="1/8"):
         utils.sem_loss(leaf(B, 133, Hc * 4, Wc * 4), sl)
+
+    # the sparse step on device-sampled lists (a stand-in sampler: the real one refuses a CPU device)
+    sampler = object.__new__(sparse.DeviceSampler)
+    sampler.device, sampler.state, sampler.last = torch.device("cpu"), torch.zeros(4, dtype=torch.int64), None
+    sk = dict(descriptor_loss="sparse", sampler=sampler, num_matching_attempts=7, num_masked_non_matches_per_match=3)
+    sfwd = ["ssp_sparse_sample", "ssp_detector_loss_fwd_pair", "ssp_transpose_batched", "ssp_transpose_batched",
+            "ssp_sparse_desc_loss_fwd", "ssp_sparse_finalize"]
+    sbwd = ["ssp_sparse_desc_loss_bwd", "ssp_transpose_batched", "ssp_transpose_batched"]
+    assert run(**sk) == sfwd + ["ssp_detector_loss_bwd_pair"] + sbwd
+    assert run(grad_on=(D, Dw), **sk) == sfwd + sbwd
+    unfused = run(fused=False, **sk)
+    assert unfused[:6] == sfwd and sorted(unfused[6:]) == sorted(sbwd + ["ssp_detector_loss_bwd_pair"])
+    assert sampler.last[0].shape == (B, 7 * 4)
+
+    # the descriptors saved for the backward are still checked by autograd for in-place modification
+    Dn = D * 1.0
+    loss, _mask, _pos, _neg = utils.descriptor_loss(Dn, Dw, H)
+    Dn.add_(1.0)
+    with pytest.raises(RuntimeError, match="modified by an inplace operation"):
+        loss.backward()
