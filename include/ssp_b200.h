@@ -22,7 +22,6 @@ extern "C" {
 
 int ssp_version(void);
 const char* ssp_last_error(void);
-int ssp_sm_count(void);
 
 /* ---- a1 / a10: warp_points (utils/utils.py:315-343), filter_points (:303-311),
  *      warp_keypoints / keep_true_keypoints (evaluations/detector_evaluation.py:139-191) ---- */
@@ -117,8 +116,8 @@ int ssp_desc_pos_fwd(const float* D /*[B,Dch,Hc,Wc]*/, const float* Dw, const fl
                      int Hc, int Wc, int Dch, int cell, float dist, float lamda, float mpos, float mneg,
                      double* partials, int* rowcol, float* rowdot, int* colcnt, int* colrow, float* coldot,
                      void* stream);
-/* Same contract from the packed hi/lo planes [B,Nc_pad,256] bf16 of D (A*) and Dw (B*) written by ssp_desc_pack2 (bf16x3
- * engine): a cell's descriptor is 2 x 512 contiguous bytes there instead of 256 channels 4*Nc bytes apart. */
+/* Same contract from the packed hi/lo planes [B,Nc_pad,256] bf16 of D (A*) and Dw (B*) written by ssp_desc_pack2_geometry
+ * (bf16x3 engine): a cell's descriptor is 2 x 512 contiguous bytes there instead of 256 channels 4*Nc bytes apart. */
 int ssp_desc_pos_planes_nblocks(int B, int Nc);
 int ssp_desc_pos_fwd_planes(const void* Ahi, const void* Alo, const void* Bhi, const void* Blo, const float* wpts,
                             const float* mv_pad, int B, int Hc, int Wc, int cell, float dist, float lamda, float mpos,
@@ -130,21 +129,19 @@ int ssp_desc_dense_fwd_simt(const float* D, const float* Dw, const float* mv_pad
                             float* dbgS /*[B,Nc,Nc] or NULL*/, void* stream);
 int ssp_desc_pack(const float* src /*[B,Dch,Nc]*/, const float* scale /*[B,Nc_pad] or NULL*/, int B, int Dch, int Nc,
                   void* hi /*bf16 [B,Nc_pad,Dch]*/, void* lo /*or NULL*/, void* stream);
-int ssp_desc_pack2(const float* src0, const float* src1 /*or NULL*/, const float* scale, int B, int Dch, int Nc, void* hi0,
-                   void* lo0, void* hi1, void* lo1, void* stream);
-/* ssp_desc_pack2 (both tensors, unscaled) and ssp_desc_geometry as ONE launch: they do not depend on each other */
+/* ssp_desc_pack of two tensors (unscaled) and ssp_desc_geometry as ONE launch: they do not depend on each other */
 int ssp_desc_pack2_geometry(const float* src0, const float* src1, int B, int Dch, int Hc, int Wc, void* hi0, void* lo0 /*or NULL*/,
                             void* hi1, void* lo1 /*or NULL*/, const float* H /*[B,3,3]*/, const float* mask_valid /*or NULL*/,
                             const float* mask2d /*or NULL*/, int cell, float* wpts, float* mv_pad, double* mv_part,
                             uint32_t* mvbits /*or NULL*/, void* stream);
 int ssp_desc_dense_tc_nblocks(int B, int Nc);
-/* tcgen05 forward (CTA-pair MMAs, M=256): negative hinge over all pairs + indicator words; bitsC = transpose of bitsR
- * (second kernel of the same call).  The lo planes must lie above their hi planes in memory (one allocation).
+/* tcgen05 forward (CTA-pair MMAs, M=256): negative hinge over all pairs + row-orientation indicator words bitsR (their
+ * transpose bitsC comes from ssp_desc_pos_coef).  The lo planes must lie above their hi planes in memory (one allocation).
  * mvbits != NULL ("fold"): the indicator words drop the columns whose mask_valid is 0, so the dD indicator GEMM can take
  * the unscaled forward planes of Dw and one scalar (valid when mask_valid is binary and g_neg = 0). */
 int ssp_desc_dense_fwd_tc(const void* Ahi, const void* Alo, const void* Bhi, const void* Blo, const float* mv_pad,
                           const uint32_t* mvbits /*or NULL*/, int B, int Hc, int Wc, float mneg, double* partials,
-                          uint32_t* bitsR, uint32_t* bitsC, float* dbgS, void* stream);
+                          uint32_t* bitsR, float* dbgS, void* stream);
 /* overflow (optional) = &colcnt[B*Nc_pad], the counter of positive pairs that did not fit the sparse lists: non-zero
  * makes loss / pos_sum NaN (loud without a host sync) */
 int ssp_desc_finalize(const double* pos_part, int npos, const double* neg_part, int nneg, const double* mv_part,
@@ -154,13 +151,13 @@ int ssp_desc_finalize(const double* pos_part, int npos, const double* neg_part, 
 int ssp_desc_pair_mask(const float* wpts, int B, int Hc, int Wc, int cell, float dist, float* mask /*[B,Nc,Nc]*/,
                        void* stream);
 int ssp_desc_alpha(const float* mv_pad, const float* g3 /*[3] dL/d(loss,pos,neg)*/, const float* out8, int B,
-                   int Nc_pad, float* alpha /*[B,Nc_pad]*/, float* srow /*or NULL: [B,Nc_pad], alpha for mask_valid = 1*/,
-                   void* stream);
+                   int Nc_pad, float* alpha /*[B,Nc_pad]*/, void* stream);
 /* backward coefficients of the positive pairs (and removal of their negative term).  colrow_sorted receives the column
  * lists ordered by row index (deterministic summation order) with their coefficients in colcoef; the forward's lists
  * are left untouched, so a second backward over the same graph sees the same inputs.
  * g3: gmode 0 -> {dL/dloss, dL/dpos, dL/dneg}; gmode 1 -> g3[0] = dL/dloss only (fused step); both scaled by gscale.
- * alpha_out / srow_out (optional, [B,Nc_pad]): what ssp_desc_alpha would write for the same scaled gradients.
+ * alpha_out (optional, [B,Nc_pad]): what ssp_desc_alpha would write for the same scaled gradients; srow_out (optional,
+ * [B,Nc_pad]): the same coefficient at mask_valid = 1, the row scale of the folded backward.
  * bitsC_out (optional, then Nc = unpadded cell count): bitsC transposed from bitsR by extra blocks of the same launch. */
 int ssp_desc_pos_coef(const int* rowcol, const float* rowdot, const int* colcnt, const int* colrow, const float* coldot,
                       const uint32_t* bitsR, const float* mv_pad, const float* g3, float gscale, int gmode,
@@ -178,19 +175,14 @@ int ssp_step_bwd_prologue(const float* semi0, const float* labels0, const float*
                           float* alpha_out, float* srow_out, uint32_t* bitsC_out, void* stream);
 /* dD[b,:,r] += sum_n rowcoef[b,r,n] Dw[b,:,rowcol[b,r,n]];  dDw[b,:,c] += sum_n colcoef[b,c,n] D[b,:,colrow[b,c,n]] */
 int ssp_desc_pos_apply(const int* rowcol, const float* rowcoef, const int* colrow, const float* colcoef, const float* D,
-                       const float* Dw, int B, int Dch, int Nc, int which /*0 both, 1 dD, 2 dDw*/, float* dD, float* dDw,
-                       void* stream);
-/* indicator GEMM  out[b,d,r] = rowscale[b,r] * sum_k bit(r,k) * colscale[b,k] * src[b,d,k]
- *                            + sum_n pcoef[b,r,n] * possrc[b,d,plist[b,r,n]]   (plist may be NULL) */
+                       const float* Dw, int B, int Dch, int Nc, float* dD, float* dDw, void* stream);
+/* indicator GEMM  out[b,d,r] = rowscale[b,r] * sum_k bit(r,k) * colscale[b,k] * src[b,d,k]  (scales may be NULL) */
 int ssp_desc_bits_gemm_simt(const uint32_t* bits, const float* src /*[B,Dch,Nc]*/, const float* colscale,
-                            const float* rowscale, const int* plist, const float* pcoef, const float* possrc, int B,
-                            int Dch, int Nc, float* out /*[B,Dch,Nc]*/, void* stream);
-/* tcgen05 indicator GEMM (CTA-pair MMAs, A = indicator bits expanded into TMEM, B = packed planes [B,Nc_pad,256] bf16,
- * Blo above Bhi in memory or NULL); positive-pair partners read from packed planes pos_hi (+ pos_lo). */
-int ssp_desc_bits_gemm_tc_planes(const uint32_t* bits, const void* Bhi, const void* Blo, const float* rowscale,
-                                 const int* plist, const float* pcoef, const void* pos_hi, const void* pos_lo, int B,
-                                 int Nc, float* out /*[B,256,Nc]*/, void* stream);
-/* both indicator GEMMs of the backward (job 0: dD, job 1: dDw) in ONE persistent launch */
+                            const float* rowscale, int B, int Dch, int Nc, float* out /*[B,Dch,Nc]*/, void* stream);
+/* tcgen05 indicator GEMMs of the backward (job 0: dD, job 1: dDw) in ONE persistent launch (CTA-pair MMAs, A = indicator
+ * bits expanded into TMEM, B = packed planes [B,Nc_pad,256] bf16, Blo above Bhi in memory or NULL), out [B,256,Nc]
+ *   out[b,d,r] = rowscale[b,r] * sum_k bit(r,k) * B[b,k,d] + sum_n pcoef[b,r,n] * pos[b,plist[b,r,n],d]
+ * with the positive-pair partners read from the packed planes pos_hi (+ pos_lo); plist may be NULL. */
 int ssp_desc_bits_gemm_tc_pair(const uint32_t* bits0, const void* Bhi0, const void* Blo0, const float* rowscale0,
                                const int* plist0, const float* pcoef0, const void* pos_hi0, const void* pos_lo0,
                                float* out0, const uint32_t* bits1, const void* Bhi1, const void* Blo1,
@@ -281,7 +273,6 @@ int ssp_warp_labels(const float* pnts, const int* counts, int B, int Pmax, int H
  * {loss, sum, count} in place with the global-batch values (any of them may be NULL).  Stream-ordered, graph
  * capturable, no NCCL.  A peer that does not arrive within timeout_s poisons the outputs with NaN and sets the
  * sticky error that ssp_xchg_status reports (it synchronises the stream). ---- */
-size_t ssp_xchg_bytes(void);
 int ssp_xchg_max_ranks(void);
 int ssp_xchg_alloc(void** buf, void* ipc_handle64_host);
 int ssp_xchg_open(const void* ipc_handle64_host, void** peer_buf);

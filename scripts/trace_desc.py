@@ -26,26 +26,33 @@ mv = torch.ones((B, Ncp), device=dev)
 PA = torch.empty((2, B, Ncp, Dch), dtype=torch.bfloat16, device=dev)  # hi, lo planes of D (lo above hi)
 PB = torch.empty_like(PA)                                             # hi, lo planes of Dw
 st = stream_of(D)
-call("ssp_desc_pack2", ptr(D), ptr(Dw), None, B, Dch, Nc, ptr(PA[0]), ptr(PA[1]), ptr(PB[0]), ptr(PB[1]), st)
+call("ssp_desc_pack", ptr(D), None, B, Dch, Nc, ptr(PA[0]), ptr(PA[1]), st)
+call("ssp_desc_pack", ptr(Dw), None, B, Dch, Nc, ptr(PB[0]), ptr(PB[1]), st)
 nneg = lib.ssp_desc_dense_tc_nblocks(B, Nc)
 part = torch.empty((nneg, 2), dtype=torch.float64, device=dev)
 bitsR = torch.empty((B, Ncp // 32, Ncp), dtype=torch.int32, device=dev)
 bitsC = torch.empty_like(bitsR)
 out = torch.empty((B, Dch, Nc), device=dev)
 out2 = torch.empty((B, Dch, Nc), device=dev)
-plist = torch.full((B, Ncp, 16), -1, dtype=torch.int32, device=dev)
+maxp = lib.ssp_desc_maxp()
+plist = torch.full((B, Ncp, maxp), -1, dtype=torch.int32, device=dev)
 plist[:, :Nc, 0] = torch.arange(Nc, device=dev, dtype=torch.int32)[None]
-pcoef = torch.ones((B, Ncp, 16), device=dev)
+pcoef = torch.ones((B, Ncp, maxp), device=dev)
 
 
-def fwd(bits=True, split=True, transpose=True):
+def fwd(bits=True, split=True):
     call("ssp_desc_dense_fwd_tc", ptr(PA[0]), ptr(PA[1]) if split else None, ptr(PB[0]), ptr(PB[1]) if split else None, ptr(mv), None,
-         B, Hc, Wc, 0.2, ptr(part), ptr(bitsR) if bits else None, ptr(bitsC) if (bits and transpose) else None, None, st)
+         B, Hc, Wc, 0.2, ptr(part), ptr(bitsR) if bits else None, None, st)
 
 
-def bwd1(pos=True, split=True):
-    call("ssp_desc_bits_gemm_tc_planes", ptr(bitsR), ptr(PB[0]), ptr(PB[1]) if split else None, None, ptr(plist) if pos else None,
-         ptr(pcoef) if pos else None, ptr(PB[0]), ptr(PB[1]) if split else None, B, Nc, ptr(out), st)
+def transpose_bits():
+    """bitsC from bitsR the way the backward makes it: the transpose blocks of the coefficient launch (empty pair lists)."""
+    nolist = torch.full((B, Ncp, maxp), -1, dtype=torch.int32, device=dev)
+    zi, zf = torch.zeros((B, Ncp), dtype=torch.int32, device=dev), torch.zeros((B, Ncp, maxp), device=dev)
+    g3, out8 = torch.zeros(3, device=dev), torch.ones(8, device=dev)
+    coef, srt = torch.empty((2, B, Ncp, maxp), device=dev), torch.empty_like(nolist)
+    call("ssp_desc_pos_coef", ptr(nolist), ptr(zf), ptr(zi), ptr(nolist), ptr(zf), ptr(bitsR), ptr(mv), ptr(g3), 1.0, 0,
+         ptr(out8), B, Ncp, 1.0, 1.0, ptr(coef[0]), ptr(srt), ptr(coef[1]), None, None, ptr(bitsC), Nc, st)
 
 
 def bwd2(pos=True, split=True):
@@ -57,6 +64,8 @@ def bwd2(pos=True, split=True):
 CAP = lib.ssp_debug_trace_cap()
 flush = torch.empty((64 << 20,), dtype=torch.float32, device=dev)  # 256 MB > L2
 res = {}
+fwd()
+transpose_bits()
 for name, fn in (("fwd", fwd), ("bwd", bwd2)):
     for _ in range(3):
         fn()

@@ -22,7 +22,6 @@ _Z = _c.c_size_t
 SIGNATURES = {
     "ssp_version": (_I, []),
     "ssp_last_error": (_c.c_char_p, []),
-    "ssp_sm_count": (_I, []),
     "ssp_warp_points": (_I, [_P, _I, _P, _I, _P, _P]),
     "ssp_warp_points_mask": (_I, [_P, _I, _P, _I, _F, _F, _P, _P, _P]),
     "ssp_warp_keypoints_f64": (_I, [_P, _I, _P, _D, _D, _P, _P, _P]),
@@ -52,18 +51,16 @@ SIGNATURES = {
     "ssp_desc_dense_simt_nblocks": (_I, [_I, _I]),
     "ssp_desc_dense_fwd_simt": (_I, [_P, _P, _P, _I, _I, _I, _I, _F, _P, _P, _P, _P, _P]),
     "ssp_desc_pack": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
-    "ssp_desc_pack2": (_I, [_P, _P, _P, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_desc_pack2_geometry": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P, _I, _P, _P, _P, _P, _P]),
     "ssp_desc_dense_tc_nblocks": (_I, [_I, _I]),
-    "ssp_desc_dense_fwd_tc": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P, _P, _P, _P, _P]),
+    "ssp_desc_dense_fwd_tc": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _F, _P, _P, _P, _P]),
     "ssp_desc_finalize": (_I, [_P, _I, _P, _I, _P, _I, _I, _I, _I, _P, _P, _P, _P, _F, _P, _P]),
     "ssp_desc_pair_mask": (_I, [_P, _I, _I, _I, _I, _F, _P, _P]),
-    "ssp_desc_alpha": (_I, [_P, _P, _P, _I, _I, _P, _P, _P]),
+    "ssp_desc_alpha": (_I, [_P, _P, _P, _I, _I, _P, _P]),
     "ssp_desc_pos_coef": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _F, _I, _P, _I, _I, _F, _F, _P, _P, _P, _P, _P, _P, _I, _P]),
     "ssp_step_bwd_prologue": (_I, [_P] * 6 + [_I] * 3 + [_P] * 5 + [_P] * 8 + [_F, _I, _P, _F, _F] + [_P] * 7),
-    "ssp_desc_pos_apply": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P]),
-    "ssp_desc_bits_gemm_simt": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P]),
-    "ssp_desc_bits_gemm_tc_planes": (_I, [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _P, _P]),
+    "ssp_desc_pos_apply": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _P, _P, _P]),
+    "ssp_desc_bits_gemm_simt": (_I, [_P, _P, _P, _P, _I, _I, _I, _P, _P]),
     "ssp_desc_bits_gemm_tc_pair": (_I, [_P] * 18 + [_I, _I, _P]),
     "ssp_sem_ce_ws_bytes": (_Z, [_I, _I, _I, _I, _I]),
     "ssp_sem_ce_fwd": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _Z, _P]),
@@ -81,7 +78,6 @@ SIGNATURES = {
     "ssp_warp_labels": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "ssp_debug_trace": (_I, [_P]),
     "ssp_debug_trace_cap": (_I, []),
-    "ssp_xchg_bytes": (_Z, []),
     "ssp_xchg_max_ranks": (_I, []),
     "ssp_xchg_alloc": (_I, [_c.POINTER(_P), _P]),
     "ssp_xchg_open": (_I, [_P, _c.POINTER(_P)]),
@@ -149,9 +145,19 @@ def profile_end():
     return out
 
 
+def check_arity(name, args):
+    """Raise TypeError unless args fits the entry point's SIGNATURES entry.  ctypes rejects too few arguments but passes
+    surplus ones on silently: a call site not updated after a parameter was removed would run with its arguments shifted
+    by one slot (its stream dropped as the surplus) and no error anywhere."""
+    want = len(SIGNATURES[name][1])
+    if len(args) != want:
+        raise TypeError("%s takes %d arguments, got %d" % (name, want, len(args)))
+
+
 def call(name, *args):
     """Invoke an int-returning entry point and raise RuntimeError(ssp_last_error()) on failure."""
     global launch_count, kernel_count
+    check_arity(name, args)
     launch_count += 1
     kernel_count += KERNELS_PER_CALL.get(name, 1)
     fn = getattr(load(), name)

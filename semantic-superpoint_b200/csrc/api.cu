@@ -1,4 +1,4 @@
-// Library-level entry points: version, last-error text, device properties.
+// Library-level entry points (version, last-error text) and the SM count the persistent kernels size their grids by.
 #include "common.cuh"
 #include <string.h>
 
@@ -23,4 +23,3 @@ int ssp_num_sms() {
 
 extern "C" const char* ssp_last_error(void) { return g_err; }
 extern "C" int ssp_version(void) { return 100; }  // 0.1.0
-extern "C" int ssp_sm_count(void) { return ssp_num_sms(); }

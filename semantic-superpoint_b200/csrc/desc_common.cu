@@ -544,22 +544,17 @@ extern "C" int ssp_desc_pair_mask(const float* wpts, int B, int Hc, int Wc, int 
 // ----------------------------------------------------------------------------------------------
 // backward scales: alpha[b,c] = (g_loss * mv[b,c] + g_neg) / norm   (coefficient of the negative hinge)
 // ----------------------------------------------------------------------------------------------
-// srow (optional) = the same coefficient for mv = 1: the row scale of the folded backward (mask already inside the bits)
 __global__ void desc_alpha_kernel(const float* __restrict__ mv_pad, const float* __restrict__ g3,
-                                  const float* __restrict__ out4, size_t n, float* __restrict__ alpha,
-                                  float* __restrict__ srow) {
+                                  const float* __restrict__ out4, size_t n, float* __restrict__ alpha) {
   size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) {
-    alpha[i] = (g3[0] * mv_pad[i] + g3[2]) / out4[3];
-    if (srow) srow[i] = (g3[0] * 1.0f + g3[2]) / out4[3];
-  }
+  if (i < n) alpha[i] = (g3[0] * mv_pad[i] + g3[2]) / out4[3];
 }
 
-extern "C" int ssp_desc_alpha(const float* mv_pad, const float* g3, const float* out4, int B, int Nc_pad,
-                              float* alpha, float* srow, void* stream) {
+extern "C" int ssp_desc_alpha(const float* mv_pad, const float* g3, const float* out4, int B, int Nc_pad, float* alpha,
+                              void* stream) {
   SSP_REQUIRE(mv_pad && g3 && out4 && alpha, "ssp_desc_alpha: null pointer");
   size_t n = (size_t)B * Nc_pad;
-  desc_alpha_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(mv_pad, g3, out4, n, alpha, srow);
+  desc_alpha_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(mv_pad, g3, out4, n, alpha);
   SSP_CUDA_CHECK_LAUNCH("desc_alpha_kernel");
   return SSP_OK;
 }
@@ -578,8 +573,9 @@ __global__ void __launch_bounds__(128) desc_pos_coef_kernel(const __grid_constan
   desc_pos_coef_block(A, blockIdx.x, blockIdx.y, blockIdx.z, gridDim.x);
 }
 
-// alpha_out / srow_out (optional, [B, Nc_pad]): the vectors ssp_desc_alpha would write for the same (scaled) gradients -- the
-// fused step gets them from this launch and skips that kernel.
+// alpha_out (optional, [B, Nc_pad]): the vector ssp_desc_alpha would write for the same (scaled) gradients -- the fused step
+// gets it from this launch and skips that kernel; srow_out (optional, [B, Nc_pad]): the same coefficient at mask_valid = 1,
+// the row scale of the folded backward (mask already inside the bits).
 // bitsC_out (optional, with Nc = the unpadded cell count): the column-orientation indicator words, transposed from bitsR by
 // extra blocks of the same launch (the tensor-core forward then needs no transpose kernel).
 extern "C" int ssp_desc_pos_coef(const int* rowcol, const float* rowdot, const int* colcnt, const int* colrow,
@@ -607,12 +603,12 @@ extern "C" int ssp_desc_pos_coef(const int* rowcol, const float* rowdot, const i
 __global__ void __launch_bounds__(256)
 desc_pos_apply_kernel(const int* __restrict__ rowcol, const float* __restrict__ rowcoef, const int* __restrict__ colrow,
                       const float* __restrict__ colcoef, const float* __restrict__ D, const float* __restrict__ Dw,
-                      int Dch, int Nc, int Nc_pad, int which, float* __restrict__ dD, float* __restrict__ dDw) {
+                      int Dch, int Nc, int Nc_pad, float* __restrict__ dD, float* __restrict__ dDw) {
   // block = 128 consecutive cells x 2 sub-groups of 16 channels: 512 contiguous bytes per channel row per block
   const int b = blockIdx.y;
   const int r = blockIdx.x * 128 + (threadIdx.x & 127), sub = threadIdx.x >> 7;
   const int nd32 = (Dch + 31) / 32;
-  const bool second = which == 2 || (which == 0 && (int)blockIdx.z >= nd32);
+  const bool second = (int)blockIdx.z >= nd32;
   const int d0 = ((int)blockIdx.z % nd32) * 32 + sub * 16;
   if (r >= Nc || d0 >= Dch) return;
   const int* list = (second ? colrow : rowcol) + ((size_t)b * Nc_pad + r) * DESC_MAXP;
@@ -637,15 +633,14 @@ desc_pos_apply_kernel(const int* __restrict__ rowcol, const float* __restrict__ 
   }
 }
 
-// which: 0 = both gradients, 1 = dD only, 2 = dDw only (lets the two halves run on different streams)
 extern "C" int ssp_desc_pos_apply(const int* rowcol, const float* rowcoef, const int* colrow, const float* colcoef,
-                                  const float* D, const float* Dw, int B, int Dch, int Nc, int which, float* dD,
-                                  float* dDw, void* stream) {
+                                  const float* D, const float* Dw, int B, int Dch, int Nc, float* dD, float* dDw,
+                                  void* stream) {
   SSP_REQUIRE(rowcol && rowcoef && colrow && colcoef && D && Dw && dD && dDw, "ssp_desc_pos_apply: null pointer");
-  SSP_REQUIRE(B > 0 && B <= 65535 && Dch > 0 && Nc > 0 && which >= 0 && which <= 2, "ssp_desc_pos_apply: bad sizes");
-  dim3 grid(ssp_ceil_div(Nc, 128), B, (which == 0 ? 2 : 1) * ssp_ceil_div(Dch, 32));
+  SSP_REQUIRE(B > 0 && B <= 65535 && Dch > 0 && Nc > 0, "ssp_desc_pos_apply: bad sizes");
+  dim3 grid(ssp_ceil_div(Nc, 128), B, 2 * ssp_ceil_div(Dch, 32));
   desc_pos_apply_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(rowcol, rowcoef, colrow, colcoef, D, Dw, Dch, Nc,
-                                                                desc_nc_pad(Nc), which, dD, dDw);
+                                                                desc_nc_pad(Nc), dD, dDw);
   SSP_CUDA_CHECK_LAUNCH("desc_pos_apply_kernel");
   return SSP_OK;
 }
@@ -743,22 +738,22 @@ desc_pack_geometry_kernel(const __grid_constant__ PackArgs P, const __grid_const
   }
 }
 
-// Packs one (src1 == NULL) or two tensors in one launch; `scale` applies to both.
-extern "C" int ssp_desc_pack2(const float* src0, const float* src1, const float* scale, int B, int Dch, int Nc, void* hi0,
-                              void* lo0, void* hi1, void* lo1, void* stream) {
-  SSP_REQUIRE(src0 && hi0 && (!src1 || hi1), "ssp_desc_pack: null pointer");
+// One tensor; `scale` (optional) multiplies its cells.
+extern "C" int ssp_desc_pack(const float* src, const float* scale, int B, int Dch, int Nc, void* hi, void* lo,
+                             void* stream) {
+  SSP_REQUIRE(src && hi, "ssp_desc_pack: null pointer");
   SSP_REQUIRE(B > 0 && B <= 65535 && Dch > 0 && Dch % 2 == 0 && Nc > 0, "ssp_desc_pack: bad sizes (Dch must be even)");
   int Nc_pad = desc_nc_pad(Nc);
   const int nchb = (Dch + PK_CH - 1) / PK_CH;
-  SSP_REQUIRE(2 * nchb <= 65535, "ssp_desc_pack: descriptor dim %d too large", Dch);
-  dim3 grid(Nc_pad / PK_CELLS, B, (src1 ? 2 : 1) * nchb);
-  PackArgs A = {src0, src1, scale, Dch, Nc, Nc_pad, (__nv_bfloat16*)hi0, (__nv_bfloat16*)lo0, (__nv_bfloat16*)hi1, (__nv_bfloat16*)lo1};
+  SSP_REQUIRE(nchb <= 65535, "ssp_desc_pack: descriptor dim %d too large", Dch);
+  dim3 grid(Nc_pad / PK_CELLS, B, nchb);
+  PackArgs A = {src, nullptr, scale, Dch, Nc, Nc_pad, (__nv_bfloat16*)hi, (__nv_bfloat16*)lo, nullptr, nullptr};
   desc_pack_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(A);
   SSP_CUDA_CHECK_LAUNCH("desc_pack_kernel");
   return SSP_OK;
 }
 
-// ssp_desc_pack2 (both tensors, no scale) and ssp_desc_geometry as ONE launch (arguments = those two calls')
+// two ssp_desc_pack calls (no scale) and ssp_desc_geometry as ONE launch (arguments = those calls')
 extern "C" int ssp_desc_pack2_geometry(const float* src0, const float* src1, int B, int Dch, int Hc, int Wc, void* hi0, void* lo0,
                                        void* hi1, void* lo1, const float* Hm, const float* mask_valid, const float* mask2d,
                                        int cell, float* wpts, float* mv_pad, double* mv_part, uint32_t* mvbits, void* stream) {
@@ -775,9 +770,4 @@ extern "C" int ssp_desc_pack2_geometry(const float* src0, const float* src1, int
   desc_pack_geometry_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(P, G, npack, Nc_pad / GEOM_THREADS);
   SSP_CUDA_CHECK_LAUNCH("desc_pack_geometry_kernel");
   return SSP_OK;
-}
-
-extern "C" int ssp_desc_pack(const float* src, const float* scale, int B, int Dch, int Nc, void* hi, void* lo,
-                             void* stream) {
-  return ssp_desc_pack2(src, nullptr, scale, B, Dch, Nc, hi, lo, nullptr, nullptr, stream);
 }

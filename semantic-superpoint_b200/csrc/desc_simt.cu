@@ -112,9 +112,8 @@ extern "C" int ssp_desc_dense_fwd_simt(const float* D, const float* Dw, const fl
 // ----------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 desc_bits_gemm_simt_kernel(const uint32_t* __restrict__ bits, const float* __restrict__ src,
-                           const float* __restrict__ colscale, const float* __restrict__ rowscale,
-                           const int* __restrict__ plist, const float* __restrict__ pcoef,
-                           const float* __restrict__ possrc, int Dch, int Nc, int Nc_pad, float* __restrict__ out) {
+                           const float* __restrict__ colscale, const float* __restrict__ rowscale, int Dch, int Nc,
+                           int Nc_pad, float* __restrict__ out) {
   __shared__ float sv[256][33];
   __shared__ uint32_t wb[32];
   int b = blockIdx.y, r0 = blockIdx.x * 32, d0 = blockIdx.z * 256;
@@ -154,34 +153,20 @@ desc_bits_gemm_simt_kernel(const uint32_t* __restrict__ bits, const float* __res
   int r = r0 + lane;
   if (r < Nc) {
     float rs = rowscale ? rowscale[(size_t)b * Nc_pad + r] : 1.f;
-    // sparse positive pairs of this row (and removal of their negative term), see desc_pos_coef_kernel
-    int npos = 0;
-    if (plist) {
-      for (int n = 0; n < DESC_MAXP; ++n)
-        if (plist[((size_t)b * Nc_pad + r) * DESC_MAXP + n] >= 0) npos = n + 1;
-    }
     for (int dd = w; dd < 256; dd += 8) {
       int d = d0 + dd;
-      if (d >= Dch) continue;
-      float v = sv[dd][lane] * rs;
-      for (int n = 0; n < npos; ++n) {
-        int pc = plist[((size_t)b * Nc_pad + r) * DESC_MAXP + n];
-        if (pc >= 0) v = fmaf(pcoef[((size_t)b * Nc_pad + r) * DESC_MAXP + n], __ldg(possrc + ((size_t)b * Dch + d) * Nc + pc), v);
-      }
-      out[((size_t)b * Dch + d) * Nc + r] = v;
+      if (d < Dch) out[((size_t)b * Dch + d) * Nc + r] = sv[dd][lane] * rs;
     }
   }
 }
 
 extern "C" int ssp_desc_bits_gemm_simt(const uint32_t* bits, const float* src, const float* colscale,
-                                       const float* rowscale, const int* plist, const float* pcoef,
-                                       const float* possrc, int B, int Dch, int Nc, float* out, void* stream) {
+                                       const float* rowscale, int B, int Dch, int Nc, float* out, void* stream) {
   SSP_REQUIRE(bits && src && out, "ssp_desc_bits_gemm_simt: null pointer");
-  SSP_REQUIRE(!plist || (pcoef && possrc), "ssp_desc_bits_gemm_simt: plist needs pcoef and possrc");
   SSP_REQUIRE(B > 0 && B <= 65535 && Dch > 0 && Nc > 0, "ssp_desc_bits_gemm_simt: bad sizes");
   int Nc_pad = desc_nc_pad(Nc);
   dim3 grid(Nc_pad / 32, B, ssp_ceil_div(Dch, 256));
-  desc_bits_gemm_simt_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(bits, src, colscale, rowscale, plist, pcoef, possrc, Dch, Nc, Nc_pad, out);
+  desc_bits_gemm_simt_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(bits, src, colscale, rowscale, Dch, Nc, Nc_pad, out);
   SSP_CUDA_CHECK_LAUNCH("desc_bits_gemm_simt_kernel");
   return SSP_OK;
 }

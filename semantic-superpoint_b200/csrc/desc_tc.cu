@@ -20,9 +20,10 @@
 //   warps 0-7   epilogue: tcgen05.ld 32x32b, hinge, mask_valid weighting (packed fp32x2 math), running sums and the
 //               row-orientation indicator words (sign bits funnel-shifted into place).  No geometry here: the sparse
 //               positive pairs are corrected by the pos kernels.  The pair matrix never reaches HBM.
-//   The column-orientation indicator words are produced from the row-orientation ones by a bit-matrix transpose kernel.
+//   The column-orientation indicator words are transposed from the row-orientation ones by blocks of the backward's
+//   coefficient launch (desc_pos_coef.cuh).
 //
-// Backward kernel = indicator GEMM  out[b, d, r] = rowscale[r] * sum_k bit(r,k) * Bp[b, k, d] for up to two independent
+// Backward kernel = indicator GEMM  out[b, d, r] = rowscale[r] * sum_k bit(r,k) * Bp[b, k, d] for the two independent
 // jobs (dD and dDw) in one launch, work item = (pair, job, 256-row tile, channel half):
 //   warps 0-7   expand 64 indicator bits per row into bf16 {0, 2} (one shift + one and per register; the bit order of
 //               the words is chosen for that, DESC_BITPOS) and tcgen05.st them as the A operand into TMEM; warps 0-3 take
@@ -376,36 +377,6 @@ desc_dense_fwd_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
 }
 
 // ------------------------------------------------------------------------------------------------
-// bitsC from bitsR: transpose of the indicator bit matrix (both in DESC_BITPOS order).
-//   bitsR[b][cw][r]: bit DESC_BITPOS(j) = indicator(row r, column 32 cw + j)
-//   bitsC[b][rw][c]: bit DESC_BITPOS(i) = indicator(row 32 rw + i, column c)
-// One warp per 32 x 32 tile: lane L holds the word of row 32 rw + inv(L) (inv = inverse of DESC_BITPOS), the tile is
-// transposed in five shuffle / mask stages (block-swap recursion), and lane L then holds the word of column 32 cw + inv(L).
-// ------------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256)
-desc_bits_transpose_kernel(const uint32_t* __restrict__ bitsR, uint32_t* __restrict__ bitsC, int NW, int NWv, int Nc_pad) {
-  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-  const int rw = blockIdx.x, b = blockIdx.y;
-  const int rl = ((lane & 15) << 1) | (lane >> 4);
-  // a warp walks the column words cw = warp, warp + 8, ... four at a time: the four loads are in flight together
-  for (int cw0 = warp; cw0 < NW; cw0 += 32) {
-    uint32_t w[4];
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const int cw = cw0 + 8 * u;
-      // words beyond the valid range were never written by the forward: they transpose to zero
-      w[u] = (cw < NWv && rw < NWv) ? __ldg(bitsR + ((size_t)b * NW + cw) * Nc_pad + rw * 32 + rl) : 0u;
-    }
-#pragma unroll
-    for (int u = 0; u < 4; ++u) {
-      const int cw = cw0 + 8 * u;
-      if (cw >= NW) break;
-      bitsC[((size_t)b * NW + rw) * Nc_pad + cw * 32 + rl] = warp_transpose32(w[u], lane);
-    }
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
 // indicator GEMM (backward)
 // ------------------------------------------------------------------------------------------------
 constexpr int KT = 128;                      // cells (GEMM K) per stage: 8 K=16 steps per plane, i.e. up to 16 MMAs behind ONE pair
@@ -415,6 +386,7 @@ constexpr int BG_PLANE_BYTES = KT * 128;     // one [128 cells x 64 channels] bo
 constexpr int BG_N = 128;                    // channels per work item (half of the descriptor)
 constexpr int BG_THREADS = 576;              // warps 0-7 expanders (two sets), 8-15 epilogue, 16 TMA producer, 17 MMA issuer
 constexpr int BG_W_EPI = 8, BG_W_TMA = 16, BG_W_MMA = 17;
+constexpr int BG_JOBS = 2;                   // dD and dDw
 constexpr int BG_NS = 4;                     // ring depth: TMEM holds 2 x 128 accumulator columns + 4 x 64 columns of A
 constexpr int BG_ACOLS = KT / 2;             // TMEM columns of one A stage (two bf16 per column)
 
@@ -443,7 +415,7 @@ struct BgJob {
 template <int P>
 __global__ void __launch_bounds__(BG_THREADS, 1)
 desc_bits_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_constant__ CUtensorMap tm1, BgJob job0,
-                         BgJob job1, int njobs, int B, int Nc, int Nc_pad) {
+                         BgJob job1, int B, int Nc, int Nc_pad) {
   using Cfg = BgCfg<P>;
   constexpr int NS = BG_NS;
   static_assert(256 + BG_ACOLS * NS <= 512, "TMEM A ring does not fit");
@@ -464,7 +436,7 @@ desc_bits_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_c
   const uint32_t cta_rank = tc::cluster_ctarank();
   const bool leader = cta_rank == 0;
   const int ncluster = gridDim.x >> 1, cid = blockIdx.x >> 1;
-  const int T = B * njobs * MP * 2;
+  const int T = B * BG_JOBS * MP * 2;
   constexpr uint32_t A_COL0 = 256;  // TMEM: accumulators at columns [0,128) and [128,256), then NS x 64 columns of A
 
   // item -> (b, job, mp, dh)
@@ -473,13 +445,13 @@ desc_bits_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_c
     int t = it >> 1;
     mp = t % MP;
     t /= MP;
-    jb = t % njobs;
-    b = t / njobs;
+    jb = t % BG_JOBS;
+    b = t / BG_JOBS;
   };
 
   if (warp == BG_W_TMA && lane == 0) {
     tc::prefetch_tmap(&tm0);
-    if (njobs > 1) tc::prefetch_tmap(&tm1);
+    tc::prefetch_tmap(&tm1);
   }
   if (warp == BG_W_MMA) {
     if (lane == 0) {
@@ -840,14 +812,13 @@ extern "C" int ssp_desc_dense_tc_nblocks(int B, int Nc) {
 
 // Ahi/Alo: packed planes of `descriptors`, Bhi/Blo: packed planes of `descriptors_warped` ([B, Nc_pad, 256] bf16).
 // Alo == Blo == NULL selects single-pass bf16; otherwise bf16x3.  bitsR (optional) receives the row-orientation indicator
-// words, bitsC (optional, needs bitsR) their transpose.  mvbits (optional, [B, Nc_pad/32] words of mask_valid != 0 in
+// words (their transpose bitsC comes from ssp_desc_pos_coef).  mvbits (optional, [B, Nc_pad/32] words of mask_valid != 0 in
 // DESC_BITPOS order, from ssp_desc_geometry): the indicator words drop the columns whose mask_valid is 0 ("fold").
 extern "C" int ssp_desc_dense_fwd_tc(const void* Ahi, const void* Alo, const void* Bhi, const void* Blo,
                                      const float* mv_pad, const uint32_t* mvbits, int B, int Hc, int Wc, float mneg,
-                                     double* partials, uint32_t* bitsR, uint32_t* bitsC, float* dbgS, void* stream) {
+                                     double* partials, uint32_t* bitsR, float* dbgS, void* stream) {
   SSP_REQUIRE(Ahi && Bhi && mv_pad && partials, "ssp_desc_dense_fwd_tc: null pointer");
   SSP_REQUIRE((Alo == nullptr) == (Blo == nullptr), "ssp_desc_dense_fwd_tc: lo planes must both be given or both null");
-  SSP_REQUIRE(!bitsC || bitsR, "ssp_desc_dense_fwd_tc: bitsC needs bitsR");
   SSP_REQUIRE(B > 0 && B <= 65535 && Hc > 0 && Wc > 0, "ssp_desc_dense_fwd_tc: bad sizes");
   SSP_REQUIRE(mneg > 0.f, "ssp_desc_dense_fwd_tc: margin_neg must be > 0 (zero padding relies on it)");
   SSP_REQUIRE((((uintptr_t)Ahi | (uintptr_t)Bhi | (uintptr_t)Alo | (uintptr_t)Blo | (uintptr_t)mv_pad) & 15) == 0,
@@ -878,74 +849,48 @@ extern "C" int ssp_desc_dense_fwd_tc(const void* Ahi, const void* Alo, const voi
   else     { if (bitsR) LAUNCH_FWD(1, true); else LAUNCH_FWD(1, false); }
 #undef LAUNCH_FWD
   SSP_CUDA_CHECK_LAUNCH("desc_dense_fwd_tc_kernel");
-  if (bitsC) {
-    const int NW = g.Nc_pad / 32, NWv = (g.Nc + 31) / 32;
-    dim3 tg(NW, B);
-    desc_bits_transpose_kernel<<<tg, 256, 0, st>>>(bitsR, bitsC, NW, NWv, g.Nc_pad);
-    SSP_CUDA_CHECK_LAUNCH("desc_bits_transpose_kernel");
-  }
   return SSP_OK;
 }
 
-// out[b, d, r] = rowscale[b, r] * sum_k bit(r, k) * (Bhi + Blo)[b, k, d]      (out is [B, 256, Nc] fp32)
-//                + sum_n pcoef[b, r, n] * (pos_hi + pos_lo)[b, plist[b, r, n], d]   (sparse positive pairs; plist may be NULL)
-struct BgHostJob {
-  const uint32_t* bits; const void* Bhi; const void* Blo; const float* rowscale; const int* plist; const float* pcoef;
-  const void* pos_hi; const void* pos_lo; float* out;
-};
-
-static int bits_gemm_tc_launch(const BgHostJob* jobs, int njobs, int B, int Nc, void* stream) {
-  SSP_REQUIRE(B > 0 && Nc > 0, "ssp_desc_bits_gemm_tc: bad sizes");
-  int Nc_pad = desc_nc_pad(Nc);
-  uint64_t rows = (uint64_t)B * Nc_pad;
-  CUtensorMap maps[2];
-  BgJob dj[2] = {};
-  int rc;
-  for (int j = 0; j < njobs; ++j) {
-    const BgHostJob& h = jobs[j];
-    SSP_REQUIRE(h.bits && h.Bhi && h.out, "ssp_desc_bits_gemm_tc: null pointer");
-    SSP_REQUIRE(!h.plist || (h.pcoef && h.pos_hi), "ssp_desc_bits_gemm_tc: plist needs pcoef and the partner planes");
-    SSP_REQUIRE((((uintptr_t)h.Bhi | (uintptr_t)h.Blo | (uintptr_t)h.pos_hi | (uintptr_t)h.pos_lo) & 15) == 0,
-                "ssp_desc_bits_gemm_tc: operands must be 16-byte aligned");
-    SSP_REQUIRE((h.Blo == nullptr) == (jobs[0].Blo == nullptr), "ssp_desc_bits_gemm_tc: both jobs must use the same engine (lo planes)");
-    if ((rc = make_planes_map3(&maps[j], h.Bhi, h.Blo, rows, KT))) return rc;
-    dj[j].bits = h.bits; dj[j].rowscale = h.rowscale; dj[j].plist = h.plist; dj[j].pcoef = h.pcoef;
-    dj[j].pos_hi = (const uint4*)h.pos_hi; dj[j].pos_lo = (const uint4*)h.pos_lo; dj[j].out = h.out;
-  }
-  if (njobs == 1) { maps[1] = maps[0]; dj[1] = dj[0]; }
-  long long items = (long long)B * njobs * (Nc_pad / (2 * BM)) * 2;
-  int nclusters = (int)std::min<long long>(items, std::max(1, ssp_num_sms() / 2));
-  int grid = 2 * nclusters;
-  cudaStream_t st = (cudaStream_t)stream;
-  if (jobs[0].Blo) {
-    if ((rc = set_smem(desc_bits_gemm_tc_kernel<2>, BgCfg<2>::SMEM))) return rc;
-    if ((rc = launch_cluster2(desc_bits_gemm_tc_kernel<2>, grid, BG_THREADS, BgCfg<2>::SMEM, st, maps[0], maps[1], dj[0], dj[1], njobs,
-                              B, Nc, Nc_pad))) return rc;
-  } else {
-    if ((rc = set_smem(desc_bits_gemm_tc_kernel<1>, BgCfg<1>::SMEM))) return rc;
-    if ((rc = launch_cluster2(desc_bits_gemm_tc_kernel<1>, grid, BG_THREADS, BgCfg<1>::SMEM, st, maps[0], maps[1], dj[0], dj[1], njobs,
-                              B, Nc, Nc_pad))) return rc;
-  }
-  SSP_CUDA_CHECK_LAUNCH("desc_bits_gemm_tc_kernel");
-  return SSP_OK;
-}
-
-// One indicator GEMM (pos_lo / Blo may be NULL: single-pass bf16 engine).
-extern "C" int ssp_desc_bits_gemm_tc_planes(const uint32_t* bits, const void* Bhi, const void* Blo, const float* rowscale,
-                                            const int* plist, const float* pcoef, const void* pos_hi, const void* pos_lo,
-                                            int B, int Nc, float* out, void* stream) {
-  BgHostJob j = {bits, Bhi, Blo, rowscale, plist, pcoef, pos_hi, pos_lo, out};
-  return bits_gemm_tc_launch(&j, 1, B, Nc, stream);
-}
-
-// Both indicator GEMMs of the backward (job 0: dD, job 1: dDw) in ONE launch: 2x the work items per launch, so the
-// persistent clusters end within one item of each other (4.3 items per cluster for one job at B = 32, 8.6 for two).
+// Both indicator GEMMs of the backward in ONE launch (job 0: dD, job 1: dDw; Blo / pos_lo NULL: single-pass bf16 engine):
+//   out[b, d, r] = rowscale[b, r] * sum_k bit(r, k) * (Bhi + Blo)[b, k, d]      (out is [B, 256, Nc] fp32)
+//                  + sum_n pcoef[b, r, n] * (pos_hi + pos_lo)[b, plist[b, r, n], d]   (sparse positive pairs; plist may be NULL)
+// Two jobs per launch give 2x the work items, so the persistent clusters end within one item of each other (4.3 items per
+// cluster for one job at B = 32, 8.6 for two).
 extern "C" int ssp_desc_bits_gemm_tc_pair(const uint32_t* bits0, const void* Bhi0, const void* Blo0, const float* rowscale0,
                                           const int* plist0, const float* pcoef0, const void* pos_hi0, const void* pos_lo0,
                                           float* out0, const uint32_t* bits1, const void* Bhi1, const void* Blo1,
                                           const float* rowscale1, const int* plist1, const float* pcoef1, const void* pos_hi1,
                                           const void* pos_lo1, float* out1, int B, int Nc, void* stream) {
-  BgHostJob j[2] = {{bits0, Bhi0, Blo0, rowscale0, plist0, pcoef0, pos_hi0, pos_lo0, out0},
-                    {bits1, Bhi1, Blo1, rowscale1, plist1, pcoef1, pos_hi1, pos_lo1, out1}};
-  return bits_gemm_tc_launch(j, 2, B, Nc, stream);
+  SSP_REQUIRE(B > 0 && Nc > 0, "ssp_desc_bits_gemm_tc_pair: bad sizes");
+  SSP_REQUIRE(bits0 && Bhi0 && out0 && bits1 && Bhi1 && out1, "ssp_desc_bits_gemm_tc_pair: null pointer");
+  SSP_REQUIRE((!plist0 || (pcoef0 && pos_hi0)) && (!plist1 || (pcoef1 && pos_hi1)),
+              "ssp_desc_bits_gemm_tc_pair: plist needs pcoef and the partner planes");
+  SSP_REQUIRE((((uintptr_t)Bhi0 | (uintptr_t)Blo0 | (uintptr_t)pos_hi0 | (uintptr_t)pos_lo0 | (uintptr_t)Bhi1 | (uintptr_t)Blo1 |
+                (uintptr_t)pos_hi1 | (uintptr_t)pos_lo1) & 15) == 0,
+              "ssp_desc_bits_gemm_tc_pair: operands must be 16-byte aligned");
+  SSP_REQUIRE((Blo0 == nullptr) == (Blo1 == nullptr), "ssp_desc_bits_gemm_tc_pair: both jobs must use the same engine (lo planes)");
+  const int Nc_pad = desc_nc_pad(Nc);
+  const uint64_t rows = (uint64_t)B * Nc_pad;
+  CUtensorMap m0, m1;
+  int rc;
+  if ((rc = make_planes_map3(&m0, Bhi0, Blo0, rows, KT))) return rc;
+  if ((rc = make_planes_map3(&m1, Bhi1, Blo1, rows, KT))) return rc;
+  const BgJob j0 = {bits0, rowscale0, plist0, pcoef0, (const uint4*)pos_hi0, (const uint4*)pos_lo0, out0};
+  const BgJob j1 = {bits1, rowscale1, plist1, pcoef1, (const uint4*)pos_hi1, (const uint4*)pos_lo1, out1};
+  long long items = (long long)B * BG_JOBS * (Nc_pad / (2 * BM)) * 2;
+  int nclusters = (int)std::min<long long>(items, std::max(1, ssp_num_sms() / 2));
+  int grid = 2 * nclusters;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (Blo0) {
+    if ((rc = set_smem(desc_bits_gemm_tc_kernel<2>, BgCfg<2>::SMEM))) return rc;
+    if ((rc = launch_cluster2(desc_bits_gemm_tc_kernel<2>, grid, BG_THREADS, BgCfg<2>::SMEM, st, m0, m1, j0, j1, B, Nc, Nc_pad)))
+      return rc;
+  } else {
+    if ((rc = set_smem(desc_bits_gemm_tc_kernel<1>, BgCfg<1>::SMEM))) return rc;
+    if ((rc = launch_cluster2(desc_bits_gemm_tc_kernel<1>, grid, BG_THREADS, BgCfg<1>::SMEM, st, m0, m1, j0, j1, B, Nc, Nc_pad)))
+      return rc;
+  }
+  SSP_CUDA_CHECK_LAUNCH("desc_bits_gemm_tc_kernel");
+  return SSP_OK;
 }

@@ -140,7 +140,6 @@ loss_exchange_kernel(XchgPeers peers, int rank, int world, float* __restrict__ d
   }
 }
 
-extern "C" size_t ssp_xchg_bytes(void) { return sizeof(XchgBuf); }
 extern "C" int ssp_xchg_max_ranks(void) { return XCHG_MAXR; }
 
 // The one allocation this library makes: IPC export needs a cudaMalloc'ed base pointer (a sub-block of a caching

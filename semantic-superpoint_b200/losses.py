@@ -326,7 +326,7 @@ def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist,
         # bitsC (the column-orientation indicator words) is only read by the backward GEMM: it is transposed from bitsR by
         # extra blocks of the backward's coefficient launch, not here
         call("ssp_desc_dense_fwd_tc", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(mv_pad), ptr(mvbits), B, Hc, Wc, _MNEG,
-             ptr(neg_part), ptr(bitsR), None, ptr(debug_S), s)
+             ptr(neg_part), ptr(bitsR), ptr(debug_S), s)
     else:
         # the HBM-bound exact positive-pair kernel overlaps the pack + tensor-core kernels
         if engine != "fp32":  # single-pass bf16: pack + geometry first (the positive-pair kernel needs the warped points)
@@ -339,7 +339,7 @@ def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist,
                  ptr(bitsR), ptr(bitsC), ptr(debug_S), s)
         else:
             call("ssp_desc_dense_fwd_tc", ptr(Ahi), None, ptr(Bhi), None, ptr(mv_pad), ptr(mvbits), B, Hc, Wc, _MNEG,
-                 ptr(neg_part), ptr(bitsR), None, ptr(debug_S), s)
+                 ptr(neg_part), ptr(bitsR), ptr(debug_S), s)
         fork.join()
     st = DescState((Dc, Dwc, mv_pad, bitsR, bitsC, lists_i, lists_f, Ahi, Alo, Bhi, Blo), out8, (B, Dch, Hc, Wc), lamda,
                    engine, fold)
@@ -379,7 +379,7 @@ def desc_backward(st, g3, gscale=1.0, gmode=0, det=None):
     alpha = torch.empty((B, Ncp), dtype=torch.float32, device=dev)
     srow = torch.empty((B, Ncp), dtype=torch.float32, device=dev) if fold else None
     if not fold:
-        call("ssp_desc_alpha", ptr(mv_pad), ptr(g3), ptr(out8), B, Ncp, ptr(alpha), None, s)
+        call("ssp_desc_alpha", ptr(mv_pad), ptr(g3), ptr(out8), B, Ncp, ptr(alpha), s)
     rowcol, colrow, colcnt = lists_i[0], lists_i[1], lists_i[2]
     rowdot, coldot = lists_f[0], lists_f[1]
     coefs = torch.empty((2,) + tuple(rowdot.shape), dtype=torch.float32, device=dev)
@@ -417,11 +417,11 @@ def desc_backward(st, g3, gscale=1.0, gmode=0, det=None):
                  ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted),
                  ptr(coefs[1]), None, None, ptr(bitsC) if tc_engine else None, Nc if tc_engine else 0, stream_of(Dc))
         if not tc_engine:
-            call("ssp_desc_bits_gemm_simt", ptr(bitsR), ptr(Dwc), ptr(alpha), None, None, None, None, B, Dch, Nc, ptr(dD), s)
-            call("ssp_desc_bits_gemm_simt", ptr(bitsC), ptr(Dc), None, ptr(alpha), None, None, None, B, Dch, Nc, ptr(dDw), s)
+            call("ssp_desc_bits_gemm_simt", ptr(bitsR), ptr(Dwc), ptr(alpha), None, B, Dch, Nc, ptr(dD), s)
+            call("ssp_desc_bits_gemm_simt", ptr(bitsC), ptr(Dc), None, ptr(alpha), B, Dch, Nc, ptr(dDw), s)
             f1.join()
             call("ssp_desc_pos_apply", ptr(rowcol), ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(Dc), ptr(Dwc), B, Dch,
-                 Nc, 0, ptr(dD), ptr(dDw), s)
+                 Nc, ptr(dD), ptr(dDw), s)
             return dD, dDw
         call("ssp_desc_pack", ptr(Dwc), ptr(alpha), B, Dch, Nc, ptr(Shi), ptr(Slo), s)
         f1.join()

@@ -4,6 +4,7 @@ import os
 import re
 import subprocess
 
+import pytest
 from conftest import ROOT
 
 
@@ -46,6 +47,37 @@ def test_header_argument_counts_match_ctypes():
     for name, args in re.findall(r"\b(ssp_[a-z0-9_]+)\s*\(([^)]*)\)\s*;", src):
         n = 0 if args.strip() in ("", "void") else len(args.split(","))
         assert n == len(_lib.SIGNATURES[name][1]), name
+
+
+# entry points of the SSP_TRACE build that only scripts/trace_desc.py calls (a profiling aid, not part of the package)
+_SCRIPT_ONLY = {"ssp_debug_trace", "ssp_debug_trace_cap"}
+
+
+def test_every_entry_point_has_a_caller():
+    """Every entry point of the ctypes table is called from the package (or __graft_entry__.py): the ABI carries no dead
+    surface that its readers would still have to keep consistent."""
+    from ssp_b200 import _lib
+    pkg = os.path.join(ROOT, "semantic-superpoint_b200")
+    texts = [open(os.path.join(ROOT, "__graft_entry__.py")).read()]
+    for f in sorted(os.listdir(pkg)):
+        if f.endswith(".py"):
+            text = open(os.path.join(pkg, f)).read()
+            if f == "_lib.py":  # the table itself is not a caller
+                text, n = re.subn(r"^SIGNATURES = \{.*?^\}$", "", text, flags=re.S | re.M)
+                assert n == 1
+            texts.append(text)
+    src = "\n".join(texts)
+    orphans = [n for n in _lib.SIGNATURES if n not in _SCRIPT_ONLY and not re.search(r"\b%s\b" % n, src)]
+    assert not orphans, orphans
+
+
+def test_python_call_checks_argument_count():
+    """ctypes ignores surplus arguments: _lib.call must refuse them (and missing ones) before anything runs."""
+    from ssp_b200 import _lib
+    with pytest.raises(TypeError, match="ssp_desc_alpha"):
+        _lib.call("ssp_desc_alpha", None, None, None, 1, 256, None, None, None)
+    with pytest.raises(TypeError, match="ssp_desc_alpha"):
+        _lib.call("ssp_desc_alpha", None, None, None, 1, 256, None)
 
 
 def test_argument_errors_without_gpu():

@@ -130,13 +130,19 @@ def test_shard_range_covers_everything():
 
 
 def test_orchestration_call_sequences(monkeypatch):
-    """The host side of the loss step with the C library faked out (every entry point recorded, nothing computed): the
-    Python orchestration -- buffer shapes, autograd plumbing, engine dispatch, fused / unfused / semantic / sparse variants,
-    partial gradients -- runs on a CPU-only box and issues the documented kernel sequence (DESIGN 4.3)."""
+    """The host side of the loss step with the C library faked out (every entry point recorded and its argument count
+    checked, nothing computed): the Python orchestration -- buffer shapes, autograd plumbing, engine dispatch, fused /
+    unfused / semantic / sparse variants, partial gradients -- runs on a CPU-only box and issues the documented kernel
+    sequence (DESIGN 4.3)."""
     from ssp_b200 import _lib, losses, sparse, step, utils
     calls = []
+
+    def fake_call(name, *args):
+        _lib.check_arity(name, args)  # every call site passes exactly the arguments its entry point declares
+        calls.append(name)
+
     for m in (_lib, losses, sparse, utils):
-        monkeypatch.setattr(m, "call", lambda name, *a: calls.append(name))
+        monkeypatch.setattr(m, "call", fake_call)
         monkeypatch.setattr(m, "stream_of", lambda t: None)
     monkeypatch.setattr(_lib, "require_cuda", lambda *t: None)
     monkeypatch.setattr(utils, "_cuda_device", lambda device, *t: torch.device("cpu"))
