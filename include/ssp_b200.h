@@ -251,6 +251,18 @@ int ssp_sparse_sample(const float* mat_H /*[B,3,3]*/, int B, int Hc, int Wc, int
 int ssp_sparse_finalize(const int* M /*[B] or NULL*/, int B, float* out3, const float* det0, const float* det1,
                         float lambda_loss, float* total /*or NULL*/, void* stream);
 
+/* ---- homography sampler (SURVEY 8f rank 4): sample_homography_np (utils/homographies.py:12-141) on the device, at the
+ * arguments of its call sites (datasets/Coco.py:261-277, :342-347): shape [2,2], shift -1, allow_artifacts, no translation
+ * overflow.  The distribution of the reference, not its RNG stream; one thread per homography, float64 arithmetic.
+ * flags: 1 perspective, 2 scaling, 4 rotation, 8 translation.  homographies [B,3,3] = the inverse of the sampled transform
+ * (the callers' convention, Coco.py:345), inv_homographies [B,3,3] = the inverse of that fp32 matrix; with group > 0 every
+ * index that is a multiple of group is the identity (Coco.py:271, one group per source image).  state [4] uint64 device:
+ * {seed, launch counter, 0, unused}; the launch reads the counter and advances it by one, as ssp_sparse_sample does, from
+ * disjoint Philox counters (one seed serves both samplers). ---- */
+int ssp_sample_homography(int B, int flags, int n_scales, int n_angles, double scaling_amplitude,
+                          double perspective_amplitude_x, double perspective_amplitude_y, double patch_ratio, double max_angle,
+                          int group, unsigned long long* state, float* homographies, float* inv_homographies, void* stream);
+
 /* ---- label warping of the warped training pair (SURVEY 8f rank 4): datasets/data_tools.py:37-63 warpLabels (+ :6-34
  * get_labels_bi), call sites datasets/Coco.py:330,367.  pnts [B,Pmax,2] (x, y) fp32, counts[b] valid points per image
  * (device), Hpix [B,3,3] = homography_scaling_torch(homography, H, W) (pixel coordinates, computed by the host like the

@@ -74,6 +74,7 @@ SIGNATURES = {
     "ssp_sparse_desc_loss_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _P, _P, _P]),
     "ssp_sparse_sample": (_I, [_P, _I, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_sparse_finalize": (_I, [_P, _I, _P, _P, _P, _F, _P, _P]),
+    "ssp_sample_homography": (_I, [_I, _I, _I, _I, _D, _D, _D, _D, _D, _I, _P, _P, _P, _P]),
     "ssp_warp_labels_ws_bytes": (_Z, [_I, _I, _I]),
     "ssp_warp_labels": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
     "ssp_debug_trace": (_I, [_P]),

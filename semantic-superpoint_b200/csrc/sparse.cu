@@ -12,6 +12,7 @@
 // apart), one warp per sampled pair for the dot products, a fixed-order per-image reduction, and for the backward a
 // warp-per-pair scatter (fp32 atomics into cell-major gradient buffers) followed by the transpose back.
 #include "common.cuh"
+#include "philox.cuh"
 #include <cub/block/block_radix_sort.cuh>
 
 // [B, Dch, Nc] <-> [B, Nc, Dch] through a 32 x 32 shared tile (both directions coalesced)
@@ -180,24 +181,8 @@ extern "C" int ssp_sparse_desc_loss_bwd(const float* Dt, const float* Dwt, const
 // Random numbers: Philox4x32-10, key = seed, counter = (item, image << 2 | purpose, launch counter).  The seed and the launch
 // counter live in the caller's state buffer; every block reads the counter, and the last block to finish advances it, so
 // consecutive launches (and graph replays) draw fresh lists with no host involvement.
+// The purpose tags here (the low two bits of the counter's second word) are 0, 1 and 2; 3 belongs to homography.cu.
 constexpr int SAMPLE_THREADS = 1024, SAMPLE_ITEMS = 8, SAMPLE_MAX_CELLS = SAMPLE_THREADS * SAMPLE_ITEMS;
-
-__device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const unsigned lo0 = 0xD2511F53u * c.x, hi0 = __umulhi(0xD2511F53u, c.x);
-    const unsigned lo1 = 0xCD9E8D57u * c.z, hi1 = __umulhi(0xCD9E8D57u, c.z);
-    c = make_uint4(hi1 ^ c.y ^ k.x, lo1, hi0 ^ c.w ^ k.y, lo0);
-    k.x += 0x9E3779B9u;
-    k.y += 0xBB67AE85u;
-  }
-  return c;
-}
-
-// uniform integer in [0, n) from 64 random bits (bias below n / 2^64)
-__device__ __forceinline__ int uniform_below(unsigned lo, unsigned hi, int n) {
-  return (int)__umul64hi(((unsigned long long)hi << 32) | lo, (unsigned long long)n);
-}
 
 __global__ void __launch_bounds__(SAMPLE_THREADS, 1)
 sparse_sample_kernel(const float* __restrict__ mat_H, int Hc, int Wc, int K, int nper, unsigned long long* state, int* ia,

@@ -23,6 +23,7 @@ from torch.autograd.function import once_differentiable
 from . import _lib
 from ._lib import call, f32c, ptr, stream_of
 from .losses import grad_vector
+from .rng import DeviceRng
 
 CHECK_EMPTY_IMAGES = False  # DeviceSampler.sample raises when an image had no candidate (costs a host sync per call)
 
@@ -75,25 +76,19 @@ def sample_correspondences(homography, Hc, Wc, num_matching_attempts=1000, num_m
     return matches_a, matches_b, non_a.long(), non_b.long()
 
 
-class DeviceSampler(object):
+class DeviceSampler(DeviceRng):
     """Correspondence lists of the sparse loss drawn on the device (ssp_sparse_sample, csrc/sparse.cu): per image, the cells
     whose warp lands in the image are the candidates; K matches are a random K-subset of them (or all of them plus draws
     with replacement when there are fewer than K), and every match gets n non-matches at uniform cells.
 
-    The random numbers are Philox4x32-10 keyed by (seed, image, launch counter).  The seed and the counter live in a device
-    buffer that every launch reads and advances, so eager calls and graph replays draw fresh lists without the host, and
-    get_state() / set_state() reproduce a sequence bit for bit.  An image whose homography maps no cell into the image turns
+    The random numbers are Philox4x32-10 keyed by (seed, image, launch counter), with the state handling of rng.DeviceRng:
+    eager calls and graph replays draw fresh lists without the host, and get_state() / set_state() reproduce a sequence bit
+    for bit.  An image whose homography maps no cell into the image turns
     the loss into NaN and counts in a device flag (empty_images(); CHECK_EMPTY_IMAGES raises on it).  Grids up to 8192
     cells (one block of 1024 threads x 8 cells per image: 30x40, 60x80 and KITTI's 47x155 fit); larger ones are an error."""
 
     def __init__(self, seed=0, device="cuda"):
-        self.device = torch.device(device)
-        if self.device.type != "cuda":
-            raise RuntimeError("DeviceSampler samples on a CUDA device, got %s" % self.device)
-        seed = int(seed) & 0xFFFFFFFFFFFFFFFF
-        seed = seed - (1 << 64) if seed >= (1 << 63) else seed
-        # {seed, launch counter, blocks done (0 between launches), images with M = 0 so far}, as uint64 bits
-        self.state = torch.tensor([seed, 0, 0, 0], dtype=torch.int64).to(self.device)
+        super().__init__(seed, device)  # state[3]: images with M = 0 so far
         self.last = None  # (ia, ib, M) of the last call
 
     def sample(self, mat_H, Hc, Wc, K=1000, n=10):
@@ -111,13 +106,6 @@ class DeviceSampler(object):
             self.state[3] = 0
             raise RuntimeError("DeviceSampler: the homography maps no cell into the image (%d images)" % n_empty)
         return ia, ib, M
-
-    def get_state(self):
-        """{seed, launch counter} as a device int64 tensor [2] (a copy)."""
-        return self.state[:2].clone()
-
-    def set_state(self, state):
-        self.state[:2].copy_(torch.as_tensor(state, dtype=torch.int64))
 
     def empty_images(self):
         """Images that had no candidate since the sampler was created (host sync)."""

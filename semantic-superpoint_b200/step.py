@@ -7,6 +7,7 @@ Both are free of host synchronisation except the final keypoint read-back of ada
 """
 import torch
 
+from . import _lib
 from . import utils as U
 
 
@@ -123,18 +124,27 @@ def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist
 
 
 @torch.no_grad()
-def collate_warped_pair(img, pnts_list, homographies, erosion_radius=3, bilinear=True):
+def collate_warped_pair(img, pnts_list, homographies=None, erosion_radius=3, bilinear=True, sampler=None,
+                        **homography_params):
     """The warped half of a training batch, built on the device from the unwarped images and their keypoints -- what
     datasets/Coco.py:341-392 does per sample in the DataLoader workers (inv_warp_image, warpLabels, compute_valid_mask):
     img [B,1,H,W], pnts_list = B arrays [P,2] (x, y), homographies [B,3,3] (normalised coordinates, already inverted as in
     Coco.py:345).  Returns the batch keys of the reference: warped_img, warped_labels, warped_res [B,2,H,W],
     warped_labels_bi, warped_valid_mask [B,1,H,W], homographies, inv_homographies.  (Photometric augmentation and the
-    gaussian label blur are imgaug calls and stay where they are.)"""
+    gaussian label blur are imgaug calls and stay where they are.)
+    sampler (a homography.HomographySampler) instead of homographies: the batch's homographies are drawn on the device with
+    homography_params (sample_homography_np's keywords, e.g. the config's warped_pair params) and inv_homographies comes
+    from the same kernel, with no host round trip."""
     dev = img.device
     B, _, H, W = img.shape
-    Hm = torch.as_tensor(homographies, dtype=torch.float32).reshape(B, 3, 3)
-    Hinv = torch.inverse(Hm.cpu()).to(dev)  # the reference inverts on the CPU (np.linalg.inv / torch.inverse per sample)
-    Hm = Hm.to(dev)
+    if (homographies is None) == (sampler is None):
+        raise ValueError("collate_warped_pair: pass either homographies or sampler")
+    if sampler is not None:
+        Hm, Hinv = sampler.sample(B, **homography_params)
+    else:
+        Hm = torch.as_tensor(homographies, dtype=torch.float32).reshape(B, 3, 3)
+        Hinv = torch.inverse(Hm.cpu()).to(dev)  # the reference inverts on the CPU (np.linalg.inv / torch.inverse per sample)
+        Hm = Hm.to(dev)
     warped_img = U.inv_warp_image_batch(img, Hinv, device=dev, mode="bilinear")
     lab = U.warp_labels_batch(pnts_list, H, W, Hm, bilinear=bilinear, device=dev)
     mask = U.compute_valid_mask(torch.tensor([H, W]), Hinv, device=dev, erosion_radius=erosion_radius).unsqueeze(1)
@@ -143,6 +153,31 @@ def collate_warped_pair(img, pnts_list, homographies, erosion_radius=3, bilinear
     if bilinear:
         out["warped_labels_bi"] = lab["labels_bi"]
     return out
+
+
+@torch.no_grad()
+def adaptation_views(img, sampler, num=100, erosion_radius=0, **homography_params):
+    """The homography-adaptation branch of the dataset (datasets/Coco.py:258-291) on the device, for I source images at
+    once: img [I,1,H,W], sampler a homography.HomographySampler, homography_params sample_homography_np's keywords (the
+    export config's homography_adaptation.homographies.params).  Draws I*num homographies, the first of every image the
+    identity, warps num bilinear views of each image by inv_homographies and builds their valid masks
+    (compute_valid_mask with erosion_radius, the config's valid_border_margin).  No host synchronisation.
+
+    Returns the sample keys of the reference: image [I,num,H,W], valid_mask [I,num,H,W], homographies [I,num,3,3],
+    inv_homographies [I,num,3,3].  export.py:284-287 swaps the two names when it reads a sample (the aggregation warps the
+    detections back with `homographies`), so the heads' logits semi [I,num,65,H/8,W/8] of out["image"] go to
+    adaptation_step(semi, out["homographies"], out["valid_mask"], binary_mask=True)."""
+    _lib.require_cuda(img)
+    I, C, H, W = img.shape
+    if C != 1:
+        raise ValueError("adaptation_views: img must be [I, 1, H, W], got %s" % (tuple(img.shape),))
+    num = int(num)
+    Hm, Hinv = sampler.sample(I * num, group=num, **homography_params)
+    views = img.expand(I, num, H, W).reshape(I * num, 1, H, W)  # img.repeat(N, 1, 1, 1) of Coco.py:280
+    image = U.inv_warp_image_batch(views, Hinv, device=img.device, mode="bilinear")
+    valid = U.compute_valid_mask(torch.tensor([H, W]), Hinv, device=img.device, erosion_radius=erosion_radius)
+    return {"image": image.reshape(I, num, H, W), "valid_mask": valid.reshape(I, num, H, W),
+            "homographies": Hm.reshape(I, num, 3, 3), "inv_homographies": Hinv.reshape(I, num, 3, 3)}
 
 
 class GraphedLossStep(object):
