@@ -91,10 +91,24 @@ int ssp_combine_heatmap_signed(const float* heat_signed /*[I,N,H,W]*/, const flo
  *      stencil: device (2R+1)^2 bytes, 1 = suppressed offset.  pts: [I,3,capacity] float64 rows x,y,conf,
  *      confidence-descending.  counts_host: HOST int[I]. ---- */
 size_t ssp_nms_ws_bytes(int I, int H, int W, int capacity);
+/* byte offset in ssp_nms_fast's workspace of its per-image keypoint counts (device unsigned int[I], valid after the call) */
+size_t ssp_nms_ws_counts_offset(int I, int H, int W);
 int ssp_nms_fast(const float* heat /*[I,H,W]*/, int I, int H, int W, float conf_thresh, int R, const uint8_t* stencil,
                  int border, int capacity, double* pts, int* counts_host, void* ws, size_t ws_bytes, void* stream);
 int ssp_box_nms(const float* prob /*[I,H,W]*/, int I, int H, int W, float min_prob, int R, const uint8_t* stencil,
                 float* out /*[I,H,W]*/, void* ws, size_t ws_bytes, void* stream);
+
+/* ---- sub-pixel keypoints (SURVEY 8a): SuperPointFrontend_torch.soft_argmax_points (models/model_wrap.py:212-248) with
+ *      extract_patch_from_points / norm_patches / do_log / soft_argmax_2d (utils/losses.py; torchgeometry 0.1.2
+ *      SpatialSoftArgmax2d, normalized_coordinates=False), the step the shipped COCO export config runs between NMS and
+ *      top-k (configs/magicpoint_coco_export.yaml:44-45, export.py:309-314).  pts: the [I,3,capacity] float64 layout of
+ *      ssp_nms_fast, refined in place; image i refines its first min(counts[i], limit, capacity) points.  counts: device
+ *      unsigned int[I], e.g. ssp_nms_fast's own (ssp_nms_ws_counts_offset), so no host round trip.  Per point,
+ *      (xi, yi) = (int)(x, y), patch = heat[yi - patch/2 + r, xi - patch/2 + c] (zero outside the image), q = patch /
+ *      (sum + 1e-6), q < 0 -> 1e-6, l = log q, e = exp(l - max l), s = 1 / (sum e + 1e-6), then in float64
+ *      x += sum((c * e) * s) - patch/2 and y += sum((r * e) * s) - patch/2; conf is unchanged.  1 <= patch <= 15. ---- */
+int ssp_soft_argmax_points(const float* heat /*[I,H,W]*/, int I, int H, int W, double* pts, int capacity,
+                           const unsigned int* counts, int limit, int patch, void* stream);
 
 /* ---- a5: descriptor_loss (utils/utils.py:779-893), forward and backward, split into stages.
  *      Nc = Hc*Wc, Nc_pad = ceil(Nc/256)*256.  wpts [B,Nc_pad,2], mv_pad [B,Nc_pad],

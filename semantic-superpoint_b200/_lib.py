@@ -39,7 +39,9 @@ SIGNATURES = {
     "ssp_combine_heatmap": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
     "ssp_combine_heatmap_signed": (_I, [_P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_nms_ws_bytes": (_Z, [_I, _I, _I, _I]),
+    "ssp_nms_ws_counts_offset": (_Z, [_I, _I, _I]),
     "ssp_nms_fast": (_I, [_P, _I, _I, _I, _F, _I, _P, _I, _I, _P, _P, _P, _Z, _P]),
+    "ssp_soft_argmax_points": (_I, [_P, _I, _I, _I, _P, _I, _P, _I, _I, _P]),
     "ssp_box_nms": (_I, [_P, _I, _I, _I, _F, _I, _P, _P, _P, _Z, _P]),
     "ssp_desc_geometry_nblocks": (_I, [_I, _I]),
     "ssp_desc_geometry": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),

@@ -422,6 +422,11 @@ extern "C" size_t ssp_nms_ws_bytes(int I, int H, int W, int capacity) {
   return state + ctr + lists + 256;
 }
 
+// workspace: state map (rounded to 256 B) | round counter (256 B) | per-image keypoint counts | candidate lists
+extern "C" size_t ssp_nms_ws_counts_offset(int I, int H, int W) {
+  return ((size_t)I * H * W + 255) / 256 * 256 + 256;
+}
+
 struct NmsWs {
   uint8_t* state;
   unsigned int* remaining;
@@ -435,9 +440,8 @@ static NmsWs nms_carve(void* ws, int I, int H, int W, int capacity) {
   size_t n = (size_t)I * H * W;
   char* p = (char*)ws;
   w.state = (uint8_t*)p;
-  p += (n + 255) / 256 * 256;
-  w.remaining = (unsigned int*)p;
-  p += 256;
+  w.remaining = (unsigned int*)(p + (n + 255) / 256 * 256);
+  p += ssp_nms_ws_counts_offset(I, H, W);
   w.count = (unsigned int*)p;
   p += (((size_t)I * 4 + 255) / 256) * 256;
   w.lval = (float*)p;

@@ -58,7 +58,7 @@ def install(utils_module=None, trainer_class=None, frontend_class=None, export_m
             sparse_module=None, data_tools_module=None):
     """Patch `utils.utils` (imported from sys.path unless given) and, when passed, the trainer class
     (`Train_model_heatmap_all`: detector_loss, getMasks, sem_loss), the inference front-end class
-    (`SuperPointFrontend_torch`: getPtsFromHeatmap, nms_fast, sample_desc_from_points), the tracker class
+    (`SuperPointFrontend_torch`: getPtsFromHeatmap, nms_fast, sample_desc_from_points, soft_argmax_points), the tracker class
     (`PointTracker`: nn_match_two_way), the `export` module (combine_heatmap), `utils.loss_functions.sparse_loss`
     (batch_descriptor_loss_sparse / descriptor_loss_sparse) and `datasets.data_tools` (warpLabels)."""
     bound = []
@@ -81,6 +81,13 @@ def install(utils_module=None, trainer_class=None, frontend_class=None, export_m
               lambda self, in_corners, H, W, dist_thresh: _u.nms_fast(in_corners, H, W, dist_thresh), bound)
         _bind(frontend_class, "sample_desc_from_points",
               lambda self, coarse_desc, pts: _u.sample_desc_from_points(coarse_desc, pts, self.cell), bound)
+
+        def _soft_argmax(self, pts, patch_size=5):
+            # the reference also keeps its log-patches in self.patches (debug only); that attribute is not produced
+            self.pts_subpixel = _u.soft_argmax_points(self.heatmap, pts, patch_size)
+            return self.pts_subpixel.copy()
+
+        _bind(frontend_class, "soft_argmax_points", _soft_argmax, bound)
     if tracker_class is not None:  # models/model_wrap.py PointTracker
 
         def _nn(self, desc1, desc2, nn_thresh):

@@ -2,7 +2,7 @@
 
 loss_step          = Train_model_heatmap_all.train_val_sample lines 295-365 (detector loss x2 + descriptor loss,
                      optionally the two semantic cross entropies of the SSp configuration)
-adaptation_step    = export.export_detector_homoAdapt_gpu lines 304-323 (flatten -> aggregate -> NMS -> top-k)
+adaptation_step    = export.export_detector_homoAdapt_gpu lines 304-323 (flatten -> aggregate -> NMS [-> sub-pixel] -> top-k)
 Both are free of host synchronisation except the final keypoint read-back of adaptation_step.
 """
 import torch
@@ -104,12 +104,16 @@ def _sparse_loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels
 
 
 @torch.no_grad()
-def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist=4, top_k=600, binary_mask=False):
+def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist=4, top_k=600, binary_mask=False,
+                    subpixel=False, patch_size=5):
     """semi [I,N,65,Hc,Wc] (or [N,65,Hc,Wc]), inv_homographies [I,N,3,3], mask_2D [I,N,H,W] -> list of [K,3] arrays
     (x, y, prob), K <= top_k, per source image.
     mask_2D is the stack of valid masks of the warped views; binary_mask=True promises a 0/1 mask (compute_valid_mask's output,
     what the export path always passes): the mask is folded into the flattened heatmap as its sign and the aggregation gathers
-    one array instead of two (bit-identical results; a non-binary mask then yields NaN heatmaps)."""
+    one array instead of two (bit-identical results; a non-binary mask then yields NaN heatmaps).
+    subpixel=True (the export config's model.subpixel.enable, export.py:309-314) refines x and y of the kept points by
+    utils.soft_argmax_points on the aggregated heatmap with patch_size, on the device before the read-back; count, order
+    and prob are those of subpixel=False."""
     if semi.dim() == 4:
         semi, inv_homographies = semi.unsqueeze(0), inv_homographies.reshape(1, -1, 3, 3)
         mask_2D = mask_2D.reshape(1, semi.shape[1], mask_2D.shape[-2], mask_2D.shape[-1])
@@ -119,7 +123,7 @@ def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist
     else:
         heat = U.flattenDetection(semi.reshape(I * N, C, Hc, Wc)).reshape(I, N, Hc * 8, Wc * 8)
         agg = U.combine_heatmap_batch(heat, inv_homographies, mask_2D)
-    pts = U.heatmap_to_pts_batch(agg, conf_thresh, nms_dist, top_k=top_k)
+    pts = U.heatmap_to_pts_batch(agg, conf_thresh, nms_dist, top_k=top_k, subpixel=subpixel, patch_size=patch_size)
     return [p.transpose() for p in pts]
 
 

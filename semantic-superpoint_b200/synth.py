@@ -105,3 +105,12 @@ def sample_homography(rng, shift=-1, perspective=True, scaling=True, rotation=Tr
     h = np.linalg.solve(np.array(A), np.array(bvec))
     Hm = np.append(h, 1.0).reshape(3, 3)
     return Hm  # pts1 -> pts2, as cv2.getPerspectiveTransform(pts1, pts2) (homographies.py:140); callers invert it
+
+
+def adaptation_workload(I0, N, Hc, Wc, seed=0):
+    """Host inputs of bench.py's homography-adaptation workload: logits semi [I0,N,65,Hc,Wc] (3 x pseudo-normal) and
+    homographies [I0,N,3,3] of N views per source image, the identity first (float32)."""
+    rng = np.random.default_rng(500 + seed)
+    Hs = np.stack([[np.linalg.inv(sample_homography(rng, max_angle=3.14 / 2)) for _ in range(N)] for _ in range(I0)])
+    Hs[:, 0] = np.eye(3)
+    return pseudo_normal((I0, N, 65, Hc, Wc), 7000 + seed) * 3, Hs.astype(np.float32)

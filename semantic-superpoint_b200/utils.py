@@ -18,8 +18,8 @@ from .losses import (DescriptorLossFn, DetectorLossFn, DetectorLossPairFn, LazyP
 __all__ = [
     "warp_points", "filter_points", "warp_points_filter", "warp_keypoints", "inv_warp_image_batch", "inv_warp_image",
     "compute_valid_mask", "ellipse_kernel", "labels2Dto3D", "getMasks", "detector_loss", "flattenDetection",
-    "combine_heatmap", "getPtsFromHeatmap", "nms_fast", "box_nms", "descriptor_loss", "normPts", "denormPts",
-    "homography_scaling_torch", "homography_scaling", "warpLabels", "warp_labels_batch",
+    "combine_heatmap", "getPtsFromHeatmap", "nms_fast", "box_nms", "soft_argmax_points", "descriptor_loss", "normPts",
+    "denormPts", "homography_scaling_torch", "homography_scaling", "warpLabels", "warp_labels_batch",
 ]
 
 _grid_cache = {}
@@ -425,10 +425,14 @@ def _nms_ws(I, H, W, capacity, dev):
     return torch.empty((nbytes,), dtype=torch.uint8, device=dev), nbytes
 
 
-def heatmap_to_pts_batch(heat, conf_thresh, nms_dist, border_remove=4, capacity=None, top_k=None):
+def heatmap_to_pts_batch(heat, conf_thresh, nms_dist, border_remove=4, capacity=None, top_k=None, subpixel=False,
+                         patch_size=5):
     """getPtsFromHeatmap for a stack [I,H,W] of CUDA heatmaps in one call.  Returns a list of [3,K] float64 arrays.
     top_k: only the top_k most confident points of every image are copied back (the list is confidence-descending, so this is
-    what the export's `pts[:top_k]` keeps, export.py:317-323)."""
+    what the export's `pts[:top_k]` keeps, export.py:317-323).
+    subpixel: x and y of the points that are copied back are refined by soft_argmax_points(heat, pts, patch_size) on the
+    device before the read-back (export.py:309-314); each point is refined on its own, so refining only the top_k is the
+    reference's refine-then-truncate."""
     dev = _cuda_device("cuda", heat)
     x = f32c(heat, dev)
     I, H, W = x.shape
@@ -442,6 +446,10 @@ def heatmap_to_pts_batch(heat, conf_thresh, nms_dist, border_remove=4, capacity=
          capacity, ptr(pts), counts, ptr(ws), nbytes, stream_of(x))
     cnt = [min(c, top_k) for c in counts] if top_k else list(counts)
     kmax = max(cnt) if I else 0
+    if subpixel and kmax:
+        # per-image counts straight from the NMS workspace: no copy, no sync
+        counts_dev = _lib._c.c_void_p(ws.data_ptr() + _lib.load().ssp_nms_ws_counts_offset(I, H, W))
+        call("ssp_soft_argmax_points", ptr(x), I, H, W, ptr(pts), capacity, counts_dev, kmax, int(patch_size), stream_of(x))
     host = pts[:, :, :kmax].cpu().numpy() if kmax else np.zeros((I, 3, 0))
     return [host[i, :, :cnt[i]] for i in range(I)]
 
@@ -462,6 +470,36 @@ def getPtsFromHeatmap(heatmap, conf_thresh, nms_dist):
     dev = _cuda_device("cuda", t)
     out = heatmap_to_pts_batch(t.to(dev).reshape(1, t.shape[-2], t.shape[-1]), conf_thresh, nms_dist)[0]
     return out if out.shape[1] else np.zeros((3, 0))
+
+
+def soft_argmax_points(heatmap, pts, patch_size=5):
+    """reference: models/model_wrap.py:212-248 (SuperPointFrontend_torch.soft_argmax_points(self, pts, patch_size=5), which
+    reads the heatmap from self.heatmap), with utils/losses.py's extract_patch_from_points, norm_patches, do_log and the
+    soft arg-max of torchgeometry's SpatialSoftArgmax2d(normalized_coordinates=False).
+
+    heatmap: torch (any device) or numpy, squeezed to [H,W].  pts: numpy float64 [3,K] (x, y, conf) or a one-element list of
+    it.  Returns a one-element list holding the refined [3,K] float64 array: x and y moved to the soft arg-max of the
+    patch_size x patch_size patch around (int(x), int(y)) (zeros outside the image), conf unchanged.  K = 0 -> [zeros((3,0))]
+    (the reference crashes in np.stack)."""
+    if isinstance(pts, (list, tuple)):
+        pts = pts[0]
+    p = np.ascontiguousarray(pts, dtype=np.float64)  # the kernel reads rows x, y of a row-major [3,K]
+    if p.ndim != 2 or p.shape[0] != 3:
+        raise RuntimeError("soft_argmax_points: pts must be [3, K] (x, y, conf), got %s" % (p.shape,))
+    K = p.shape[1]
+    if K == 0:
+        return [np.zeros((3, 0))]
+    if isinstance(heatmap, np.ndarray):
+        heatmap = torch.from_numpy(np.ascontiguousarray(heatmap, dtype=np.float32))
+    dev = _cuda_device("cuda", heatmap)
+    h = f32c(heatmap.detach().squeeze(), dev)
+    if h.dim() != 2:
+        raise RuntimeError("soft_argmax_points: heatmap must squeeze to [H, W], got %s" % (tuple(heatmap.shape),))
+    H, W = h.shape
+    pd = torch.from_numpy(p).to(dev)
+    counts = torch.tensor([K], dtype=torch.int32).to(dev)
+    call("ssp_soft_argmax_points", ptr(h), 1, H, W, ptr(pd), K, ptr(counts), K, int(patch_size), stream_of(pd))
+    return [pd.cpu().numpy()]
 
 
 def nms_fast(in_corners, H, W, dist_thresh):
