@@ -235,6 +235,22 @@ int ssp_sample_desc(const float* coarse, const double* pts, int K, int D, int Hc
                     void* stream);
 int ssp_nn_match(const float* desc1 /*[D,K1]*/, const float* desc2 /*[D,K2]*/, int D, int K1, int K2,
                  unsigned long long* best1 /*[K1]*/, unsigned long long* best2 /*[K2]*/, void* stream);
+/* Batched forms for the descriptor export of a batch of image pairs.
+ * ssp_sample_desc_batch: coarse [I,D,Hc,Wc], pts [I,3,capacity] float64 (ssp_nms_fast's layout), counts device unsigned[I]
+ *   (e.g. ssp_nms_fast's own, ssp_nms_ws_counts_offset).  Image i samples its first min(counts[i], limit) points into
+ *   desc [I,D,limit] with ssp_sample_desc's arithmetic (bit-identical results); its later columns are zeros.  limit <= capacity.
+ * ssp_nn_match_batch: P pairs on the tensor cores.  hi1/lo1 [P,R1,256], hi2/lo2 [P,R2,256] = ssp_desc_pack's bf16 planes of
+ *   [P,256,limit] fp32 descriptors (R = ceil(limit/256)*256, lo above hi), multiplied as hi*hi + lo*hi + hi*lo (fp32-grade
+ *   dots).  Pair p matches its first n1 = min(counts1[p], limit, R1) points against the first n2 = min(counts2[p], limit, R2):
+ *   dist, ties and the mutual test of ssp_nn_match / nn_match_two_way, dist < nn_thresh compared in fp32.  matches
+ *   [P,3,R1] float64 receives (index 1, index 2, dist) of pair p's nmatch[p] matches (device unsigned[P]) in increasing
+ *   index-1 order.  ws: ssp_nn_match_batch_ws_bytes(P, R1, R2) bytes, 8-byte aligned. */
+int ssp_sample_desc_batch(const float* coarse, const double* pts, int capacity, const unsigned int* counts, int limit,
+                          int I, int D, int Hc, int Wc, int cell, float* desc, void* stream);
+size_t ssp_nn_match_batch_ws_bytes(int P, int R1, int R2);
+int ssp_nn_match_batch(const void* hi1, const void* lo1, int R1, const void* hi2, const void* lo2, int R2,
+                       const unsigned int* counts1, const unsigned int* counts2, int limit, int P, float nn_thresh,
+                       double* matches, unsigned int* nmatch, void* ws, size_t ws_bytes, void* stream);
 
 /* ---- sparse descriptor loss (SURVEY 8f rank 2): utils/loss_functions/sparse_loss.py:65-284 with
  * pixelwise_contrastive_loss.py:140-265 (dist "cos", method "1d").  The reference samples K matches and Kn non-matches per

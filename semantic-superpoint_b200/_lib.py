@@ -71,6 +71,9 @@ SIGNATURES = {
     "ssp_sem_ce_up8_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P]),
     "ssp_sample_desc": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P]),
     "ssp_nn_match": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
+    "ssp_sample_desc_batch": (_I, [_P, _P, _I, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
+    "ssp_nn_match_batch_ws_bytes": (_Z, [_I, _I, _I]),
+    "ssp_nn_match_batch": (_I, [_P, _P, _I, _P, _P, _I, _P, _P, _I, _I, _F, _P, _P, _P, _Z, _P]),
     "ssp_transpose_batched": (_I, [_P, _I, _I, _I, _P, _P]),
     "ssp_sparse_desc_loss_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _P, _P, _P, _P]),
     "ssp_sparse_desc_loss_bwd": (_I, [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _P, _P, _P]),
@@ -128,7 +131,7 @@ def check(rc, what):
 # kernels launched per entry point (memsets / copies not counted); the NMS drivers launch init + >= 2 rounds +
 # compact + rank, counted at their minimum
 KERNELS_PER_CALL = {"ssp_nms_fast": 5, "ssp_box_nms": 4, "ssp_detector_loss_fwd": 2, "ssp_detector_loss_fwd_pair": 2,
-                    "ssp_sem_ce_fwd": 2, "ssp_sem_ce_up8": 2}
+                    "ssp_sem_ce_fwd": 2, "ssp_sem_ce_up8": 2, "ssp_nn_match_batch": 2}
 kernel_count = 0
 _prof = None
 

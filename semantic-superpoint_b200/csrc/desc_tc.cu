@@ -35,6 +35,7 @@
 //   warp 17     MMA issuer (leader), M=256 N=128 K=16, A from TMEM
 #include "desc_common.cuh"
 #include "tc_ptx.cuh"
+#include "tma_map.cuh"
 #include <algorithm>
 #include <cstdlib>
 
@@ -712,49 +713,6 @@ desc_bits_gemm_tc_kernel(const __grid_constant__ CUtensorMap tm0, const __grid_c
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_tiled() {
-  static EncodeTiledFn fn = nullptr;
-  if (!fn) {
-    void* p = nullptr;
-    cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-        qres == cudaDriverEntryPointSuccess)
-      fn = reinterpret_cast<EncodeTiledFn>(p);
-  }
-  return fn;
-}
-
-// hi (+ lo) planes [rows, 256] bf16 as ONE 3-D tensor {256 channels, rows, planes}: a [64 ch x box_rows x planes] box brings
-// the same cells of both planes with one TMA instruction.  The planes may live anywhere as long as lo is above hi and the
-// distance is a multiple of 16 bytes (the Python host allocates them back to back).
-int make_planes_map3(CUtensorMap* m, const void* hi, const void* lo, uint64_t rows, uint32_t box_rows) {
-  EncodeTiledFn enc = get_encode_tiled();
-  if (!enc) { ssp_set_error("cuTensorMapEncodeTiled unavailable (driver too old?)"); return SSP_EUNSUPPORTED; }
-  const uint64_t plane_bytes = rows * KD * 2;
-  uint64_t pstride = plane_bytes;
-  if (lo) {
-    if ((uintptr_t)lo <= (uintptr_t)hi || (((uintptr_t)lo - (uintptr_t)hi) & 15) || ((uintptr_t)lo - (uintptr_t)hi) < plane_bytes ||
-        ((uintptr_t)lo - (uintptr_t)hi) >= (1ull << 40)) {
-      ssp_set_error("tcgen05 descriptor kernels: the lo plane must lie above the hi plane (distance a multiple of 16 bytes)");
-      return SSP_EARG;
-    }
-    pstride = (uintptr_t)lo - (uintptr_t)hi;
-  }
-  cuuint64_t dims[3] = {(cuuint64_t)KD, (cuuint64_t)rows, (cuuint64_t)(lo ? 2 : 1)};
-  cuuint64_t strides[2] = {(cuuint64_t)KD * 2, (cuuint64_t)pstride};
-  cuuint32_t box[3] = {(cuuint32_t)KC, box_rows, (cuuint32_t)(lo ? 2 : 1)};
-  cuuint32_t estr[3] = {1, 1, 1};
-  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(hi), dims, strides, box, estr,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-  if (r != CUDA_SUCCESS) { ssp_set_error("cuTensorMapEncodeTiled (3-D planes) failed with CUresult %d", (int)r); return SSP_EARG; }
-  return SSP_OK;
-}
-
 // launch with thread-block clusters of 2 along x
 template <typename... KArgs, typename... Args>
 int launch_cluster2(void (*kernel)(KArgs...), int grid, int block, int smem, cudaStream_t st, Args... args) {

@@ -12,17 +12,28 @@
 #include "common.cuh"
 
 // ----------------------------------------------------------------------------------------------
-// descriptor sampling: block = one keypoint, thread = channel (strided)
+// descriptor sampling: block (k, i) = keypoint k of image i, thread = channel (strided).  Image i samples its first
+// n_i = min(counts[i], limit) points (counts NULL: all `limit`); its columns k >= n_i are written as zeros.
 // ----------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
-sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ pts, int K, int D, int Hc, int Wc,
-                   int cell, float* __restrict__ desc) {
+sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ pts, int capacity,
+                   const unsigned int* __restrict__ counts, int limit, int D, int Hc, int Wc, int cell,
+                   float* __restrict__ desc) {
   __shared__ float red[32];
-  const int k = blockIdx.x;
+  const int k = blockIdx.x, img = blockIdx.y;
+  const size_t plane = (size_t)Hc * Wc;
+  coarse += (size_t)img * D * plane;
+  pts += (size_t)img * 3 * capacity;
+  desc += (size_t)img * D * limit;
+  const unsigned int cnt = counts ? counts[img] : (unsigned int)limit;
+  if (k >= (int)min(cnt, (unsigned int)limit)) {
+    for (int c = threadIdx.x; c < D; c += blockDim.x) desc[(size_t)c * limit + k] = 0.f;
+    return;
+  }
   const double Wd = (double)(Wc * cell), Hd = (double)(Hc * cell);
-  // pts is the reference's [3,K] (x row, y row, conf row) float64 array
+  // pts is the reference's [3,K] (x row, y row, conf row) float64 array, rows `capacity` apart
   const float xn = (float)(pts[k] / (Wd / 2.0) - 1.0);
-  const float yn = (float)(pts[(size_t)K + k] / (Hd / 2.0) - 1.0);
+  const float yn = (float)(pts[(size_t)capacity + k] / (Hd / 2.0) - 1.0);
   const float ix = ((xn + 1.f) / 2.f) * (float)(Wc - 1);
   const float iy = ((yn + 1.f) / 2.f) * (float)(Hc - 1);
   const float fx = floorf(ix), fy = floorf(iy);
@@ -30,7 +41,6 @@ sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ 
   const int x0 = any ? (int)fx : 0, y0 = any ? (int)fy : 0, x1 = x0 + 1, y1 = y0 + 1;
   const float wx1 = ix - fx, wx0 = (fx + 1.f) - ix, wy1 = iy - fy, wy0 = (fy + 1.f) - iy;
   const bool xin0 = any && x0 >= 0, xin1 = any && x1 < Wc, yin0 = any && y0 >= 0, yin1 = any && y1 < Hc;
-  const size_t plane = (size_t)Hc * Wc;
   float ss = 0.f;
   for (int c = threadIdx.x; c < D; c += blockDim.x) {
     const float* p = coarse + (size_t)c * plane;
@@ -39,7 +49,7 @@ sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ 
     if (yin0 && xin1) v += __ldg(p + (size_t)y0 * Wc + x1) * (wx1 * wy0);
     if (yin1 && xin0) v += __ldg(p + (size_t)y1 * Wc + x0) * (wx0 * wy1);
     if (yin1 && xin1) v += __ldg(p + (size_t)y1 * Wc + x1) * (wx1 * wy1);
-    desc[(size_t)c * K + k] = v;
+    desc[(size_t)c * limit + k] = v;
     ss = fmaf(v, v, ss);
   }
   ss = warp_sum(ss);
@@ -49,7 +59,7 @@ sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ 
   for (int w = 0; w < (int)(blockDim.x + 31) / 32; ++w) tot += red[w];
   const float nrm = sqrtf(tot);
   for (int c = threadIdx.x; c < D; c += blockDim.x) {  // each thread rescales the values it wrote
-    float* o = desc + (size_t)c * K + k;
+    float* o = desc + (size_t)c * limit + k;
     *o = *o / nrm;  // 0/0 = NaN for a point sampled entirely outside, like the reference
   }
 }
@@ -58,7 +68,18 @@ extern "C" int ssp_sample_desc(const float* coarse, const double* pts, int K, in
                                float* desc, void* stream) {
   SSP_REQUIRE(coarse && pts && desc, "ssp_sample_desc: null pointer");
   SSP_REQUIRE(K > 0 && D > 0 && Hc > 0 && Wc > 0 && cell > 0, "ssp_sample_desc: bad sizes K=%d D=%d Hc=%d Wc=%d", K, D, Hc, Wc);
-  sample_desc_kernel<<<K, 256, 0, (cudaStream_t)stream>>>(coarse, pts, K, D, Hc, Wc, cell, desc);
+  sample_desc_kernel<<<dim3(K, 1), 256, 0, (cudaStream_t)stream>>>(coarse, pts, K, nullptr, K, D, Hc, Wc, cell, desc);
+  SSP_CUDA_CHECK_LAUNCH("sample_desc_kernel");
+  return SSP_OK;
+}
+
+extern "C" int ssp_sample_desc_batch(const float* coarse, const double* pts, int capacity, const unsigned int* counts,
+                                     int limit, int I, int D, int Hc, int Wc, int cell, float* desc, void* stream) {
+  SSP_REQUIRE(coarse && pts && counts && desc, "ssp_sample_desc_batch: null pointer");
+  SSP_REQUIRE(I > 0 && I <= 65535 && D > 0 && Hc > 0 && Wc > 0 && cell > 0 && limit > 0 && capacity >= limit,
+              "ssp_sample_desc_batch: bad sizes I=%d D=%d Hc=%d Wc=%d limit=%d capacity=%d", I, D, Hc, Wc, limit, capacity);
+  sample_desc_kernel<<<dim3(limit, I), 256, 0, (cudaStream_t)stream>>>(coarse, pts, capacity, counts, limit, D, Hc, Wc,
+                                                                      cell, desc);
   SSP_CUDA_CHECK_LAUNCH("sample_desc_kernel");
   return SSP_OK;
 }

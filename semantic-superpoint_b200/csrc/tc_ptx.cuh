@@ -57,6 +57,15 @@ __device__ __forceinline__ void tma_load_2d(const CUtensorMap* m, uint64_t* bar,
       : "memory");
 }
 
+// 3-D tiled load global -> shared (this CTA), completes `bytes` on the mbarrier
+__device__ __forceinline__ void tma_load_3d(const CUtensorMap* m, uint64_t* bar, void* dst, int x, int y, int z) {
+  asm volatile(
+      "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];" ::"r"(
+          smem_u32(dst)),
+      "l"(m), "r"(smem_u32(bar)), "r"(x), "r"(y), "r"(z)
+      : "memory");
+}
+
 // same, delivered to the same smem / mbarrier offsets of every CTA in `cta_mask` of the cluster (L2 read once)
 __device__ __forceinline__ void tma_load_2d_mc(const CUtensorMap* m, uint64_t* bar, void* dst, int x, int y, uint16_t cta_mask) {
   asm volatile(

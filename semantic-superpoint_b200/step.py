@@ -1,14 +1,18 @@
-"""The two hot loops of the reference, expressed over the kernels (no backbone: heads' outputs come in).
+"""The hot loops of the reference, expressed over the kernels (no backbone: heads' outputs come in).
 
 loss_step          = Train_model_heatmap_all.train_val_sample lines 295-365 (detector loss x2 + descriptor loss,
                      optionally the two semantic cross entropies of the SSp configuration)
 adaptation_step    = export.export_detector_homoAdapt_gpu lines 304-323 (flatten -> aggregate -> NMS [-> sub-pixel] -> top-k)
-Both are free of host synchronisation except the final keypoint read-back of adaptation_step.
+match_step         = export.export_descriptor lines 66-189 for a batch of image pairs (flatten -> NMS -> descriptors -> matches)
+The first two are free of host synchronisation except the final keypoint read-back of adaptation_step; match_step
+synchronises twice (NMS counts, read-back).
 """
+import numpy as np
 import torch
 
 from . import _lib
 from . import utils as U
+from ._lib import call, ptr
 
 
 def loss_step(semi, semi_warp, desc, desc_warp, labels_2D, warped_labels, mask_2D, mask_warp_2D, mat_H,
@@ -125,6 +129,82 @@ def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist
         agg = U.combine_heatmap_batch(heat, inv_homographies, mask_2D)
     pts = U.heatmap_to_pts_batch(agg, conf_thresh, nms_dist, top_k=top_k, subpixel=subpixel, patch_size=patch_size)
     return [p.transpose() for p in pts]
+
+
+@torch.no_grad()
+def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, top_k=None, nn_thresh=0.7):
+    """The descriptor export of P image pairs (export.py:66-189, export_descriptor) as one call: keypoints, descriptors and
+    two-way matches of every pair.  semi, semi_warp [P,65,Hc,Wc] logits; desc, desc_warp [P,256,Hc,Wc] coarse descriptors
+    (the head's normalised output); CUDA tensors.  Returns P dicts with
+      pts, warped_pts      [3,K] float64 (x, y, conf), confidence-descending, K <= top_k (None: every NMS point)
+      desc, warped_desc    [256,K] float32
+      matches              [3,L] float64 (index in pts, index in warped_pts, distance), increasing index-1 order
+    equal, pair by pair, to getPtsFromHeatmap(flattenDetection(semi[p]), conf_thresh, nms_dist)[:, :top_k],
+    sample_desc_from_points(desc[p:p+1], pts), the same for the warped image, and nn_match_two_way(desc, warped_desc,
+    nn_thresh), the matching on the tensor cores (nn_match_two_way_batch).  Two host synchronisations: the NMS reads its
+    counts (which also size every later buffer) and the single read-back of all results."""
+    U._check_nn_thresh(nn_thresh)
+    P, C, Hc, Wc = semi.shape
+    if C != 65 or tuple(semi_warp.shape) != (P, C, Hc, Wc):
+        raise ValueError("match_step: semi and semi_warp must be [P,65,Hc,Wc], got %s and %s"
+                         % (tuple(semi.shape), tuple(semi_warp.shape)))
+    if desc.shape[1] != 256 or tuple(desc.shape) != (P, 256, Hc, Wc) or tuple(desc_warp.shape) != (P, 256, Hc, Wc):
+        raise ValueError("match_step: desc and desc_warp must be [P,256,Hc,Wc] (the tensor-core matcher takes 256-dimensional "
+                         "descriptors), got %s and %s" % (tuple(desc.shape), tuple(desc_warp.shape)))
+    _lib.require_cuda(semi, desc, semi_warp, desc_warp)
+    dev = semi.device
+    st = _lib.stream_of(semi)
+    H, W = Hc * 8, Wc * 8
+    # 1. both flattened heatmaps into the halves of one [2P,1,H,W] buffer
+    heat = torch.empty((2 * P, 1, H, W), dtype=torch.float32, device=dev)
+    for h, s in enumerate((semi, semi_warp)):
+        call("ssp_flatten_detection", ptr(_lib.f32c(s.detach(), dev)), P, Hc, Wc, ptr(heat[h * P:(h + 1) * P]), st)
+    # 2. one NMS over the 2P heatmaps (host sync 1: the counts)
+    pts, counts, counts_dev = U._nms_batch(heat.view(2 * P, H, W), conf_thresh, nms_dist)
+    cnt = [min(c, top_k) for c in counts] if top_k is not None else counts
+    kmax = max(cnt)
+    if kmax == 0:
+        empty = {"pts": np.zeros((3, 0)), "desc": np.zeros((256, 0)), "warped_pts": np.zeros((3, 0)),
+                 "warped_desc": np.zeros((256, 0)), "matches": np.zeros((3, 0))}
+        return [{k: v.copy() for k, v in empty.items()} for _ in range(P)]
+    R = (kmax + 255) // 256 * 256
+    # every result lands in one device buffer, read back with one copy
+    sizes = {"pts": 2 * P * 3 * kmax * 8, "desc": 2 * P * 256 * kmax * 4, "matches": P * 3 * R * 8, "nmatch": P * 4}
+    offs, total = {}, 0
+    for k, n in sizes.items():
+        offs[k] = total
+        total += (n + 255) // 256 * 256
+    stage = torch.empty((total,), dtype=torch.uint8, device=dev)
+    region = lambda k, dtype, shape: stage[offs[k]:offs[k] + sizes[k]].view(dtype).view(shape)
+    d_all = region("desc", torch.float32, (2 * P, 256, kmax))
+    matches = region("matches", torch.float64, (P, 3, R))
+    nmatch = region("nmatch", torch.int32, (P,))
+    # 3. descriptors at the first min(count, kmax) points of every image (zeros after them)
+    cap = pts.shape[2]
+    for h, d in enumerate((desc, desc_warp)):
+        call("ssp_sample_desc_batch", ptr(_lib.f32c(d.detach(), dev)), ptr(pts[h * P:]), cap, ptr(counts_dev[h * P:]), kmax,
+             P, 256, Hc, Wc, 8, ptr(d_all[h * P:]), st)
+    # 4. + 5. operand planes and the matcher
+    planes = U._pack_planes(d_all)
+    U._nn_match_planes(planes[:, :P], planes[:, P:], counts_dev[:P], counts_dev[P:], kmax, nn_thresh, matches, nmatch)
+    region("pts", torch.float64, (2 * P, 3, kmax)).copy_(pts[:, :, :kmax])
+    # 6. the read-back (host sync 2), into page-locked memory: a pageable copy of the descriptors runs at a fraction of the
+    # link's rate, and torch's pinned-memory cache reuses the block once the previous call's results are released
+    host = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
+    host.copy_(stage)
+    host = host.numpy()
+    view = lambda k, dtype, shape: host[offs[k]:offs[k] + sizes[k]].view(dtype).reshape(shape)
+    hp, hd = view("pts", np.float64, (2 * P, 3, kmax)), view("desc", np.float32, (2 * P, 256, kmax))
+    hm, hn = view("matches", np.float64, (P, 3, R)), view("nmatch", np.int32, (P,))
+    out = []
+    for p in range(P):
+        k1, k2 = cnt[p], cnt[P + p]
+        out.append({"pts": hp[p, :, :k1] if k1 else np.zeros((3, 0)),
+                    "desc": hd[p, :, :k1] if k1 else np.zeros((256, 0)),
+                    "warped_pts": hp[P + p, :, :k2] if k2 else np.zeros((3, 0)),
+                    "warped_desc": hd[P + p, :, :k2] if k2 else np.zeros((256, 0)),
+                    "matches": hm[p, :, :hn[p]] if hn[p] else np.zeros((3, 0))})
+    return out
 
 
 @torch.no_grad()

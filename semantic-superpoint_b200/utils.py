@@ -425,6 +425,23 @@ def _nms_ws(I, H, W, capacity, dev):
     return torch.empty((nbytes,), dtype=torch.uint8, device=dev), nbytes
 
 
+def _nms_batch(x, conf_thresh, nms_dist, border_remove=4, capacity=None):
+    """Device part of getPtsFromHeatmap for a stack x [I,H,W] of fp32 CUDA heatmaps: one ssp_nms_fast call, whose sync also
+    reads the per-image counts.  Returns (pts [I,3,capacity] float64 on the device, confidence-descending; host list of
+    the counts; the same counts on the device as an int32 [I] view of the NMS workspace)."""
+    I, H, W = x.shape
+    R = int(nms_dist)
+    if capacity is None:
+        capacity = (H // (R + 1) + 1) * (W // (R + 1) + 1)  # kept points are > R apart in Chebyshev distance
+    pts = torch.empty((I, 3, capacity), dtype=torch.float64, device=x.device)
+    counts = (_lib._c.c_int * I)()
+    ws, nbytes = _nms_ws(I, H, W, capacity, x.device)
+    call("ssp_nms_fast", ptr(x), I, H, W, float(conf_thresh), R, ptr(_cheb_stencil(R, x.device)), int(border_remove),
+         capacity, ptr(pts), counts, ptr(ws), nbytes, stream_of(x))
+    off = _lib.load().ssp_nms_ws_counts_offset(I, H, W)
+    return pts, list(counts), ws[off:off + 4 * I].view(torch.int32)
+
+
 def heatmap_to_pts_batch(heat, conf_thresh, nms_dist, border_remove=4, capacity=None, top_k=None, subpixel=False,
                          patch_size=5):
     """getPtsFromHeatmap for a stack [I,H,W] of CUDA heatmaps in one call.  Returns a list of [3,K] float64 arrays.
@@ -436,20 +453,13 @@ def heatmap_to_pts_batch(heat, conf_thresh, nms_dist, border_remove=4, capacity=
     dev = _cuda_device("cuda", heat)
     x = f32c(heat, dev)
     I, H, W = x.shape
-    R = int(nms_dist)
-    if capacity is None:
-        capacity = (H // (R + 1) + 1) * (W // (R + 1) + 1)  # kept points are > R apart in Chebyshev distance
-    pts = torch.empty((I, 3, capacity), dtype=torch.float64, device=dev)
-    counts = (_lib._c.c_int * I)()
-    ws, nbytes = _nms_ws(I, H, W, capacity, dev)
-    call("ssp_nms_fast", ptr(x), I, H, W, float(conf_thresh), R, ptr(_cheb_stencil(R, dev)), int(border_remove),
-         capacity, ptr(pts), counts, ptr(ws), nbytes, stream_of(x))
-    cnt = [min(c, top_k) for c in counts] if top_k else list(counts)
+    pts, counts, counts_dev = _nms_batch(x, conf_thresh, nms_dist, border_remove, capacity)
+    cnt = [min(c, top_k) for c in counts] if top_k else counts
     kmax = max(cnt) if I else 0
     if subpixel and kmax:
         # per-image counts straight from the NMS workspace: no copy, no sync
-        counts_dev = _lib._c.c_void_p(ws.data_ptr() + _lib.load().ssp_nms_ws_counts_offset(I, H, W))
-        call("ssp_soft_argmax_points", ptr(x), I, H, W, ptr(pts), capacity, counts_dev, kmax, int(patch_size), stream_of(x))
+        call("ssp_soft_argmax_points", ptr(x), I, H, W, ptr(pts), pts.shape[2], ptr(counts_dev), kmax, int(patch_size),
+             stream_of(x))
     host = pts[:, :, :kmax].cpu().numpy() if kmax else np.zeros((I, 3, 0))
     return [host[i, :, :cnt[i]] for i in range(I)]
 
@@ -645,6 +655,66 @@ def nn_match_two_way(desc1, desc2, nn_thresh):
     matches[1, :] = idx[keep]
     matches[2, :] = scores[keep]
     return matches
+
+
+def _pack_planes(desc):
+    """[I,256,K] fp32 CUDA descriptors -> the matcher's bf16 hi / lo planes [2,I,R,256] (R = ceil(K/256)*256, zero rows
+    past K) from one ssp_desc_pack launch; [0] is hi, [1] is lo (above hi in memory, as the tensor maps need)."""
+    I, D, K = desc.shape
+    R = (K + 255) // 256 * 256
+    planes = torch.empty((2, I, R, D), dtype=torch.bfloat16, device=desc.device)
+    call("ssp_desc_pack", ptr(desc), None, I, D, K, ptr(planes[0]), ptr(planes[1]), stream_of(desc))
+    return planes
+
+
+def _nn_match_planes(planes1, planes2, counts1, counts2, limit, nn_thresh, matches, nmatch):
+    """ssp_nn_match_batch on planes [2,P,R,256] from _pack_planes: pair p matches its first min(counts[p], limit) points of
+    each set.  matches [P,3,R1] float64 and nmatch [P] int32 are device outputs."""
+    P, R1, R2 = planes1.shape[1], planes1.shape[2], planes2.shape[2]
+    nbytes = _lib.load().ssp_nn_match_batch_ws_bytes(P, R1, R2)
+    ws = torch.empty((nbytes // 8,), dtype=torch.int64, device=planes1.device)
+    call("ssp_nn_match_batch", ptr(planes1[0]), ptr(planes1[1]), R1, ptr(planes2[0]), ptr(planes2[1]), R2, ptr(counts1),
+         ptr(counts2), int(limit), P, float(nn_thresh), ptr(matches), ptr(nmatch), ptr(ws), nbytes, stream_of(matches))
+
+
+def _check_nn_thresh(nn_thresh):
+    if not nn_thresh >= 0.0:
+        raise ValueError("'nn_thresh' should be non-negative")
+
+
+def nn_match_two_way_batch(desc1, desc2, nn_thresh, counts1=None, counts2=None):
+    """nn_match_two_way for P pairs at once, on the tensor cores.
+
+    desc1 [P,256,K1], desc2 [P,256,K2] unit descriptors (CUDA tensors); counts1 / counts2 (optional, length P: sequences or
+    integer tensors): pair p uses its first counts[p] columns (capped at K), the rest are ignored.  Returns P numpy float64
+    [3,L] arrays (index in 1, index in 2, distance) of the mutual nearest neighbours closer than nn_thresh, in increasing
+    index-1 order.  Products are fp32-grade (bf16 hi / lo split, three MMA passes); the threshold is compared in fp32."""
+    _check_nn_thresh(nn_thresh)
+    if desc1.dim() != 3 or desc2.dim() != 3 or desc1.shape[0] != desc2.shape[0]:
+        raise ValueError("nn_match_two_way_batch: expected desc1 [P,256,K1] and desc2 [P,256,K2]")
+    if desc1.shape[1] != 256 or desc2.shape[1] != 256:
+        raise ValueError("nn_match_two_way_batch: the tensor-core matcher takes 256-dimensional descriptors")
+    _lib.require_cuda(desc1, desc2)
+    P, K1, K2 = int(desc1.shape[0]), int(desc1.shape[2]), int(desc2.shape[2])
+    if P == 0 or K1 == 0 or K2 == 0:
+        return [np.zeros((3, 0)) for _ in range(P)]
+    dev = desc1.device
+
+    def cnt(c, K):
+        if c is None:
+            return torch.full((P,), K, dtype=torch.int32, device=dev)
+        c = torch.as_tensor(c).to(device=dev, dtype=torch.int32).reshape(-1)
+        if c.numel() != P:
+            raise ValueError("nn_match_two_way_batch: %d counts for %d pairs" % (c.numel(), P))
+        return c.clamp(min=0, max=K)
+
+    c1, c2 = cnt(counts1, K1), cnt(counts2, K2)
+    p1, p2 = _pack_planes(f32c(desc1.detach(), dev)), _pack_planes(f32c(desc2.detach(), dev))
+    matches = torch.empty((P, 3, p1.shape[2]), dtype=torch.float64, device=dev)
+    nmatch = torch.empty((P,), dtype=torch.int32, device=dev)
+    _nn_match_planes(p1, p2, c1, c2, max(K1, K2), nn_thresh, matches, nmatch)
+    m, n = matches.cpu().numpy(), nmatch.cpu().numpy()
+    return [m[p, :, :n[p]] if n[p] else np.zeros((3, 0)) for p in range(P)]
 
 
 # ------------------------------------------------------------------------------------------------
