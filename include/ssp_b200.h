@@ -25,10 +25,9 @@ const char* ssp_last_error(void);
 
 /* ---- a1 / a10: warp_points (utils/utils.py:315-343), filter_points (:303-311),
  *      warp_keypoints / keep_true_keypoints (evaluations/detector_evaluation.py:139-191) ---- */
-int ssp_warp_points(const float* pts /*[P,2] x,y*/, int P, const float* H /*[B,3,3]*/, int B,
-                    float* out /*[B,P,2]*/, void* stream);
-int ssp_warp_points_mask(const float* pts, int P, const float* H, int B, float shape_x, float shape_y,
-                         float* out /*[B,P,2]*/, uint8_t* keep /*[B,P] 0<=p<=shape-1*/, void* stream);
+int ssp_warp_points_mask(const float* pts /*[P,2] x,y*/, int P, const float* H /*[B,3,3]*/, int B, float shape_x,
+                         float shape_y, float* out /*[B,P,2]*/, uint8_t* keep /*[B,P] 0<=p<=shape-1, or NULL*/,
+                         void* stream);
 int ssp_warp_keypoints_f64(const double* kp /*[K,2] x,y pixels*/, int K, const double* H /*[3,3]*/, double W,
                            double Hh, double* out /*[K,2]*/, uint8_t* keep /*[K] 0<=x<W,0<=y<H*/, void* stream);
 
@@ -54,11 +53,8 @@ int ssp_labels2d_to_3d(const float* labels /*[B,1,H,W]*/, int B, int H, int W, i
                        float* out /*[B,64|65,H/8,W/8]*/, void* stream);
 int ssp_cell_mask(const float* mask2d /*[B,1,H,W]*/, int B, int H, int W, float* out /*[B,H/8,W/8]*/, void* stream);
 size_t ssp_detector_loss_ws_bytes(int B, int Hc, int Wc);
-int ssp_detector_loss_fwd(const float* semi /*[B,65,Hc,Wc]*/, const float* target, const float* mask, int B, int Hc,
-                          int Wc, int fused2d, float* out3, void* ws, size_t ws_bytes, void* stream);
-int ssp_detector_loss_bwd(const float* semi, const float* target, const float* mask, int B, int Hc, int Wc,
-                          int fused2d, const float* fwd_out3, const float* gout /*[1]*/, float* dsemi, void* stream);
-/* both losses of a training pair (image, warped image) in one launch; ws = 2 regions of ws_bytes rounded up to 16;
+/* one loss (semi1 == NULL: problem 1's pointers are ignored) or both losses of a training pair (image, warped image) in
+ * one launch; semi [B,65,Hc,Wc], gout [1]; ws = one region of ws_bytes rounded up to 16 per loss;
  * cellmask1 (optional, [B,Hc,Wc]) receives getMasks() of problem 1 as a by-product */
 int ssp_detector_loss_fwd_pair(const float* semi0, const float* target0, const float* mask0, const float* semi1,
                                const float* target1, const float* mask1, int B, int Hc, int Wc, int fused2d,
@@ -89,7 +85,7 @@ int ssp_combine_heatmap_signed(const float* heat_signed /*[I,N,H,W]*/, const flo
 
 /* ---- a8 / a9: getPtsFromHeatmap + nms_fast (utils/utils.py:581-609, 653-712), box_nms (:612-650).
  *      stencil: device (2R+1)^2 bytes, 1 = suppressed offset.  pts: [I,3,capacity] float64 rows x,y,conf,
- *      confidence-descending.  counts_host: HOST int[I]. ---- */
+ *      confidence-descending.  counts_host: HOST int[I].  0 <= R <= 48. ---- */
 size_t ssp_nms_ws_bytes(int I, int H, int W, int capacity);
 /* byte offset in ssp_nms_fast's workspace of its per-image keypoint counts (device unsigned int[I], valid after the call) */
 size_t ssp_nms_ws_counts_offset(int I, int H, int W);
@@ -225,20 +221,19 @@ int ssp_sem_ce_up8_bwd(const float* gsum, const float* out3, const float* gout, 
                        float* dlogits /*[B,C,Hc,Wc]*/, void* stream);
 
 /* ---- sparse descriptors: sampling at keypoints and two-way nearest-neighbour matching (SURVEY 8f rank 3) ---------
- * ssp_sample_desc replaces SuperPointFrontend_torch.sample_desc_from_points (models/model_wrap.py:295-313):
- *   coarse [D,Hc,Wc] fp32, pts = the reference's [3,K] float64 array (x row, y row, conf row; device memory),
- *   desc [D,K] fp32 = bilinear samples (grid_sample align_corners=True, zero padding), L2-normalised per point.
+ * ssp_sample_desc_batch replaces SuperPointFrontend_torch.sample_desc_from_points (models/model_wrap.py:295-313); with
+ *   I = 1 and capacity = limit = K: coarse [D,Hc,Wc] fp32, pts = the reference's [3,K] float64 array (x row, y row,
+ *   conf row; device memory), desc [D,K] fp32 = bilinear samples (grid_sample align_corners=True, zero padding),
+ *   L2-normalised per point.
  * ssp_nn_match replaces the K1 x K2 part of PointTracker.nn_match_two_way (models/model_wrap.py:451-494):
  *   best1[i] = (bits(min_j dist(i,j)) << 32 | argmin_j), best2[j] likewise over i, dist = sqrt(2 - 2 clip(d1_i . d2_j, -1, 1));
  *   ties go to the lowest index (np.argmin).  The threshold / mutual test on 2K numbers stays with the caller. */
-int ssp_sample_desc(const float* coarse, const double* pts, int K, int D, int Hc, int Wc, int cell, float* desc,
-                    void* stream);
 int ssp_nn_match(const float* desc1 /*[D,K1]*/, const float* desc2 /*[D,K2]*/, int D, int K1, int K2,
                  unsigned long long* best1 /*[K1]*/, unsigned long long* best2 /*[K2]*/, void* stream);
 /* Batched forms for the descriptor export of a batch of image pairs.
  * ssp_sample_desc_batch: coarse [I,D,Hc,Wc], pts [I,3,capacity] float64 (ssp_nms_fast's layout), counts device unsigned[I]
  *   (e.g. ssp_nms_fast's own, ssp_nms_ws_counts_offset).  Image i samples its first min(counts[i], limit) points into
- *   desc [I,D,limit] with ssp_sample_desc's arithmetic (bit-identical results); its later columns are zeros.  limit <= capacity.
+ *   desc [I,D,limit]; its later columns are zeros.  limit <= capacity.
  * ssp_nn_match_batch: P pairs on the tensor cores.  hi1/lo1 [P,R1,256], hi2/lo2 [P,R2,256] = ssp_desc_pack's bf16 planes of
  *   [P,256,limit] fp32 descriptors (R = ceil(limit/256)*256, lo above hi), multiplied as hi*hi + lo*hi + hi*lo (fp32-grade
  *   dots).  Pair p matches its first n1 = min(counts1[p], limit, R1) points against the first n2 = min(counts2[p], limit, R2):

@@ -22,7 +22,6 @@ _Z = _c.c_size_t
 SIGNATURES = {
     "ssp_version": (_I, []),
     "ssp_last_error": (_c.c_char_p, []),
-    "ssp_warp_points": (_I, [_P, _I, _P, _I, _P, _P]),
     "ssp_warp_points_mask": (_I, [_P, _I, _P, _I, _F, _F, _P, _P, _P]),
     "ssp_warp_keypoints_f64": (_I, [_P, _I, _P, _D, _D, _P, _P, _P]),
     "ssp_inv_warp_image": (_I, [_P, _I, _I, _I, _I, _P, _P, _P, _I, _P, _P]),
@@ -30,8 +29,6 @@ SIGNATURES = {
     "ssp_labels2d_to_3d": (_I, [_P, _I, _I, _I, _I, _P, _P]),
     "ssp_cell_mask": (_I, [_P, _I, _I, _I, _P, _P]),
     "ssp_detector_loss_ws_bytes": (_Z, [_I, _I, _I]),
-    "ssp_detector_loss_fwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _Z, _P]),
-    "ssp_detector_loss_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P]),
     "ssp_detector_loss_fwd_pair": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _Z, _P]),
     "ssp_detector_loss_bwd_pair": (_I, [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P, _P, _P]),
     "ssp_flatten_detection": (_I, [_P, _I, _I, _I, _P, _P]),
@@ -69,7 +66,6 @@ SIGNATURES = {
     "ssp_sem_ce_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _P]),
     "ssp_sem_ce_up8": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P, _P, _Z, _P]),
     "ssp_sem_ce_up8_bwd": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P]),
-    "ssp_sample_desc": (_I, [_P, _P, _I, _I, _I, _I, _I, _P, _P]),
     "ssp_nn_match": (_I, [_P, _P, _I, _I, _I, _P, _P, _P]),
     "ssp_sample_desc_batch": (_I, [_P, _P, _I, _P, _I, _I, _I, _I, _I, _I, _P, _P]),
     "ssp_nn_match_batch_ws_bytes": (_Z, [_I, _I, _I]),
@@ -130,8 +126,8 @@ def check(rc, what):
 
 # kernels launched per entry point (memsets / copies not counted); the NMS drivers launch init + >= 2 rounds +
 # compact + rank, counted at their minimum
-KERNELS_PER_CALL = {"ssp_nms_fast": 5, "ssp_box_nms": 4, "ssp_detector_loss_fwd": 2, "ssp_detector_loss_fwd_pair": 2,
-                    "ssp_sem_ce_fwd": 2, "ssp_sem_ce_up8": 2, "ssp_nn_match_batch": 2}
+KERNELS_PER_CALL = {"ssp_nms_fast": 5, "ssp_box_nms": 4, "ssp_detector_loss_fwd_pair": 2, "ssp_sem_ce_fwd": 2,
+                    "ssp_sem_ce_up8": 2, "ssp_nn_match_batch": 2}
 kernel_count = 0
 _prof = None
 

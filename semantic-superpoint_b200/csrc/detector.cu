@@ -407,13 +407,13 @@ extern "C" int ssp_detector_loss_fwd_pair(const float* semi0, const float* targe
                                           int Wc, int fused2d, float* out3_0, float* out3_1, float* cellmask1, void* ws,
                                           size_t ws_bytes, void* stream) {
   int rc;
-  if ((rc = det_check("ssp_detector_loss_fwd", semi0, target0, mask0, B, Hc, Wc, fused2d))) return rc;
+  if ((rc = det_check("ssp_detector_loss_fwd_pair", semi0, target0, mask0, B, Hc, Wc, fused2d))) return rc;
   int np = semi1 ? 2 : 1;
-  if (np == 2 && (rc = det_check("ssp_detector_loss_fwd", semi1, target1, mask1, B, Hc, Wc, fused2d))) return rc;
-  SSP_REQUIRE(out3_0 && ws && (np == 1 || out3_1), "ssp_detector_loss_fwd: null pointer");
+  if (np == 2 && (rc = det_check("ssp_detector_loss_fwd_pair", semi1, target1, mask1, B, Hc, Wc, fused2d))) return rc;
+  SSP_REQUIRE(out3_0 && ws && (np == 1 || out3_1), "ssp_detector_loss_fwd_pair: null pointer");
   size_t per = (ssp_detector_loss_ws_bytes(B, Hc, Wc) + 15) / 16 * 16;
-  SSP_REQUIRE(ws_bytes >= per * np, "ssp_detector_loss_fwd: workspace too small");
-  SSP_REQUIRE(((uintptr_t)ws & 15) == 0, "ssp_detector_loss_fwd: workspace must be 16-byte aligned");
+  SSP_REQUIRE(ws_bytes >= per * np, "ssp_detector_loss_fwd_pair: workspace too small");
+  SSP_REQUIRE(((uintptr_t)ws & 15) == 0, "ssp_detector_loss_fwd_pair: workspace must be 16-byte aligned");
   cudaStream_t st = (cudaStream_t)stream;
   DetProblems pb = {};
   for (int i = 0; i < np; ++i) {
@@ -437,21 +437,15 @@ extern "C" int ssp_detector_loss_fwd_pair(const float* semi0, const float* targe
   return SSP_OK;
 }
 
-extern "C" int ssp_detector_loss_fwd(const float* semi, const float* target, const float* mask, int B, int Hc,
-                                     int Wc, int fused2d, float* out3, void* ws, size_t ws_bytes, void* stream) {
-  return ssp_detector_loss_fwd_pair(semi, target, mask, nullptr, nullptr, nullptr, B, Hc, Wc, fused2d, out3, nullptr,
-                                    nullptr, ws, ws_bytes, stream);
-}
-
 extern "C" int ssp_detector_loss_bwd_pair(const float* semi0, const float* target0, const float* mask0,
                                           const float* semi1, const float* target1, const float* mask1, int B, int Hc,
                                           int Wc, int fused2d, const float* fwd0, const float* fwd1, const float* gout0,
                                           const float* gout1, float* dsemi0, float* dsemi1, void* stream) {
   int rc;
-  if ((rc = det_check("ssp_detector_loss_bwd", semi0, target0, mask0, B, Hc, Wc, fused2d))) return rc;
+  if ((rc = det_check("ssp_detector_loss_bwd_pair", semi0, target0, mask0, B, Hc, Wc, fused2d))) return rc;
   int np = semi1 ? 2 : 1;
-  if (np == 2 && (rc = det_check("ssp_detector_loss_bwd", semi1, target1, mask1, B, Hc, Wc, fused2d))) return rc;
-  SSP_REQUIRE(fwd0 && gout0 && dsemi0 && (np == 1 || (fwd1 && gout1 && dsemi1)), "ssp_detector_loss_bwd: null pointer");
+  if (np == 2 && (rc = det_check("ssp_detector_loss_bwd_pair", semi1, target1, mask1, B, Hc, Wc, fused2d))) return rc;
+  SSP_REQUIRE(fwd0 && gout0 && dsemi0 && (np == 1 || (fwd1 && gout1 && dsemi1)), "ssp_detector_loss_bwd_pair: null pointer");
   DetProblems pb = {};
   for (int i = 0; i < np; ++i) {
     pb.p[i].semi = i ? semi1 : semi0;
@@ -469,13 +463,6 @@ extern "C" int ssp_detector_loss_bwd_pair(const float* semi0, const float* targe
     detector_loss_bwd_kernel<0><<<grid, 128, 0, st>>>(pb, B, Hc, Wc);
   SSP_CUDA_CHECK_LAUNCH("detector_loss_bwd_kernel");
   return SSP_OK;
-}
-
-extern "C" int ssp_detector_loss_bwd(const float* semi, const float* target, const float* mask, int B, int Hc,
-                                     int Wc, int fused2d, const float* fwd_out3, const float* gout, float* dsemi,
-                                     void* stream) {
-  return ssp_detector_loss_bwd_pair(semi, target, mask, nullptr, nullptr, nullptr, B, Hc, Wc, fused2d, fwd_out3, nullptr, gout,
-                                    nullptr, dsemi, nullptr, stream);
 }
 
 // Fused-step backward prologue: ssp_detector_loss_bwd_pair (fused2d = 1, both images) and ssp_desc_pos_coef (with alpha / srow

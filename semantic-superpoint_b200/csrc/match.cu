@@ -13,7 +13,7 @@
 
 // ----------------------------------------------------------------------------------------------
 // descriptor sampling: block (k, i) = keypoint k of image i, thread = channel (strided).  Image i samples its first
-// n_i = min(counts[i], limit) points (counts NULL: all `limit`); its columns k >= n_i are written as zeros.
+// n_i = min(counts[i], limit) points; its columns k >= n_i are written as zeros.
 // ----------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ pts, int capacity,
@@ -25,8 +25,7 @@ sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ 
   coarse += (size_t)img * D * plane;
   pts += (size_t)img * 3 * capacity;
   desc += (size_t)img * D * limit;
-  const unsigned int cnt = counts ? counts[img] : (unsigned int)limit;
-  if (k >= (int)min(cnt, (unsigned int)limit)) {
+  if (k >= (int)min(counts[img], (unsigned int)limit)) {
     for (int c = threadIdx.x; c < D; c += blockDim.x) desc[(size_t)c * limit + k] = 0.f;
     return;
   }
@@ -62,15 +61,6 @@ sample_desc_kernel(const float* __restrict__ coarse, const double* __restrict__ 
     float* o = desc + (size_t)c * limit + k;
     *o = *o / nrm;  // 0/0 = NaN for a point sampled entirely outside, like the reference
   }
-}
-
-extern "C" int ssp_sample_desc(const float* coarse, const double* pts, int K, int D, int Hc, int Wc, int cell,
-                               float* desc, void* stream) {
-  SSP_REQUIRE(coarse && pts && desc, "ssp_sample_desc: null pointer");
-  SSP_REQUIRE(K > 0 && D > 0 && Hc > 0 && Wc > 0 && cell > 0, "ssp_sample_desc: bad sizes K=%d D=%d Hc=%d Wc=%d", K, D, Hc, Wc);
-  sample_desc_kernel<<<dim3(K, 1), 256, 0, (cudaStream_t)stream>>>(coarse, pts, K, nullptr, K, D, Hc, Wc, cell, desc);
-  SSP_CUDA_CHECK_LAUNCH("sample_desc_kernel");
-  return SSP_OK;
 }
 
 extern "C" int ssp_sample_desc_batch(const float* coarse, const double* pts, int capacity, const unsigned int* counts,

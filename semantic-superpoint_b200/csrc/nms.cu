@@ -116,108 +116,11 @@ nms_round_kernel(const float* __restrict__ heat, uint8_t* __restrict__ state, in
   if (left) atomicAdd(remaining, (unsigned int)left);
 }
 
-// Square-window rounds (nms_fast): the two questions of a round -- "is a kept point in my (2R+1)^2 window?" and
-// "am I the highest-priority undecided point of my window?" -- are a dilation and a max filter, both separable:
-// 2 x (2R+1) shared-memory reads per pixel instead of (2R+1)^2.  Priority is a unique 64-bit key
-// (order-preserving float bits << 32 | ~linear index), so "am I the max" is one compare.
+// Priority as one unique 64-bit key (order-preserving float bits << 32 | ~linear index): larger key = higher priority.
 __device__ __forceinline__ unsigned long long nms_key(float v, unsigned int idx) {
   unsigned int u = __float_as_uint(v);
   u = (u & 0x80000000u) ? ~u : (u | 0x80000000u);
   return ((unsigned long long)u << 32) | (unsigned long long)(0xFFFFFFFFu - idx);
-}
-
-__global__ void __launch_bounds__(256)
-nms_round_square_kernel(const float* __restrict__ heat, uint8_t* __restrict__ state, int H, int W, int R,
-                        unsigned int* __restrict__ remaining) {
-  extern __shared__ unsigned char smem_raw[];
-  const int TW = NT + 2 * R;
-  unsigned long long* key = reinterpret_cast<unsigned long long*>(smem_raw);  // TW*TW
-  unsigned long long* rm = key + TW * TW;                                     // TW*NT row maxima
-  float* sv = reinterpret_cast<float*>(rm + TW * NT);                         // TW*TW values
-  uint8_t* ss = reinterpret_cast<uint8_t*>(sv + TW * TW);                     // TW*TW states
-  uint8_t* rk = ss + TW * TW;                                                 // TW*NT row-dilated kept flags
-  __shared__ int any_undecided;
-  const int tid = threadIdx.x;
-  const size_t img = (size_t)blockIdx.z * H * W;
-  heat += img;
-  state += img;
-  const int ty0 = blockIdx.y * NT, tx0 = blockIdx.x * NT;
-  if (tid == 0) any_undecided = 0;
-  __syncthreads();
-  int found = 0;
-  for (int i = tid; i < NT * NT; i += 256) {
-    int y = ty0 + i / NT, x = tx0 + i % NT;
-    if (y < H && x < W && state[(size_t)y * W + x] == ST_UNDECIDED) found = 1;
-  }
-  if (found) any_undecided = 1;
-  __syncthreads();
-  if (!any_undecided) return;
-  for (int i = tid; i < TW * TW; i += 256) {
-    int y = ty0 - R + i / TW, x = tx0 - R + i % TW;
-    uint8_t st = ST_NONE;
-    float v = 0.f;
-    if (y >= 0 && y < H && x >= 0 && x < W) {
-      st = state[(size_t)y * W + x];
-      if (st != ST_NONE) v = heat[(size_t)y * W + x];
-    }
-    ss[i] = st;
-    sv[i] = v;
-  }
-  __syncthreads();
-  int left = 0;
-  for (int it = 0; it < NMS_LOCAL_ITERS; ++it) {
-    for (int i = tid; i < TW * TW; i += 256) {
-      int y = ty0 - R + i / TW, x = tx0 - R + i % TW;
-      key[i] = ss[i] == ST_UNDECIDED ? nms_key(sv[i], (unsigned int)(y * W + x)) : 0ull;
-    }
-    __syncthreads();
-    for (int i = tid; i < TW * NT; i += 256) {  // row pass over all TW rows, interior columns
-      int row = i / NT, col = i % NT;
-      const unsigned long long* kr = key + row * TW + col;
-      const uint8_t* sr = ss + row * TW + col;
-      unsigned long long m = 0ull;
-      uint8_t k = 0;
-      for (int dx = 0; dx <= 2 * R; ++dx) {
-        m = max(m, kr[dx]);
-        k |= (sr[dx] == ST_KEPT);
-      }
-      rm[i] = m;
-      rk[i] = k;
-    }
-    __syncthreads();
-    uint8_t ns[4];
-    left = 0;
-#pragma unroll
-    for (int qd = 0; qd < 4; ++qd) {  // column pass, interior pixels
-      int i = tid + qd * 256;
-      int ly = i / NT, lx = i % NT;
-      int c = (ly + R) * TW + (lx + R);
-      uint8_t st = ss[c];
-      ns[qd] = st;
-      if (st != ST_UNDECIDED) continue;
-      unsigned long long m = 0ull;
-      uint8_t k = 0;
-      for (int dy = 0; dy <= 2 * R; ++dy) {
-        m = max(m, rm[(ly + dy) * NT + lx]);
-        k |= rk[(ly + dy) * NT + lx];
-      }
-      if (k) ns[qd] = ST_NONE;
-      else if (key[c] == m) ns[qd] = ST_KEPT;
-      else left++;
-    }
-    __syncthreads();
-#pragma unroll
-    for (int qd = 0; qd < 4; ++qd) {
-      int i = tid + qd * 256;
-      ss[(i / NT + R) * TW + (i % NT + R)] = ns[qd];
-    }
-    __syncthreads();
-  }
-  for (int i = tid; i < NT * NT; i += 256) {
-    int y = ty0 + i / NT, x = tx0 + i % NT;
-    if (y < H && x < W) state[(size_t)y * W + x] = ss[(i / NT + R) * TW + (i % NT + R)];
-  }
-  if (left) atomicAdd(remaining, (unsigned int)left);
 }
 
 // Square-window rounds, sliding-window form (R known at compile time).  One 64-bit array carries everything a round needs:
@@ -337,6 +240,7 @@ static bool nms_launch_sliding(int R, dim3 grid, const float* heat, uint8_t* sta
     case 4: launch_sliding<4>(grid, heat, state, H, W, remaining, st); return true;
     case 5: launch_sliding<5>(grid, heat, state, H, W, remaining, st); return true;
     case 6: launch_sliding<6>(grid, heat, state, H, W, remaining, st); return true;
+    case 7: launch_sliding<7>(grid, heat, state, H, W, remaining, st); return true;
     case 8: launch_sliding<8>(grid, heat, state, H, W, remaining, st); return true;
     default: return false;
   }
@@ -452,15 +356,18 @@ static NmsWs nms_carve(void* ws, int I, int H, int W, int capacity) {
 
 // Runs the rounds to the fixed point.  Synchronises the stream every `batch` rounds to read the
 // number of still-undecided pixels (the reference API returns host data, so a sync is inherent).
+// square: the stencil is the full (2R+1)^2 window (nms_fast), so radii 1..8 run the sliding-window kernel; every other
+// radius, and every box_nms footprint, runs the stencil kernel.  Both reach the greedy result for the order (confidence
+// desc, linear index asc); the only difference is that the 64-bit key orders -0.0 below +0.0 where the float compare of
+// the stencil kernel ties them.  That matters only when both signed zeros are candidates at once, which no caller
+// produces: flattenDetection heatmaps are >= +0, and utils.nms_fast has one -0.0 among negative ranks and NaN.
 static int nms_run_rounds(const float* heat, const NmsWs& w, int I, int H, int W, int R, const uint8_t* stencil,
-                          bool square, cudaStream_t st, int* rounds_out) {
+                          bool square, cudaStream_t st) {
   dim3 grid(ssp_ceil_div(W, NT), ssp_ceil_div(H, NT), I);
   int TW = NT + 2 * R;
-  size_t smem = square ? (size_t)TW * TW * 13 + (size_t)TW * NT * 9 + 16
-                       : (size_t)TW * TW * 5 + (size_t)(2 * R + 1) * (2 * R + 1);
+  size_t smem = (size_t)TW * TW * 5 + (size_t)(2 * R + 1) * (2 * R + 1);
   if (smem > 48 * 1024) {
-    cudaError_t e = square ? cudaFuncSetAttribute(nms_round_square_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                           : cudaFuncSetAttribute(nms_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    cudaError_t e = cudaFuncSetAttribute(nms_round_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) { ssp_set_error("nms: window radius %d needs %zu B shared memory: %s", R, smem, cudaGetErrorString(e)); return (int)e; }
   }
   int rounds = 0;
@@ -471,10 +378,7 @@ static int nms_run_rounds(const float* heat, const NmsWs& w, int I, int H, int W
   while (remaining) {
     for (int k = 0; k < batch; ++k) {
       if (k == batch - 1) SSP_CUDA_CALL(cudaMemsetAsync(w.remaining, 0, 4, st));
-      if (square && nms_launch_sliding(R, grid, heat, w.state, H, W, w.remaining, st)) {
-      } else if (square)
-        nms_round_square_kernel<<<grid, 256, smem, st>>>(heat, w.state, H, W, R, w.remaining);
-      else
+      if (!(square && nms_launch_sliding(R, grid, heat, w.state, H, W, w.remaining, st)))
         nms_round_kernel<<<grid, 256, smem, st>>>(heat, w.state, H, W, R, stencil, w.remaining);
       SSP_CUDA_CHECK_LAUNCH("nms_round_kernel");
       ++rounds;
@@ -484,7 +388,6 @@ static int nms_run_rounds(const float* heat, const NmsWs& w, int I, int H, int W
     SSP_CUDA_CALL(cudaStreamSynchronize(st));
     if (rounds > 4 * (H + W) * I + 64) { ssp_set_error("nms: rounds did not converge"); return SSP_EUNSUPPORTED; }
   }
-  if (rounds_out) *rounds_out = rounds;
   return SSP_OK;
 }
 
@@ -503,8 +406,8 @@ extern "C" int ssp_nms_fast(const float* heat, int I, int H, int W, float conf_t
   size_t n = (size_t)I * H * W;
   nms_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(heat, n, conf_thresh, 0, w.state);
   SSP_CUDA_CHECK_LAUNCH("nms_init_kernel");
-  // the stencil of nms_fast is the full (2R+1)^2 square (all ones): separable rounds
-  int rc = nms_run_rounds(heat, w, I, H, W, R, stencil, true, st, nullptr);
+  // the stencil of nms_fast is the full (2R+1)^2 square (all ones)
+  int rc = nms_run_rounds(heat, w, I, H, W, R, stencil, true, st);
   if (rc) return rc;
   SSP_CUDA_CALL(cudaMemsetAsync(w.count, 0, (size_t)I * 4, st));
   dim3 cg(ssp_ceil_div(H * W, 256), I);
@@ -536,7 +439,7 @@ extern "C" int ssp_box_nms(const float* prob, int I, int H, int W, float min_pro
   size_t n = (size_t)I * H * W;
   nms_init_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(prob, n, min_prob, 1, w.state);
   SSP_CUDA_CHECK_LAUNCH("nms_init_kernel");
-  int rc = nms_run_rounds(prob, w, I, H, W, R, stencil, false, st, nullptr);
+  int rc = nms_run_rounds(prob, w, I, H, W, R, stencil, false, st);
   if (rc) return rc;
   nms_dense_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(prob, w.state, n, out);
   SSP_CUDA_CHECK_LAUNCH("nms_dense_kernel");

@@ -5,33 +5,9 @@
 #include "common.cuh"
 
 // ----------------------------------------------------------------------------------------------
-// a1: warp_points   out[b,p,:] = (H_b [x,y,1]^T)[:2] / (H_b [x,y,1]^T)[2]
+// a1 / a10: warp_points   out[b,p,:] = (H_b [x,y,1]^T)[:2] / (H_b [x,y,1]^T)[2]
+// keep (optional) = the in-bounds predicate of filter_points: 0 <= p <= shape-1, inclusive.
 // ----------------------------------------------------------------------------------------------
-__global__ void warp_points_kernel(const float* __restrict__ pts, int P, const float* __restrict__ Hm,
-                                   float* __restrict__ out) {
-  int b = blockIdx.y;
-  __shared__ float h[9];
-  if (threadIdx.x < 9) h[threadIdx.x] = Hm[b * 9 + threadIdx.x];
-  __syncthreads();
-  for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < P; p += gridDim.x * blockDim.x) {
-    float2 xy = reinterpret_cast<const float2*>(pts)[p];
-    float ox, oy;
-    homography_apply(h, xy.x, xy.y, ox, oy);
-    reinterpret_cast<float2*>(out)[(size_t)b * P + p] = make_float2(ox, oy);
-  }
-}
-
-extern "C" int ssp_warp_points(const float* pts, int P, const float* Hm, int B, float* out, void* stream) {
-  SSP_REQUIRE(pts && Hm && out, "ssp_warp_points: null pointer");
-  SSP_REQUIRE(P >= 0 && B > 0, "ssp_warp_points: bad sizes P=%d B=%d", P, B);
-  if (P == 0) return SSP_OK;
-  dim3 grid(min(ssp_ceil_div(P, 256), 148 * 8), B);
-  warp_points_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(pts, P, Hm, out);
-  SSP_CUDA_CHECK_LAUNCH("warp_points_kernel");
-  return SSP_OK;
-}
-
-// a10: fused warp + in-bounds predicate (filter_points semantics: 0 <= p <= shape-1, inclusive).
 __global__ void warp_points_mask_kernel(const float* __restrict__ pts, int P, const float* __restrict__ Hm,
                                         float sx, float sy, float* __restrict__ out,
                                         uint8_t* __restrict__ keep) {
@@ -44,13 +20,13 @@ __global__ void warp_points_mask_kernel(const float* __restrict__ pts, int P, co
     float ox, oy;
     homography_apply(h, xy.x, xy.y, ox, oy);
     reinterpret_cast<float2*>(out)[(size_t)b * P + p] = make_float2(ox, oy);
-    keep[(size_t)b * P + p] = (ox >= 0.f && ox <= sx - 1.f && oy >= 0.f && oy <= sy - 1.f) ? 1 : 0;
+    if (keep) keep[(size_t)b * P + p] = (ox >= 0.f && ox <= sx - 1.f && oy >= 0.f && oy <= sy - 1.f) ? 1 : 0;
   }
 }
 
 extern "C" int ssp_warp_points_mask(const float* pts, int P, const float* Hm, int B, float shape_x,
                                     float shape_y, float* out, uint8_t* keep, void* stream) {
-  SSP_REQUIRE(pts && Hm && out && keep, "ssp_warp_points_mask: null pointer");
+  SSP_REQUIRE(pts && Hm && out, "ssp_warp_points_mask: null pointer");
   SSP_REQUIRE(P >= 0 && B > 0, "ssp_warp_points_mask: bad sizes P=%d B=%d", P, B);
   if (P == 0) return SSP_OK;
   dim3 grid(min(ssp_ceil_div(P, 256), 148 * 8), B);

@@ -89,8 +89,8 @@ class DetectorLossFn(torch.autograd.Function):
         out3 = torch.empty((3,), dtype=torch.float32, device=dev)
         nbytes = _lib.load().ssp_detector_loss_ws_bytes(B, Hc, Wc)
         ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-        call("ssp_detector_loss_fwd", ptr(x), ptr(t), ptr(m), B, Hc, Wc, 1 if fused2d else 0, ptr(out3), ptr(ws),
-             nbytes, stream_of(x))
+        call("ssp_detector_loss_fwd_pair", ptr(x), ptr(t), ptr(m), None, None, None, B, Hc, Wc, 1 if fused2d else 0,
+             ptr(out3), None, None, ptr(ws), nbytes, stream_of(x))
         ctx.save_for_backward(x, t, m)
         ctx.out3 = out3  # attribute, not a saved tensor (the exchange rewrites it in place)
         ctx.fused2d = fused2d
@@ -107,8 +107,8 @@ class DetectorLossFn(torch.autograd.Function):
         B, C, Hc, Wc = x.shape
         g = f32c(gout.reshape(1), x.device)
         dsemi = torch.empty_like(x)
-        call("ssp_detector_loss_bwd", ptr(x), ptr(t), ptr(m), B, Hc, Wc, 1 if ctx.fused2d else 0, ptr(out3), ptr(g),
-             ptr(dsemi), stream_of(x))
+        call("ssp_detector_loss_bwd_pair", ptr(x), ptr(t), ptr(m), None, None, None, B, Hc, Wc, 1 if ctx.fused2d else 0,
+             ptr(out3), None, ptr(g), None, ptr(dsemi), None, stream_of(x))
         return dsemi, None, None, None, None
 
 

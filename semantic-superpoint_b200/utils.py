@@ -83,7 +83,7 @@ def warp_points(points, homographies, device="cpu"):
     B, P = Hm.shape[0], pts.shape[0]
     out = torch.empty((B, P, 2), dtype=torch.float32, device=dev)
     if P > 0:
-        call("ssp_warp_points", ptr(pts), P, ptr(Hm), B, ptr(out), stream_of(out))
+        call("ssp_warp_points_mask", ptr(pts), P, ptr(Hm), B, 0.0, 0.0, ptr(out), None, stream_of(out))
     out = out.to(out_dev)
     return out[0, :, :] if no_batches else out
 
@@ -346,10 +346,7 @@ def combine_heatmap(heatmap, inv_homographies, mask_2D, device="cpu"):
     N, C, H, W = h.shape
     if C != 1 or m.shape != h.shape or Hm.shape[0] != N:
         raise RuntimeError("combine_heatmap: expected heatmap/mask [N,1,H,W] and homographies [1,N,3,3]")
-    out = torch.empty((1, H, W), dtype=torch.float32, device=dev)
-    call("ssp_combine_heatmap", ptr(h), ptr(m), ptr(Hm), 1, N, H, W, ptr(_linspace_grid(W, dev)),
-         ptr(_linspace_grid(H, dev)), ptr(out), stream_of(out))
-    return out.to(out_dev)
+    return combine_heatmap_batch(h.view(1, N, H, W), Hm[None], m.view(1, N, H, W)).to(out_dev)
 
 
 def combine_heatmap_batch(heatmap, inv_homographies, mask_2D):
@@ -624,7 +621,9 @@ def sample_desc_from_points(coarse_desc, pts, cell=8):
         raise RuntimeError("sample_desc_from_points: coarse_desc must be [1,D,Hc,Wc], got %s" % (tuple(coarse_desc.shape),))
     p = torch.from_numpy(np.ascontiguousarray(pts, dtype=np.float64)).to(dev)
     out = torch.empty((D, K), dtype=torch.float32, device=dev)
-    call("ssp_sample_desc", ptr(cd), ptr(p), K, D, int(cd.shape[2]), int(cd.shape[3]), int(cell), ptr(out), stream_of(out))
+    count = torch.full((1,), K, dtype=torch.int32, device=dev)
+    call("ssp_sample_desc_batch", ptr(cd), ptr(p), K, ptr(count), K, 1, D, int(cd.shape[2]), int(cd.shape[3]), int(cell),
+         ptr(out), stream_of(out))
     return out.cpu().numpy()
 
 

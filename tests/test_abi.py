@@ -84,7 +84,7 @@ def test_argument_errors_without_gpu():
     """Argument validation happens before any CUDA call, so it is testable on a CPU-only box."""
     from ssp_b200 import _lib
     lib = _lib.load()
-    assert lib.ssp_warp_points(None, 1, None, 1, None, None) < 0
+    assert lib.ssp_warp_points_mask(None, 1, None, 1, 0.0, 0.0, None, None, None) < 0
     assert b"null pointer" in lib.ssp_last_error()
     assert lib.ssp_labels2d_to_3d(ctypes.c_void_p(16), 1, 12, 12, 1, ctypes.c_void_p(16), None) < 0
     assert b"multiples of 8" in lib.ssp_last_error()

@@ -298,6 +298,24 @@ def test_nms_480x640_and_batch():
         assert np.array_equal(outs[i], O.getPtsFromHeatmap(stack[i], 0.015, 4))
 
 
+@pytest.mark.parametrize("r", [0, 7, 9, 16, 48])
+def test_nms_radii_off_the_benchmark(r):
+    """Radii 0 and 9..48 run the stencil kernel, 7 the sliding kernel: getPtsFromHeatmap, heatmap_to_pts_batch and nms_fast
+    equal the oracle exactly on a tie-free map and on the tied map above, up to the largest radius nms_fast accepts."""
+    tied = np.round(synth.uniform((96, 128), 5) * 8).astype(np.float32) / 8
+    maps = ((synth.unique_heatmap(96, 128, 40 + r), 0.015), (tied, 0.3))
+    for heat, thr in maps:
+        assert np.array_equal(S.getPtsFromHeatmap(heat, thr, r), O.getPtsFromHeatmap(heat, thr, r))
+        ys, xs = np.nonzero(heat >= thr)
+        corners = np.stack([xs, ys, heat[ys, xs]]).astype(np.float64)
+        out, inds = S.nms_fast(corners, 96, 128, r)
+        ref, rinds = O.nms_fast(corners, 96, 128, r)
+        assert np.array_equal(out, ref) and np.array_equal(inds, rinds)
+    outs = S.heatmap_to_pts_batch(cu(np.stack([m for m, _ in maps])), 0.015, r)
+    for (heat, _), got in zip(maps, outs):
+        assert np.array_equal(got, O.getPtsFromHeatmap(heat, 0.015, r))
+
+
 def test_box_nms(golden):
     g = golden("box_nms")
     out = S.box_nms(cu(g["prob"]), 4, iou=0.1, min_prob=0.01, keep_top_k=1000)
@@ -633,7 +651,7 @@ def test_sample_desc_and_nn_match(golden):
 def test_abi_errors():
     from ssp_b200 import _lib
     lib = _lib.load()
-    assert lib.ssp_warp_points(None, 4, None, 1, None, None) < 0
+    assert lib.ssp_warp_points_mask(None, 4, None, 1, 0.0, 0.0, None, None, None) < 0
     assert b"null" in lib.ssp_last_error()
     x = torch.zeros((1, 1, 12, 16), device=DEV)
     with pytest.raises(RuntimeError):
