@@ -113,11 +113,7 @@ int ssp_soft_argmax_points(const float* heat /*[I,H,W]*/, int I, int H, int W, d
  *      out8 = { loss, pos_sum, neg_sum, norm, num_loss, num_pos, num_neg, sum(mask_valid) }
  *      mvbits (optional, [B,Nc_pad/32] u32): mask_valid != 0 per cell in the same bit order, for the "fold" mode of the
  *      tensor-core engine (mask folded into the indicator words; a non-binary mask then poisons the normaliser: NaN) ---- */
-int ssp_desc_geometry_nblocks(int B, int Nc);
-int ssp_desc_geometry(const float* H /*[B,3,3]*/, const float* mask_valid /*[B,Nc] or NULL*/,
-                      const float* mask2d /*or NULL; used when mask_valid is NULL: [B,1,8Hc,8Wc], getMasks fused in*/, int B,
-                      int Hc, int Wc, int cell, float* wpts, float* mv_pad, double* mv_part /*[geometry_nblocks]*/,
-                      uint32_t* mvbits /*or NULL*/, void* stream);
+int ssp_desc_geometry_nblocks(int B, int Nc); /* length of ssp_desc_pack2_geometry's mv_part */
 int ssp_desc_pos_nblocks(int B, int Nc);
 int ssp_desc_maxp(void); /* DESC_MAXP: list slots per row / column */
 /* sparse positive pairs: exact fp32 dots, partial sums (4 doubles per block: pos_u, pos_w, negcorr_u, negcorr_w)
@@ -139,11 +135,14 @@ int ssp_desc_dense_fwd_simt(const float* D, const float* Dw, const float* mv_pad
                             float* dbgS /*[B,Nc,Nc] or NULL*/, void* stream);
 int ssp_desc_pack(const float* src /*[B,Dch,Nc]*/, const float* scale /*[B,Nc_pad] or NULL*/, int B, int Dch, int Nc,
                   void* hi /*bf16 [B,Nc_pad,Dch]*/, void* lo /*or NULL*/, void* stream);
-/* ssp_desc_pack of two tensors (unscaled) and ssp_desc_geometry as ONE launch: they do not depend on each other */
-int ssp_desc_pack2_geometry(const float* src0, const float* src1, int B, int Dch, int Hc, int Wc, void* hi0, void* lo0 /*or NULL*/,
-                            void* hi1, void* lo1 /*or NULL*/, const float* H /*[B,3,3]*/, const float* mask_valid /*or NULL*/,
-                            const float* mask2d /*or NULL*/, int cell, float* wpts, float* mv_pad, double* mv_part,
-                            uint32_t* mvbits /*or NULL*/, void* stream);
+/* ssp_desc_pack of two tensors (unscaled) and the geometry (warped cell centres wpts, mv_pad and the per-block sums mv_part
+ * of mask_valid) as ONE launch: they do not depend on each other.  hi0 == hi1 == NULL: the geometry alone (src*, lo* and
+ * Dch unused).  mask2d is used when mask_valid is NULL: [B,1,8Hc,8Wc], getMasks fused in (cell must be 8). */
+int ssp_desc_pack2_geometry(const float* src0, const float* src1, int B, int Dch, int Hc, int Wc, void* hi0 /*or NULL*/,
+                            void* lo0 /*or NULL*/, void* hi1 /*or NULL*/, void* lo1 /*or NULL*/, const float* H /*[B,3,3]*/,
+                            const float* mask_valid /*[B,Nc] or NULL*/, const float* mask2d /*or NULL*/, int cell,
+                            float* wpts, float* mv_pad, double* mv_part /*[geometry_nblocks]*/, uint32_t* mvbits /*or NULL*/,
+                            void* stream);
 int ssp_desc_dense_tc_nblocks(int B, int Nc);
 /* tcgen05 forward (CTA-pair MMAs, M=256): negative hinge over all pairs + row-orientation indicator words bitsR (their
  * transpose bitsC comes from ssp_desc_pos_coef).  The lo planes must lie above their hi planes in memory (one allocation).

@@ -41,7 +41,6 @@ SIGNATURES = {
     "ssp_soft_argmax_points": (_I, [_P, _I, _I, _I, _P, _I, _P, _I, _I, _P]),
     "ssp_box_nms": (_I, [_P, _I, _I, _I, _F, _I, _P, _P, _P, _Z, _P]),
     "ssp_desc_geometry_nblocks": (_I, [_I, _I]),
-    "ssp_desc_geometry": (_I, [_P, _P, _P, _I, _I, _I, _I, _P, _P, _P, _P, _P]),
     "ssp_desc_pos_nblocks": (_I, [_I, _I]),
     "ssp_desc_maxp": (_I, []),
     "ssp_desc_pos_fwd": (_I, [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _F, _F, _F, _P, _P, _P, _P, _P, _P, _P]),

@@ -80,24 +80,6 @@ __global__ void __launch_bounds__(GEOM_THREADS) desc_geometry_kernel(const __gri
 
 extern "C" int ssp_desc_geometry_nblocks(int B, int Nc) { return B * (desc_nc_pad(Nc) / GEOM_THREADS); }
 
-// mvbits (optional): [B, Nc_pad/32] words of mask_valid != 0 in DESC_BITPOS order for the "fold" mode of the tensor-core
-// engine; requesting them also makes a non-binary mask poison the normaliser with NaN.
-// mask2d (optional, used when mask_valid is NULL): the pixel-resolution mask [B,1,8Hc,8Wc] the cell mask is the product of
-// (getMasks fused in; cell must be 8).
-extern "C" int ssp_desc_geometry(const float* Hm, const float* mask_valid, const float* mask2d, int B, int Hc, int Wc, int cell,
-                                 float* wpts, float* mv_pad, double* mv_part, uint32_t* mvbits, void* stream) {
-  SSP_REQUIRE(Hm && wpts && mv_pad && mv_part, "ssp_desc_geometry: null pointer");
-  SSP_REQUIRE(B > 0 && B <= 65535 && Hc > 0 && Wc > 0 && cell > 0, "ssp_desc_geometry: bad sizes");
-  SSP_REQUIRE(!mask2d || mask_valid || (cell == 8 && ((uintptr_t)mask2d & 15) == 0),
-              "ssp_desc_geometry: the fused pixel mask needs cell_size 8 and a 16-byte aligned mask");
-  int Nc_pad = desc_nc_pad(Hc * Wc);
-  dim3 grid(Nc_pad / GEOM_THREADS, B);
-  GeomArgs A = {Hm, mask_valid, mask2d, B, Hc, Wc, cell, Nc_pad, reinterpret_cast<float2*>(wpts), mv_pad, mv_part, mvbits};
-  desc_geometry_kernel<<<grid, GEOM_THREADS, 0, (cudaStream_t)stream>>>(A);
-  SSP_CUDA_CHECK_LAUNCH("desc_geometry_kernel");
-  return SSP_OK;
-}
-
 // candidate window of cell indices whose centre can be within `dist` of (wx, wy): a centre k*cell + half qualifies only if
 // |k*cell + half - w| <= dist, i.e. k in [(w - dist - half)/cell, (w + dist - half)/cell]; the window is that interval
 // widened by 0.01 cell (0.08 px at cell = 8: three orders of magnitude above the fp32 rounding of pixel coordinates), the
@@ -753,19 +735,33 @@ extern "C" int ssp_desc_pack(const float* src, const float* scale, int B, int Dc
   return SSP_OK;
 }
 
-// two ssp_desc_pack calls (no scale) and ssp_desc_geometry as ONE launch (arguments = those calls')
+// two ssp_desc_pack calls (no scale) and the descriptor-loss geometry as ONE launch.  hi0 == hi1 == NULL: the geometry
+// alone (src*, lo* and Dch unused), for the fp32 engine, which reads no planes.
+// mvbits (optional): [B, Nc_pad/32] words of mask_valid != 0 in DESC_BITPOS order for the "fold" mode of the tensor-core
+// engine; requesting them also makes a non-binary mask poison the normaliser with NaN.
+// mask2d (optional, used when mask_valid is NULL): the pixel-resolution mask [B,1,8Hc,8Wc] the cell mask is the product of
+// (getMasks fused in; cell must be 8).
 extern "C" int ssp_desc_pack2_geometry(const float* src0, const float* src1, int B, int Dch, int Hc, int Wc, void* hi0, void* lo0,
                                        void* hi1, void* lo1, const float* Hm, const float* mask_valid, const float* mask2d,
                                        int cell, float* wpts, float* mv_pad, double* mv_part, uint32_t* mvbits, void* stream) {
-  SSP_REQUIRE(src0 && src1 && hi0 && hi1 && Hm && wpts && mv_pad && mv_part, "ssp_desc_pack2_geometry: null pointer");
-  SSP_REQUIRE(B > 0 && B <= 65535 && Dch > 0 && Dch % 2 == 0 && Hc > 0 && Wc > 0 && cell > 0, "ssp_desc_pack2_geometry: bad sizes");
+  const bool pack = hi0 || hi1;
+  SSP_REQUIRE((!pack || (src0 && src1 && hi0 && hi1)) && Hm && wpts && mv_pad && mv_part, "ssp_desc_pack2_geometry: null pointer");
+  SSP_REQUIRE(B > 0 && B <= 65535 && (!pack || (Dch > 0 && Dch % 2 == 0)) && Hc > 0 && Wc > 0 && cell > 0,
+              "ssp_desc_pack2_geometry: bad sizes");
   SSP_REQUIRE(!mask2d || mask_valid || (cell == 8 && ((uintptr_t)mask2d & 15) == 0),
               "ssp_desc_pack2_geometry: the fused pixel mask needs cell_size 8 and a 16-byte aligned mask");
   const int Nc = Hc * Wc, Nc_pad = desc_nc_pad(Nc);
-  const int nchb = (Dch + PK_CH - 1) / PK_CH, npack = 2 * nchb;
+  GeomArgs G = {Hm, mask_valid, mask2d, B, Hc, Wc, cell, Nc_pad, reinterpret_cast<float2*>(wpts), mv_pad, mv_part, mvbits};
+  if (!pack) {
+    // not desc_pack_geometry_kernel with npack = 0: its 33 KB pack tile made the geometry 7.4 instead of 5.3 us and the
+    // positive-pair kernel after it 52.3 instead of 51.0 us (fp32 engine, B = 32 of 30 x 40 cells, NVIDIA B200 at 1000 W)
+    desc_geometry_kernel<<<dim3(Nc_pad / GEOM_THREADS, B), GEOM_THREADS, 0, (cudaStream_t)stream>>>(G);
+    SSP_CUDA_CHECK_LAUNCH("desc_geometry_kernel");
+    return SSP_OK;
+  }
+  const int npack = 2 * ((Dch + PK_CH - 1) / PK_CH);
   SSP_REQUIRE(npack + 1 <= 65535, "ssp_desc_pack2_geometry: descriptor dim %d too large", Dch);
   PackArgs P = {src0, src1, nullptr, Dch, Nc, Nc_pad, (__nv_bfloat16*)hi0, (__nv_bfloat16*)lo0, (__nv_bfloat16*)hi1, (__nv_bfloat16*)lo1};
-  GeomArgs G = {Hm, mask_valid, mask2d, B, Hc, Wc, cell, Nc_pad, reinterpret_cast<float2*>(wpts), mv_pad, mv_part, mvbits};
   dim3 grid(Nc_pad / PK_CELLS, B, npack + 1);
   desc_pack_geometry_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(P, G, npack, Nc_pad / GEOM_THREADS);
   SSP_CUDA_CHECK_LAUNCH("desc_pack_geometry_kernel");

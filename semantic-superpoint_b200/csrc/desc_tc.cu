@@ -771,7 +771,7 @@ extern "C" int ssp_desc_dense_tc_nblocks(int B, int Nc) {
 // Ahi/Alo: packed planes of `descriptors`, Bhi/Blo: packed planes of `descriptors_warped` ([B, Nc_pad, 256] bf16).
 // Alo == Blo == NULL selects single-pass bf16; otherwise bf16x3.  bitsR (optional) receives the row-orientation indicator
 // words (their transpose bitsC comes from ssp_desc_pos_coef).  mvbits (optional, [B, Nc_pad/32] words of mask_valid != 0 in
-// DESC_BITPOS order, from ssp_desc_geometry): the indicator words drop the columns whose mask_valid is 0 ("fold").
+// DESC_BITPOS order, from ssp_desc_pack2_geometry): the indicator words drop the columns whose mask_valid is 0 ("fold").
 extern "C" int ssp_desc_dense_fwd_tc(const void* Ahi, const void* Alo, const void* Bhi, const void* Blo,
                                      const float* mv_pad, const uint32_t* mvbits, int B, int Hc, int Wc, float mneg,
                                      double* partials, uint32_t* bitsR, float* dbgS, void* stream) {

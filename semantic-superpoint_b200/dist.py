@@ -55,6 +55,9 @@ class LossExchange(object):
       det*  = out3 of a detector loss   {loss, numerator, sum(mask) + 1e-5}
       desc8 = out8 of the descriptor loss {loss, pos, neg, norm, num_loss, num_pos, num_neg, sum(mask_valid)}
       sem*  = out3 of a semantic loss   {loss, sum, count}
+    B_local, Hc, Wc: the descriptor loss's shard size and cell grid; its global normaliser is
+      B_global * (sum_global(mask_valid) + 1) * Hc * Wc  (utils/utils.py:886-887), B_global the SUM of the ranks' B_local
+      (shards may differ by one pair).
     backend "p2p": the peer-memory kernel (CUDA tensors, ranks on one node); "allreduce": one torch all-reduce.
     """
 
@@ -186,26 +189,6 @@ def close_exchanges():
     for ex in list(_exchanges.values()):
         ex.close()
     _exchanges.clear()
-
-
-def globalize_detector(out3, group):
-    """out3 = [loss, numerator, sum(mask) + 1e-5] of the local shard -> same triple for the global batch (in place)."""
-    get_exchange(group).run(det0=out3)
-    return out3
-
-
-def globalize_semantic(out3, group):
-    """out3 = [loss, sum, count] of the local shard -> global batch (mean over every counted pixel of every rank)."""
-    get_exchange(group).run(sem0=out3)
-    return out3
-
-
-def globalize_descriptor(out8, B_local, Hc, Wc, group):
-    """out8 = [loss, pos, neg, norm, num_loss, num_pos, num_neg, sum(mask_valid)] of the local shard -> global batch.
-    norm_global = B_global * (sum_global(mask_valid) + 1) * Hc * Wc  (utils/utils.py:886-887); B_global is the SUM of the
-    ranks' shard sizes (shards may differ by one pair)."""
-    get_exchange(group).run(desc8=out8, B_local=B_local, Hc=Hc, Wc=Wc)
-    return out8
 
 
 def max_over_ranks(value, device):

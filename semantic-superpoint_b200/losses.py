@@ -6,6 +6,7 @@ numerators / mask sums are exchanged by ONE peer-memory kernel (dist.LossExchang
 the loss scalars and normalisers in place, stream ordered, before the forward returns; the backward kernels
 scale by the global normaliser.
 """
+import contextlib
 import functools
 from collections import namedtuple
 
@@ -63,55 +64,6 @@ class _Fork(object):
 
 
 # ------------------------------------------------------------------------------------------------
-class DetectorLossFn(torch.autograd.Function):
-    """loss = sum_cells mask * sum_c BCE(softmax(semi)_c, target_c) / (sum mask + 1e-5)
-
-    fused2d=False: target [B,65,Hc,Wc], mask [B,Hc,Wc]  (reference signature)
-    fused2d=True : target = labels_2D [B,1,H,W], mask = mask_2D [B,1,H,W] (labels2Dto3D + getMasks fused)
-    """
-
-    @staticmethod
-    def forward(ctx, semi, target, mask, fused2d, dist_group=None):
-        _lib.require_cuda(semi)
-        dev = semi.device
-        x = f32c(semi.detach(), dev)
-        t = f32c(target.detach(), dev)
-        m = f32c(mask.detach(), dev)
-        B, C, Hc, Wc = x.shape
-        if C != 65:
-            raise RuntimeError("detector_loss: input must have 65 channels, got %d" % C)
-        if fused2d:
-            if t.numel() != B * Hc * Wc * 64 or m.numel() != B * Hc * Wc * 64:
-                raise RuntimeError("detector_loss_2d: labels_2D / mask_2D must be [B,1,8Hc,8Wc]")
-        else:
-            if t.shape != x.shape or m.numel() != B * Hc * Wc:
-                raise RuntimeError("detector_loss: target must be [B,65,Hc,Wc] and mask [B,Hc,Wc]")
-        out3 = torch.empty((3,), dtype=torch.float32, device=dev)
-        nbytes = _lib.load().ssp_detector_loss_ws_bytes(B, Hc, Wc)
-        ws = torch.empty((nbytes,), dtype=torch.uint8, device=dev)
-        call("ssp_detector_loss_fwd_pair", ptr(x), ptr(t), ptr(m), None, None, None, B, Hc, Wc, 1 if fused2d else 0,
-             ptr(out3), None, None, ptr(ws), nbytes, stream_of(x))
-        ctx.save_for_backward(x, t, m)
-        ctx.out3 = out3  # attribute, not a saved tensor (the exchange rewrites it in place)
-        ctx.fused2d = fused2d
-        if dist_group is not None:
-            from .dist import globalize_detector
-            globalize_detector(out3, dist_group)
-        return out3[0]
-
-    @staticmethod
-    @once_differentiable
-    def backward(ctx, gout):
-        x, t, m = ctx.saved_tensors
-        out3 = ctx.out3
-        B, C, Hc, Wc = x.shape
-        g = f32c(gout.reshape(1), x.device)
-        dsemi = torch.empty_like(x)
-        call("ssp_detector_loss_bwd_pair", ptr(x), ptr(t), ptr(m), None, None, None, B, Hc, Wc, 1 if ctx.fused2d else 0,
-             ptr(out3), None, ptr(g), None, ptr(dsemi), None, stream_of(x))
-        return dsemi, None, None, None, None
-
-
 class SemanticLossFn(torch.autograd.Function):
     """Cross entropy of the semantic head with ignore_index (Train_model_heatmap_all.py:181-193).
 
@@ -149,10 +101,10 @@ class SemanticLossFn(torch.autograd.Function):
                  stream_of(x))
             ctx.saved = (x, lab, lse2)
         ctx.up, ctx.shape, ctx.ignore = up, (B, C, h, w), int(ignore_index)
-        ctx.out3 = out3  # attribute, see DetectorLossFn
+        ctx.out3 = out3  # attribute, see DetectorLossPairFn
         if dist_group is not None:
-            from .dist import globalize_semantic
-            globalize_semantic(out3, dist_group)
+            from .dist import get_exchange
+            get_exchange(dist_group).run(sem0=out3)
         return out3[0]
 
     @staticmethod
@@ -186,63 +138,79 @@ def _lam3_vector(lam, dev):
 
 
 # ------------------------------------------------------------------------------------------------
-DetPair = namedtuple("DetPair", "saved out fused2d")  # saved = fp32 (x0, t0, m0, x1, t1, m1); out [2,3]: a triple per image
+# saved = fp32 (x0, t0, m0, x1, t1, m1), the last three None for one loss; out [n,3]: a triple per image
+DetPair = namedtuple("DetPair", "saved out fused2d")
 
 
 def det_pair_forward(semi, target, mask, semi_w, target_w, mask_w, fused2d):
-    """Both detector losses in one launch -> (DetPair, getMasks() of the warped mask [B,Hc,Wc])."""
+    """One detector loss (semi_w None) or both of a pair in one launch -> (DetPair, getMasks() of the warped mask
+    [B,Hc,Wc], None for one loss)."""
     _lib.require_cuda(semi, semi_w)
     dev = semi.device
-    x0, t0, m0 = f32c(semi.detach(), dev), f32c(target.detach(), dev), f32c(mask.detach(), dev)
-    x1, t1, m1 = f32c(semi_w.detach(), dev), f32c(target_w.detach(), dev), f32c(mask_w.detach(), dev)
+    pair = semi_w is not None
+    n = 2 if pair else 1
+    fc = lambda a: f32c(a.detach(), dev)
+    x0, t0, m0 = fc(semi), fc(target), fc(mask)
+    x1, t1, m1 = (fc(semi_w), fc(target_w), fc(mask_w)) if pair else (None, None, None)
     B, C, Hc, Wc = x0.shape
-    if C != 65 or x1.shape != x0.shape:
-        raise RuntimeError("detector_loss: inputs must be two [B,65,Hc,Wc] tensors of the same shape")
+    if C != 65 or (pair and x1.shape != x0.shape):
+        raise RuntimeError("detector_loss: logits must be [B,65,Hc,Wc], the same shape for both images of a pair")
     n2d = B * Hc * Wc * 64
-    for t, m in ((t0, m0), (t1, m1)):
+    for t, m in ((t0, m0), (t1, m1))[:n]:
         ok = (t.numel() == n2d and m.numel() == n2d) if fused2d else (t.shape == x0.shape and m.numel() == B * Hc * Wc)
         if not ok:
             raise RuntimeError("detector_loss: target / mask shapes do not match the logits")
-    out = torch.empty((2, 3), dtype=torch.float32, device=dev)
-    cellmask = torch.empty((B, Hc, Wc), dtype=torch.float32, device=dev)
+    out = torch.empty((n, 3), dtype=torch.float32, device=dev)
+    cellmask = torch.empty((B, Hc, Wc), dtype=torch.float32, device=dev) if pair else None
     per = (_lib.load().ssp_detector_loss_ws_bytes(B, Hc, Wc) + 15) // 16 * 16
-    ws = torch.empty((2 * per,), dtype=torch.uint8, device=dev)
+    ws = torch.empty((n * per,), dtype=torch.uint8, device=dev)
     call("ssp_detector_loss_fwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
-         1 if fused2d else 0, ptr(out[0]), ptr(out[1]), ptr(cellmask), ptr(ws), 2 * per, stream_of(x0))
+         1 if fused2d else 0, ptr(out[0]), ptr(out[1]) if pair else None, ptr(cellmask), ptr(ws), n * per, stream_of(x0))
     return DetPair((x0, t0, m0, x1, t1, m1), out, fused2d), cellmask
 
 
-def det_pair_backward(st, g0, g1):
-    """(d semi, d semi_w) for upstream gradients g0, g1: 1-element device tensors (the fused step passes one twice)."""
+def det_pair_backward(st, g0, g1=None):
+    """(d semi, d semi_w) for upstream gradients g0, g1: 1-element device tensors (the fused step passes one twice).
+    One loss: g1 and d semi_w are None."""
     x0, t0, m0, x1, t1, m1 = st.saved
+    pair = x1 is not None
     B, C, Hc, Wc = x0.shape
-    d0, d1 = torch.empty_like(x0), torch.empty_like(x1)
+    d0, d1 = torch.empty_like(x0), (torch.empty_like(x1) if pair else None)
     call("ssp_detector_loss_bwd_pair", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc,
-         1 if st.fused2d else 0, ptr(st.out[0]), ptr(st.out[1]), ptr(g0), ptr(g1), ptr(d0), ptr(d1), stream_of(x0))
+         1 if st.fused2d else 0, ptr(st.out[0]), ptr(st.out[1]) if pair else None, ptr(g0), ptr(g1), ptr(d0), ptr(d1),
+         stream_of(x0))
     return d0, d1
 
 
 class DetectorLossPairFn(torch.autograd.Function):
-    """Both detector losses of a training pair (image, warped image) in ONE launch each way, plus getMasks() of the
-    warped mask as a by-product (it is the descriptor loss's mask_valid).  Returns (loss, loss_warp, cell_mask_warp)."""
+    """loss = sum_cells mask * sum_c BCE(softmax(semi)_c, target_c) / (sum mask + 1e-5) of one image (semi_w None) or of
+    both images of a training pair (image, warped image), in ONE launch each way.
+
+    fused2d=False: target [B,65,Hc,Wc], mask [B,Hc,Wc]  (reference signature)
+    fused2d=True : target = labels_2D [B,1,H,W], mask = mask_2D [B,1,H,W] (labels2Dto3D + getMasks fused)
+    Returns loss for one image; (loss, loss_warp, cell_mask_warp) for a pair, where cell_mask_warp = getMasks() of the
+    warped mask is a by-product (it is the descriptor loss's mask_valid)."""
 
     @staticmethod
     def forward(ctx, semi, target, mask, semi_w, target_w, mask_w, fused2d, dist_group=None):
+        pair = semi_w is not None
         st, cellmask = det_pair_forward(semi, target, mask, semi_w, target_w, mask_w, fused2d)
         ctx.save_for_backward(*st.saved)
-        ctx.st = st._replace(saved=None)  # out is an attribute, see DetectorLossFn
-        ctx.mark_non_differentiable(cellmask)
+        ctx.st = st._replace(saved=None)  # out is an attribute, not a saved tensor (the exchange rewrites it in place)
         if dist_group is not None:
             from .dist import get_exchange
-            get_exchange(dist_group).run(det0=st.out[0], det1=st.out[1])
+            get_exchange(dist_group).run(det0=st.out[0], det1=st.out[1] if pair else None)
+        if not pair:
+            return st.out[0, 0]
+        ctx.mark_non_differentiable(cellmask)
         return st.out[0, 0], st.out[1, 0], cellmask
 
     @staticmethod
     @once_differentiable
-    def backward(ctx, g0, g1, _gm):
+    def backward(ctx, g0, g1=None, _gm=None):
         st = ctx.st._replace(saved=ctx.saved_tensors)
-        g = grad_vector((g0, g1), st.out.device)
-        d0, d1 = det_pair_backward(st, g[0:1], g[1:2])
+        g = grad_vector((g0, g1)[:len(st.out)], st.out.device)
+        d0, d1 = det_pair_backward(st, *g.split(1))
         return d0, None, None, d1, None, None, None, None
 
 
@@ -286,10 +254,6 @@ def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist,
     mvbits = torch.empty((B, Ncp // 32), dtype=torch.int32, device=dev) if fold else None
     nmv = lib.ssp_desc_geometry_nblocks(B, Nc)
     mv_part = torch.empty((nmv,), dtype=torch.float64, device=dev)
-    geom_args = (ptr(Hm), ptr(mask_valid), ptr(mask_2d), cell, ptr(wpts), ptr(mv_pad), ptr(mv_part), ptr(mvbits))
-    if engine == "fp32":
-        call("ssp_desc_geometry", geom_args[0], geom_args[1], geom_args[2], B, Hc, Wc, *geom_args[3:], s)
-    # tensor-core engines: the geometry blocks ride in the operand pack's launch (independent work, one launch instead of two)
 
     # sparse positive pairs: exact dots, partial sums, pair lists for the backward
     maxp = lib.ssp_desc_maxp()
@@ -317,10 +281,13 @@ def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist,
         Bhi, Blo = PB[0], (PB[1] if split else None)
     neg_part = torch.empty((nneg, 2), dtype=torch.float64, device=dev)
     out8 = torch.empty((8,), dtype=torch.float32, device=dev)
+    # geometry (warped cell centres, mask) and, on the tensor-core engines, the operand pack in one launch (independent work):
+    # every positive-pair kernel needs the warped points.  The fp32 engine packs nothing (hi planes NULL).
+    call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(Hm),
+         ptr(mask_valid), ptr(mask_2d), cell, ptr(wpts), ptr(mv_pad), ptr(mv_part), ptr(mvbits), s)
     if split:
         # bf16x3: the positive pairs read the packed hi/lo planes (2 x 512 contiguous bytes per cell instead of 256
         # strided channels), so they run right after the pack, in front of the tensor-core kernel
-        call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), *geom_args, s)
         call("ssp_desc_pos_fwd_planes", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(wpts), ptr(mv_pad), B, Hc, Wc, cell,
              dist, lamda, _MPOS, _MNEG, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), s)
         # bitsC (the column-orientation indicator words) is only read by the backward GEMM: it is transposed from bitsR by
@@ -328,9 +295,7 @@ def desc_forward(D, Dw, Hm, *, mask_valid=None, mask_2d=None, cell, lamda, dist,
         call("ssp_desc_dense_fwd_tc", ptr(Ahi), ptr(Alo), ptr(Bhi), ptr(Blo), ptr(mv_pad), ptr(mvbits), B, Hc, Wc, _MNEG,
              ptr(neg_part), ptr(bitsR), ptr(debug_S), s)
     else:
-        # the HBM-bound exact positive-pair kernel overlaps the pack + tensor-core kernels
-        if engine != "fp32":  # single-pass bf16: pack + geometry first (the positive-pair kernel needs the warped points)
-            call("ssp_desc_pack2_geometry", ptr(Dc), ptr(Dwc), B, Dch, Hc, Wc, ptr(Ahi), None, ptr(Bhi), None, *geom_args, s)
+        # the HBM-bound exact positive-pair kernel overlaps the GEMM kernel
         with _Fork(dev) as fork:
             call("ssp_desc_pos_fwd", ptr(Dc), ptr(Dwc), ptr(wpts), ptr(mv_pad), B, Hc, Wc, Dch, cell, dist, lamda, _MPOS,
                  _MNEG, ptr(pos_part), ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), stream_of(Dc))
@@ -395,36 +360,35 @@ def desc_backward(st, g3, gscale=1.0, gmode=0, det=None):
     # epilogues (dedicated epilogue warps hide the gathers behind the next item's main loop);
     # fp32 engine: one streaming apply kernel after the GEMMs.
     # stream plan:  [pos_coef]  ||  [pack(alpha * Dw), unless folded]  ->  GEMM pair
-    if fold:
-        # bitsR / bitsC already exclude the columns with mask_valid = 0: dD = srow * (I' @ Dw) on the forward planes
-        if det is not None:
-            # fused step: the detector-loss backward of both images rides in the same launch (heterogeneous blocks)
-            dst, dg, d0, d1 = det
-            x0, t0, m0, x1, t1, m1 = dst.saved
-            call("ssp_step_bwd_prologue", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc, ptr(dst.out[0]),
-                 ptr(dst.out[1]), ptr(dg), ptr(d0), ptr(d1),
-                 ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR), ptr(mv_pad), ptr(g3), gscale,
-                 gmode, ptr(out8), lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(alpha), ptr(srow),
-                 ptr(bitsC), s)
-        else:
-            call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
-                 ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted),
-                 ptr(coefs[1]), ptr(alpha), ptr(srow), ptr(bitsC), Nc, s)
+    # folded: bitsR / bitsC already exclude the columns with mask_valid = 0, dD = srow * (I' @ Dw) on the forward planes
+    if det is not None:
+        # fused step: the detector-loss backward of both images rides in the same launch (heterogeneous blocks)
+        dst, dg, d0, d1 = det
+        x0, t0, m0, x1, t1, m1 = dst.saved
+        call("ssp_step_bwd_prologue", ptr(x0), ptr(t0), ptr(m0), ptr(x1), ptr(t1), ptr(m1), B, Hc, Wc, ptr(dst.out[0]),
+             ptr(dst.out[1]), ptr(dg), ptr(d0), ptr(d1),
+             ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR), ptr(mv_pad), ptr(g3), gscale,
+             gmode, ptr(out8), lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(alpha), ptr(srow),
+             ptr(bitsC), s)
     else:
-        # on the tensor-core engines the coefficient launch also transposes bitsR into bitsC (fp32: the forward wrote it)
-        with _Fork(dev) as f1:
+        # folded, the coefficient launch also writes alpha and srow; on the tensor-core engines it transposes bitsR into
+        # bitsC (fp32: the forward wrote it).  Unfolded, it runs on a side stream next to alpha and the pack.
+        side = contextlib.nullcontext() if fold else _Fork(dev)
+        with side:
             call("ssp_desc_pos_coef", ptr(rowcol), ptr(rowdot), ptr(colcnt), ptr(colrow), ptr(coldot), ptr(bitsR),
                  ptr(mv_pad), ptr(g3), gscale, gmode, ptr(out8), B, Ncp, lamda, _MPOS, ptr(coefs[0]), ptr(colrow_sorted),
-                 ptr(coefs[1]), None, None, ptr(bitsC) if tc_engine else None, Nc if tc_engine else 0, stream_of(Dc))
+                 ptr(coefs[1]), ptr(alpha) if fold else None, ptr(srow), ptr(bitsC) if tc_engine else None,
+                 Nc if tc_engine else 0, stream_of(Dc))
+    if not fold:
         if not tc_engine:
             call("ssp_desc_bits_gemm_simt", ptr(bitsR), ptr(Dwc), ptr(alpha), None, B, Dch, Nc, ptr(dD), s)
             call("ssp_desc_bits_gemm_simt", ptr(bitsC), ptr(Dc), None, ptr(alpha), B, Dch, Nc, ptr(dDw), s)
-            f1.join()
+            side.join()
             call("ssp_desc_pos_apply", ptr(rowcol), ptr(coefs[0]), ptr(colrow_sorted), ptr(coefs[1]), ptr(Dc), ptr(Dwc), B, Dch,
                  Nc, ptr(dD), ptr(dDw), s)
             return dD, dDw
         call("ssp_desc_pack", ptr(Dwc), ptr(alpha), B, Dch, Nc, ptr(Shi), ptr(Slo), s)
-        f1.join()
+        side.join()
     # the dD GEMM reads the forward planes of Dw (rows scaled by srow) when folded, the packed alpha * Dw otherwise; the
     # positive-pair partners come from the packed planes of the forward (Dw for dD, D for dDw)
     Whi, Wlo = (Bhi, Blo) if fold else (Shi, Slo)
@@ -446,12 +410,12 @@ class DescriptorLossFn(torch.autograd.Function):
                                        need_grad=need_grad, fold=False, debug_S=debug_S)
         desc_finalize(st, parts)
         if dist_group is not None:
-            from .dist import globalize_descriptor
+            from .dist import get_exchange
             B, _, Hc, Wc = st.dims
-            globalize_descriptor(st.out8, B, Hc, Wc, dist_group)
+            get_exchange(dist_group).run(desc8=st.out8, B_local=B, Hc=Hc, Wc=Wc)
         if need_grad:
             ctx.save_for_backward(*st.saved)
-        ctx.st = st._replace(saved=None)  # out8 is an attribute, see DetectorLossFn
+        ctx.st = st._replace(saved=None)  # out8 is an attribute, see DetectorLossPairFn
         ctx.mark_non_differentiable(wpts)
         return st.out8[0], st.out8[1], st.out8[2], wpts
 

@@ -12,8 +12,7 @@ import torch
 
 from . import _lib
 from ._lib import call, f32c, ptr, stream_of
-from .losses import (DescriptorLossFn, DetectorLossFn, DetectorLossPairFn, LazyPairMask, SemanticLossFn,
-                     get_descriptor_engine)
+from .losses import DescriptorLossFn, DetectorLossPairFn, LazyPairMask, SemanticLossFn, get_descriptor_engine
 
 __all__ = [
     "warp_points", "filter_points", "warp_points_filter", "warp_keypoints", "inv_warp_image_batch", "inv_warp_image",
@@ -287,13 +286,13 @@ def detector_loss(input, target, mask=None, loss_type="softmax", dist_group=None
     _lib.require_cuda(input)
     if mask is None:
         mask = torch.ones((input.shape[0],) + tuple(input.shape[2:]), device=input.device)
-    return DetectorLossFn.apply(input, target, mask, False, dist_group)
+    return DetectorLossPairFn.apply(input, target, mask, None, None, None, False, dist_group)
 
 
 def detector_loss_2d(semi, labels_2D, mask_2D, dist_group=None):
     """Fused labels2Dto3D(add_dustbin=True) + getMasks + detector_loss from the 2-D maps (one kernel)."""
     _lib.require_cuda(semi)
-    return DetectorLossFn.apply(semi, labels_2D, mask_2D, True, dist_group)
+    return DetectorLossPairFn.apply(semi, labels_2D, mask_2D, None, None, None, True, dist_group)
 
 
 def detector_loss_pair_2d(semi, labels_2D, mask_2D, semi_warp, warped_labels, mask_warp_2D, dist_group=None):

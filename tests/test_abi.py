@@ -91,6 +91,9 @@ def test_argument_errors_without_gpu():
     p = ctypes.c_void_p(16)
     assert lib.ssp_inv_warp_image(p, 1, 1, 8, 8, p, p, p, 2, p, None) < 0  # mode is 0 (bilinear) or 1 (nearest)
     assert b"mode" in lib.ssp_last_error()
+    # the pack planes are given for both tensors (operand pack + geometry) or for neither (geometry alone)
+    assert lib.ssp_desc_pack2_geometry(p, p, 1, 256, 30, 40, p, None, None, None, p, None, None, 8, p, p, p, None, None) < 0
+    assert b"null pointer" in lib.ssp_last_error()
     assert lib.ssp_detector_loss_ws_bytes(32, 30, 40) >= 16 + 300 * 16
 
 

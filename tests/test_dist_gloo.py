@@ -41,8 +41,7 @@ def _worker(rank, world, port, q):
         # drives the torch.distributed form with CPU tensors
         os.environ["SSP_EXCHANGE"] = "allreduce"
     import torch.distributed as tdist
-    from ssp_b200.dist import (LossExchange, get_exchange, globalize_descriptor, globalize_detector, globalize_semantic,
-                               init_from_env, shard_range)
+    from ssp_b200.dist import LossExchange, get_exchange, init_from_env, shard_range
     init_from_env(backend="gloo")
     assert get_exchange(True).backend == "allreduce"  # CPU tensors / gloo: the torch.distributed form of the exchange
     Hs, D, Dw, mv, semi, lab, m3 = _inputs()
@@ -51,11 +50,11 @@ def _worker(rank, world, port, q):
     l, _, p, n = O.descriptor_loss(D[lo:hi], Dw[lo:hi], Hs[lo:hi], mv[lo:hi])
     norm = np.float32(hi - lo) * (mv[lo:hi].sum() + 1) * HC * WC
     out8 = torch.tensor([l, p, n, norm, l * norm, p * norm, n * norm, mv[lo:hi].sum()], dtype=torch.float32)
-    globalize_descriptor(out8, hi - lo, HC, WC, True)
+    get_exchange(True).run(desc8=out8, B_local=hi - lo, Hc=HC, Wc=WC)
     ld = O.detector_loss(semi[lo:hi], lab[lo:hi], m3[lo:hi])
     den = np.float32(m3[lo:hi].sum() + 1e-5)
     out3 = torch.tensor([ld, ld * den, den], dtype=torch.float32)
-    globalize_detector(out3, True)
+    get_exchange(True).run(det0=out3)
     # the fused step exchanges everything in ONE call: same numbers
     out8d = torch.tensor([l, p, n, norm, l * norm, p * norm, n * norm, mv[lo:hi].sum()], dtype=torch.float32)
     out3d = torch.tensor([ld, ld * den, den], dtype=torch.float32)
@@ -67,7 +66,7 @@ def _worker(rank, world, port, q):
     ls = O.sem_loss(sl[lo:hi], slab[lo:hi])
     cnt = np.float32((slab[lo:hi] != 133).sum())
     outs = torch.tensor([ls, ls * cnt, cnt], dtype=torch.float32)
-    globalize_semantic(outs, True)
+    get_exchange(True).run(sem0=outs)
     q.put((rank, out8.numpy().copy(), out3.numpy().copy(), outs.numpy().copy()))
     tdist.barrier()
     tdist.destroy_process_group()

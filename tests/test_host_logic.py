@@ -195,7 +195,7 @@ def test_orchestration_call_sequences(monkeypatch):
     assert multi[:5] == fwd and sorted(multi[5:]) == sorted(bwd_desc + ["ssp_detector_loss_bwd_pair"])
     assert run(fused=False, grad_on=(D, Dw), loss_keys=("positive_dist", "negative_dist")) == fwd + bwd_desc
     assert [c for c in run(engine="fp32") if "_desc_" in c] == [
-        "ssp_desc_geometry", "ssp_desc_pos_fwd", "ssp_desc_dense_fwd_simt", "ssp_desc_finalize", "ssp_desc_alpha",
+        "ssp_desc_pack2_geometry", "ssp_desc_pos_fwd", "ssp_desc_dense_fwd_simt", "ssp_desc_finalize", "ssp_desc_alpha",
         "ssp_desc_pos_coef", "ssp_desc_bits_gemm_simt", "ssp_desc_bits_gemm_simt", "ssp_desc_pos_apply"]
     assert "ssp_desc_pos_fwd" in run(engine="bf16") and "ssp_desc_pos_fwd_planes" not in run(engine="bf16")
     sp, sl = leaf(B, 133, Hc, Wc), torch.randint(0, 134, (B, Hc * 8, Wc * 8))
