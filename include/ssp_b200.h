@@ -298,6 +298,48 @@ int ssp_warp_labels(const float* pnts, const int* counts, int B, int Pmax, int H
                     float* labels, float* res, float* labels_bi /*or NULL*/, float* warped, int* kept, void* ws,
                     size_t ws_bytes, void* stream);
 
+/* ---- evaluation of exported image pairs (evaluation.py:86-499 of the reference lineage, with
+ * evaluations/detector_evaluation.py and evaluations/descriptor_evaluation.py).  Pair p's points are pts1 / pts2
+ * [P,3,cap] float64 (x, y, conf rows, as ssp_nms_fast writes them); it uses its first min(counts[p], limit) points of each
+ * image.  Hs [P,2,9] float64: H (image 1 -> image 2, pixel coordinates) and its inverse as the caller computes it.  Matches
+ * [P,3,Lmax] float64 (index 1, index 2, distance) with nmatch[p] valid entries: ssp_nn_match_batch's output.
+ *
+ * ssp_ransac_homography: n = n_sets * P problems; problem q = set * P + p takes pair p's matches, all of them (set 0) or, in
+ * set 1, those with distance < subset_dist, in list order; Lmax <= 8192.  M hypotheses per problem, all evaluated: 4
+ * distinct matches from Philox4x32-10 (key seed, counter (q, hypothesis, draw block, 1 << 31)), OpenCV's
+ * haveCollinearPoints (every triple, both images) and checkSubset sign test, the 4-point DLT (h33 = 1) in float64; a
+ * rejected sample scores nothing.  Match j is an inlier when ||pi(H p1_j) - p2_j||^2 <= thresh^2 (|w| <= FLT_EPSILON: an
+ * outlier); coordinates enter as fp32 (exact for integer positions).  The hypothesis with the most inliers wins, the lowest
+ * index on ties; H [n,9] is OpenCV's normalised DLT refit on its inliers (h33 = 1, no Levenberg-Marquardt step), ninl [n]
+ * and mask [n,Lmax] (uint8, over the problem's list) its inliers, best [n] its index.  No estimate (fewer than 4 matches,
+ * no hypothesis with 4 inliers, a degenerate refit): H all NaN, ninl 0, mask 0, best -1.  samples [n,M,4] int32 (the drawn
+ * indices, -1 when the problem has fewer than 4 matches) and hyp_inliers [n,M] int32 (-1 = rejected sample) are optional
+ * outputs (NULL in production).  ws: ssp_ransac_homography_ws_bytes(n, M).
+ *
+ * ssp_eval_repeatability: out [P,2] = (repeatability, localisation error) of compute_repeatability
+ * (detector_evaluation.py:152-283): float64 warps, strict in-bounds masks, the keep_k most confident points of each side
+ * (ties at the cut resolved as a stable sort), mutual nearest distances <= dist_thresh; (0, -1) when nothing matches.
+ *
+ * ssp_eval_match_metrics: out [P,3+T] = (mean corner distance of H_est[p] from H, matching score, NN mAP, then
+ * mean_dist <= correctness_thresh[t] as 0 / 1), from the RANSAC results of ssp_ransac_homography (problems 0..P-1 on all
+ * matches; with map_gt == 0 problems P..2P-1 on the matches closer than subset_dist, whose inlier masks label the mAP
+ * matches; map_gt == 1 labels them by ||pi(H p1) - p2|| < 3).  correctness_thresh: HOST array of T <= 8 values.  The
+ * matching score is 2 ninl / (K1 + K2'), K2' counting image 2's points whose integer-truncated back-warp by fp32(H^-1)
+ * lies inside the image (warpLabels' arithmetic); AP is average_precision_score with score = -distance. ---- */
+size_t ssp_ransac_homography_ws_bytes(int n, int M);
+int ssp_ransac_homography(const double* pts1, int cap1, const double* pts2, int cap2, const double* matches,
+                          const unsigned int* nmatch, int Lmax, int P, int n_sets, double subset_dist, int M, double thresh,
+                          unsigned long long seed, double* H, int* ninl, unsigned char* mask, int* best,
+                          int* samples /*or NULL*/, int* hyp_inliers /*or NULL*/, void* ws, size_t ws_bytes, void* stream);
+int ssp_eval_repeatability(const double* pts1, int cap1, const unsigned int* counts1, const double* pts2, int cap2,
+                           const unsigned int* counts2, int limit, int P, const double* Hs, int Himg, int Wimg, int keep_k,
+                           double dist_thresh, double* out, void* stream);
+int ssp_eval_match_metrics(const double* pts1, int cap1, const unsigned int* counts1, const double* pts2, int cap2,
+                           const unsigned int* counts2, int limit, int P, const double* Hs, int Himg, int Wimg,
+                           const double* matches, const unsigned int* nmatch, int Lmax, double subset_dist,
+                           const double* H_est, const int* ninl, const unsigned char* mask, int map_gt,
+                           const double* correctness_thresh, int T, double* out, void* stream);
+
 /* ---- multi-GPU (SURVEY 8e): exchange of the global-batch normalisers of the loss step as ONE kernel over peer memory.
  * The reference is single-GPU; what has to agree with it on a batch sharded by pair is the whole-batch divisors of
  * detector_loss (Train_model_heatmap_all.py:178), descriptor_loss (utils/utils.py:886-887) and sem_loss (:181-193).

@@ -77,6 +77,11 @@ SIGNATURES = {
     "ssp_sample_homography": (_I, [_I, _I, _I, _I, _D, _D, _D, _D, _D, _I, _P, _P, _P, _P]),
     "ssp_warp_labels_ws_bytes": (_Z, [_I, _I, _I]),
     "ssp_warp_labels": (_I, [_P, _P, _I, _I, _I, _I, _P, _I, _P, _P, _P, _P, _P, _P, _Z, _P]),
+    "ssp_ransac_homography_ws_bytes": (_Z, [_I, _I]),
+    "ssp_ransac_homography": (_I, [_P, _I, _P, _I, _P, _P, _I, _I, _I, _D, _I, _D, _c.c_ulonglong] + [_P] * 7 + [_Z, _P]),
+    "ssp_eval_repeatability": (_I, [_P, _I, _P, _P, _I, _P, _I, _I, _P, _I, _I, _I, _D, _P, _P]),
+    "ssp_eval_match_metrics": (_I, [_P, _I, _P, _P, _I, _P, _I, _I, _P, _I, _I, _P, _P, _I, _D, _P, _P, _P, _I, _P, _I, _P,
+                                    _P]),
     "ssp_debug_trace": (_I, [_P]),
     "ssp_debug_trace_cap": (_I, []),
     "ssp_xchg_max_ranks": (_I, []),
@@ -126,7 +131,8 @@ def check(rc, what):
 # kernels launched per entry point (memsets / copies not counted); the NMS drivers launch init + >= 2 rounds +
 # compact + rank, counted at their minimum
 KERNELS_PER_CALL = {"ssp_nms_fast": 5, "ssp_box_nms": 4, "ssp_detector_loss_fwd_pair": 2, "ssp_sem_ce_fwd": 2,
-                    "ssp_sem_ce_up8": 2, "ssp_nn_match_batch": 2}
+                    "ssp_sem_ce_up8": 2, "ssp_nn_match_batch": 2,
+                    "ssp_ransac_homography": 2}
 kernel_count = 0
 _prof = None
 

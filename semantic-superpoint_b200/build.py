@@ -18,7 +18,7 @@ TRACE = os.environ.get("SSP_TRACE") == "1"
 LIB_PATH = os.path.join(LIB_DIR, "libssp_b200_trace.so" if TRACE else "libssp_b200.so")
 OBJ_DIR = os.path.join(HERE, "build_trace" if TRACE else "build")
 
-SOURCES = ["api.cu", "warp.cu", "detector.cu", "semantic.cu", "match.cu", "match_tc.cu", "heatmap.cu", "nms.cu", "subpixel.cu", "desc_common.cu", "desc_simt.cu", "desc_tc.cu", "exchange.cu", "labels.cu", "sparse.cu", "homography.cu"]
+SOURCES = ["api.cu", "warp.cu", "detector.cu", "semantic.cu", "match.cu", "match_tc.cu", "heatmap.cu", "nms.cu", "subpixel.cu", "desc_common.cu", "desc_simt.cu", "desc_tc.cu", "exchange.cu", "labels.cu", "sparse.cu", "homography.cu", "eval.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
     "-Xcompiler", "-fPIC", "--use_fast_math=false",

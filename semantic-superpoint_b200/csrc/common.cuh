@@ -80,3 +80,13 @@ __device__ __forceinline__ void homography_apply(const float* __restrict__ h, fl
   ox = X / Z;
   oy = Y / Z;
 }
+
+// float64 pixel-coordinate warp of the evaluation side, [x, y, 1] H^T / z (evaluations/detector_evaluation.py:139-150);
+// warp_keypoints_f64_kernel and the evaluation kernels share it
+__device__ __forceinline__ void warp_keypoint_f64(const double* __restrict__ Hm, double x, double y, double& ox, double& oy) {
+  double X = Hm[0] * x + Hm[1] * y + Hm[2];
+  double Y = Hm[3] * x + Hm[4] * y + Hm[5];
+  double Z = Hm[6] * x + Hm[7] * y + Hm[8];
+  ox = X / Z;
+  oy = Y / Z;
+}

@@ -1,6 +1,11 @@
 // Counter-based random numbers shared by the device samplers (sparse.cu, homography.cu).  Every sampler keys Philox4x32-10
 // with its seed and puts (item, purpose tag, launch counter) in the counter; the purpose tags of different samplers are kept
 // disjoint, so two samplers built from the same seed draw unrelated numbers.
+// Counter layout (x, y, z, w):
+//   sparse.cu      (item, image << 2 | tag 0..2, launch counter lo, launch counter hi)
+//   homography.cu  (homography, block << 2 | 3, launch counter lo, launch counter hi)
+//   eval.cu        (problem, hypothesis, draw block, 0x80000000): the RANSAC sampler keeps no launch counter; bit 31 of the
+//                  fourth word is set, which a sampler's launch counter (its high word) never reaches
 #pragma once
 #include <cuda_runtime.h>
 

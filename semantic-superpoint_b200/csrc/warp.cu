@@ -42,11 +42,8 @@ __global__ void warp_keypoints_f64_kernel(const double* __restrict__ kp, int K, 
                                           uint8_t* __restrict__ keep) {
   int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= K) return;
-  double x = kp[2 * i], y = kp[2 * i + 1];
-  double X = Hm[0] * x + Hm[1] * y + Hm[2];
-  double Y = Hm[3] * x + Hm[4] * y + Hm[5];
-  double Z = Hm[6] * x + Hm[7] * y + Hm[8];
-  double ox = X / Z, oy = Y / Z;
+  double ox, oy;
+  warp_keypoint_f64(Hm, kp[2 * i], kp[2 * i + 1], ox, oy);
   out[2 * i] = ox;
   out[2 * i + 1] = oy;
   keep[i] = (ox >= 0.0 && ox < W && oy >= 0.0 && oy < Hh) ? 1 : 0;

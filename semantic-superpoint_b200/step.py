@@ -3,7 +3,8 @@
 loss_step          = Train_model_heatmap_all.train_val_sample lines 295-365 (detector loss x2 + descriptor loss,
                      optionally the two semantic cross entropies of the SSp configuration)
 adaptation_step    = export.export_detector_homoAdapt_gpu lines 304-323 (flatten -> aggregate -> NMS [-> sub-pixel] -> top-k)
-match_step         = export.export_descriptor lines 66-189 for a batch of image pairs (flatten -> NMS -> descriptors -> matches)
+match_step         = export.export_descriptor lines 66-189 for a batch of image pairs (flatten -> NMS -> descriptors -> matches),
+                     optionally followed by evaluation.py's metrics of the pairs (utils.evaluate_pairs)
 The first two are free of host synchronisation except the final keypoint read-back of adaptation_step; match_step
 synchronises twice (NMS counts, read-back).
 """
@@ -132,7 +133,8 @@ def adaptation_step(semi, inv_homographies, mask_2D, conf_thresh=0.015, nms_dist
 
 
 @torch.no_grad()
-def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, top_k=None, nn_thresh=0.7):
+def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, top_k=None, nn_thresh=0.7,
+               homographies=None, shape_eval=None, **eval_kw):
     """The descriptor export of P image pairs (export.py:66-189, export_descriptor) as one call: keypoints, descriptors and
     two-way matches of every pair.  semi, semi_warp [P,65,Hc,Wc] logits; desc, desc_warp [P,256,Hc,Wc] coarse descriptors
     (the head's normalised output); CUDA tensors.  Returns P dicts with
@@ -142,7 +144,12 @@ def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, 
     equal, pair by pair, to getPtsFromHeatmap(flattenDetection(semi[p]), conf_thresh, nms_dist)[:, :top_k],
     sample_desc_from_points(desc[p:p+1], pts), the same for the warped image, and nn_match_two_way(desc, warped_desc,
     nn_thresh), the matching on the tensor cores (nn_match_two_way_batch).  Two host synchronisations: the NMS reads its
-    counts (which also size every later buffer) and the single read-back of all results."""
+    counts (which also size every later buffer) and the single read-back of all results.
+    homographies [P,3,3] (pixel coordinates, image 1 -> image 2) runs utils.evaluate_pairs on the device buffers before the
+    read-back (same host synchronisations, no descriptor round trip) and adds "metrics" to every result: that pair's entries
+    of evaluate_pairs' dict.  shape_eval (H, W) defaults to the image shape; eval_kw are evaluate_pairs' keywords.  The
+    evaluation's cross-check matches reuse the export's matcher launch when nn_thresh > 2 (every distance is <= 2), else
+    one more ssp_nn_match_batch runs without a threshold; the export's own results do not change."""
     U._check_nn_thresh(nn_thresh)
     P, C, Hc, Wc = semi.shape
     if C != 65 or tuple(semi_warp.shape) != (P, C, Hc, Wc):
@@ -155,6 +162,11 @@ def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, 
     dev = semi.device
     st = _lib.stream_of(semi)
     H, W = Hc * 8, Wc * 8
+    if homographies is not None:
+        params = U._eval_params(**eval_kw)
+        shape_eval = (H, W) if shape_eval is None else tuple(int(v) for v in shape_eval)
+        Hs_host = U._homography_pairs(homographies, P)
+        Hs = torch.from_numpy(Hs_host).pin_memory().to(dev, non_blocking=True)
     # 1. both flattened heatmaps into the halves of one [2P,1,H,W] buffer
     heat = torch.empty((2 * P, 1, H, W), dtype=torch.float32, device=dev)
     for h, s in enumerate((semi, semi_warp)):
@@ -166,10 +178,23 @@ def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, 
     if kmax == 0:
         empty = {"pts": np.zeros((3, 0)), "desc": np.zeros((256, 0)), "warped_pts": np.zeros((3, 0)),
                  "warped_desc": np.zeros((256, 0)), "matches": np.zeros((3, 0))}
-        return [{k: v.copy() for k, v in empty.items()} for _ in range(P)]
+        out = [{k: v.copy() for k, v in empty.items()} for _ in range(P)]
+        if homographies is not None:
+            keys = ("keep_k_points", "distance_thresh", "correctness_thresh", "map_nn_thresh", "map_inliers", "seed")
+            m = U.evaluate_pairs([r["pts"] for r in out], [r["warped_pts"] for r in out], [r["desc"] for r in out],
+                                 [r["warped_desc"] for r in out], Hs_host[:, 0].reshape(P, 3, 3), shape_eval,
+                                 **dict(zip(keys, params)))
+            _attach_metrics(out, m)
+        return out
     R = (kmax + 255) // 256 * 256
     # every result lands in one device buffer, read back with one copy
     sizes = {"pts": 2 * P * 3 * kmax * 8, "desc": 2 * P * 256 * kmax * 4, "matches": P * 3 * R * 8, "nmatch": P * 4}
+    if homographies is not None:
+        T, n_sets = len(params[0]), 1 if params[1] else 2
+        sizes.update(U._eval_sizes(P, R, T, n_sets))
+        own_matches = nn_thresh <= 2.0  # a distance of exactly 2 fails the matcher's strict test
+        if own_matches:
+            sizes["ev_nmatch"] = P * 4
     offs, total = {}, 0
     for k, n in sizes.items():
         offs[k] = total
@@ -188,6 +213,15 @@ def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, 
     planes = U._pack_planes(d_all)
     U._nn_match_planes(planes[:, :P], planes[:, P:], counts_dev[:P], counts_dev[P:], kmax, nn_thresh, matches, nmatch)
     region("pts", torch.float64, (2 * P, 3, kmax)).copy_(pts[:, :, :kmax])
+    if homographies is not None:
+        ev_matches, ev_nmatch = matches, nmatch
+        if own_matches:
+            ev_matches = torch.empty((P, 3, R), dtype=torch.float64, device=dev)
+            ev_nmatch = region("ev_nmatch", torch.int32, (P,))
+            U._nn_match_planes(planes[:, :P], planes[:, P:], counts_dev[:P], counts_dev[P:], kmax, float("inf"), ev_matches,
+                               ev_nmatch)
+        U._eval_launch(region("pts", torch.float64, (2 * P, 3, kmax)), kmax, counts_dev, P, ev_matches, ev_nmatch, Hs,
+                       shape_eval, params, region)
     # 6. the read-back (host sync 2), into page-locked memory: a pageable copy of the descriptors runs at a fraction of the
     # link's rate, and torch's pinned-memory cache reuses the block once the previous call's results are released
     host = torch.empty((total,), dtype=torch.uint8, pin_memory=True)
@@ -204,7 +238,16 @@ def match_step(semi, desc, semi_warp, desc_warp, conf_thresh=0.015, nms_dist=4, 
                     "warped_pts": hp[P + p, :, :k2] if k2 else np.zeros((3, 0)),
                     "warped_desc": hd[P + p, :, :k2] if k2 else np.zeros((256, 0)),
                     "matches": hm[p, :, :hn[p]] if hn[p] else np.zeros((3, 0))})
+    if homographies is not None:
+        nm = view("ev_nmatch", np.int32, (P,)) if own_matches else hn
+        _attach_metrics(out, U._eval_results(view, nm, P, R, T, n_sets))
     return out
+
+
+def _attach_metrics(results, m):
+    """results[p]["metrics"] = pair p's entries of an evaluate_pairs dict."""
+    for p, r in enumerate(results):
+        r["metrics"] = {k: (v[p] if k == "inliers" else v[p].copy() if v[p].ndim else v[p].item()) for k, v in m.items()}
 
 
 @torch.no_grad()

@@ -761,3 +761,169 @@ def warpLabels(pnts, H, W, homography, bilinear=False):
     if bilinear:
         out["labels_bi"] = o["labels_bi"][0].cpu()
     return out
+
+
+# ------------------------------------------------------------------------------------------------
+# evaluation of exported image pairs (evaluation.py:86-499 of the reference lineage)
+# ------------------------------------------------------------------------------------------------
+RANSAC_HYPOTHESES = 2000   # cv2.findHomography(RANSAC)'s maxIters, every hypothesis evaluated
+RANSAC_THRESH = 3.0        # its ransacReprojThreshold
+RANSAC_MAX_MATCHES = 8192  # matches per RANSAC problem (include/ssp_b200.h); all-points HPatches pairs hold ~6.2 k
+
+
+def _eval_params(keep_k_points=1000, distance_thresh=3, correctness_thresh=(1, 3, 5), map_nn_thresh=1.2,
+                 map_inliers="ransac", seed=0):
+    """Validated evaluation settings (evaluate_pairs' keywords): (thresholds, map_gt flag, keep_k, distance_thresh,
+    map_nn_thresh, seed)."""
+    thr = tuple(float(t) for t in np.atleast_1d(correctness_thresh))
+    if not 1 <= len(thr) <= 8:
+        raise ValueError("correctness_thresh: 1 to 8 thresholds, got %d" % len(thr))
+    if map_inliers not in ("ransac", "gt"):
+        raise ValueError("map_inliers must be 'ransac' or 'gt', got %r" % (map_inliers,))
+    if int(keep_k_points) < 1 or not distance_thresh >= 0 or not map_nn_thresh >= 0:
+        raise ValueError("keep_k_points must be positive, distance_thresh and map_nn_thresh non-negative")
+    return thr, int(map_inliers == "gt"), int(keep_k_points), float(distance_thresh), float(map_nn_thresh), int(seed)
+
+
+def _homography_pairs(homographies, P):
+    """[P,2,9] float64 host array: each pair's pixel homography and its inverse (np.linalg.inv, as evaluation.py)."""
+    Hm = np.asarray(homographies, dtype=np.float64).reshape(-1, 3, 3)
+    if Hm.shape[0] != P:
+        raise ValueError("%d homographies for %d pairs" % (Hm.shape[0], P))
+    return np.stack([Hm.reshape(P, 9), np.linalg.inv(Hm).reshape(P, 9)], axis=1)
+
+
+def _eval_sizes(P, R, T, n_sets):
+    """Byte sizes of the device results of _eval_launch (P pairs, match lists R long)."""
+    n = n_sets * P
+    return {"ev_rep": P * 2 * 8, "ev_met": P * (3 + T) * 8, "ev_H": n * 9 * 8, "ev_ninl": n * 4, "ev_mask": n * R}
+
+
+def _eval_launch(pts, kmax, counts, P, matches, nmatch, Hs, shape, params, region):
+    """The evaluation kernels on device buffers: pts [2P,3,kmax] float64 (image 1 then image 2 of every pair), counts [2P]
+    int32 (each capped at kmax), matches [P,3,R] / nmatch [P] the cross-check matches, Hs [P,2,9] float64.  region(key, dtype,
+    shape) gives the output buffers named by _eval_sizes."""
+    thr, map_gt, keep_k, dthr, nn, seed = params
+    R = matches.shape[2]
+    n_sets = 1 if map_gt else 2
+    st = stream_of(pts)
+    H, W = int(shape[0]), int(shape[1])
+    p1, p2, c1, c2 = ptr(pts), ptr(pts[P:]), ptr(counts), ptr(counts[P:])
+    call("ssp_eval_repeatability", p1, kmax, c1, p2, kmax, c2, kmax, P, ptr(Hs), H, W, keep_k, dthr,
+         ptr(region("ev_rep", torch.float64, (P, 2))), st)
+    nbytes = _lib.load().ssp_ransac_homography_ws_bytes(n_sets * P, RANSAC_HYPOTHESES)
+    ws = torch.empty((nbytes // 8,), dtype=torch.float64, device=pts.device)
+    Hest, ninl = region("ev_H", torch.float64, (n_sets * P, 9)), region("ev_ninl", torch.int32, (n_sets * P,))
+    mask = region("ev_mask", torch.uint8, (n_sets * P, R))
+    best = torch.empty((n_sets * P,), dtype=torch.int32, device=pts.device)
+    call("ssp_ransac_homography", p1, kmax, p2, kmax, ptr(matches), ptr(nmatch), R, P, n_sets, nn, RANSAC_HYPOTHESES,
+         RANSAC_THRESH, int(seed) & (2 ** 64 - 1), ptr(Hest), ptr(ninl), ptr(mask), ptr(best), None, None,
+         ptr(ws), nbytes, st)
+    call("ssp_eval_match_metrics", p1, kmax, c1, p2, kmax, c2, kmax, P, ptr(Hs), H, W, ptr(matches), ptr(nmatch), R, nn,
+         ptr(Hest), ptr(ninl), ptr(mask), map_gt, (_lib._c.c_double * len(thr))(*thr), len(thr),
+         ptr(region("ev_met", torch.float64, (P, 3 + len(thr)))), st)
+
+
+def _eval_results(view, nm, P, R, T, n_sets):
+    """evaluate_pairs' result dict from the host copies of _eval_launch's outputs (view(key, dtype, shape)); nm [P] holds
+    the number of cross-check matches of every pair."""
+    rep, met = view("ev_rep", np.float64, (P, 2)), view("ev_met", np.float64, (P, 3 + T))
+    mask = view("ev_mask", np.uint8, (n_sets * P, R))
+    return {"repeatability": rep[:, 0].copy(), "localization_err": rep[:, 1].copy(), "mean_dist": met[:, 0].copy(),
+            "correctness": met[:, 3:] > 0.5, "matching_score": met[:, 1].copy(), "ap": met[:, 2].copy(),
+            "homography": view("ev_H", np.float64, (n_sets * P, 9))[:P].reshape(P, 3, 3).copy(),
+            "inliers": [mask[p, :nm[p]].astype(bool) for p in range(P)]}
+
+
+def _as_columns(pts, desc, name, p):
+    """One image's points [3,K] float64 and descriptors [256,K] float32 from match_step's layout ([3,K], [256,K]) or the
+    exported npz files' ([K,3], [K,256])."""
+    pts, desc = np.asarray(pts), np.asarray(desc)
+    if pts.ndim == 2 and desc.ndim == 2:
+        if pts.shape[0] == 3 and desc.shape == (256, pts.shape[1]):
+            return pts.astype(np.float64), desc.astype(np.float32)
+        if pts.shape[1] == 3 and desc.shape == (pts.shape[0], 256):
+            return pts.T.astype(np.float64), desc.T.astype(np.float32)
+    raise ValueError("evaluate_pairs: pair %d: %s %s and descriptors %s are neither [3,K] / [256,K] nor [K,3] / [K,256]"
+                     % (p, name, tuple(pts.shape), tuple(desc.shape)))
+
+
+@torch.no_grad()
+def evaluate_pairs(pts, warped_pts, desc, warped_desc, homographies, shape, keep_k_points=1000, distance_thresh=3,
+                   correctness_thresh=(1, 3, 5), map_nn_thresh=1.2, map_inliers="ransac", seed=0):
+    """The metrics of evaluation.py for P exported image pairs, on the device in one pass.
+
+    pts / warped_pts: P arrays [3,K] (x, y, conf) as match_step returns them, or [K,3] as the exported npz files hold them;
+    desc / warped_desc: P arrays [256,K] (or [K,256]); homographies [P,3,3] float64, pixel coordinates, image 1 -> image 2;
+    shape = (H, W).  Up to RANSAC_MAX_MATCHES points per image.  Per pair:
+      repeatability, localization_err   compute_repeatability(pts, warped_pts, H, shape, keep_k_points, distance_thresh)
+                                        (detector_evaluation.py), the golden-pinned definition; its select_k_best uses
+                                        numpy's default (unstable) argsort, whose order among equal confidences is
+                                        unspecified, so where confidences tie at the keep_k cut this keeps the tied points
+                                        a stable sort would (the later ones) and may pick other points than the reference
+      homography [3,3], inliers         RANSAC on the cross-check matches (mutual L2 nearest neighbours, no threshold, as
+                                        BFMatcher(NORM_L2, crossCheck=True)): RANSAC_HYPOTHESES hypotheses from `seed`,
+                                        RANSAC_THRESH px, refit by the normalised DLT on the best hypothesis's inliers
+                                        (OpenCV's LM refinement is not run); NaN and no inliers without an estimate
+      mean_dist, correctness [T]        mean corner distance of the estimate from H, and mean_dist <= each threshold
+      matching_score                    2 * inliers / (K1 + K2'), K2' = warped points whose truncated back-warp lies inside
+      ap                                average_precision_score of the matches closer than map_nn_thresh, score = -distance,
+                                        labelled by a second RANSAC on them ("ransac", evaluation.py's inliers_method 'cv')
+                                        or by ||H p1 - p2|| < 3 ("gt")
+    Everything but repeatability is restated from the evaluation code this project forked (its inliers_method 'cv',
+    nn_thresh 1.2, top_K 1000, rep_thd 3, the truncation in warpLabels, corners from the image shape), not pinned by a
+    fixture of the reference; a detail that turns out to differ is a default to change.  Descriptor matching runs on the
+    tensor cores (fp32-grade dots), so near-tied nearest neighbours may resolve differently from an fp32 BLAS matcher.
+    Returns a dict of per-pair numpy arrays (averaging over pairs is left to the caller)."""
+    params = _eval_params(keep_k_points, distance_thresh, correctness_thresh, map_nn_thresh, map_inliers, seed)
+    P = len(pts)
+    if P == 0 or not (len(warped_pts) == len(desc) == len(warped_desc) == P):
+        raise ValueError("evaluate_pairs: pts, warped_pts, desc and warped_desc must be P > 0 arrays each")
+    cols = [_as_columns(pts[p], desc[p], "pts", p) for p in range(P)] + \
+           [_as_columns(warped_pts[p], warped_desc[p], "warped_pts", p) for p in range(P)]
+    counts = np.array([c[0].shape[1] for c in cols], dtype=np.int32)
+    kmax = max(int(counts.max()), 1)
+    if kmax > RANSAC_MAX_MATCHES:
+        raise ValueError("evaluate_pairs: %d points in one image, at most %d are supported" % (kmax, RANSAC_MAX_MATCHES))
+    Hs = _homography_pairs(homographies, P)
+    dev = _cuda_device("cuda")
+    # one upload of every input from one page-locked buffer
+    up = {"pts": (np.float64, (2 * P, 3, kmax)), "desc": (np.float32, (2 * P, 256, kmax)), "counts": (np.int32, (2 * P,)),
+          "Hs": (np.float64, (P, 2, 9))}
+    offs, total = {}, 0
+    for k, (dt, shp) in up.items():
+        offs[k] = total
+        total += (int(np.prod(shp)) * np.dtype(dt).itemsize + 255) // 256 * 256
+    host = torch.zeros((total,), dtype=torch.uint8, pin_memory=True)
+    hv = lambda k: host.numpy()[offs[k]:offs[k] + int(np.prod(up[k][1])) * np.dtype(up[k][0]).itemsize].view(
+        up[k][0]).reshape(up[k][1])
+    hp, hd = hv("pts"), hv("desc")
+    for i, (pp, dd) in enumerate(cols):
+        hp[i, :, :pp.shape[1]] = pp
+        hd[i, :, :dd.shape[1]] = dd
+    hv("counts")[:] = counts
+    hv("Hs")[:] = Hs
+    buf = host.to(dev, non_blocking=True)
+    dv = lambda k, dtype: buf[offs[k]:offs[k] + int(np.prod(up[k][1])) * np.dtype(up[k][0]).itemsize].view(dtype).view(
+        up[k][1])
+    d_pts, d_desc, d_cnt, d_H = dv("pts", torch.float64), dv("desc", torch.float32), dv("counts", torch.int32), dv(
+        "Hs", torch.float64)
+    planes = _pack_planes(d_desc)
+    R = planes.shape[2]
+    matches = torch.empty((P, 3, R), dtype=torch.float64, device=dev)
+    T, n_sets = len(params[0]), 1 if params[1] else 2
+    sizes = dict(_eval_sizes(P, R, T, n_sets), nmatch=P * 4)
+    ooffs, ototal = {}, 0
+    for k, n in sizes.items():
+        ooffs[k] = ototal
+        ototal += (n + 255) // 256 * 256
+    stage = torch.empty((ototal,), dtype=torch.uint8, device=dev)
+    region = lambda k, dtype, shape: stage[ooffs[k]:ooffs[k] + sizes[k]].view(dtype).view(shape)
+    nmatch = region("nmatch", torch.int32, (P,))
+    _nn_match_planes(planes[:, :P], planes[:, P:], d_cnt[:P], d_cnt[P:], kmax, float("inf"), matches, nmatch)
+    _eval_launch(d_pts, kmax, d_cnt, P, matches, nmatch, d_H, shape, params, region)
+    out = torch.empty((ototal,), dtype=torch.uint8, pin_memory=True)
+    out.copy_(stage)
+    out = out.numpy()
+    view = lambda k, dtype, shp: out[ooffs[k]:ooffs[k] + sizes[k]].view(dtype).reshape(shp)
+    return _eval_results(view, view("nmatch", np.int32, (P,)), P, R, T, n_sets)
